@@ -2,12 +2,12 @@
 """bench.py -- `fastF bam2db` hot path on B200: reads/s through libfastf_gpu.so, roofline of the dominant kernel, the
 reference's CPU path timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R] [--base-reads B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--reads R] [--base-reads B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2]): synthetic 10x-v3 BAM, 10k cells, 36k genes, `-c 1.0 -r 0.3 -s 926`, R reads per GPU
-(default 500M).  The BAM is a zlib-6 BGZF image of B DISTINCT reads per rank (--base-reads; default 0 = as many as the host
-cores of this rank generate in ~90 s, between 8 M and 64 M: 64 M reads = 9.6 GB compressed / 26 GB inflated; data seed
+(default 500M).  The BAM is a zlib-6 BGZF image of B DISTINCT reads per rank (--base-reads; default 0 = 64 M / ranks, between
+8 M and 64 M and at most R, whatever the host: 64 M reads = 9.6 GB compressed / 26 GB inflated; data seed
 DATA_SEED + rank) whose record blocks are cycled T = ceil(R/B) times through the same job -- 5e8 distinct reads would take
 ~12 min of host zlib time per GPU.  The MT19937 draw ordinal keeps running across cycles, so every cycle keeps a different
 30 % of its reads.  One step = one whole job (begin -> feed all cycles -> sample -> sort -> dedup/count -> COO on the host).
@@ -20,6 +20,8 @@ Before timing, the job's counters and COO of a bounded prefix (--check-reads) ar
           launch's CUDA-event duration, against MEASURED_PEAKS.json hbm_gbs
   cpu_baseline : oracle/_ref/fastF_ref (the unmodified reference compiled against the header shims) on a bounded prefix of the
           same BAM, 1 core (the reference path is single-threaded)
+  --dump-outputs DIR : after the timed steps, what the last timed job returned to its caller as float64 .npy files (see
+          dump_outputs), so that two builds can be compared output for output on the same input
 """
 import argparse
 import ctypes as C
@@ -210,6 +212,24 @@ def cpu_model():
     return "unknown"
 
 
+DUMP_BYTES, DUMP_SEED = 64 << 20, 926
+
+
+def dump_outputs(d, stats, coo):
+    """Writes a bam2db job's result as float64 .npy files under d: counters.npy (total, cb_valid, sampled, valid, nnz) and the COO
+    matrix m_gene.npy, m_cell.npy, m_count.npy.  A COO too large for DUMP_BYTES is cut to a fixed, seeded sample of its entries
+    (sorted, so file order is kept); coo_index.npy holds the positions of the entries written, in every case."""
+    os.makedirs(d, exist_ok=True)
+    nnz = len(coo["m_gene"])
+    cap = (DUMP_BYTES - (1 << 20)) // (4 * 8)   # four float64 arrays of cap entries, 1 MB left for the counters and the .npy headers
+    idx = np.arange(nnz) if nnz <= cap else np.sort(np.random.default_rng(DUMP_SEED).choice(nnz, cap, replace=False))
+    np.save(os.path.join(d, "counters.npy"), np.array([stats[k] for k in ("total", "cb_valid", "sampled", "valid", "nnz")], dtype=np.float64))
+    np.save(os.path.join(d, "coo_index.npy"), idx.astype(np.float64))
+    for k in ("m_gene", "m_cell", "m_count"):
+        np.save(os.path.join(d, k + ".npy"), coo[k][idx].astype(np.float64))   # uint32 values: exact in float64
+    log(f"[bench] --dump-outputs: {len(idx)} of {nnz} COO entries and the counters written to {d}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -218,7 +238,7 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--reads", type=int, default=500_000_000, help="reads per GPU per step")
     ap.add_argument("--base-reads", type=int, default=0, help="DISTINCT reads generated per GPU (a zlib-6 BGZF image, every rank its own data seed) and cycled ceil(reads/base) times per step; "
-                    "0 = as many as the host cores of this rank generate in ~90 s, between 8 M and 64 M")
+                    "0 = 64 M / ranks, between 8 M and 64 M")
     ap.add_argument("--check-reads", type=int, default=2_000_000, help="prefix of the data whose single-GPU result is compared with the CPU oracle before anything is timed (0 = skip)")
     ap.add_argument("--cli-reads", type=int, default=0, help="also time `fastF bam2db` (file in /dev/shm -> sqlite + gz files) against the reference CLI on a file of this many reads, outputs compared (0 = on the cpu_baseline sample)")
     ap.add_argument("--freq-reads", type=int, default=32_000_000, help="reads of the `freq` run reported as the `secondary` object of the line (0 = skip)")
@@ -233,7 +253,11 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 3], help="BASELINE.json configs[N] shape: 2 = 10k cells, -c 1.0 -r 0.3 (the headline); 3 = 50k cells, -c 0.2 -r 0.5 (the sharded 2 B-read case: --gpus 8 --reads 250000000)")
     ap.add_argument("--depth-sweep", action="store_true", help="after the main line: -r 0.1..1.0 over the same resident input (BASELINE.json configs[4])")
     ap.add_argument("--workload", default="bam2db", choices=["bam2db", "freq", "crb", "extract"], help="bam2db = BASELINE.json configs[2] (the headline); freq = configs[1] (use --reads 100000000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the counters and COO matrix of the last timed job to DIR/*.npy (float64; "
+                    "a fixed, seeded sample of the COO when it exceeds 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "bam2db"):
+        ap.error("--dump-outputs writes the results of the bam2db timed path (--impl ours --workload bam2db)")
     global N_CELLS, RATE_CELL, RATE_DEPTH
     if args.config == 3:
         N_CELLS, RATE_CELL, RATE_DEPTH = 50000, 0.2, 0.5
@@ -242,9 +266,9 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     threads = os.cpu_count() or 1
     if args.base_reads <= 0:
-        # zlib-6 generation runs at ~44 k reads/s per host thread; every rank generates its own distinct segment on its share of the cores
-        per_rank_threads = max(1, threads // max(1, world))
-        args.base_reads = int(min(64_000_000, max(8_000_000, per_rank_threads * 4_000_000), max(args.reads, 1_000_000)))
+        # zlib-6 generation runs at ~44 k reads/s per host thread, so 64 M reads over all ranks take ~90 s on 16 host cores.  The
+        # size does not depend on the host's core count: the same arguments give the same input everywhere.
+        args.base_reads = int(min(64_000_000, max(8_000_000, 64_000_000 // max(1, world)), max(args.reads, 1_000_000)))
     workload = f"bam2db synthetic 10x-v3 BAM: {args.reads} reads/GPU, {N_CELLS} cells, {N_GENES} genes, -c {RATE_CELL} -r {RATE_DEPTH} -s {SEED} (BASELINE.json configs[{args.config}])"
 
     # ------------------------------------------------------------------ reference arm: the reference's own CPU path
@@ -426,7 +450,9 @@ def main():
                 assert tile_stats["nnz"] <= st_["nnz"], ("nnz below one tile's", st_["nnz"], tile_stats["nnz"])
             assert st_["status"] == 0, ("status", st_["status"])
 
-        def one_job(device_resident, want_copy=False):
+        kept = []   # --dump-outputs: (stats, COO) of the last timed job
+
+        def one_job(device_resident, want_copy=False, keep=False):
             with B.Bam2dbJob(ctx, inputs, rate["depth"], SEED, want_rows=False, inflate_lanes=engine["lanes"], chunk_inflated_bytes=chunk, headerless=(rank != 0)) as job:
                 for t in range(tiles):
                     if device_resident:
@@ -436,10 +462,20 @@ def main():
                         lo = 0 if (t == 0 and rank == 0) else hdr_end
                         job.feed(hptr.value + lo, eof_start - lo)
                 if world > 1:
-                    return multi_gpu_tail(job, dist, torch, ctx, rank, world, inputs)
-                return job.finish(copy=want_copy)
+                    st_, out_ = multi_gpu_tail(job, dist, torch, ctx, rank, world, inputs)   # out_: rank 0's gathered COO (numpy)
+                    if keep:
+                        kept.append((st_, out_))
+                    return st_, out_
+                if not keep:
+                    return job.finish(copy=want_copy)
+                # the library's result arrays are held until after the timed region instead of being copied inside it
+                res = _lib.Bam2dbResult()
+                ctx.check(lib.fastf_bam2db_finish(job.job, C.byref(res)), "bam2db_finish")
+                st_ = {f: getattr(res, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+                kept.append((st_, res))
+                return st_, None
 
-        def timed(device_resident, steps, warmup, sampler=None):
+        def timed(device_resident, steps, warmup, sampler=None, keep_last=False):
             for _ in range(warmup):
                 one_job(device_resident)
             if dist:
@@ -454,8 +490,8 @@ def main():
             t0 = time.time()
             e0.record(lib_stream)
             stats_all = []
-            for _ in range(steps):
-                st, _out = one_job(device_resident)
+            for i in range(steps):
+                st, _out = one_job(device_resident, keep=keep_last and i == steps - 1)
                 stats_all.append(st)
             for st in stats_all:
                 check_job(st)
@@ -471,7 +507,16 @@ def main():
 
         lib_stream = torch.cuda.ExternalStream(lib.fastf_compute_stream(ctx.h), device=torch.device("cuda", local_rank))
         sampler = ClockSampler(local_rank) if rank == 0 else None
-        wall, stats_all, launches, clocks, dev_ms_total = timed(True, args.steps, args.warmup, sampler)
+        wall, stats_all, launches, clocks, dev_ms_total = timed(True, args.steps, args.warmup, sampler, keep_last=bool(args.dump_outputs))
+        if args.dump_outputs:
+            kst, kout = kept.pop()
+            if world == 1:
+                res = kout
+                kout = {k: np.ctypeslib.as_array(getattr(res, k), (res.nnz,)) if res.nnz else np.zeros(0, np.uint32) for k in ("m_gene", "m_cell", "m_count")}
+                dump_outputs(args.dump_outputs, kst, kout)
+                lib.fastf_bam2db_result_free(C.byref(res))
+            elif rank == 0:
+                dump_outputs(args.dump_outputs, kst, kout)
         ms_step = dev_ms_total / args.steps
         ms_step_wall = 1e3 * wall / args.steps
         ms_job_dev = float(np.mean([s["ms_device_total"] for s in stats_all]))   # library's own first-chunk -> last-kernel clock

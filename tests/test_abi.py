@@ -28,15 +28,23 @@ def test_header_symbols_exported(lib):
     assert lib.fastf_abi_version() == 1
 
 
-def test_no_cpu_fallback(lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from fastf_b200 import _lib
-    with pytest.raises(_lib.FastfError, match="no CUDA device"):
-        _lib.Context(0)
-    import fastf_b200
-    assert fastf_b200.freq(os.path.join(ROOT, "tests", "golden", "freq", "synth.fastq.gz"), "/tmp", 16, 12) == 1
+def test_no_cpu_fallback(lib, tmp_path):
+    """without a visible CUDA device (hidden by CUDA_VISIBLE_DEVICES on a machine that has one) every entry point refuses"""
+    import subprocess
+    import sys
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "import fastf_b200\n"
+            "from fastf_b200 import _lib\n"
+            "try:\n"
+            "    _lib.Context(0)\n"
+            "    raise SystemExit('a context was created without a device')\n"
+            "except _lib.FastfError as e:\n"
+            "    assert 'no CUDA device' in str(e), e\n"
+            "assert fastf_b200.freq(%r, %r, 16, 12) == 1\n"
+            "print('OK refused')\n") % (ROOT, os.path.join(ROOT, "tests", "golden", "freq", "synth.fastq.gz"), str(tmp_path))
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=300)
+    assert r.returncode == 0 and "OK refused" in r.stdout, r.stdout[-2000:]
+    assert not os.path.exists(tmp_path / "whitelist.txt")
 
 
 def test_keep_threshold_matches_reference_rule(lib, oracle):
