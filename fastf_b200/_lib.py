@@ -29,6 +29,14 @@ class Bam2dbResult(C.Structure):
                 ("ms_sample", C.c_float), ("ms_sort", C.c_float), ("ms_count", C.c_float), ("ms_device_total", C.c_float), ("ms_crc", C.c_float)]
 
 
+SWEEP_MAX_RATES = 32   # FASTF_SWEEP_MAX_RATES
+
+
+class Bam2dbSweepResult(C.Structure):
+    _fields_ = [("n_rates", C.c_uint32), ("rate", Bam2dbResult * SWEEP_MAX_RATES),
+                ("n_rows", C.c_uint64), ("row_keys", c_u64p), ("row_rate", c_u8p)]
+
+
 class FreqResult(C.Structure):
     _fields_ = [("n_reads", C.c_uint64), ("n_keys", C.c_uint64), ("key", c_u64p), ("count", c_u32p), ("first", c_u32p),
                 ("n_exceptions", C.c_uint64), ("exc_ordinal", c_u32p), ("exc_bytes", c_u8p), ("exc_stride", C.c_uint32),
@@ -76,6 +84,8 @@ _SIGS = {
     "fastf_bam2db_sample_counts": (C.c_int, [C.c_void_p, c_u64p, c_u64p]),
     "fastf_bam2db_key_layout": (C.c_int, [C.c_void_p, c_u32p, c_u32p, c_u32p]),
     "fastf_bam2db_finish": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbResult)]),
+    "fastf_bam2db_finish_sweep": (C.c_int, [C.c_void_p, C.c_uint32, c_u64p, C.POINTER(Bam2dbSweepResult)]),
+    "fastf_bam2db_sweep_result_free": (None, [C.POINTER(Bam2dbSweepResult)]),
     "fastf_bam2db_stats": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbResult)]),
     "fastf_bam2db_job_free": (None, [C.c_void_p]),
     "fastf_bam2db_result_free": (None, [C.POINTER(Bam2dbResult)]),

@@ -239,6 +239,33 @@ class Bam2dbJob:
         self.lib.fastf_bam2db_result_free(C.byref(res))
         return stats, out
 
+    def finish_sweep(self, rates):
+        """The depth sweep instead of finish(): one result per depth rate, in the order given.  Returns [(stats, arrays)], each
+        what finish() returns for a job begun with that rate (counters, COO, that rate's rows and n_rows with want_rows); the stage
+        clocks are the sweep job's, the same for every rate."""
+        thr = np.array([self.lib.fastf_keep_threshold(C.c_float(r)) for r in rates], dtype=np.uint64)
+        res = _lib.Bam2dbSweepResult()
+        try:
+            self.ctx.check(self.lib.fastf_bam2db_finish_sweep(self.job, len(thr), thr.ctypes.data_as(_lib.c_u64p), C.byref(res)), "bam2db_finish_sweep")
+            rows = np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if (self.want_rows and res.n_rows) else np.zeros(0, np.uint64)
+            row_rate = np.ctypeslib.as_array(res.row_rate, (res.n_rows,)).copy() if (self.want_rows and res.n_rows) else np.zeros(0, np.uint8)
+            out = []
+            for i in range(len(thr)):
+                r = res.rate[i]
+                z32 = np.zeros(0, np.uint32)
+                arrays = {
+                    "m_gene": np.ctypeslib.as_array(r.m_gene, (r.nnz,)).copy() if r.nnz else z32,
+                    "m_cell": np.ctypeslib.as_array(r.m_cell, (r.nnz,)).copy() if r.nnz else z32,
+                    "m_count": np.ctypeslib.as_array(r.m_count, (r.nnz,)).copy() if r.nnz else z32,
+                    "row_keys": rows[thr[row_rate] <= thr[i]],
+                }
+                stats = {f: getattr(r, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+                stats["n_rows"] = len(arrays["row_keys"])
+                out.append((stats, arrays))
+            return out
+        finally:
+            self.lib.fastf_bam2db_sweep_result_free(C.byref(res))
+
     def stats(self):
         res = _lib.Bam2dbResult()
         self.ctx.check(self.lib.fastf_bam2db_stats(self.job, C.byref(res)), "bam2db_stats")
@@ -256,16 +283,27 @@ class Bam2dbJob:
         self.close()
 
 
+def _feed_all(job, bam_bytes, feed_piece):
+    buf = np.frombuffer(bam_bytes, dtype=np.uint8)
+    n = buf.size
+    step = feed_piece if feed_piece else max(n, 1)
+    for lo in range(0, n, step):
+        hi = min(n, lo + step)
+        job.feed(buf.ctypes.data + lo, hi - lo)
+
+
 def run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
     """The C-ABI call sequence for one BAM image in host memory.  Returns (stats dict, dict of numpy result arrays)."""
     with Bam2dbJob(ctx, inputs, rate_depth, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes) as job:
-        buf = np.frombuffer(bam_bytes, dtype=np.uint8)
-        n = buf.size
-        step = feed_piece if feed_piece else max(n, 1)
-        for lo in range(0, n, step):
-            hi = min(n, lo + step)
-            job.feed(buf.ctypes.data + lo, hi - lo)
+        _feed_all(job, bam_bytes, feed_piece)
         return job.finish()
+
+
+def run_device_sweep(ctx, bam_bytes, inputs, rates, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
+    """run_device for several depth rates out of one job: [(stats, arrays)] in the order of `rates`."""
+    with Bam2dbJob(ctx, inputs, 0.0, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes) as job:
+        _feed_all(job, bam_bytes, feed_piece)
+        return job.finish_sweep(rates)
 
 
 def matrix_header(bam_file, rate_cell, rate_depth, total, sampled, valid):
@@ -318,6 +356,15 @@ def open_database(db_file, bam_file, barcodes_file, features_file):
     return db
 
 
+def insert_lists(db, inputs):
+    db.execute("BEGIN TRANSACTION")
+    db.executemany("INSERT INTO cell VALUES (?);", ((c.decode("latin-1"),) for c in inputs.cells))
+    db.execute("END TRANSACTION")
+    db.execute("BEGIN TRANSACTION")
+    db.executemany("INSERT INTO feature VALUES (?, ?, ?);", ((f[1].decode("latin-1"), f[2].decode("latin-1"), f[3].decode("latin-1")) for f in inputs.features))
+    db.execute("END TRANSACTION")
+
+
 def load_lists(db, lib, barcodes_file, features_file, rate_cell, seed):
     inputs = Bam2dbInputs(lib, barcodes_file, features_file, rate_cell, seed)
     print("Total number of cells: %d" % inputs.n_cells)
@@ -327,12 +374,7 @@ def load_lists(db, lib, barcodes_file, features_file, rate_cell, seed):
     if inputs.duplicate_features:
         print("Warning: Duplicate feature names were found in %s!" % features_file)
     if db is not None:
-        db.execute("BEGIN TRANSACTION")
-        db.executemany("INSERT INTO cell VALUES (?);", ((c.decode("latin-1"),) for c in inputs.cells))
-        db.execute("END TRANSACTION")
-        db.execute("BEGIN TRANSACTION")
-        db.executemany("INSERT INTO feature VALUES (?, ?, ?);", ((f[1].decode("latin-1"), f[2].decode("latin-1"), f[3].decode("latin-1")) for f in inputs.features))
-        db.execute("END TRANSACTION")
+        insert_lists(db, inputs)
     return inputs
 
 
@@ -408,6 +450,21 @@ def write_outputs(db, bam_file, path_out, inputs, rate_cell, rate_depth, stats, 
     return 0
 
 
+def _run_with_retries(run):
+    """run(umi_max_bytes, inflate_lanes), retried the way the reference's inputs need it"""
+    flags, umi_bytes = 0, 3   # 10x UMIs: 10 or 12 bases; room for 16 on demand
+    while True:
+        try:
+            return run(umi_bytes, flags)
+        except _lib.FastfError as e:
+            if "umi-too-long" in str(e) and umi_bytes == 3:
+                umi_bytes = 4
+            elif "record-straddles-bgzf-block" in str(e) and not flags:
+                flags = BAM_STRADDLE   # not an htslib-written file: guess and verify the record starts per block (one chunk)
+            else:
+                raise
+
+
 def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell, rate_depth, seed=926, device=0, ctx=None):
     own = ctx is None
     try:
@@ -420,18 +477,7 @@ def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell,
         print("Start to convert bam file to sqlite3 database...")
         sys.stdout.flush()
         bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
-        flags, umi_bytes = 0, 3   # 10x UMIs: 10 or 12 bases; room for 16 on demand
-        while True:
-            try:
-                stats, out = run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, umi_max_bytes=umi_bytes, inflate_lanes=flags)
-                break
-            except _lib.FastfError as e:
-                if "umi-too-long" in str(e) and umi_bytes == 3:
-                    umi_bytes = 4
-                elif "record-straddles-bgzf-block" in str(e) and not flags:
-                    flags = BAM_STRADDLE   # not an htslib-written file: guess and verify the record starts per block (one chunk)
-                else:
-                    raise
+        stats, out = _run_with_retries(lambda mb, fl: run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
         rc = write_outputs(db, bam_file, path_out, inputs, rate_cell, rate_depth, stats, out, ctx=ctx)
         db.close()
         return rc
@@ -439,5 +485,63 @@ def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell,
         sys.stderr.write("bam2db: %s\n" % e)
         return 1
     finally:
+        if own and ctx is not None:
+            ctx.close()
+
+
+def sweep_layout(db_name, path_out, rates):
+    """(name, float32 value, output directory, database) per rate: rate r writes into path_out/depth_<r as given>/, its database
+    is that directory's <basename of db_name>.  Raises ValueError on what the sweep refuses."""
+    if not 1 <= len(rates) <= _lib.SWEEP_MAX_RATES:
+        raise ValueError("the depth sweep takes 1..%d rates" % _lib.SWEEP_MAX_RATES)
+    out, seen = [], set()
+    for r in rates:
+        name = r if isinstance(r, str) else str(r)
+        val = np.float32(float(r))
+        if name in seen or val.tobytes() in seen:
+            raise ValueError("the rate %s is listed twice" % name)
+        seen.update((name, val.tobytes()))
+        d = os.path.join(path_out, "depth_" + name)
+        out.append((name, float(val), d, os.path.join(d, os.path.basename(db_name))))
+    for _, _, _, db in out:
+        if os.path.exists(db):
+            raise ValueError("database: %s already exists, change the name of database in -d argument!" % db)
+    return out
+
+
+def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, rates, seed=926, device=0, ctx=None):
+    """bam2db at several depth rates out of one pass over the BAM (one GPU).  Rate r's output set is exactly what
+    bam2db(bam_file, <its database>, <its directory>, ..., rate_cell, r, seed) writes; see sweep_layout for where it goes.
+    Returns 0 / 1 like bam2db."""
+    own = ctx is None
+    dbs = []
+    try:
+        layout = sweep_layout(db_name, path_out, rates)
+        if own:
+            ctx = _lib.Context(device)
+        for _, _, d, dbf in layout:
+            os.makedirs(d, exist_ok=True)
+            db = open_database(dbf, bam_file, barcodes_file, features_file)
+            if db is None:
+                return 1
+            dbs.append(db)
+        inputs = load_lists(None, ctx.lib, barcodes_file, features_file, rate_cell, seed)
+        for db in dbs:
+            insert_lists(db, inputs)
+        print("Start to convert bam file to sqlite3 database...")
+        sys.stdout.flush()
+        bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
+        results = _run_with_retries(lambda mb, fl: run_device_sweep(ctx, bam_bytes, inputs, [v for _, v, _, _ in layout], seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+        for (name, val, d, _), db, (stats, out) in zip(layout, dbs, results):
+            print("Depth rate %s -> %s" % (name, d))
+            if write_outputs(db, bam_file, d, inputs, rate_cell, val, stats, out, ctx=ctx):
+                return 1
+        return 0
+    except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
+        sys.stderr.write("bam2db: %s\n" % e)
+        return 1
+    finally:
+        for db in dbs:
+            db.close()
         if own and ctx is not None:
             ctx.close()

@@ -1,5 +1,6 @@
 // Part of the libfastf_gpu translation unit (capi.cu includes it, in this order; it is not a header of its own):
-// the bam2db job: chunk pipeline (copy ring, inflate / CRC / parse / gather per chunk), MT19937 keep bits, sampling, sort, dedup / count, results.
+// the bam2db job: chunk pipeline (copy ring, inflate / CRC / parse / gather per chunk), MT19937 keep bits, sampling, sort, dedup / count, results;
+// the depth sweep (several rates out of one job).
 #pragma once
 
 // ---------------------------------------------------------------------------------------------------
@@ -62,15 +63,17 @@ struct fastf_bam2db_job {
     u32 status = 0;
     bool header_done = false;
     std::vector<u8> carry;    // partial BGZF block left over by fastf_bam2db_feed
-    // MT19937 keep bits
+    // MT19937 keep bits (the depth sweep: tempered words, one u32 per draw)
     DevBuf mt_state, keepbits, mt_states, mt_scratch;
     u64 mt_pairs_done = 0;     // twist pairs generated since mt_origin
-    u64 mt_origin = 0;         // stream index of bit 0 of keepbits (0 unless the job jumped ahead)
+    u64 mt_origin = 0;         // stream index of bit (word) 0 of keepbits (0 unless the job jumped ahead)
     bool mt_seeded = false;
     cudaEvent_t ev_mt = nullptr;
     // sampling / sort / count
     bool sampled_done = false;
     DevBuf tile_valid, tile_tot, sample_counters, kept, orand;
+    DevBuf kept_rate, rate_alt;   // depth sweep: rate index of every kept row, and its sort ping-pong buffer
+    RleScratch rateS;             // depth sweep: the per-rate count over the distinct keys (held in rleS)
     PinBuf small_host;
     u64 n_sampled = 0, n_valid = 0;
     SortScratch sortS;
@@ -121,9 +124,11 @@ extern "C" void fastf_bam2db_job_free(fastf_bam2db_job *job)
     dev_release(ctx, job->cells.slots); dev_release(ctx, job->cells.pool); dev_release(ctx, job->genes.slots); dev_release(ctx, job->genes.pool);
     dev_release(ctx, job->counters); dev_release(ctx, job->hdr_off); dev_release(ctx, job->cand); dev_release(ctx, job->mt_state); dev_release(ctx, job->keepbits); dev_release(ctx, job->mt_states); dev_release(ctx, job->mt_scratch);
     dev_release(ctx, job->tile_valid); dev_release(ctx, job->tile_tot); dev_release(ctx, job->sample_counters); dev_release(ctx, job->kept); dev_release(ctx, job->orand);
+    dev_release(ctx, job->kept_rate); dev_release(ctx, job->rate_alt);
     pin_release(ctx, job->small_host);
     sort_scratch_release(ctx, job->sortS);
     rle_scratch_release(ctx, job->rleS);
+    rle_scratch_release(ctx, job->rateS);
     delete job;
 }
 
@@ -195,24 +200,25 @@ extern "C" int fastf_bam2db_begin(fastf_ctx *ctx, const fastf_bam2db_params *p, 
     return 0;
 }
 
-// Extend the keep-bit stream so that it covers stream indices [mt_origin, n_draws).  Runs on the mt stream.
-static int mt_extend(fastf_bam2db_job *job, u64 n_draws)
+// Extend the keep-bit stream (words: the tempered words) so that it covers stream indices [mt_origin, n_draws).  Runs on the mt stream.
+static int mt_extend(fastf_bam2db_job *job, u64 n_draws, bool words = false)
 {
     fastf_ctx *ctx = job->ctx;
     if (n_draws <= job->mt_origin) return 0;
     const u64 pairs = (n_draws - job->mt_origin + 1247) / 1248;
     if (pairs <= job->mt_pairs_done) return 0;
-    const size_t need = (size_t)pairs * 39 * sizeof(u32);
+    const size_t per_pair = (words ? 1248 : 39) * sizeof(u32);
+    const size_t need = (size_t)pairs * per_pair;
     if (need > job->keepbits.cap) {
         // grow geometrically; the copy keeps the bits produced so far
         size_t want = std::max(std::max(need + need / 2, (size_t)(64u << 20)), ctx->hint_keepbits);
-        TRY(dev_reserve(ctx, job->keepbits, want, (size_t)job->mt_pairs_done * 39 * sizeof(u32), ctx->mt));
+        TRY(dev_reserve(ctx, job->keepbits, want, (size_t)job->mt_pairs_done * per_pair, ctx->mt));
     }
     Timer &tm = job->t_mt[job->mt_launches++ & 1u];   // the launch two extensions back has long finished
     tm.collect(&job->ms_mt);
     tm.start(ctx->mt);
     FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->mt, job->prm.seed, job->mt_state.as<u32>(), job->mt_seeded ? 0u : 1u, job->mt_pairs_done, pairs - job->mt_pairs_done,
-                 job->prm.keep_threshold, (u32 *)nullptr, job->keepbits.as<u32>());
+                 job->prm.keep_threshold, words ? job->keepbits.as<u32>() : (u32 *)nullptr, words ? (u32 *)nullptr : job->keepbits.as<u32>());
     CKL("mt19937");
     tm.stop(ctx->mt);
     job->mt_seeded = true;
@@ -260,11 +266,12 @@ static int mt_jump_to(fastf_bam2db_job *job, u64 origin)
     return 0;
 }
 
-// Keep bits for stream indices [first, first + n) generated by FASTF_MT_SEGMENTS CTAs at once: every CTA jumps to the start of
-// its own segment, then runs the normal twist.  Used once the number of draws is known (fastf_bam2db_sample); replaces whatever
-// the job had generated speculatively.  Returns 1 when the jump tables are unavailable (caller falls back to one sequential CTA).
+// Keep bits (words: tempered words) for stream indices [first, first + n) generated by FASTF_MT_SEGMENTS CTAs at once: every CTA
+// jumps to the start of its own segment, then runs the normal twist.  Used once the number of draws is known (fastf_bam2db_sample,
+// the depth sweep); replaces whatever the job had generated speculatively.  Returns 1 when the jump tables are unavailable (caller
+// falls back to one sequential CTA).
 #define FASTF_MT_SEGMENTS 32
-static int mt_generate_parallel(fastf_bam2db_job *job, u64 first, u64 n, cudaStream_t s)
+static int mt_generate_parallel(fastf_bam2db_job *job, u64 first, u64 n, cudaStream_t s, bool words = false)
 {
     fastf_ctx *ctx = job->ctx;
     const fastf_mtj::Tables &T = fastf_mtj::tables();
@@ -282,14 +289,15 @@ static int mt_generate_parallel(fastf_bam2db_job *job, u64 first, u64 n, cudaStr
     }
     TRY(dev_reserve(ctx, job->mt_states, (size_t)K * 624 * sizeof(u32)));
     TRY(dev_reserve(ctx, job->mt_scratch, (size_t)K * FASTF_MTJ_SCRATCH * sizeof(u32)));
-    TRY(dev_reserve(ctx, job->keepbits, (size_t)K * ppc * 39 * sizeof(u32)));
+    TRY(dev_reserve(ctx, job->keepbits, (size_t)K * ppc * (words ? 1248 : 39) * sizeof(u32)));
     Timer &tm = job->t_mt[job->mt_launches++ & 1u];
     tm.collect(&job->ms_mt);
     tm.start(s);
     FASTF_LAUNCH(fastf_mt_jump_batch_kernel, K, FASTF_MTJ_THREADS, 0, s, job->prm.seed, (const u64 *)ctx->mtj_polys, (u32)T.pow2.size(), first, ppc * 1248ull, job->mt_states.as<u32>(),
                  job->mt_scratch.as<u32>());
     CKL("mt_jump_batch");
-    FASTF_LAUNCH(fastf_mt19937_kernel, K, FASTF_MT_THREADS, 0, s, job->prm.seed, job->mt_states.as<u32>(), 0u, (u64)0, ppc, job->prm.keep_threshold, (u32 *)nullptr, job->keepbits.as<u32>());
+    FASTF_LAUNCH(fastf_mt19937_kernel, K, FASTF_MT_THREADS, 0, s, job->prm.seed, job->mt_states.as<u32>(), 0u, (u64)0, ppc, job->prm.keep_threshold,
+                 words ? job->keepbits.as<u32>() : (u32 *)nullptr, words ? (u32 *)nullptr : job->keepbits.as<u32>());
     CKL("mt19937");
     tm.stop(s);
     job->mt_seeded = true;
@@ -774,13 +782,12 @@ extern "C" int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *re
     return fill_stats(job, res);
 }
 
-extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *res)
+// FASTF_FEED_TIMING=1: the host-fed job's copy / inflate / parse timeline on stderr (once, at finish); releases its events
+static int report_feed_timing(fastf_bam2db_job *job)
 {
     fastf_ctx *ctx = job->ctx;
-    CK(cudaSetDevice(ctx->device));
-    memset(res, 0, sizeof *res);
-    if (!job->sampled_done) TRY(fastf_bam2db_sample(job, 0));
-    if (job->feed_timing && !job->ft_copy_ev.empty()) {
+    if (!job->feed_timing || job->ft_copy_ev.empty()) return 0;
+    {
         CK(cudaStreamSynchronize(ctx->copy));
         double ms = 0, span = 0;
         for (auto &e : job->ft_copy_ev) { float t = 0; cudaEventElapsedTime(&t, e.first, e.second); ms += t; }
@@ -809,6 +816,16 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
         for (auto &e : job->ft_parse_ev) cudaEventDestroy(e);
         job->ft_copy_ev.clear(); job->ft_infl_ev.clear(); job->ft_parse_ev.clear();
     }
+    return 0;
+}
+
+extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *res)
+{
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof *res);
+    if (!job->sampled_done) TRY(fastf_bam2db_sample(job, 0));
+    TRY(report_feed_timing(job));
     const u64 n = job->n_valid;
     const FastfKeyLayout &L = job->L;
     if (job->prm.want_rows) {
@@ -840,6 +857,148 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
     TRY(fill_stats(job, res));
     res->nnz = nnz;
     return 0;
+}
+
+// Depth sweep (include/fastf_gpu.h): draws as words -> per-rate histograms + (key, rate index) rows in file order -> ONE sort with the
+// rate index as least significant digit -> distinct keys with their smallest rate index -> per rate, a predicated count over them.
+extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+{
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof *res);
+    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES || !keep_thresholds) return ctx_fail(ctx, "bam2db_finish_sweep: 1..%u keep thresholds", (unsigned)FASTF_SWEEP_MAX_RATES);
+    for (u32 i = 0; i < n_rates; i++)
+        if (keep_thresholds[i] > 4294967296ull) return ctx_fail(ctx, "bam2db_finish_sweep: keep_thresholds[%u] > 2^32", i);
+    if (job->sampled_done) return ctx_fail(ctx, "bam2db_finish_sweep: the job was already sampled at one rate");
+    TRY(drain_chunks(job));
+    TRY(report_feed_timing(job));
+    const u64 n = job->n_cand;
+    if (n >= 0xffffffffull) return ctx_fail(ctx, "bam2db_finish_sweep: %llu CB-valid reads exceed the 2^32-1 limit of one device", (unsigned long long)n);
+    const u32 K = n_rates;
+    // sorted position p <-> caller index order[p]; ties keep caller order, so a row's rate index maps to the first of equal thresholds
+    u32 order[FASTF_SWEEP_MAX_RATES], pos[FASTF_SWEEP_MAX_RATES];
+    for (u32 i = 0; i < K; i++) order[i] = i;
+    std::stable_sort(order, order + K, [&](u32 a, u32 b) { return keep_thresholds[a] < keep_thresholds[b]; });
+    FastfSweepRates R;
+    memset(&R, 0, sizeof R);
+    R.k = K;
+    for (u32 p = 0; p < K; p++) { R.t[p] = keep_thresholds[order[p]]; pos[order[p]] = p; }
+    const u64 first_draw = job->prm.d0;
+    const FastfKeyLayout &L = job->L;
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+    memset(hist, 0, sizeof hist);
+    u64 nk = 0;   // valid rows kept by the largest threshold
+    if (n) {
+        if (mt_generate_parallel(job, first_draw, n, ctx->mt, true)) TRY(mt_extend(job, first_draw + n, true));
+        CK(cudaEventRecord(job->ev_mt, ctx->mt));
+        CK(cudaStreamWaitEvent(ctx->compute, job->ev_mt, 0));
+        const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
+        TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
+        TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
+        TRY(dev_reserve(ctx, job->sample_counters, sizeof hist));
+        TRY(pin_reserve(ctx, job->small_host, sizeof hist));
+        CK(cudaMemsetAsync(job->sample_counters.p, 0, sizeof hist, ctx->compute));
+        job->t_sample.start(ctx->compute);
+        FASTF_LAUNCH(fastf_sweep_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin, R,
+                     job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
+        CKL("sweep_count");
+        TRY(launch_scan_rows(ctx, job->tile_valid.as<u32>(), ntiles, 1, job->tile_tot.as<u32>(), ctx->compute));
+        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, sizeof hist, cudaMemcpyDeviceToHost, ctx->compute));
+        CK(cudaStreamSynchronize(ctx->compute));
+        memcpy(hist, job->small_host.p, sizeof hist);
+        for (u32 p = 0; p < K; p++) nk += hist[FASTF_SWEEP_MAX_RATES + p];
+        TRY(dev_reserve(ctx, job->kept, std::max<u64>(nk, 1) * sizeof(u64)));
+        TRY(dev_reserve(ctx, job->kept_rate, std::max<u64>(nk, 1) * sizeof(u32)));
+        TRY(dev_reserve(ctx, job->rate_alt, std::max<u64>(nk, 1) * sizeof(u32)));
+        FASTF_LAUNCH(fastf_sweep_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin, R,
+                     (const u32 *)job->tile_valid.as<u32>(), job->kept.as<u64>(), job->kept_rate.as<u32>());
+        CKL("sweep_scatter");
+        job->t_sample.stop(ctx->compute);
+        CK(cudaEventRecord(job->ev_last, ctx->compute));
+    }
+    job->sampled_done = true;
+    // the rows in file order, each with the caller index of its rate
+    if (job->prm.want_rows) {
+        res->row_keys = (u64 *)malloc(std::max<u64>(nk, 1) * sizeof(u64));
+        res->row_rate = (u8 *)malloc(std::max<u64>(nk, 1));
+        u32 *rb = (u32 *)malloc(std::max<u64>(nk, 1) * sizeof(u32));
+        if (!res->row_keys || !res->row_rate || !rb) { free(rb); return ctx_fail(ctx, "out of host memory for %llu rows", (unsigned long long)nk); }
+        int rc = 0;
+        if (nk) rc = d2h_pageable(ctx, res->row_keys, job->kept.p, nk * sizeof(u64), ctx->compute) || d2h_pageable(ctx, rb, job->kept_rate.p, nk * sizeof(u32), ctx->compute);
+        for (u64 r = 0; r < nk && !rc; r++) res->row_rate[r] = (u8)order[rb[r]];
+        free(rb);
+        if (rc) return rc;
+        res->n_rows = nk;
+    }
+    // one sort of (key, rate index), the rate index as the least significant digit: the first row of a run of equal keys carries
+    // the key's smallest rate index, and the run heads are the distinct keys (rleS.grp_key) with it (rleS.grp_val)
+    u64 nheads = 0;
+    const u32 *grate = nullptr;   // FastfRatePred::grate of the distinct keys
+    if (nk) {
+        u64 varying = 0;
+        job->t_sort.start(ctx->compute);
+        TRY(varying_bits(ctx, job->orand, job->small_host, job->kept.as<u64>(), nk, &varying, ctx->compute));
+        u32 shifts[9];
+        shifts[0] = FASTF_SORT_VAL_DIGIT;
+        const int npass = 1 + plan_windows(varying, shifts + 1);
+        bool in_alt = false;
+        TRY(sort_keys(ctx, job->sortS, job->kept.as<u64>(), job->cand.as<u64>(), job->kept_rate.as<u32>(), job->rate_alt.as<u32>(), nk, shifts, npass, &in_alt, ctx->compute));
+        const u64 *sorted = in_alt ? job->cand.as<u64>() : job->kept.as<u64>();
+        const u32 *sorted_rate = in_alt ? job->rate_alt.as<u32>() : job->kept_rate.as<u32>();
+        u32 *gr = in_alt ? job->kept_rate.as<u32>() : job->rate_alt.as<u32>();   // the ping-pong buffer the sort left free
+        TRY(rle_groups(ctx, job->rleS, sorted, sorted_rate, nk, 0, 64, 0, &nheads, nullptr, ctx->compute));
+        FASTF_LAUNCH(fastf_group_rate_kernel, (u32)((nheads + 255) / 256), 256, 0, ctx->compute, (const u64 *)job->rleS.grp_key.as<u64>(), (const u32 *)job->rleS.grp_val.as<u32>(), nheads, L.bits_umi, gr);
+        grate = gr;
+        CKL("group_rate");
+        job->t_sort.stop(ctx->compute);
+    }
+    // per rate (sorted position p): one predicated count over the distinct keys; its COO goes to the host before the next rate's
+    fastf_bam2db_result *out = res->rate;
+    u64 sampled = 0, valid = 0;
+    for (u32 p = 0; p < K; p++) {
+        fastf_bam2db_result &r = out[order[p]];
+        sampled += hist[p];
+        valid += hist[FASTF_SWEEP_MAX_RATES + p];
+        r.sampled = sampled;
+        r.valid = valid;
+        u64 nnz = 0;
+        if (nheads) {
+            job->t_count.start(ctx->compute);
+            TRY(rle_groups(ctx, job->rateS, job->rleS.grp_key.as<u64>(), nullptr, nheads, L.bits_umi, L.bits_umi - 1, L.bits_gene, &nnz, nullptr, ctx->compute,
+                           FastfRatePred{job->rleS.grp_val.as<u32>(), grate, p}));
+            job->t_count.stop(ctx->compute);
+            job->t_count.collect(&job->ms_count);
+        }
+        TRY(coo_to_host(ctx, job->rateS, nnz, &r.m_gene, &r.m_cell, &r.m_count, ctx->compute));
+        r.nnz = nnz;
+    }
+    CK(cudaEventRecord(job->ev_last, ctx->compute));
+    CK(cudaStreamSynchronize(ctx->compute));
+    CK(cudaStreamSynchronize(ctx->mt));
+    job->n_sampled = sampled;
+    job->n_valid = valid;
+    fastf_bam2db_result st;
+    memset(&st, 0, sizeof st);
+    TRY(fill_stats(job, &st));
+    res->n_rates = K;
+    for (u32 i = 0; i < K; i++) {
+        fastf_bam2db_result &r = out[i];
+        const fastf_bam2db_result keep = r;
+        r = st;
+        r.sampled = keep.sampled; r.valid = keep.valid; r.nnz = keep.nnz;
+        r.m_gene = keep.m_gene; r.m_cell = keep.m_cell; r.m_count = keep.m_count;
+    }
+    return 0;
+}
+
+extern "C" void fastf_bam2db_sweep_result_free(fastf_bam2db_sweep_result *res)
+{
+    if (!res) return;
+    for (u32 i = 0; i < FASTF_SWEEP_MAX_RATES; i++) fastf_bam2db_result_free(&res->rate[i]);
+    free(res->row_keys); free(res->row_rate);
+    res->row_keys = nullptr;
+    res->row_rate = nullptr;
+    res->n_rows = 0;
 }
 
 extern "C" void fastf_bam2db_result_free(fastf_bam2db_result *res)

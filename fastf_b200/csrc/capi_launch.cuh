@@ -144,7 +144,7 @@ static int plan_windows(u64 varying, u32 *shifts)
     return n;
 }
 // Sorts n keys (and optional u32 payload).  keys/alt (and vals/vals_alt) are ping-pong buffers of n elements;
-// *sorted_in_alt tells where the result ended up.
+// *sorted_in_alt tells where the result ended up.  A pass whose shift is FASTF_SORT_VAL_DIGIT sorts by the payload's low byte.
 static int sort_keys(fastf_ctx *ctx, SortScratch &S, u64 *keys, u64 *alt, u32 *vals, u32 *vals_alt, u64 n, const u32 *shifts, int npass, bool *sorted_in_alt, cudaStream_t s)
 {
     *sorted_in_alt = false;
@@ -157,7 +157,8 @@ static int sort_keys(fastf_ctx *ctx, SortScratch &S, u64 *keys, u64 *alt, u32 *v
     u64 *src = keys, *dst = alt;
     u32 *vsrc = vals, *vdst = vals_alt;
     for (int p = 0; p < npass; p++) {
-        FASTF_LAUNCH(fastf_radix_hist_kernel, ntiles, FASTF_RS_THREADS, 0, s, (const u64 *)src, n, shifts[p], S.hist.as<u32>(), ntiles);
+        if (shifts[p] == FASTF_SORT_VAL_DIGIT && !vals) return ctx_fail(ctx, "sort: a payload-digit pass needs a payload");
+        FASTF_LAUNCH(fastf_radix_hist_kernel, ntiles, FASTF_RS_THREADS, 0, s, (const u64 *)src, (const u32 *)vsrc, n, shifts[p], S.hist.as<u32>(), ntiles);
         CKL("radix_hist");
         TRY(launch_scan_rows(ctx, S.hist.as<u32>(), ntiles, 256, S.totals.as<u32>(), s));
         FASTF_LAUNCH(fastf_radix_digit_base_kernel, 1, 256, 0, s, (const u32 *)S.totals.as<u32>(), S.dbase.as<u32>());
@@ -199,9 +200,9 @@ static void rle_scratch_release(fastf_ctx *ctx, RleScratch &R)
     pin_release(ctx, R.totals_host);
 }
 // After this: R.grp_key/grp_first/grp_dstart(/grp_val)/count hold ngroups entries on device; with split_bits_gene > 0
-// R.out_gene / R.out_cell hold the split group key.
+// R.out_gene / R.out_cell hold the split group key.  pred: the depth sweep's rate predicate (radix_dedup.cuh), off by default.
 static int rle_groups(fastf_ctx *ctx, RleScratch &R, const u64 *sorted, const u32 *vals, u64 n, u32 group_shift, u32 nn_bit, u32 split_bits_gene, u64 *ngroups_out, u64 *ndistinct_out,
-                      cudaStream_t s)
+                      cudaStream_t s, FastfRatePred pred = FastfRatePred{nullptr, nullptr, 0u})
 {
     *ngroups_out = 0;
     if (ndistinct_out) *ndistinct_out = 0;
@@ -211,7 +212,7 @@ static int rle_groups(fastf_ctx *ctx, RleScratch &R, const u64 *sorted, const u3
     TRY(dev_reserve(ctx, R.tile_counts, (size_t)2 * ntiles * sizeof(u32)));
     TRY(dev_reserve(ctx, R.tile_totals, 2 * sizeof(u32)));
     TRY(pin_reserve(ctx, R.totals_host, 2 * sizeof(u32)));
-    FASTF_LAUNCH(fastf_rle_count_kernel, ntiles, FASTF_RLE_THREADS, 0, s, sorted, n, group_shift, nn_bit, R.tile_counts.as<u32>(), ntiles);
+    FASTF_LAUNCH(fastf_rle_count_kernel, ntiles, FASTF_RLE_THREADS, 0, s, sorted, n, group_shift, nn_bit, pred, R.tile_counts.as<u32>(), ntiles);
     CKL("rle_count");
     TRY(launch_scan_rows(ctx, R.tile_counts.as<u32>(), ntiles, 2, R.tile_totals.as<u32>(), s));
     CK(cudaMemcpyAsync(R.totals_host.p, R.tile_totals.p, 2 * sizeof(u32), cudaMemcpyDeviceToHost, s));
@@ -223,7 +224,7 @@ static int rle_groups(fastf_ctx *ctx, RleScratch &R, const u64 *sorted, const u3
     TRY(dev_reserve(ctx, R.count, (size_t)ngroups * sizeof(u32)));
     if (vals) TRY(dev_reserve(ctx, R.grp_val, (size_t)ngroups * sizeof(u32)));
     if (split_bits_gene) { TRY(dev_reserve(ctx, R.out_gene, (size_t)ngroups * sizeof(u32))); TRY(dev_reserve(ctx, R.out_cell, (size_t)ngroups * sizeof(u32))); }
-    FASTF_LAUNCH(fastf_rle_emit_kernel, ntiles, FASTF_RLE_THREADS, 0, s, sorted, vals, n, group_shift, nn_bit, (const u32 *)R.tile_counts.as<u32>(), ntiles, R.grp_key.as<u64>(),
+    FASTF_LAUNCH(fastf_rle_emit_kernel, ntiles, FASTF_RLE_THREADS, 0, s, sorted, vals, n, group_shift, nn_bit, pred, (const u32 *)R.tile_counts.as<u32>(), ntiles, R.grp_key.as<u64>(),
                  R.grp_first.as<u32>(), R.grp_dstart.as<u32>(), vals ? R.grp_val.as<u32>() : (u32 *)nullptr);
     CKL("rle_emit");
     if (ngroups) {

@@ -1,4 +1,4 @@
-// Prefix sums, the MT19937 keep-bit stream (K3) and the depth-sampling compaction (K3b).
+// Prefix sums, the MT19937 keep-bit stream (K3), the depth-sampling compaction (K3b) and its several-rate form (the depth sweep).
 #pragma once
 #include "common.cuh"
 
@@ -271,4 +271,91 @@ fastf_sample_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__re
 #pragma unroll
     for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++)
         if (flags & (1u << k)) kept[o++] = keys[k];
+}
+
+// ------------------------------------------------------------------------------------------------
+// Depth sweep: one pass samples at K rates.  The draws arrive as tempered words u (fastf_mt19937_kernel
+// out_words); the K keep thresholds are sorted ascending, and the rate index of a draw is
+//     b(u) = min{ i : u < T_i }  (K when there is none)  =  number of thresholds <= u,
+// so a read is kept at rate i <=> b <= i: the reads kept at a lower rate are a subset of those kept
+// at a higher one.  Counts go into per-rate histograms (their prefix sums are the per-rate counters);
+// the valid candidates with b < K are compacted in file order as (key, b).
+// ------------------------------------------------------------------------------------------------
+struct FastfSweepRates {
+    u64 t[FASTF_SWEEP_MAX_RATES];   // ascending thresholds, t[0..k)
+    u32 k;
+};
+
+__device__ __forceinline__ u32 fastf_rate_index(const u64 *t, u32 k, u32 u)
+{
+    u32 b = 0;
+    for (u32 j = 0; j < k; j++) b += (u64)u >= t[j];
+    return b;
+}
+
+// hist: u64[2][FASTF_SWEEP_MAX_RATES]: row 0 = CB-valid reads with rate index b, row 1 = those whose key is insertable
+__global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
+fastf_sweep_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, u64 first_draw, FastfSweepRates R, u32 *__restrict__ tile_valid, u64 *__restrict__ hist)
+{
+    __shared__ u64 s_t[FASTF_SWEEP_MAX_RATES];
+    __shared__ u32 s_h[2][FASTF_SWEEP_MAX_RATES];
+    __shared__ u32 s_valid;
+    const u32 K = R.k;
+    if (threadIdx.x < FASTF_SWEEP_MAX_RATES) { s_t[threadIdx.x] = R.t[threadIdx.x]; s_h[0][threadIdx.x] = 0; s_h[1][threadIdx.x] = 0; }
+    if (threadIdx.x == 0) s_valid = 0;
+    __syncthreads();
+    const u64 base = (u64)blockIdx.x * FASTF_SAMPLE_TILE;
+    u32 valid = 0;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
+        u64 i = base + (u64)k * FASTF_SAMPLE_THREADS + threadIdx.x;
+        if (i < n) {
+            const u32 b = fastf_rate_index(s_t, K, words[first_draw + i]);
+            if (b < K) {
+                atomicAdd(&s_h[0][b], 1u);
+                if (cand[i] != FASTF_INVALID_KEY) { atomicAdd(&s_h[1][b], 1u); valid++; }
+            }
+        }
+    }
+    valid = __reduce_add_sync(FASTF_FULL_MASK, valid);
+    if ((threadIdx.x & 31u) == 0) atomicAdd(&s_valid, valid);
+    __syncthreads();
+    if (threadIdx.x == 0) tile_valid[blockIdx.x] = s_valid;
+    if (threadIdx.x < K) {
+        if (s_h[0][threadIdx.x]) atomicAdd((unsigned long long *)&hist[threadIdx.x], (unsigned long long)s_h[0][threadIdx.x]);
+        if (s_h[1][threadIdx.x]) atomicAdd((unsigned long long *)&hist[FASTF_SWEEP_MAX_RATES + threadIdx.x], (unsigned long long)s_h[1][threadIdx.x]);
+    }
+}
+
+__global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
+fastf_sweep_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, u64 first_draw, FastfSweepRates R, const u32 *__restrict__ tile_off, u64 *__restrict__ kept,
+                           u32 *__restrict__ kept_rate)
+{
+    __shared__ u64 s_t[FASTF_SWEEP_MAX_RATES];
+    const u32 K = R.k;
+    if (threadIdx.x < FASTF_SWEEP_MAX_RATES) s_t[threadIdx.x] = R.t[threadIdx.x];
+    __syncthreads();
+    // blocked arrangement as in fastf_sample_scatter_kernel: file order under a single block scan
+    const u64 base = (u64)blockIdx.x * FASTF_SAMPLE_TILE + (u64)threadIdx.x * FASTF_SAMPLE_ITEMS;
+    u64 keys[FASTF_SAMPLE_ITEMS];
+    u32 rb[FASTF_SAMPLE_ITEMS];
+    u32 flags = 0, cnt = 0;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
+        u64 i = base + k;
+        bool v = false;
+        rb[k] = K;
+        if (i < n) {
+            rb[k] = fastf_rate_index(s_t, K, words[first_draw + i]);
+            if (rb[k] < K) { keys[k] = cand[i]; v = keys[k] != FASTF_INVALID_KEY; }
+        }
+        flags |= (u32)v << k;
+        cnt += v;
+    }
+    u32 tot;
+    u32 ex = fastf_block_exscan<FASTF_SAMPLE_THREADS>(cnt, &tot);
+    u64 o = (u64)tile_off[blockIdx.x] + ex;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++)
+        if (flags & (1u << k)) { kept[o] = keys[k]; kept_rate[o] = rb[k]; o++; }
 }

@@ -14,6 +14,10 @@ extern int _umi_copies_flag;   /* reference src/bam2db_ds.h:23 */
 extern int fastf_device;       /* CUDA device ordinal (env FASTF_DEVICE, default 0) */
 extern int fastf_gpus;         /* bam2db over this many GPUs of the node (env FASTF_GPUS or --gpus N, default 1) */
 int bam2db(char *bam_file, char *db_file, char *path_out, char *barcodes_file, char *features_file, float rate_cell, float rate_depth, unsigned int seed);
+/* the depth sweep (not a reference entry point): one device job, output set i = what bam2db(..., rates[i], seed) writes, into
+ * out_dirs[i] with database db_files[i]; 1..32 rates, one GPU.  rate_names[i] names rate i on stdout. */
+int bam2db_sweep(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
+                 const float *rates, unsigned int seed);
 /* cell_counts + print_tree in one call: histogram of the first l+u bases of every read of R1 (BGZF or plain text), written to fp
  * in the reference's BST pre-order.  Returns 0 / 1. */
 int freq_whitelist(const char *r1_path, size_t len_cellbarcode, size_t len_umi, FILE *fp);

@@ -1,13 +1,17 @@
 /* fastF (B200 build): the reference's command line for the GPU subcommands (reference src/main.c:30-92, 231-402, 404-443).
  *   fastF bam2db  -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL -r RATE_DEPTH [-o OUT] [-s SEED] [-u]
+ *   fastF bam2db  -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL --depths R1,R2,... [-o OUT] [-s SEED] [-u]
+ *                 (the depth sweep, not a reference option: one pass, rate Ri written into OUT/depth_<Ri>/ with database OUT/depth_<Ri>/<basename of DB>)
  *   fastF freq    -R R1 -o OUT [-l LEN] [-u UMI]
  *   fastF crb     -b BAM -o OUT.gz
  *   fastF extract -b BAM -t TAG [-T 0|1]
  * Long options (--bam --feature --barcode --dbname --cell --depth --out --seed --umicopies; --R1 --out --len --umi; --tag --type) as
  * in the reference.  filter is not part of this build (out of scope: see DESIGN.md). */
 #include "fastf_host.h"
+#include <errno.h>
 #include <stdlib.h>
 #include <string.h>
+#include <sys/stat.h>
 #include <unistd.h>
 
 typedef struct { char s; const char *l; int has_arg; } optdef;
@@ -67,32 +71,78 @@ static int cmd_freq(int argc, const char **argv)
     return rc;
 }
 
+#define MAX_DEPTHS 32   /* FASTF_SWEEP_MAX_RATES */
+
+/* --depths R1,R2,...: one device pass, one output set per rate (bam2db_sweep) */
+static int depth_sweep(const char *bam, const char *feat, const char *bc, const char *db, const char *out, float rate_cell, const char *list, unsigned seed)
+{
+    char *names[MAX_DEPTHS + 1], *dirs[MAX_DEPTHS], *dbs[MAX_DEPTHS];
+    float rates[MAX_DEPTHS];
+    uint32_t n = 0;
+    char *copy = strdup(list);
+    for (char *save = NULL, *t = strtok_r(copy, ",", &save); t; t = strtok_r(NULL, ",", &save)) {
+        if (n == MAX_DEPTHS) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths takes at most %d rates.\n", MAX_DEPTHS); exit(1); }
+        names[n] = t;
+        rates[n] = strtof(t, NULL);   /* as -r */
+        for (uint32_t k = 0; k < n; k++)
+            if (!strcmp(names[k], t) || !memcmp(&rates[k], &rates[n], sizeof(float))) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths lists the rate %s twice.\n", t); exit(1); }
+        n++;
+    }
+    if (!n) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths needs at least one rate.\n"); exit(1); }
+    {   /* bam2db() lets FASTF_GPUS override --gpus: refuse either here, before any directory is made */
+        const char *e = getenv("FASTF_GPUS");
+        if (fastf_gpus > 1 || (e && atoi(e) > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths runs on one GPU (--gpus 1, FASTF_GPUS unset or 1).\n"); exit(1); }
+    }
+    const char *base = strrchr(db, '/') ? strrchr(db, '/') + 1 : db;
+    for (uint32_t k = 0; k < n; k++) {
+        dirs[k] = (char *)malloc(strlen(out) + strlen(names[k]) + 16);
+        dbs[k] = (char *)malloc(strlen(out) + strlen(names[k]) + strlen(base) + 17);
+        sprintf(dirs[k], "%s/depth_%s", out, names[k]);
+        sprintf(dbs[k], "%s/%s", dirs[k], base);
+        if (access(dbs[k], F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", dbs[k]); exit(1); }
+    }
+    for (uint32_t k = 0; k < n; k++)
+        if (mkdir(dirs[k], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", dirs[k]); exit(1); }
+    const int rc = bam2db_sweep((char *)bam, dbs, dirs, (char *)bc, (char *)feat, rate_cell, n, (const char *const *)names, rates, seed);
+    for (uint32_t k = 0; k < n; k++) { free(dirs[k]); free(dbs[k]); }
+    free(copy);
+    if (rc) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }
+    return 0;
+}
+
 static int cmd_bam2db(int argc, const char **argv)
 {
-    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".";
+    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".", *depths = NULL;
     float rate_cell = 0.0f, rate_depth = 0.0f;   /* the reference leaves these uninitialised (src/main.c:293-294): pass -c and -r */
+    int have_r = 0;
     unsigned seed = 926;
-    static const optdef defs[] = {{'b', "bam", 1}, {'f', "feature", 1}, {'a', "barcode", 1}, {'d', "dbname", 1}, {'c', "cell", 1}, {'r', "depth", 1}, {'o', "out", 1}, {'s', "seed", 1}, {'u', "umicopies", 0}, {'h', "help", 0}, {'g', "gpus", 1}};
+    static const optdef defs[] = {{'b', "bam", 1}, {'f', "feature", 1}, {'a', "barcode", 1}, {'d', "dbname", 1}, {'c', "cell", 1}, {'r', "depth", 1}, {'o', "out", 1}, {'s', "seed", 1}, {'u', "umicopies", 0}, {'h', "help", 0}, {'g', "gpus", 1}, {0, "depths", 1}};
     for (int i = 1; i < argc; i++) {
         const char *v;
-        switch (next_opt(argc, argv, &i, defs, 11, &v)) {
+        switch (next_opt(argc, argv, &i, defs, 12, &v)) {
         case 0: bam = v; break;
         case 1: feat = v; break;
         case 2: bc = v; break;
         case 3: db = v; break;
         case 4: rate_cell = strtof(v, NULL); break;     /* OPT_FLOAT uses strtof (src/argparse.c:101-116) */
-        case 5: rate_depth = strtof(v, NULL); break;
+        case 5: rate_depth = strtof(v, NULL); have_r = 1; break;
         case 6: out = v; break;
         case 7: seed = (unsigned)(int)strtol(v, NULL, 0); break;
         case 8: _umi_copies_flag = 1; break;
         case 10: fastf_gpus = (int)strtol(v, NULL, 0); break;   /* not a reference option: GPUs of this node to shard the BAM over */
-        default: printf("Usage: fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL -r RATE_DEPTH [-o OUT] [-s 926] [-u] [--gpus N]\n\nFilter bam file with desired cell proportion and read depth, then summarise it into UMI matrix.\n"); exit(0);
+        case 11: depths = v; break;                              /* not a reference option: the depth sweep */
+        default: printf("Usage: fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL -r RATE_DEPTH [-o OUT] [-s 926] [-u] [--gpus N]\n"
+                        "       fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL --depths R1,R2,... [-o OUT] [-s 926] [-u]\n\n"
+                        "Filter bam file with desired cell proportion and read depth, then summarise it into UMI matrix.\n"
+                        "--depths writes the result of every rate Ri (up to 32, one pass over the BAM) into OUT/depth_<Ri>/, database OUT/depth_<Ri>/<basename of DB>.\n"); exit(0);
         }
     }
+    if (depths && have_r) { fprintf(stderr, "\x1b[31mError:\x1b[0m -r/--depth and --depths exclude each other.\n"); exit(1); }
     if (!bam || access(bam, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam file: %s does not exist.\n", bam ? bam : "(null)"); exit(1); }
     if (!feat || access(feat, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m feature file: %s does not exist.\n", feat ? feat : "(null)"); exit(1); }
     if (!bc || access(bc, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m barcode file: %s does not exist.\n", bc ? bc : "(null)"); exit(1); }
     if (!db) { fprintf(stderr, "\x1b[31mError:\x1b[0m please name the database with -d.\n"); exit(1); }
+    if (depths) return depth_sweep(bam, feat, bc, db, out, rate_cell, depths, seed);
     if (access(db, F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", db); exit(1); }
     if (bam2db((char *)bam, (char *)db, (char *)out, (char *)bc, (char *)feat, rate_cell, rate_depth, seed)) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }
     return 0;

@@ -132,6 +132,25 @@ int fastf_bam2db_sample_counts(fastf_bam2db_job *job, uint64_t *sampled, uint64_
 int fastf_bam2db_key_layout(fastf_bam2db_job *job, uint32_t *bits_cell, uint32_t *bits_gene, uint32_t *bits_umi);
 /* single-GPU tail: (sample if not done) + sort + dedup + count + copy back */
 int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *res);
+/* ---- depth sweep: one job, the outputs of several depth rates (single GPU) ----
+ * For one -c / -s every read meets the same MT19937 draw u whatever the depth rate, and a larger threshold keeps a superset of the
+ * reads a smaller one keeps.  So one inflate + parse + draw pass yields the exact result of every rate: rate[i] equals what
+ * fastf_bam2db_finish returns for a job begun with keep_threshold = keep_thresholds[i].  The stage clocks are the job's, the same
+ * in every rate[i]: ms_sample covers the per-rate histograms and the (key, rate index) compaction, ms_sort the one sort plus the
+ * compaction of the distinct keys with their smallest rate index, ms_count the sum of the K per-rate count passes. */
+#define FASTF_SWEEP_MAX_RATES 32
+typedef struct {
+    uint32_t n_rates;
+    fastf_bam2db_result rate[FASTF_SWEEP_MAX_RATES]; /* rate[i] as fastf_bam2db_finish fills it for keep_thresholds[i]; row_keys NULL, n_rows 0 */
+    uint64_t n_rows;      /* valid rows kept by the largest threshold, file order (0 unless the job was begun with want_rows) */
+    uint64_t *row_keys;
+    uint8_t *row_rate;    /* per row: index into keep_thresholds of the smallest threshold that keeps it (the first such index on ties);
+                           * row r belongs to rate i's table umi <=> keep_thresholds[row_rate[r]] <= keep_thresholds[i] */
+} fastf_bam2db_sweep_result;
+/* instead of fastf_bam2db_finish (and of fastf_bam2db_sample, which must not have been called); keep_thresholds in caller order,
+ * 1..FASTF_SWEEP_MAX_RATES of them, each <= 2^32 (fastf_keep_threshold); p->keep_threshold of the job is ignored */
+int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res);
+void fastf_bam2db_sweep_result_free(fastf_bam2db_sweep_result *res);
 /* counters, sizes and per-stage device clocks so far, without finishing (multi-GPU driver); no arrays are allocated */
 int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *res);
 void fastf_bam2db_job_free(fastf_bam2db_job *job);
