@@ -86,16 +86,22 @@ _SIGS = {
     "fastf_bam2db_finish": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbResult)]),
     "fastf_bam2db_finish_sweep": (C.c_int, [C.c_void_p, C.c_uint32, c_u64p, C.POINTER(Bam2dbSweepResult)]),
     "fastf_bam2db_sweep_result_free": (None, [C.POINTER(Bam2dbSweepResult)]),
+    "fastf_bam2db_sample_sweep": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, c_u64p, c_u64p, c_u64p]),
+    "fastf_bam2db_kept_sweep_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), c_u64p]),
     "fastf_bam2db_stats": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbResult)]),
     "fastf_bam2db_job_free": (None, [C.c_void_p]),
     "fastf_bam2db_result_free": (None, [C.POINTER(Bam2dbResult)]),
     "fastf_bam2db_run_sharded": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(Bam2dbParams), C.c_void_p, C.c_size_t, C.POINTER(Bam2dbResult)]),
+    "fastf_bam2db_run_sharded_sweep": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(Bam2dbParams), C.c_void_p, C.c_size_t, C.c_uint32, c_u64p, C.POINTER(Bam2dbSweepResult)]),
     "fastf_sharded_last_error": (C.c_char_p, []),
     "fastf_sharded_exchanged": (C.c_uint64, []),
     "fastf_sort_u64_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]),
     "fastf_dedup_count_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, c_u64p, C.POINTER(c_u32p), C.POINTER(c_u32p), C.POINTER(c_u32p)]),
     "fastf_dedup_count_device_out": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, c_u64p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fastf_unique_partition_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, c_u64p]),
+    "fastf_unique_partition_rates_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, c_u64p]),
+    "fastf_sweep_count_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, c_u64p, C.POINTER(c_u32p), C.POINTER(c_u32p),
+                                           C.POINTER(c_u32p)]),
     "fastf_free": (None, [C.c_void_p]),
     "fastf_inflate_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_float)]),
     "fastf_mt19937_host": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, c_u32p]),

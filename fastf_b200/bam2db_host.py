@@ -183,6 +183,53 @@ def run_sharded(lib, bam_bytes, inputs, rate_depth, seed, n_devices, want_rows=T
     return stats, out
 
 
+def _sweep_to_python(res, thr, want_rows):
+    """[(stats, arrays)] per threshold (caller order) out of a filled Bam2dbSweepResult; rate i's rows are those whose rate's threshold is
+    <= thr[i].  The caller frees res."""
+    rows = np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if (want_rows and res.n_rows) else np.zeros(0, np.uint64)
+    row_rate = np.ctypeslib.as_array(res.row_rate, (res.n_rows,)).copy() if (want_rows and res.n_rows) else np.zeros(0, np.uint8)
+    out = []
+    for i in range(len(thr)):
+        r = res.rate[i]
+        z32 = np.zeros(0, np.uint32)
+        arrays = {
+            "m_gene": np.ctypeslib.as_array(r.m_gene, (r.nnz,)).copy() if r.nnz else z32,
+            "m_cell": np.ctypeslib.as_array(r.m_cell, (r.nnz,)).copy() if r.nnz else z32,
+            "m_count": np.ctypeslib.as_array(r.m_count, (r.nnz,)).copy() if r.nnz else z32,
+            "row_keys": rows[thr[row_rate] <= thr[i]],
+        }
+        stats = {f: getattr(r, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+        stats["n_rows"] = len(arrays["row_keys"])
+        out.append((stats, arrays))
+    return out
+
+
+def _thresholds(lib, rates):
+    return np.array([lib.fastf_keep_threshold(C.c_float(r)) for r in rates], dtype=np.uint64)
+
+
+def run_sharded_sweep(lib, bam_bytes, inputs, rates, seed, n_devices, want_rows=True, devices=None, **kw):
+    """The depth sweep over n_devices GPUs of this node in ONE process (fastf_bam2db_run_sharded_sweep).  Returns what
+    Bam2dbJob.finish_sweep returns for one job over the whole file: [(stats, arrays)] in the order of `rates`; every stats gains
+    "exchanged_keys"."""
+    p, keep = make_params(lib, inputs, 0.0, seed, want_rows, **kw)
+    thr = _thresholds(lib, rates)
+    buf = np.frombuffer(bam_bytes, dtype=np.uint8)
+    res = _lib.Bam2dbSweepResult()
+    devs = (C.c_int * n_devices)(*devices) if devices else None
+    try:
+        if lib.fastf_bam2db_run_sharded_sweep(n_devices, devs, C.byref(p), C.c_void_p(buf.ctypes.data), buf.size, len(thr), thr.ctypes.data_as(_lib.c_u64p), C.byref(res)) != 0:
+            raise _lib.FastfError("bam2db_run_sharded_sweep: " + lib.fastf_sharded_last_error().decode())
+        out = _sweep_to_python(res, thr, want_rows)
+    finally:
+        lib.fastf_bam2db_sweep_result_free(C.byref(res))
+    x = int(lib.fastf_sharded_exchanged())
+    for stats, _ in out:
+        stats["exchanged_keys"] = x
+    del keep
+    return out
+
+
 class Bam2dbJob:
     """One streaming bam2db job on one GPU: begin -> feed*/feed_device* -> (counts -> sample(base)) -> finish."""
 
@@ -243,26 +290,11 @@ class Bam2dbJob:
         """The depth sweep instead of finish(): one result per depth rate, in the order given.  Returns [(stats, arrays)], each
         what finish() returns for a job begun with that rate (counters, COO, that rate's rows and n_rows with want_rows); the stage
         clocks are the sweep job's, the same for every rate."""
-        thr = np.array([self.lib.fastf_keep_threshold(C.c_float(r)) for r in rates], dtype=np.uint64)
+        thr = _thresholds(self.lib, rates)
         res = _lib.Bam2dbSweepResult()
         try:
             self.ctx.check(self.lib.fastf_bam2db_finish_sweep(self.job, len(thr), thr.ctypes.data_as(_lib.c_u64p), C.byref(res)), "bam2db_finish_sweep")
-            rows = np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if (self.want_rows and res.n_rows) else np.zeros(0, np.uint64)
-            row_rate = np.ctypeslib.as_array(res.row_rate, (res.n_rows,)).copy() if (self.want_rows and res.n_rows) else np.zeros(0, np.uint8)
-            out = []
-            for i in range(len(thr)):
-                r = res.rate[i]
-                z32 = np.zeros(0, np.uint32)
-                arrays = {
-                    "m_gene": np.ctypeslib.as_array(r.m_gene, (r.nnz,)).copy() if r.nnz else z32,
-                    "m_cell": np.ctypeslib.as_array(r.m_cell, (r.nnz,)).copy() if r.nnz else z32,
-                    "m_count": np.ctypeslib.as_array(r.m_count, (r.nnz,)).copy() if r.nnz else z32,
-                    "row_keys": rows[thr[row_rate] <= thr[i]],
-                }
-                stats = {f: getattr(r, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
-                stats["n_rows"] = len(arrays["row_keys"])
-                out.append((stats, arrays))
-            return out
+            return _sweep_to_python(res, thr, self.want_rows)
         finally:
             self.lib.fastf_bam2db_sweep_result_free(C.byref(res))
 
@@ -509,29 +541,41 @@ def sweep_layout(db_name, path_out, rates):
     return out
 
 
-def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, rates, seed=926, device=0, ctx=None):
-    """bam2db at several depth rates out of one pass over the BAM (one GPU).  Rate r's output set is exactly what
+def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, rates, seed=926, device=0, ctx=None, gpus=1):
+    """bam2db at several depth rates out of one pass over the BAM.  Rate r's output set is exactly what
     bam2db(bam_file, <its database>, <its directory>, ..., rate_cell, r, seed) writes; see sweep_layout for where it goes.
+    gpus > 1 shards the BAM over devices 0..gpus-1 of this node (fastf_bam2db_run_sharded_sweep); `ctx` / `device` then only count
+    the copies of -u (umi.tsv, table numi).
     Returns 0 / 1 like bam2db."""
     own = ctx is None
     dbs = []
     try:
         layout = sweep_layout(db_name, path_out, rates)
-        if own:
+        if gpus < 1:
+            raise ValueError("gpus must be >= 1")
+        if own and gpus == 1:
             ctx = _lib.Context(device)
+        lib = ctx.lib if ctx is not None else _lib.load()   # gpus > 1: the driver opens one context per device itself
         for _, _, d, dbf in layout:
             os.makedirs(d, exist_ok=True)
             db = open_database(dbf, bam_file, barcodes_file, features_file)
             if db is None:
                 return 1
             dbs.append(db)
-        inputs = load_lists(None, ctx.lib, barcodes_file, features_file, rate_cell, seed)
+        inputs = load_lists(None, lib, barcodes_file, features_file, rate_cell, seed)
         for db in dbs:
             insert_lists(db, inputs)
         print("Start to convert bam file to sqlite3 database...")
         sys.stdout.flush()
         bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
-        results = _run_with_retries(lambda mb, fl: run_device_sweep(ctx, bam_bytes, inputs, [v for _, v, _, _ in layout], seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+        vals = [v for _, v, _, _ in layout]
+        if gpus > 1:
+            # a BAM whose records straddle blocks fails here: the straddle mode (BAM_STRADDLE) needs the whole file in one job
+            results = _run_with_retries(lambda mb, fl: run_sharded_sweep(lib, bam_bytes, inputs, vals, seed, gpus, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+        else:
+            results = _run_with_retries(lambda mb, fl: run_device_sweep(ctx, bam_bytes, inputs, vals, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+        if ctx is None and _umi_copies_flag:
+            ctx = _lib.Context(device)   # numi / umi.tsv: the copies of every distinct key are counted on one device
         for (name, val, d, _), db, (stats, out) in zip(layout, dbs, results):
             print("Depth rate %s -> %s" % (name, d))
             if write_outputs(db, bam_file, d, inputs, rate_cell, val, stats, out, ctx=ctx):

@@ -71,6 +71,7 @@ struct fastf_bam2db_job {
     cudaEvent_t ev_mt = nullptr;
     // sampling / sort / count
     bool sampled_done = false;
+    u32 sweep_rates = 0;          // sampled by the depth sweep at this many rates (0: at the job's one rate)
     DevBuf tile_valid, tile_tot, sample_counters, kept, orand;
     DevBuf kept_rate, rate_alt;   // depth sweep: rate index of every kept row, and its sort ping-pong buffer
     RleScratch rateS;             // depth sweep: the per-rate count over the distinct keys (held in rleS)
@@ -697,6 +698,7 @@ extern "C" int fastf_bam2db_kept_device(fastf_bam2db_job *job, uint64_t **dev_ke
 {
     fastf_ctx *ctx = job->ctx;
     if (!job->sampled_done) return ctx_fail(ctx, "bam2db_kept_device: call fastf_bam2db_sample first");
+    if (job->sweep_rates) return ctx_fail(ctx, "bam2db_kept_device: the job was sampled by the depth sweep; use fastf_bam2db_kept_sweep_device");
     *dev_keys = job->kept.as<u64>();
     *n = job->n_valid;
     return 0;
@@ -824,6 +826,7 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
     fastf_ctx *ctx = job->ctx;
     CK(cudaSetDevice(ctx->device));
     memset(res, 0, sizeof *res);
+    if (job->sweep_rates) return ctx_fail(ctx, "bam2db_finish: the job was sampled by the depth sweep");
     if (!job->sampled_done) TRY(fastf_bam2db_sample(job, 0));
     TRY(report_feed_timing(job));
     const u64 n = job->n_valid;
@@ -861,51 +864,57 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
 
 // Depth sweep (include/fastf_gpu.h): draws as words -> per-rate histograms + (key, rate index) rows in file order -> ONE sort with the
 // rate index as least significant digit -> distinct keys with their smallest rate index -> per rate, a predicated count over them.
-extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+// The front half (sweep_sample) runs per job, the back half (sweep_count) wherever the rows of a key meet: in the same job for one
+// GPU, on the receiving device of the exchange for several.
+
+// thresholds in caller order -> R (ascending) and order[p] = caller index of sorted position p; ties keep caller order, so a row's
+// rate index maps to the first of equal thresholds
+static int sweep_rates(fastf_ctx *ctx, const char *who, uint32_t n_rates, const uint64_t *keep_thresholds, FastfSweepRates *R, u32 *order)
+{
+    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES || !keep_thresholds) return ctx_fail(ctx, "%s: 1..%u keep thresholds", who, (unsigned)FASTF_SWEEP_MAX_RATES);
+    for (u32 i = 0; i < n_rates; i++)
+        if (keep_thresholds[i] > 4294967296ull) return ctx_fail(ctx, "%s: keep_thresholds[%u] > 2^32", who, i);
+    for (u32 i = 0; i < n_rates; i++) order[i] = i;
+    std::stable_sort(order, order + n_rates, [&](u32 a, u32 b) { return keep_thresholds[a] < keep_thresholds[b]; });
+    memset(R, 0, sizeof *R);
+    R->k = n_rates;
+    for (u32 p = 0; p < n_rates; p++) R->t[p] = keep_thresholds[order[p]];
+    return 0;
+}
+
+// The job's CB-valid reads meet draws d0 + ordinal_base + k.  hist[p] / hist[FASTF_SWEEP_MAX_RATES + p]: reads / valid reads whose rate
+// index is p; the valid rows kept by the largest threshold land in job->kept / job->kept_rate (file order), *n_kept of them.
+static int sweep_sample(fastf_bam2db_job *job, const char *who, u64 ordinal_base, const FastfSweepRates &R, u64 *hist, u64 *n_kept)
 {
     fastf_ctx *ctx = job->ctx;
-    CK(cudaSetDevice(ctx->device));
-    memset(res, 0, sizeof *res);
-    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES || !keep_thresholds) return ctx_fail(ctx, "bam2db_finish_sweep: 1..%u keep thresholds", (unsigned)FASTF_SWEEP_MAX_RATES);
-    for (u32 i = 0; i < n_rates; i++)
-        if (keep_thresholds[i] > 4294967296ull) return ctx_fail(ctx, "bam2db_finish_sweep: keep_thresholds[%u] > 2^32", i);
-    if (job->sampled_done) return ctx_fail(ctx, "bam2db_finish_sweep: the job was already sampled at one rate");
+    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already sampled", who);
     TRY(drain_chunks(job));
     TRY(report_feed_timing(job));
     const u64 n = job->n_cand;
-    if (n >= 0xffffffffull) return ctx_fail(ctx, "bam2db_finish_sweep: %llu CB-valid reads exceed the 2^32-1 limit of one device", (unsigned long long)n);
-    const u32 K = n_rates;
-    // sorted position p <-> caller index order[p]; ties keep caller order, so a row's rate index maps to the first of equal thresholds
-    u32 order[FASTF_SWEEP_MAX_RATES], pos[FASTF_SWEEP_MAX_RATES];
-    for (u32 i = 0; i < K; i++) order[i] = i;
-    std::stable_sort(order, order + K, [&](u32 a, u32 b) { return keep_thresholds[a] < keep_thresholds[b]; });
-    FastfSweepRates R;
-    memset(&R, 0, sizeof R);
-    R.k = K;
-    for (u32 p = 0; p < K; p++) { R.t[p] = keep_thresholds[order[p]]; pos[order[p]] = p; }
-    const u64 first_draw = job->prm.d0;
-    const FastfKeyLayout &L = job->L;
-    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
-    memset(hist, 0, sizeof hist);
-    u64 nk = 0;   // valid rows kept by the largest threshold
+    if (n >= 0xffffffffull) return ctx_fail(ctx, "%s: %llu CB-valid reads exceed the 2^32-1 limit of one device", who, (unsigned long long)n);
+    const u64 first_draw = job->prm.d0 + ordinal_base;
+    const u32 K = R.k;
+    memset(hist, 0, 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64));
+    u64 nk = 0;
     if (n) {
         if (mt_generate_parallel(job, first_draw, n, ctx->mt, true)) TRY(mt_extend(job, first_draw + n, true));
         CK(cudaEventRecord(job->ev_mt, ctx->mt));
         CK(cudaStreamWaitEvent(ctx->compute, job->ev_mt, 0));
+        const size_t hbytes = 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64);
         const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
         TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
         TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
-        TRY(dev_reserve(ctx, job->sample_counters, sizeof hist));
-        TRY(pin_reserve(ctx, job->small_host, sizeof hist));
-        CK(cudaMemsetAsync(job->sample_counters.p, 0, sizeof hist, ctx->compute));
+        TRY(dev_reserve(ctx, job->sample_counters, hbytes));
+        TRY(pin_reserve(ctx, job->small_host, hbytes));
+        CK(cudaMemsetAsync(job->sample_counters.p, 0, hbytes, ctx->compute));
         job->t_sample.start(ctx->compute);
         FASTF_LAUNCH(fastf_sweep_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin, R,
                      job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
         CKL("sweep_count");
         TRY(launch_scan_rows(ctx, job->tile_valid.as<u32>(), ntiles, 1, job->tile_tot.as<u32>(), ctx->compute));
-        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, sizeof hist, cudaMemcpyDeviceToHost, ctx->compute));
+        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, hbytes, cudaMemcpyDeviceToHost, ctx->compute));
         CK(cudaStreamSynchronize(ctx->compute));
-        memcpy(hist, job->small_host.p, sizeof hist);
+        memcpy(hist, job->small_host.p, hbytes);
         for (u32 p = 0; p < K; p++) nk += hist[FASTF_SWEEP_MAX_RATES + p];
         TRY(dev_reserve(ctx, job->kept, std::max<u64>(nk, 1) * sizeof(u64)));
         TRY(dev_reserve(ctx, job->kept_rate, std::max<u64>(nk, 1) * sizeof(u32)));
@@ -917,6 +926,70 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         CK(cudaEventRecord(job->ev_last, ctx->compute));
     }
     job->sampled_done = true;
+    job->sweep_rates = K;
+    job->n_sampled = 0;
+    for (u32 p = 0; p < K; p++) job->n_sampled += hist[p];
+    job->n_valid = nk;
+    *n_kept = nk;
+    return 0;
+}
+
+// (key, rate index) rows in any order, repeated keys allowed; alt / rate_alt are ping-pong buffers of n elements.  One sort of
+// (key, rate index), the rate index as the least significant digit: the first row of a run of equal keys carries the key's smallest
+// rate index, and the run heads are the distinct keys (rleS.grp_key) with it (rleS.grp_val).  Then the smallest rate index of every
+// (cell, gene) group, and per rate p (ascending threshold) one predicated count over the distinct keys, whose COO goes to the host
+// arrays nnz[p] / m_*[p] (malloc'ed) before the next pass.  t_sort / t_count (nullable) time the sort and the count passes.
+static int sweep_count(fastf_ctx *ctx, SortScratch &sortS, RleScratch &rleS, RleScratch &rateS, DevBuf &orand, PinBuf &host, u64 *keys, u64 *alt, u32 *rates, u32 *rate_alt, u64 n,
+                       u32 key_bits, u32 bits_gene, u32 bits_umi, u32 K, Timer *t_sort, Timer *t_count, float *ms_count, u64 *nnz, u32 **m_gene, u32 **m_cell, u32 **m_count, cudaStream_t s)
+{
+    u64 nheads = 0;
+    const u32 *grate = nullptr;   // FastfRatePred::grate of the distinct keys
+    if (n) {
+        u64 varying = 0;
+        if (t_sort) t_sort->start(s);
+        TRY(varying_bits(ctx, orand, host, keys, n, &varying, s));
+        if (key_bits < 64) varying &= (1ull << key_bits) - 1ull;
+        u32 shifts[9];
+        shifts[0] = FASTF_SORT_VAL_DIGIT;
+        const int npass = 1 + plan_windows(varying, shifts + 1);
+        bool in_alt = false;
+        TRY(sort_keys(ctx, sortS, keys, alt, rates, rate_alt, n, shifts, npass, &in_alt, s));
+        const u64 *sorted = in_alt ? alt : keys;
+        const u32 *sorted_rate = in_alt ? rate_alt : rates;
+        u32 *gr = in_alt ? rates : rate_alt;   // the ping-pong buffer the sort left free
+        TRY(rle_groups(ctx, rleS, sorted, sorted_rate, n, 0, 64, 0, &nheads, nullptr, s));
+        FASTF_LAUNCH(fastf_group_rate_kernel, (u32)((nheads + 255) / 256), 256, 0, s, (const u64 *)rleS.grp_key.as<u64>(), (const u32 *)rleS.grp_val.as<u32>(), nheads, bits_umi, gr);
+        grate = gr;
+        CKL("group_rate");
+        if (t_sort) t_sort->stop(s);
+    }
+    for (u32 p = 0; p < K; p++) {
+        nnz[p] = 0;
+        if (nheads) {
+            if (t_count) t_count->start(s);
+            TRY(rle_groups(ctx, rateS, rleS.grp_key.as<u64>(), nullptr, nheads, bits_umi, bits_umi - 1, bits_gene, &nnz[p], nullptr, s, FastfRatePred{rleS.grp_val.as<u32>(), grate, p}));
+            if (t_count) { t_count->stop(s); t_count->collect(ms_count); }
+        }
+        TRY(coo_to_host(ctx, rateS, nnz[p], &m_gene[p], &m_cell[p], &m_count[p], s));
+    }
+    return 0;
+}
+
+extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+{
+    const char *who = "bam2db_finish_sweep";
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof *res);
+    FastfSweepRates R;
+    u32 order[FASTF_SWEEP_MAX_RATES];
+    TRY(sweep_rates(ctx, who, n_rates, keep_thresholds, &R, order));
+    if (job->sampled_done) return ctx_fail(ctx, "bam2db_finish_sweep: the job was already sampled at one rate");
+    const u32 K = n_rates;
+    const FastfKeyLayout &L = job->L;
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+    u64 nk = 0;   // valid rows kept by the largest threshold
+    TRY(sweep_sample(job, who, 0, R, hist, &nk));
     // the rows in file order, each with the caller index of its rate
     if (job->prm.want_rows) {
         res->row_keys = (u64 *)malloc(std::max<u64>(nk, 1) * sizeof(u64));
@@ -930,30 +1003,14 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         if (rc) return rc;
         res->n_rows = nk;
     }
-    // one sort of (key, rate index), the rate index as the least significant digit: the first row of a run of equal keys carries
-    // the key's smallest rate index, and the run heads are the distinct keys (rleS.grp_key) with it (rleS.grp_val)
-    u64 nheads = 0;
-    const u32 *grate = nullptr;   // FastfRatePred::grate of the distinct keys
-    if (nk) {
-        u64 varying = 0;
-        job->t_sort.start(ctx->compute);
-        TRY(varying_bits(ctx, job->orand, job->small_host, job->kept.as<u64>(), nk, &varying, ctx->compute));
-        u32 shifts[9];
-        shifts[0] = FASTF_SORT_VAL_DIGIT;
-        const int npass = 1 + plan_windows(varying, shifts + 1);
-        bool in_alt = false;
-        TRY(sort_keys(ctx, job->sortS, job->kept.as<u64>(), job->cand.as<u64>(), job->kept_rate.as<u32>(), job->rate_alt.as<u32>(), nk, shifts, npass, &in_alt, ctx->compute));
-        const u64 *sorted = in_alt ? job->cand.as<u64>() : job->kept.as<u64>();
-        const u32 *sorted_rate = in_alt ? job->rate_alt.as<u32>() : job->kept_rate.as<u32>();
-        u32 *gr = in_alt ? job->kept_rate.as<u32>() : job->rate_alt.as<u32>();   // the ping-pong buffer the sort left free
-        TRY(rle_groups(ctx, job->rleS, sorted, sorted_rate, nk, 0, 64, 0, &nheads, nullptr, ctx->compute));
-        FASTF_LAUNCH(fastf_group_rate_kernel, (u32)((nheads + 255) / 256), 256, 0, ctx->compute, (const u64 *)job->rleS.grp_key.as<u64>(), (const u32 *)job->rleS.grp_val.as<u32>(), nheads, L.bits_umi, gr);
-        grate = gr;
-        CKL("group_rate");
-        job->t_sort.stop(ctx->compute);
-    }
-    // per rate (sorted position p): one predicated count over the distinct keys; its COO goes to the host before the next rate's
+    // the candidate array is dead after sampling and at least as large as `kept`: the keys' ping-pong buffer
     fastf_bam2db_result *out = res->rate;
+    u64 nnz[FASTF_SWEEP_MAX_RATES];
+    u32 *mg[FASTF_SWEEP_MAX_RATES] = {}, *mc[FASTF_SWEEP_MAX_RATES] = {}, *mn[FASTF_SWEEP_MAX_RATES] = {};
+    const int crc = sweep_count(ctx, job->sortS, job->rleS, job->rateS, job->orand, job->small_host, job->kept.as<u64>(), job->cand.as<u64>(), job->kept_rate.as<u32>(), job->rate_alt.as<u32>(), nk,
+                                L.bits_cell + L.bits_gene + L.bits_umi, L.bits_gene, L.bits_umi, K, &job->t_sort, &job->t_count, &job->ms_count, nnz, mg, mc, mn, ctx->compute);
+    for (u32 p = 0; p < K; p++) { out[order[p]].m_gene = mg[p]; out[order[p]].m_cell = mc[p]; out[order[p]].m_count = mn[p]; }
+    if (crc) return crc;
     u64 sampled = 0, valid = 0;
     for (u32 p = 0; p < K; p++) {
         fastf_bam2db_result &r = out[order[p]];
@@ -961,22 +1018,11 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         valid += hist[FASTF_SWEEP_MAX_RATES + p];
         r.sampled = sampled;
         r.valid = valid;
-        u64 nnz = 0;
-        if (nheads) {
-            job->t_count.start(ctx->compute);
-            TRY(rle_groups(ctx, job->rateS, job->rleS.grp_key.as<u64>(), nullptr, nheads, L.bits_umi, L.bits_umi - 1, L.bits_gene, &nnz, nullptr, ctx->compute,
-                           FastfRatePred{job->rleS.grp_val.as<u32>(), grate, p}));
-            job->t_count.stop(ctx->compute);
-            job->t_count.collect(&job->ms_count);
-        }
-        TRY(coo_to_host(ctx, job->rateS, nnz, &r.m_gene, &r.m_cell, &r.m_count, ctx->compute));
-        r.nnz = nnz;
+        r.nnz = nnz[p];
     }
     CK(cudaEventRecord(job->ev_last, ctx->compute));
     CK(cudaStreamSynchronize(ctx->compute));
     CK(cudaStreamSynchronize(ctx->mt));
-    job->n_sampled = sampled;
-    job->n_valid = valid;
     fastf_bam2db_result st;
     memset(&st, 0, sizeof st);
     TRY(fill_stats(job, &st));
@@ -989,6 +1035,67 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         r.m_gene = keep.m_gene; r.m_cell = keep.m_cell; r.m_count = keep.m_count;
     }
     return 0;
+}
+
+extern "C" int fastf_bam2db_sample_sweep(fastf_bam2db_job *job, uint64_t ordinal_base, uint32_t n_rates, const uint64_t *sorted_thresholds, uint64_t *sampled, uint64_t *valid)
+{
+    const char *who = "bam2db_sample_sweep";
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    FastfSweepRates R;
+    u32 order[FASTF_SWEEP_MAX_RATES];
+    TRY(sweep_rates(ctx, who, n_rates, sorted_thresholds, &R, order));
+    for (u32 i = 1; i < n_rates; i++)
+        if (sorted_thresholds[i] < sorted_thresholds[i - 1]) return ctx_fail(ctx, "%s: thresholds must be non-decreasing (sorted_thresholds[%u] < sorted_thresholds[%u])", who, i, i - 1);
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES], nk = 0;
+    TRY(sweep_sample(job, who, ordinal_base, R, hist, &nk));
+    u64 s = 0, v = 0;
+    for (u32 p = 0; p < n_rates; p++) {
+        s += hist[p];
+        v += hist[FASTF_SWEEP_MAX_RATES + p];
+        if (sampled) sampled[p] = s;
+        if (valid) valid[p] = v;
+    }
+    return 0;
+}
+
+extern "C" int fastf_bam2db_kept_sweep_device(fastf_bam2db_job *job, uint64_t **dev_keys, uint32_t **dev_rates, uint64_t *n)
+{
+    fastf_ctx *ctx = job->ctx;
+    if (!job->sweep_rates) return ctx_fail(ctx, "bam2db_kept_sweep_device: call fastf_bam2db_sample_sweep first");
+    *dev_keys = job->kept.as<u64>();
+    *dev_rates = job->kept_rate.as<u32>();
+    *n = job->n_valid;
+    return 0;
+}
+
+extern "C" int fastf_sweep_count_device(fastf_ctx *ctx, uint64_t *dev_keys, uint32_t *dev_rates, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_rates,
+                                        uint64_t *nnz, uint32_t **m_gene, uint32_t **m_cell, uint32_t **m_count)
+{
+    CK(cudaSetDevice(ctx->device));
+    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES) return ctx_fail(ctx, "sweep_count_device: 1..%u rates", (unsigned)FASTF_SWEEP_MAX_RATES);
+    if (key_bits > 64 || bits_umi < 2 || bits_gene + bits_umi > key_bits) return ctx_fail(ctx, "sweep_count_device: key layout %u / %u / %u bits", key_bits, bits_gene, bits_umi);
+    for (u32 p = 0; p < n_rates; p++) { nnz[p] = 0; m_gene[p] = m_cell[p] = m_count[p] = nullptr; }
+    cudaStream_t s = ctx->compute;
+    SortScratch S;
+    RleScratch R, RR;
+    DevBuf alt, ralt, orand;
+    PinBuf host;
+    int rc = dev_reserve(ctx, alt, std::max<u64>(n, 1) * sizeof(u64));
+    if (!rc) rc = dev_reserve(ctx, ralt, std::max<u64>(n, 1) * sizeof(u32));
+    if (!rc) rc = dev_reserve(ctx, orand, 2 * sizeof(u64));
+    if (!rc) rc = pin_reserve(ctx, host, 2 * sizeof(u64));
+    if (!rc) rc = sweep_count(ctx, S, R, RR, orand, host, dev_keys, alt.as<u64>(), dev_rates, ralt.as<u32>(), n, key_bits, bits_gene, bits_umi, n_rates, nullptr, nullptr, nullptr, nnz, m_gene, m_cell,
+                              m_count, s);
+    if (cudaStreamSynchronize(s) != cudaSuccess && !rc) rc = ctx_fail(ctx, "sweep_count_device: stream error");
+    sort_scratch_release(ctx, S);
+    rle_scratch_release(ctx, R);
+    rle_scratch_release(ctx, RR);
+    dev_release(ctx, alt); dev_release(ctx, ralt); dev_release(ctx, orand);
+    pin_release(ctx, host);
+    if (rc)
+        for (u32 p = 0; p < n_rates; p++) { free(m_gene[p]); free(m_cell[p]); free(m_count[p]); m_gene[p] = m_cell[p] = m_count[p] = nullptr; nnz[p] = 0; }
+    return rc;
 }
 
 extern "C" void fastf_bam2db_sweep_result_free(fastf_bam2db_sweep_result *res)

@@ -91,22 +91,25 @@ __global__ void __launch_bounds__(256) fastf_strip_tag_kernel(u64 *__restrict__ 
     if (i < n) keys[i] &= (1ull << key_bits) - 1ull;
 }
 
-extern "C" int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_cells, uint32_t nparts,
-                                             uint64_t *dev_out_keys, uint64_t *part_counts)
+// Tag every key with its destination, sort (with rates: the rate index first, as the least significant digit), keep the first key of
+// every run: the unique keys grouped by destination, each with its smallest rate index when rates are given.
+static int unique_partition(fastf_ctx *ctx, const char *who, u64 *dev_keys, u32 *dev_rates, u64 n, u32 key_bits, u32 bits_gene, u32 bits_umi, u32 n_cells, u32 nparts, u64 *dev_out_keys,
+                            u32 *dev_out_rates, u64 *part_counts)
 {
     CK(cudaSetDevice(ctx->device));
     for (u32 p = 0; p < nparts; p++) part_counts[p] = 0;
     if (n == 0) return 0;
     if (nparts == 0 || nparts > 256 || key_bits + (nparts > 1 ? bits_for(nparts - 1) : 0) > 64)
-        return ctx_fail(ctx, "unique_partition: %u key bits leave no room for the destination tag of %u parts", key_bits, nparts);
+        return ctx_fail(ctx, "%s: %u key bits leave no room for the destination tag of %u parts", who, key_bits, nparts);
     cudaStream_t s = ctx->compute;
     SortScratch S;
     RleScratch R;
-    DevBuf alt, orand, bounds;
+    DevBuf alt, valt, orand, bounds;
     PinBuf host;
     int rc = 0;
     auto body = [&]() -> int {
         TRY(dev_reserve(ctx, alt, n * sizeof(u64)));
+        if (dev_rates) TRY(dev_reserve(ctx, valt, n * sizeof(u32)));
         TRY(dev_reserve(ctx, orand, 2 * sizeof(u64)));
         TRY(dev_reserve(ctx, bounds, 257 * sizeof(u64)));
         TRY(pin_reserve(ctx, host, 257 * sizeof(u64)));
@@ -114,17 +117,21 @@ extern "C" int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys,
         CKL("tag_dest");
         u64 varying = 0;
         TRY(varying_bits(ctx, orand, host, dev_keys, n, &varying, s));
-        u32 shifts[8];
-        const int npass = plan_windows(varying, shifts);
+        u32 shifts[9];
+        int npass = 0;
+        if (dev_rates) shifts[npass++] = FASTF_SORT_VAL_DIGIT;
+        npass += plan_windows(varying, shifts + npass);
         bool in_alt = false;
-        TRY(sort_keys(ctx, S, dev_keys, alt.as<u64>(), nullptr, nullptr, n, shifts, npass, &in_alt, s));
+        TRY(sort_keys(ctx, S, dev_keys, alt.as<u64>(), dev_rates, dev_rates ? valt.as<u32>() : nullptr, n, shifts, npass, &in_alt, s));
         const u64 *sorted = in_alt ? alt.as<u64>() : dev_keys;
-        // unique: every key is its own group (group_shift 0); grp_key = the distinct keys in sorted order
+        const u32 *sorted_rates = dev_rates ? (in_alt ? valt.as<u32>() : dev_rates) : nullptr;
+        // unique: every key is its own group (group_shift 0); grp_key = the distinct keys in sorted order, grp_val their first rate
         u64 nuniq = 0;
-        TRY(rle_groups(ctx, R, sorted, nullptr, n, 0, 64, 0, &nuniq, nullptr, s));
+        TRY(rle_groups(ctx, R, sorted, sorted_rates, n, 0, 64, 0, &nuniq, nullptr, s));
         FASTF_LAUNCH(fastf_part_bounds_kernel, 1, 256, 0, s, (const u64 *)R.grp_key.as<u64>(), nuniq, key_bits, nparts, bounds.as<u64>());
         CKL("part_bounds");
         CK(cudaMemcpyAsync(dev_out_keys, R.grp_key.p, nuniq * sizeof(u64), cudaMemcpyDeviceToDevice, s));
+        if (dev_rates) CK(cudaMemcpyAsync(dev_out_rates, R.grp_val.p, nuniq * sizeof(u32), cudaMemcpyDeviceToDevice, s));
         FASTF_LAUNCH(fastf_strip_tag_kernel, (u32)((nuniq + 255) / 256), 256, 0, s, dev_out_keys, nuniq, key_bits);
         CKL("strip_tag");
         CK(cudaMemcpyAsync(host.p, bounds.p, (nparts + 1) * sizeof(u64), cudaMemcpyDeviceToHost, s));
@@ -136,9 +143,22 @@ extern "C" int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys,
     cudaStreamSynchronize(s);
     sort_scratch_release(ctx, S);
     rle_scratch_release(ctx, R);
-    dev_release(ctx, alt); dev_release(ctx, orand); dev_release(ctx, bounds);
+    dev_release(ctx, alt); dev_release(ctx, valt); dev_release(ctx, orand); dev_release(ctx, bounds);
     pin_release(ctx, host);
     return rc;
+}
+
+extern "C" int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_cells, uint32_t nparts,
+                                             uint64_t *dev_out_keys, uint64_t *part_counts)
+{
+    return unique_partition(ctx, "unique_partition", dev_keys, nullptr, n, key_bits, bits_gene, bits_umi, n_cells, nparts, dev_out_keys, nullptr, part_counts);
+}
+
+extern "C" int fastf_unique_partition_rates_device(fastf_ctx *ctx, uint64_t *dev_keys, uint32_t *dev_rates, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_cells,
+                                                   uint32_t nparts, uint64_t *dev_out_keys, uint32_t *dev_out_rates, uint64_t *part_counts)
+{
+    if (n && (!dev_rates || !dev_out_rates)) return ctx_fail(ctx, "unique_partition_rates: null rate arrays");
+    return unique_partition(ctx, "unique_partition_rates", dev_keys, dev_rates, n, key_bits, bits_gene, bits_umi, n_cells, nparts, dev_out_keys, dev_out_rates, part_counts);
 }
 
 // ---------------------------------------------------------------------------------------------------

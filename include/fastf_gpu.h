@@ -151,6 +151,15 @@ typedef struct {
  * 1..FASTF_SWEEP_MAX_RATES of them, each <= 2^32 (fastf_keep_threshold); p->keep_threshold of the job is ignored */
 int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res);
 void fastf_bam2db_sweep_result_free(fastf_bam2db_sweep_result *res);
+/* The depth sweep's per-shard building blocks (multi-GPU driver).  Unlike fastf_bam2db_finish_sweep these take the thresholds already
+ * sorted, non-decreasing (1..FASTF_SWEEP_MAX_RATES of them, each <= 2^32): the caller sorts once and keeps the map to its own order.
+ * The RATE INDEX of a row is its position p in that sorted list: the smallest p with u < sorted_thresholds[p] for the row's draw u,
+ * so the row belongs to the output of every rate q >= p.  Device rate arrays hold it as a u32 per key.
+ * fastf_bam2db_sample_sweep: instead of fastf_bam2db_sample (the job's CB-valid reads meet draws d0 + ordinal_base + k); sampled[p] /
+ * valid[p] (host, n_rates each) = this job's sampled_reads_counts / sampled_valid_reads_counts at sorted rate p. */
+int fastf_bam2db_sample_sweep(fastf_bam2db_job *job, uint64_t ordinal_base, uint32_t n_rates, const uint64_t *sorted_thresholds, uint64_t *sampled, uint64_t *valid);
+/* after fastf_bam2db_sample_sweep: the valid rows kept by the largest threshold (file order) and their rate indices, owned by the job */
+int fastf_bam2db_kept_sweep_device(fastf_bam2db_job *job, uint64_t **dev_keys, uint32_t **dev_rates, uint64_t *n);
 /* counters, sizes and per-stage device clocks so far, without finishing (multi-GPU driver); no arrays are allocated */
 int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *res);
 void fastf_bam2db_job_free(fastf_bam2db_job *job);
@@ -164,6 +173,15 @@ void fastf_bam2db_result_free(fastf_bam2db_result *res);
  * src/bam2db_ds.c:360-438,480-483).  devices == NULL means 0..n_devices-1.  p->want_rows / umi_max_bytes / inflate_lanes as in
  * fastf_bam2db_begin (FASTF_BAM_STRADDLE is single-GPU only).  Returns 0, or 1 with fastf_sharded_last_error(). */
 int fastf_bam2db_run_sharded(int n_devices, const int *devices, const fastf_bam2db_params *p, const void *bgzf_bytes, size_t n_bytes, fastf_bam2db_result *res);
+/* The depth sweep over the same shards: res equals what fastf_bam2db_finish_sweep returns for one job over the whole file with these
+ * keep_thresholds (caller order, validated as there): every rate[i]'s counters and COO, and n_rows / row_keys / row_rate in file order.
+ * Each shard samples its reads at all rates at once (fastf_bam2db_sample_sweep), keeps every distinct key once with its smallest rate
+ * index, and sends the rate index beside the key in the same all-to-all; the receiving device counts every rate
+ * (fastf_sweep_count_device).  Stage clocks as in fastf_bam2db_run_sharded (maximum over devices), except ms_sort = the maximum over
+ * devices of the local unique + partition, and ms_count = the maximum over devices of fastf_sweep_count_device, which includes the
+ * copies of every rate's COO piece to the host (CUDA events on fastf_compute_stream around each call); the same in every rate[i]. */
+int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices, const fastf_bam2db_params *p, const void *bgzf_bytes, size_t n_bytes, uint32_t n_rates,
+                                   const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res);
 const char *fastf_sharded_last_error(void);
 uint64_t fastf_sharded_exchanged(void);   /* keys that crossed the all-to-all in the last call (diagnostic) */
 
@@ -181,6 +199,15 @@ int fastf_dedup_count_device_out(fastf_ctx *ctx, const uint64_t *dev_sorted_keys
  * ascending; part_counts[nparts] (host) their sizes */
 int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi,
                                   uint32_t n_cells, uint32_t nparts, uint64_t *dev_out_keys, uint64_t *part_counts);
+/* the same carrying a rate index (fastf_bam2db_sample_sweep) per key: every distinct key leaves once, with the smallest rate index of
+ * its copies in dev_out_rates (device, capacity n); dev_keys and dev_rates are overwritten */
+int fastf_unique_partition_rates_device(fastf_ctx *ctx, uint64_t *dev_keys, uint32_t *dev_rates, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi,
+                                        uint32_t n_cells, uint32_t nparts, uint64_t *dev_out_keys, uint32_t *dev_out_rates, uint64_t *part_counts);
+/* the depth sweep's count over (key, rate index) rows on device, in any order, repeated keys allowed (each key counts at its smallest
+ * rate index); sorts dev_keys / dev_rates in place.  Per sorted rate p < n_rates: nnz[p] rows of table mtx, ascending (cell, gene), in
+ * host arrays m_gene[p] / m_cell[p] / m_count[p] (library-owned: free with fastf_free).  Only one rate's COO is on the device at a time. */
+int fastf_sweep_count_device(fastf_ctx *ctx, uint64_t *dev_keys, uint32_t *dev_rates, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_rates,
+                             uint64_t *nnz, uint32_t **m_gene, uint32_t **m_cell, uint32_t **m_count);
 void fastf_free(void *p);
 
 /* host-buffer wrappers around single kernels (tests, smoke) */

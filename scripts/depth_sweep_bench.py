@@ -13,7 +13,17 @@ CLI leg: the first --cli-reads reads (whole blocks) as files on /dev/shm; `fastF
 `fastF bam2db -r R` runs, host wall clock of the whole processes (CUDA start-up included); every rate's matrix.mtx.gz must be
 identical between the two.
 
-The GPU name and power limit are read with nvidia-smi in the same run.  Writes DIR/depth_sweep.json."""
+The GPU name and power limit are read with nvidia-smi in the same run.  Writes DIR/depth_sweep.json.
+
+    python scripts/depth_sweep_bench.py --out DIR --gpus G [--reads N] [--reps 3]
+
+Multi-GPU leg instead (the one-process driver of the library): one BAM image of --reads distinct reads (default 64 M per GPU) in host
+memory.  Per repetition, ten fastf_bam2db_run_sharded calls (one per rate) and one fastf_bam2db_run_sharded_sweep over the same ten
+rates run alternately over devices 0..G-1; each call is timed by the host wall clock and includes what the driver does inside it:
+context creation on every device, H2D copies of the shards, and the copy of the results to the host.  Both report the library's
+stage clocks (maximum over devices; the sweep's ms_sort / ms_count are its local unique + partition and its receiving-side count).  As
+the scaling reference, the one-GPU sweep (fastf_bam2db_finish_sweep, host-fed, context creation included) on the same image.  Every
+rate's counters and COO hash must agree between the three, or the script fails.  Writes DIR/depth_sweep_<G>gpu.json."""
 import argparse
 import ctypes as C
 import gzip
@@ -52,14 +62,94 @@ def coo_hash(arr):
     return h.hexdigest()[:16]
 
 
+def gpus_identity(n):
+    r = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
+    if r.returncode != 0:
+        raise RuntimeError("nvidia-smi failed: " + r.stderr)
+    rows = [[x.strip() for x in ln.split(",")] for ln in r.stdout.splitlines() if ln.strip()]
+    if len(rows) < n:
+        raise RuntimeError("%d GPUs requested, %d present" % (n, len(rows)))
+    return [{"index": int(i), "name": name, "power_limit": power} for i, name, power in rows[:n]]
+
+
+def main_multi(args):
+    """--gpus G: K x run_sharded against one run_sharded_sweep, and the one-GPU sweep as the scaling reference"""
+    import bench
+    from fastf_b200 import _lib, bam2db_host as B
+    G = args.gpus
+    gpus = gpus_identity(G)
+    lib = _lib.load()
+    reads = args.reads or 64_000_000 * G
+    base = bench.make_base(reads, os.cpu_count() or 1)
+    tmp = tempfile.mkdtemp(prefix="fastf_sweep_", dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
+    try:
+        paths, _ = bench.write_inputs(base, tmp, write_bam=False)
+        inputs = B.Bam2dbInputs(lib, paths["barcodes"], paths["features"], bench.RATE_CELL, bench.SEED)
+        bam = np.frombuffer(base["bam"], dtype=np.uint8)
+
+        def wall(run):
+            t = time.perf_counter()
+            out = run()
+            return 1e3 * (time.perf_counter() - t), out
+
+        def one_gpu():
+            with _lib.Context(0) as ctx:
+                return B.run_device_sweep(ctx, bam, inputs, RATES, bench.SEED, want_rows=False)
+
+        def check(what, got, ref):
+            for r, (s1, a1), (s2, a2) in zip(RATES, ref, got):
+                assert [s1[k] for k in COUNTERS] == [s2[k] for k in COUNTERS], (what, "counters differ", r)
+                assert coo_hash(a1) == coo_hash(a2), (what, "COO differs", r)
+
+        # warm-up: every path once
+        ref = one_gpu()
+        B.run_sharded(lib, bam, inputs, RATES[0], bench.SEED, G, want_rows=False)
+        B.run_sharded_sweep(lib, bam, inputs, RATES, bench.SEED, G, want_rows=False)
+        reps = []
+        for rep in range(args.reps):
+            singles, single_res = [], []
+            for r in RATES:
+                ms, res = wall(lambda: B.run_sharded(lib, bam, inputs, r, bench.SEED, G, want_rows=False))
+                singles.append(ms)
+                single_res.append(res)
+            ms_sweep, sweep = wall(lambda: B.run_sharded_sweep(lib, bam, inputs, RATES, bench.SEED, G, want_rows=False))
+            ms_one, one = wall(one_gpu)
+            check("run_sharded", single_res, ref)
+            check("run_sharded_sweep", sweep, ref)
+            check("one-GPU finish_sweep", one, ref)
+            reps.append({"run_sharded_ms": [round(x, 2) for x in singles], "ten_run_sharded_ms": round(sum(singles), 2), "run_sharded_sweep_ms": round(ms_sweep, 2),
+                         "one_gpu_sweep_ms": round(ms_one, 2),
+                         "run_sharded_stages_ms_sum": {k: round(sum(s[k] for s, _ in single_res), 2) for k in STAGES},
+                         "run_sharded_sweep_stages_ms": {k: round(sweep[0][0][k], 2) for k in STAGES},
+                         "one_gpu_sweep_stages_ms": {k: round(one[0][0][k], 2) for k in STAGES},
+                         "exchanged_keys_sweep": sweep[0][0]["exchanged_keys"]})
+            print(f"[sweep {G} GPU] rep {rep}: ten run_sharded {sum(singles):.1f} ms, one run_sharded_sweep {ms_sweep:.1f} ms, one-GPU sweep {ms_one:.1f} ms", file=sys.stderr, flush=True)
+        med = lambda k: sorted(x[k] for x in reps)[len(reps) // 2]   # noqa: E731
+        out = {"gpus": gpus, "n_devices": G, "reads": base["reads"], "bam_bytes": int(bam.size), "rates": RATES, "repetitions": reps,
+               "per_rate": [{"rate": r, **{k: int(s[k]) for k in COUNTERS}, "coo_sha256_16": coo_hash(a)} for r, (s, a) in zip(RATES, ref)],
+               "median_ten_run_sharded_ms": med("ten_run_sharded_ms"), "median_run_sharded_sweep_ms": med("run_sharded_sweep_ms"), "median_one_gpu_sweep_ms": med("one_gpu_sweep_ms"),
+               "agreement": "per rate: total, cb_valid, sampled, valid, nnz and a sha256 of (m_gene, m_cell, m_count) equal between run_sharded, run_sharded_sweep and the one-GPU sweep",
+               "timing": "host wall clock around each whole call from a BAM image in host memory: context creation, H2D of the compressed bytes, all device work, results on the host",
+               "build": _lib.build_info()}
+        with open(os.path.join(args.out, "depth_sweep_%dgpu.json" % G), "w") as f:
+            json.dump(out, f, indent=1)
+        print(json.dumps({k: out[k] for k in ("gpus", "reads", "median_ten_run_sharded_ms", "median_run_sharded_sweep_ms", "median_one_gpu_sweep_ms")}))
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
-    ap.add_argument("--reads", type=int, default=64_000_000)
+    ap.add_argument("--reads", type=int, default=None, help="distinct reads (default 64 M; with --gpus, 64 M per GPU)")
     ap.add_argument("--cli-reads", type=int, default=16_000_000)
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--gpus", type=int, default=0, help="run the multi-GPU leg over devices 0..G-1 instead")
     args = ap.parse_args()
     os.makedirs(args.out, exist_ok=True)
+    if args.gpus:
+        return main_multi(args)
+    args.reads = args.reads or 64_000_000
     import torch
     import bench
     from fastf_b200 import _lib, build, bam2db_host as B
