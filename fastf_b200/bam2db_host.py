@@ -155,17 +155,16 @@ def make_params(lib, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, 
     return p, (ckeys, coff, gkeys, goff)
 
 
-def _result_to_python(lib, res, want_rows):
-    z32 = np.zeros(0, np.uint32)
-    out = {
-        "m_gene": np.ctypeslib.as_array(res.m_gene, (res.nnz,)).copy() if res.nnz else z32,
-        "m_cell": np.ctypeslib.as_array(res.m_cell, (res.nnz,)).copy() if res.nnz else z32,
-        "m_count": np.ctypeslib.as_array(res.m_count, (res.nnz,)).copy() if res.nnz else z32,
-        "row_keys": np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if (want_rows and res.n_rows) else np.zeros(0, np.uint64),
-    }
+def _result_to_python(res, copy=True, row_keys=None):
+    """(stats, arrays) of a filled Bam2dbResult: its counters and clocks, and with `copy` numpy copies of its COO and of its rows
+    (`row_keys` instead, where given); arrays is None without `copy`.  The caller frees res."""
     stats = {f: getattr(res, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
-    lib.fastf_bam2db_result_free(C.byref(res))
-    return stats, out
+    if not copy:
+        return stats, None
+    if row_keys is None:
+        row_keys = np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if res.n_rows else np.zeros(0, np.uint64)
+    coo = {c: np.ctypeslib.as_array(getattr(res, c), (res.nnz,)).copy() if res.nnz else np.zeros(0, np.uint32) for c in ("m_gene", "m_cell", "m_count")}
+    return stats, dict(coo, row_keys=row_keys)
 
 
 def run_sharded(lib, bam_bytes, inputs, rate_depth, seed, n_devices, want_rows=True, devices=None, **kw):
@@ -177,7 +176,8 @@ def run_sharded(lib, bam_bytes, inputs, rate_depth, seed, n_devices, want_rows=T
     devs = (C.c_int * n_devices)(*devices) if devices else None
     if lib.fastf_bam2db_run_sharded(n_devices, devs, C.byref(p), C.c_void_p(buf.ctypes.data), buf.size, C.byref(res)) != 0:
         raise _lib.FastfError("bam2db_run_sharded: " + lib.fastf_sharded_last_error().decode())
-    stats, out = _result_to_python(lib, res, want_rows)
+    stats, out = _result_to_python(res)
+    lib.fastf_bam2db_result_free(C.byref(res))
     stats["exchanged_keys"] = int(lib.fastf_sharded_exchanged())
     del keep
     return stats, out
@@ -190,15 +190,7 @@ def _sweep_to_python(res, thr, want_rows):
     row_rate = np.ctypeslib.as_array(res.row_rate, (res.n_rows,)).copy() if (want_rows and res.n_rows) else np.zeros(0, np.uint8)
     out = []
     for i in range(len(thr)):
-        r = res.rate[i]
-        z32 = np.zeros(0, np.uint32)
-        arrays = {
-            "m_gene": np.ctypeslib.as_array(r.m_gene, (r.nnz,)).copy() if r.nnz else z32,
-            "m_cell": np.ctypeslib.as_array(r.m_cell, (r.nnz,)).copy() if r.nnz else z32,
-            "m_count": np.ctypeslib.as_array(r.m_count, (r.nnz,)).copy() if r.nnz else z32,
-            "row_keys": rows[thr[row_rate] <= thr[i]],
-        }
-        stats = {f: getattr(r, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+        stats, arrays = _result_to_python(res.rate[i], row_keys=rows[thr[row_rate] <= thr[i]])
         stats["n_rows"] = len(arrays["row_keys"])
         out.append((stats, arrays))
     return out
@@ -273,16 +265,7 @@ class Bam2dbJob:
     def finish(self, copy=True):
         res = _lib.Bam2dbResult()
         self.ctx.check(self.lib.fastf_bam2db_finish(self.job, C.byref(res)), "bam2db_finish")
-        out = None
-        if copy:
-            z32 = np.zeros(0, np.uint32)
-            out = {
-                "m_gene": np.ctypeslib.as_array(res.m_gene, (res.nnz,)).copy() if res.nnz else z32,
-                "m_cell": np.ctypeslib.as_array(res.m_cell, (res.nnz,)).copy() if res.nnz else z32,
-                "m_count": np.ctypeslib.as_array(res.m_count, (res.nnz,)).copy() if res.nnz else z32,
-                "row_keys": np.ctypeslib.as_array(res.row_keys, (res.n_rows,)).copy() if (self.want_rows and res.n_rows) else np.zeros(0, np.uint64),
-            }
-        stats = {f: getattr(res, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+        stats, out = _result_to_python(res, copy)
         self.lib.fastf_bam2db_result_free(C.byref(res))
         return stats, out
 
@@ -301,7 +284,7 @@ class Bam2dbJob:
     def stats(self):
         res = _lib.Bam2dbResult()
         self.ctx.check(self.lib.fastf_bam2db_stats(self.job, C.byref(res)), "bam2db_stats")
-        return {f: getattr(res, f) for f, _ in _lib.Bam2dbResult._fields_ if not f.startswith("m_") and f != "row_keys"}
+        return _result_to_python(res, copy=False)[0]
 
     def close(self):
         if self.job:

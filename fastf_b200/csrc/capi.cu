@@ -56,13 +56,12 @@ struct fastf_ctx {
     bool crc_attr_set;
     u64 taghist_chunk_blocks = 0, taghist_round0_mask = 0;   // fastf_taghist_test_hooks
     void *mtj_polys;   // device copy of x^(2^k) mod phi, k = 0..44 (uploaded on first use)
-    void *mtj_scratch;
     // size-bucketed caches of device / pinned allocations: a job's buffers are recycled by the next job on the same
     // context, so steady-state calls do not pay cudaMalloc / cudaMallocHost (both synchronise the device)
     std::vector<PoolEntry> *dev_pool, *pin_pool;
     // Sizes the buffers of the last bam2db job ended with.  A buffer that grows in mid-job drains every stream (dev_reserve) and
     // leaves the device idle while the host queues the next chunk, so the next job starts its growing buffers at these sizes.
-    size_t hint_cand = 0, hint_keepbits = 0, hint_ring = 0;
+    size_t hint_cand = 0, hint_ring = 0;
 };
 
 static int ctx_fail(fastf_ctx *ctx, const char *fmt, ...)
@@ -313,7 +312,6 @@ extern "C" void fastf_ctx_destroy(fastf_ctx *ctx)
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     if (ctx->mtj_polys) cudaFree(ctx->mtj_polys);
-    if (ctx->mtj_scratch) cudaFree(ctx->mtj_scratch);
     pools_trim(ctx);
     delete ctx->dev_pool;
     delete ctx->pin_pool;

@@ -63,16 +63,14 @@ struct fastf_bam2db_job {
     u32 status = 0;
     bool header_done = false;
     std::vector<u8> carry;    // partial BGZF block left over by fastf_bam2db_feed
-    // MT19937 keep bits (the depth sweep: tempered words, one u32 per draw)
-    DevBuf mt_state, keepbits, mt_states, mt_scratch;
-    u64 mt_pairs_done = 0;     // twist pairs generated since mt_origin
-    u64 mt_origin = 0;         // stream index of bit (word) 0 of keepbits (0 unless the job jumped ahead)
-    bool mt_seeded = false;
+    // MT19937 keep bits from the job's first draw on (the depth sweep: tempered words, one u32 per draw)
+    DevBuf keepbits, mt_states, mt_scratch;
     cudaEvent_t ev_mt = nullptr;
     // sampling / sort / count
     bool sampled_done = false;
     u32 sweep_rates = 0;          // sampled by the depth sweep at this many rates (0: at the job's one rate)
-    DevBuf tile_valid, tile_tot, sample_counters, kept, orand;
+    DevBuf tile_valid, tile_tot, kept, orand;
+    DevBuf sample_counters;       // u64[2][FASTF_SWEEP_MAX_RATES]: sampled / valid reads per rate index (one rate: [0] / [FASTF_SWEEP_MAX_RATES])
     DevBuf kept_rate, rate_alt;   // depth sweep: rate index of every kept row, and its sort ping-pong buffer
     RleScratch rateS;             // depth sweep: the per-rate count over the distinct keys (held in rleS)
     PinBuf small_host;
@@ -83,8 +81,7 @@ struct fastf_bam2db_job {
     u64 n_blocks = 0, comp_bytes = 0, infl_bytes = 0;
     u64 n_blocks_fed = 0, n_blocks_done = 0;   // blocks handed to run_blocks / blocks whose candidate counts have come back
     u32 launches0 = 0, n_chunks = 0;
-    Timer t_infl[2], t_crc[2], t_parse[2], t_gather[2], t_mt[2], t_sample, t_sort, t_count;
-    u32 mt_launches = 0;
+    Timer t_infl[2], t_crc[2], t_parse[2], t_gather[2], t_mt, t_sample, t_sort, t_count;
     cudaEvent_t ev_first = nullptr, ev_last = nullptr;
     bool first_recorded = false;
     float ms_inflate = 0, ms_crc = 0, ms_parse = 0, ms_gather = 0, ms_mt = 0, ms_sample = 0, ms_sort = 0, ms_count = 0;
@@ -111,19 +108,18 @@ extern "C" void fastf_bam2db_job_free(fastf_bam2db_job *job)
         job->t_infl[i].destroy(); job->t_crc[i].destroy(); job->t_parse[i].destroy(); job->t_gather[i].destroy();
     }
     ctx->hint_cand = std::max(ctx->hint_cand, job->cand.cap);
-    ctx->hint_keepbits = std::max(ctx->hint_keepbits, job->keepbits.cap);
     for (auto &R : job->comp_ring) ctx->hint_ring = std::max(ctx->hint_ring, R.buf.cap);
     for (auto &R : job->comp_ring) {
         dev_release(ctx, R.buf);
         if (R.ev_copy) cudaEventDestroy(R.ev_copy);
         if (R.ev_free) cudaEventDestroy(R.ev_free);
     }
-    job->t_mt[0].destroy(); job->t_mt[1].destroy(); job->t_sample.destroy(); job->t_sort.destroy(); job->t_count.destroy();
+    job->t_mt.destroy(); job->t_sample.destroy(); job->t_sort.destroy(); job->t_count.destroy();
     if (job->ev_mt) cudaEventDestroy(job->ev_mt);
     if (job->ev_first) cudaEventDestroy(job->ev_first);
     if (job->ev_last) cudaEventDestroy(job->ev_last);
     dev_release(ctx, job->cells.slots); dev_release(ctx, job->cells.pool); dev_release(ctx, job->genes.slots); dev_release(ctx, job->genes.pool);
-    dev_release(ctx, job->counters); dev_release(ctx, job->hdr_off); dev_release(ctx, job->cand); dev_release(ctx, job->mt_state); dev_release(ctx, job->keepbits); dev_release(ctx, job->mt_states); dev_release(ctx, job->mt_scratch);
+    dev_release(ctx, job->counters); dev_release(ctx, job->hdr_off); dev_release(ctx, job->cand); dev_release(ctx, job->keepbits); dev_release(ctx, job->mt_states); dev_release(ctx, job->mt_scratch);
     dev_release(ctx, job->tile_valid); dev_release(ctx, job->tile_tot); dev_release(ctx, job->sample_counters); dev_release(ctx, job->kept); dev_release(ctx, job->orand);
     dev_release(ctx, job->kept_rate); dev_release(ctx, job->rate_alt);
     pin_release(ctx, job->small_host);
@@ -174,10 +170,9 @@ extern "C" int fastf_bam2db_begin(fastf_ctx *ctx, const fastf_bam2db_params *p, 
     rc = rc || table_upload(ctx, job->genes, p->gene_keys, p->gene_off, p->n_genes);
     rc = rc || dev_reserve(ctx, job->counters, 4 * sizeof(u64));
     rc = rc || dev_reserve(ctx, job->hdr_off, sizeof(u64));
-    rc = rc || dev_reserve(ctx, job->mt_state, 624 * sizeof(u32));
-    rc = rc || dev_reserve(ctx, job->sample_counters, 2 * sizeof(u64));
+    rc = rc || dev_reserve(ctx, job->sample_counters, 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64));
     rc = rc || dev_reserve(ctx, job->orand, 2 * sizeof(u64));
-    rc = rc || pin_reserve(ctx, job->small_host, 64);
+    rc = rc || pin_reserve(ctx, job->small_host, 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64));
     for (int i = 0; i < 2 && !rc; i++) {
         rc = rc || pin_reserve(ctx, job->slot[i].snap, 4 * sizeof(u64));
         rc = rc || cudaEventCreateWithFlags(&job->slot[i].ev_copy, cudaEventDisableTiming) != cudaSuccess;
@@ -190,7 +185,7 @@ extern "C" int fastf_bam2db_begin(fastf_ctx *ctx, const fastf_bam2db_params *p, 
         rc = rc || cudaEventCreateWithFlags(&R.ev_copy, cudaEventDisableTiming) != cudaSuccess;
         rc = rc || cudaEventCreateWithFlags(&R.ev_free, cudaEventDisableTiming) != cudaSuccess;
     }
-    rc = rc || job->t_mt[0].init() || job->t_mt[1].init() || job->t_sample.init() || job->t_sort.init() || job->t_count.init();
+    rc = rc || job->t_mt.init() || job->t_sample.init() || job->t_sort.init() || job->t_count.init();
     rc = rc || cudaEventCreateWithFlags(&job->ev_mt, cudaEventDisableTiming) != cudaSuccess;
     rc = rc || cudaEventCreate(&job->ev_first) != cudaSuccess || cudaEventCreate(&job->ev_last) != cudaSuccess;
     if (!rc) rc = cudaMemsetAsync(job->counters.p, 0, 4 * sizeof(u64), ctx->compute) != cudaSuccess;
@@ -201,109 +196,49 @@ extern "C" int fastf_bam2db_begin(fastf_ctx *ctx, const fastf_bam2db_params *p, 
     return 0;
 }
 
-// Extend the keep-bit stream (words: the tempered words) so that it covers stream indices [mt_origin, n_draws).  Runs on the mt stream.
-static int mt_extend(fastf_bam2db_job *job, u64 n_draws, bool words = false)
-{
-    fastf_ctx *ctx = job->ctx;
-    if (n_draws <= job->mt_origin) return 0;
-    const u64 pairs = (n_draws - job->mt_origin + 1247) / 1248;
-    if (pairs <= job->mt_pairs_done) return 0;
-    const size_t per_pair = (words ? 1248 : 39) * sizeof(u32);
-    const size_t need = (size_t)pairs * per_pair;
-    if (need > job->keepbits.cap) {
-        // grow geometrically; the copy keeps the bits produced so far
-        size_t want = std::max(std::max(need + need / 2, (size_t)(64u << 20)), ctx->hint_keepbits);
-        TRY(dev_reserve(ctx, job->keepbits, want, (size_t)job->mt_pairs_done * per_pair, ctx->mt));
-    }
-    Timer &tm = job->t_mt[job->mt_launches++ & 1u];   // the launch two extensions back has long finished
-    tm.collect(&job->ms_mt);
-    tm.start(ctx->mt);
-    FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->mt, job->prm.seed, job->mt_state.as<u32>(), job->mt_seeded ? 0u : 1u, job->mt_pairs_done, pairs - job->mt_pairs_done,
-                 job->prm.keep_threshold, words ? job->keepbits.as<u32>() : (u32 *)nullptr, words ? (u32 *)nullptr : job->keepbits.as<u32>());
-    CKL("mt19937");
-    tm.stop(ctx->mt);
-    job->mt_seeded = true;
-    job->mt_pairs_done = pairs;
-    return 0;
-}
-
-// Leave in `state` (624 words, device) the MT19937 window at stream index `origin`: seed, then apply x^(2^k) mod phi for every
-// set bit k of origin (jump-ahead, mt_jump.h).  Returns 1 when the polynomial tables are unavailable.
-static int mt_state_at(fastf_ctx *ctx, u32 seed, u64 origin, u32 *state, cudaStream_t s)
+// The jump polynomials x^(2^k) mod phi (mt_jump.h) on the device, uploaded once per context, with their count in *n_polys.  They
+// reach stream indices below 2^n_polys; `last_origin` is the largest index the caller jumps to.  The tables are a pure function of
+// constants and the draw index of a job is d0 plus a count of reads, so a failure here is a bug, not a property of the input.
+static int mt_jump_polys(fastf_ctx *ctx, const char *who, u64 last_origin, u32 *n_polys)
 {
     const fastf_mtj::Tables &T = fastf_mtj::tables();
-    if (!T.ok || (origin >> T.pow2.size()) != 0) return 1;
+    if (!T.ok) return ctx_fail(ctx, "%s: the MT19937 jump tables could not be built (Berlekamp-Massey did not find the degree-19937 polynomial)", who);
+    if ((last_origin >> T.pow2.size()) != 0)
+        return ctx_fail(ctx, "%s: MT19937 stream index %llu is beyond the jump tables (< 2^%zu)", who, (unsigned long long)last_origin, T.pow2.size());
     if (!ctx->mtj_polys) {
         std::vector<uint64_t> flat(T.pow2.size() * FASTF_MT_POLY_WORDS);
         for (size_t k = 0; k < T.pow2.size(); k++) memcpy(flat.data() + k * FASTF_MT_POLY_WORDS, T.pow2[k].data(), FASTF_MT_POLY_WORDS * sizeof(uint64_t));
         CK(cudaMalloc(&ctx->mtj_polys, flat.size() * sizeof(uint64_t)));
-        CK(cudaMalloc(&ctx->mtj_scratch, (size_t)(FASTF_MT_DEG + 624 + 64) * sizeof(u32)));
         CK(cudaMemcpy(ctx->mtj_polys, flat.data(), flat.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
     }
-    // seed only (no pairs): leaves the window x_0 .. x_623 in state
-    FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, s, seed, state, 1u, (u64)0, (u64)0, (u64)0, (u32 *)nullptr, (u32 *)nullptr);
-    CKL("mt19937_seed");
-    for (u32 k = 0; k < T.pow2.size(); k++) {
-        if (!((origin >> k) & 1ull)) continue;
-        FASTF_LAUNCH(fastf_mt_jump_kernel, 1, FASTF_MTJ_THREADS, 0, s, state, (const u64 *)ctx->mtj_polys + (size_t)k * FASTF_MT_POLY_WORDS, (u32 *)ctx->mtj_scratch);
-        CKL("mt_jump");
-    }
+    *n_polys = (u32)T.pow2.size();
     return 0;
 }
 
-// Restart the job's keep-bit stream at stream index `origin`; whatever was generated before is dropped.
-static int mt_jump_to(fastf_bam2db_job *job, u64 origin)
-{
-    fastf_ctx *ctx = job->ctx;
-    Timer &tm = job->t_mt[job->mt_launches++ & 1u];
-    tm.collect(&job->ms_mt);
-    tm.start(ctx->mt);
-    const int rc = mt_state_at(ctx, job->prm.seed, origin, job->mt_state.as<u32>(), ctx->mt);
-    tm.stop(ctx->mt);
-    if (rc) return rc;
-    job->mt_seeded = true;
-    job->mt_origin = origin;
-    job->mt_pairs_done = 0;
-    return 0;
-}
-
-// Keep bits (words: tempered words) for stream indices [first, first + n) generated by FASTF_MT_SEGMENTS CTAs at once: every CTA
-// jumps to the start of its own segment, then runs the normal twist.  Used once the number of draws is known (fastf_bam2db_sample,
-// the depth sweep); replaces whatever the job had generated speculatively.  Returns 1 when the jump tables are unavailable (caller
-// falls back to one sequential CTA).
+// Keep bits (words: tempered words) for stream indices [first, first + n) into job->keepbits from bit (word) 0 on, generated by
+// up to FASTF_MT_SEGMENTS CTAs at once: every CTA jumps to the start of its own segment of the reference's single stream, then
+// runs the normal twist.  Runs on the mt stream.
 #define FASTF_MT_SEGMENTS 32
-static int mt_generate_parallel(fastf_bam2db_job *job, u64 first, u64 n, cudaStream_t s, bool words = false)
+static int mt_generate_parallel(fastf_bam2db_job *job, const char *who, u64 first, u64 n, bool words)
 {
     fastf_ctx *ctx = job->ctx;
-    const fastf_mtj::Tables &T = fastf_mtj::tables();
-    if (!T.ok) return 1;
+    cudaStream_t s = ctx->mt;
     const u64 pairs = (n + 1247) / 1248;
     const u32 K = (u32)std::min<u64>(FASTF_MT_SEGMENTS, std::max<u64>(1, pairs / 64));
     const u64 ppc = (pairs + K - 1) / K;
-    if (((first + (u64)K * ppc * 1248ull) >> T.pow2.size()) != 0) return 1;
-    if (!ctx->mtj_polys) {
-        std::vector<uint64_t> flat(T.pow2.size() * FASTF_MT_POLY_WORDS);
-        for (size_t k = 0; k < T.pow2.size(); k++) memcpy(flat.data() + k * FASTF_MT_POLY_WORDS, T.pow2[k].data(), FASTF_MT_POLY_WORDS * sizeof(uint64_t));
-        CK(cudaMalloc(&ctx->mtj_polys, flat.size() * sizeof(uint64_t)));
-        CK(cudaMalloc(&ctx->mtj_scratch, (size_t)(FASTF_MT_DEG + 624 + 64) * sizeof(u32)));
-        CK(cudaMemcpy(ctx->mtj_polys, flat.data(), flat.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
-    }
+    u32 n_polys = 0;
+    TRY(mt_jump_polys(ctx, who, first + (u64)K * ppc * 1248ull, &n_polys));
     TRY(dev_reserve(ctx, job->mt_states, (size_t)K * 624 * sizeof(u32)));
     TRY(dev_reserve(ctx, job->mt_scratch, (size_t)K * FASTF_MTJ_SCRATCH * sizeof(u32)));
     TRY(dev_reserve(ctx, job->keepbits, (size_t)K * ppc * (words ? 1248 : 39) * sizeof(u32)));
-    Timer &tm = job->t_mt[job->mt_launches++ & 1u];
-    tm.collect(&job->ms_mt);
-    tm.start(s);
-    FASTF_LAUNCH(fastf_mt_jump_batch_kernel, K, FASTF_MTJ_THREADS, 0, s, job->prm.seed, (const u64 *)ctx->mtj_polys, (u32)T.pow2.size(), first, ppc * 1248ull, job->mt_states.as<u32>(),
+    job->t_mt.start(s);
+    FASTF_LAUNCH(fastf_mt_jump_batch_kernel, K, FASTF_MTJ_THREADS, 0, s, job->prm.seed, (const u64 *)ctx->mtj_polys, n_polys, first, ppc * 1248ull, job->mt_states.as<u32>(),
                  job->mt_scratch.as<u32>());
     CKL("mt_jump_batch");
     FASTF_LAUNCH(fastf_mt19937_kernel, K, FASTF_MT_THREADS, 0, s, job->prm.seed, job->mt_states.as<u32>(), 0u, (u64)0, ppc, job->prm.keep_threshold,
                  words ? job->keepbits.as<u32>() : (u32 *)nullptr, words ? (u32 *)nullptr : job->keepbits.as<u32>());
     CKL("mt19937");
-    tm.stop(s);
-    job->mt_seeded = true;
-    job->mt_origin = first;
-    job->mt_pairs_done = (u64)K * ppc;
+    job->t_mt.stop(s);
     return 0;
 }
 
@@ -653,45 +588,71 @@ extern "C" int fastf_bam2db_counts(fastf_bam2db_job *job, uint64_t *n_records, u
     return 0;
 }
 
-extern "C" int fastf_bam2db_sample(fastf_bam2db_job *job, uint64_t ordinal_base)
+static int report_feed_timing(fastf_bam2db_job *job);
+
+// The sampling pass of a job whose CB-valid reads meet draws d0 + ordinal_base + k: at the job's keep threshold (R null; draws as
+// keep bits), or at the depth sweep's sorted thresholds R (draws as tempered words).  hist[p] / hist[FASTF_SWEEP_MAX_RATES + p]: reads
+// / valid reads whose rate index is p (one rate: p = 0); the valid rows kept by the largest threshold land in job->kept, with the
+// sweep's rate indices in job->kept_rate (file order).
+static int sample_pass(fastf_bam2db_job *job, const char *who, u64 ordinal_base, const FastfSweepRates *R, u64 *hist)
 {
     fastf_ctx *ctx = job->ctx;
-    CK(cudaSetDevice(ctx->device));
-    if (job->sampled_done) return ctx_fail(ctx, "bam2db_sample: already sampled");
+    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already sampled", who);
     TRY(drain_chunks(job));
+    TRY(report_feed_timing(job));
     const u64 n = job->n_cand;
-    const u64 first_draw = job->prm.d0 + ordinal_base;
-    job->n_sampled = job->n_valid = 0;
-    if (n >= 0xffffffffull) return ctx_fail(ctx, "bam2db_sample: %llu CB-valid reads exceed the 2^32-1 limit of one device; shard over more GPUs", (unsigned long long)n);
+    if (n >= 0xffffffffull) return ctx_fail(ctx, "%s: %llu CB-valid reads exceed the 2^32-1 limit of one device; shard over more GPUs", who, (unsigned long long)n);
+    const u32 K = R ? R->k : 1;
+    const size_t hbytes = 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64);
+    memset(hist, 0, hbytes);
+    u64 nk = 0;
     if (n) {
-        // the number of draws is known now: generate exactly the keep bits [first_draw, first_draw + n) with 32 CTAs that each
-        // jump (GF(2) jump-ahead) to their own segment of the reference's single stream.  Fallback without the jump tables: one
-        // CTA generates the stream sequentially from the seed.
-        if (mt_generate_parallel(job, first_draw, n, ctx->mt)) TRY(mt_extend(job, first_draw + n));
+        // the number of draws is known now: generate exactly [d0 + ordinal_base, + n)
+        TRY(mt_generate_parallel(job, who, job->prm.d0 + ordinal_base, n, R != nullptr));
         CK(cudaEventRecord(job->ev_mt, ctx->mt));
         CK(cudaStreamWaitEvent(ctx->compute, job->ev_mt, 0));
         const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
+        const u64 *cand = job->cand.as<u64>();
+        const u32 *draws = job->keepbits.as<u32>();
         TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
         TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
-        CK(cudaMemsetAsync(job->sample_counters.p, 0, 2 * sizeof(u64), ctx->compute));
+        CK(cudaMemsetAsync(job->sample_counters.p, 0, hbytes, ctx->compute));
         job->t_sample.start(ctx->compute);
-        FASTF_LAUNCH(fastf_sample_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin,
-                     job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
-        CKL("sample_count");
+        if (R) FASTF_LAUNCH(fastf_sweep_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, cand, n, draws, *R, job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
+        else FASTF_LAUNCH(fastf_sample_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, cand, n, draws, job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
+        CKL(R ? "sweep_count" : "sample_count");
         TRY(launch_scan_rows(ctx, job->tile_valid.as<u32>(), ntiles, 1, job->tile_tot.as<u32>(), ctx->compute));
-        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, 2 * sizeof(u64), cudaMemcpyDeviceToHost, ctx->compute));
+        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, hbytes, cudaMemcpyDeviceToHost, ctx->compute));
         CK(cudaStreamSynchronize(ctx->compute));
-        job->n_sampled = job->small_host.as<u64>()[0];
-        job->n_valid = job->small_host.as<u64>()[1];
-        TRY(dev_reserve(ctx, job->kept, std::max<u64>(job->n_valid, 1) * sizeof(u64)));
-        FASTF_LAUNCH(fastf_sample_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin,
-                     (const u32 *)job->tile_valid.as<u32>(), job->kept.as<u64>());
-        CKL("sample_scatter");
+        memcpy(hist, job->small_host.p, hbytes);
+        for (u32 p = 0; p < K; p++) nk += hist[FASTF_SWEEP_MAX_RATES + p];
+        TRY(dev_reserve(ctx, job->kept, std::max<u64>(nk, 1) * sizeof(u64)));
+        const u32 *tile_off = job->tile_valid.as<u32>();
+        if (R) {
+            TRY(dev_reserve(ctx, job->kept_rate, std::max<u64>(nk, 1) * sizeof(u32)));
+            TRY(dev_reserve(ctx, job->rate_alt, std::max<u64>(nk, 1) * sizeof(u32)));
+            FASTF_LAUNCH(fastf_sweep_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, cand, n, draws, *R, tile_off, job->kept.as<u64>(), job->kept_rate.as<u32>());
+        } else {
+            FASTF_LAUNCH(fastf_sample_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, cand, n, draws, tile_off, job->kept.as<u64>());
+        }
+        CKL(R ? "sweep_scatter" : "sample_scatter");
         job->t_sample.stop(ctx->compute);
         CK(cudaEventRecord(job->ev_last, ctx->compute));
     }
     job->sampled_done = true;
+    job->sweep_rates = R ? K : 0;
+    job->n_sampled = 0;
+    for (u32 p = 0; p < K; p++) job->n_sampled += hist[p];
+    job->n_valid = nk;
     return 0;
+}
+
+extern "C" int fastf_bam2db_sample(fastf_bam2db_job *job, uint64_t ordinal_base)
+{
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+    return sample_pass(job, "bam2db_sample", ordinal_base, nullptr, hist);
 }
 
 extern "C" int fastf_bam2db_kept_device(fastf_bam2db_job *job, uint64_t **dev_keys, uint64_t *n)
@@ -761,7 +722,7 @@ static int fill_stats(fastf_bam2db_job *job, fastf_bam2db_result *res)
     res->n_blocks = job->n_blocks; res->compressed_bytes = job->comp_bytes; res->inflated_bytes = job->infl_bytes;
     res->status = job->status;
     for (int i = 0; i < 2; i++) { job->t_infl[i].collect(&job->ms_inflate); job->t_crc[i].collect(&job->ms_crc); job->t_parse[i].collect(&job->ms_parse); job->t_gather[i].collect(&job->ms_gather); }
-    job->t_mt[0].collect(&job->ms_mt); job->t_mt[1].collect(&job->ms_mt); job->t_sample.collect(&job->ms_sample); job->t_sort.collect(&job->ms_sort); job->t_count.collect(&job->ms_count);
+    job->t_mt.collect(&job->ms_mt); job->t_sample.collect(&job->ms_sample); job->t_sort.collect(&job->ms_sort); job->t_count.collect(&job->ms_count);
     res->ms_inflate = job->ms_inflate; res->ms_crc = job->ms_crc; res->ms_parse = job->ms_parse; res->ms_gather = job->ms_gather; res->ms_mt = job->ms_mt;
     res->ms_sample = job->ms_sample; res->ms_sort = job->ms_sort; res->ms_count = job->ms_count;
     if (job->first_recorded) {
@@ -784,7 +745,7 @@ extern "C" int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *re
     return fill_stats(job, res);
 }
 
-// FASTF_FEED_TIMING=1: the host-fed job's copy / inflate / parse timeline on stderr (once, at finish); releases its events
+// FASTF_FEED_TIMING=1: the host-fed job's copy / inflate / parse timeline on stderr (once, when the job is sampled); releases its events
 static int report_feed_timing(fastf_bam2db_job *job)
 {
     fastf_ctx *ctx = job->ctx;
@@ -828,7 +789,6 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
     memset(res, 0, sizeof *res);
     if (job->sweep_rates) return ctx_fail(ctx, "bam2db_finish: the job was sampled by the depth sweep");
     if (!job->sampled_done) TRY(fastf_bam2db_sample(job, 0));
-    TRY(report_feed_timing(job));
     const u64 n = job->n_valid;
     const FastfKeyLayout &L = job->L;
     if (job->prm.want_rows) {
@@ -864,7 +824,7 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
 
 // Depth sweep (include/fastf_gpu.h): draws as words -> per-rate histograms + (key, rate index) rows in file order -> ONE sort with the
 // rate index as least significant digit -> distinct keys with their smallest rate index -> per rate, a predicated count over them.
-// The front half (sweep_sample) runs per job, the back half (sweep_count) wherever the rows of a key meet: in the same job for one
+// The front half (sample_pass) runs per job, the back half (sweep_count) wherever the rows of a key meet: in the same job for one
 // GPU, on the receiving device of the exchange for several.
 
 // thresholds in caller order -> R (ascending) and order[p] = caller index of sorted position p; ties keep caller order, so a row's
@@ -879,58 +839,6 @@ static int sweep_rates(fastf_ctx *ctx, const char *who, uint32_t n_rates, const 
     memset(R, 0, sizeof *R);
     R->k = n_rates;
     for (u32 p = 0; p < n_rates; p++) R->t[p] = keep_thresholds[order[p]];
-    return 0;
-}
-
-// The job's CB-valid reads meet draws d0 + ordinal_base + k.  hist[p] / hist[FASTF_SWEEP_MAX_RATES + p]: reads / valid reads whose rate
-// index is p; the valid rows kept by the largest threshold land in job->kept / job->kept_rate (file order), *n_kept of them.
-static int sweep_sample(fastf_bam2db_job *job, const char *who, u64 ordinal_base, const FastfSweepRates &R, u64 *hist, u64 *n_kept)
-{
-    fastf_ctx *ctx = job->ctx;
-    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already sampled", who);
-    TRY(drain_chunks(job));
-    TRY(report_feed_timing(job));
-    const u64 n = job->n_cand;
-    if (n >= 0xffffffffull) return ctx_fail(ctx, "%s: %llu CB-valid reads exceed the 2^32-1 limit of one device", who, (unsigned long long)n);
-    const u64 first_draw = job->prm.d0 + ordinal_base;
-    const u32 K = R.k;
-    memset(hist, 0, 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64));
-    u64 nk = 0;
-    if (n) {
-        if (mt_generate_parallel(job, first_draw, n, ctx->mt, true)) TRY(mt_extend(job, first_draw + n, true));
-        CK(cudaEventRecord(job->ev_mt, ctx->mt));
-        CK(cudaStreamWaitEvent(ctx->compute, job->ev_mt, 0));
-        const size_t hbytes = 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64);
-        const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
-        TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
-        TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
-        TRY(dev_reserve(ctx, job->sample_counters, hbytes));
-        TRY(pin_reserve(ctx, job->small_host, hbytes));
-        CK(cudaMemsetAsync(job->sample_counters.p, 0, hbytes, ctx->compute));
-        job->t_sample.start(ctx->compute);
-        FASTF_LAUNCH(fastf_sweep_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin, R,
-                     job->tile_valid.as<u32>(), job->sample_counters.as<u64>());
-        CKL("sweep_count");
-        TRY(launch_scan_rows(ctx, job->tile_valid.as<u32>(), ntiles, 1, job->tile_tot.as<u32>(), ctx->compute));
-        CK(cudaMemcpyAsync(job->small_host.p, job->sample_counters.p, hbytes, cudaMemcpyDeviceToHost, ctx->compute));
-        CK(cudaStreamSynchronize(ctx->compute));
-        memcpy(hist, job->small_host.p, hbytes);
-        for (u32 p = 0; p < K; p++) nk += hist[FASTF_SWEEP_MAX_RATES + p];
-        TRY(dev_reserve(ctx, job->kept, std::max<u64>(nk, 1) * sizeof(u64)));
-        TRY(dev_reserve(ctx, job->kept_rate, std::max<u64>(nk, 1) * sizeof(u32)));
-        TRY(dev_reserve(ctx, job->rate_alt, std::max<u64>(nk, 1) * sizeof(u32)));
-        FASTF_LAUNCH(fastf_sweep_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->keepbits.as<u32>(), first_draw - job->mt_origin, R,
-                     (const u32 *)job->tile_valid.as<u32>(), job->kept.as<u64>(), job->kept_rate.as<u32>());
-        CKL("sweep_scatter");
-        job->t_sample.stop(ctx->compute);
-        CK(cudaEventRecord(job->ev_last, ctx->compute));
-    }
-    job->sampled_done = true;
-    job->sweep_rates = K;
-    job->n_sampled = 0;
-    for (u32 p = 0; p < K; p++) job->n_sampled += hist[p];
-    job->n_valid = nk;
-    *n_kept = nk;
     return 0;
 }
 
@@ -988,8 +896,8 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
     const u32 K = n_rates;
     const FastfKeyLayout &L = job->L;
     u64 hist[2 * FASTF_SWEEP_MAX_RATES];
-    u64 nk = 0;   // valid rows kept by the largest threshold
-    TRY(sweep_sample(job, who, 0, R, hist, &nk));
+    TRY(sample_pass(job, who, 0, &R, hist));
+    const u64 nk = job->n_valid;   // valid rows kept by the largest threshold
     // the rows in file order, each with the caller index of its rate
     if (job->prm.want_rows) {
         res->row_keys = (u64 *)malloc(std::max<u64>(nk, 1) * sizeof(u64));
@@ -1047,8 +955,8 @@ extern "C" int fastf_bam2db_sample_sweep(fastf_bam2db_job *job, uint64_t ordinal
     TRY(sweep_rates(ctx, who, n_rates, sorted_thresholds, &R, order));
     for (u32 i = 1; i < n_rates; i++)
         if (sorted_thresholds[i] < sorted_thresholds[i - 1]) return ctx_fail(ctx, "%s: thresholds must be non-decreasing (sorted_thresholds[%u] < sorted_thresholds[%u])", who, i, i - 1);
-    u64 hist[2 * FASTF_SWEEP_MAX_RATES], nk = 0;
-    TRY(sweep_sample(job, who, ordinal_base, R, hist, &nk));
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+    TRY(sample_pass(job, who, ordinal_base, &R, hist));
     u64 s = 0, v = 0;
     for (u32 p = 0; p < n_rates; p++) {
         s += hist[p];

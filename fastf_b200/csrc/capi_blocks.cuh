@@ -304,18 +304,23 @@ extern "C" int fastf_mt19937_host_from(fastf_ctx *ctx, uint32_t seed, uint64_t f
     CK(cudaSetDevice(ctx->device));
     if (n == 0) return 0;
     const u64 pairs = (n + 1247) / 1248;
-    DevBuf state, out;
+    u32 n_polys = 0;
+    TRY(mt_jump_polys(ctx, "mt19937_host_from", first, &n_polys));
+    DevBuf state, scratch, out;
     int rc = dev_reserve(ctx, state, 624 * sizeof(u32));
+    if (!rc) rc = dev_reserve(ctx, scratch, FASTF_MTJ_SCRATCH * sizeof(u32));
     if (!rc) rc = dev_reserve(ctx, out, (size_t)pairs * 1248 * sizeof(u32));
-    if (!rc) rc = mt_state_at(ctx, seed, first, state.as<u32>(), ctx->compute);
-    if (rc == 1 && !ctx->err[0]) ctx_fail(ctx, "mt19937_host_from: jump tables unavailable");
     if (!rc) {
+        // one CTA of the batched jump leaves the window at stream index `first`; the twist continues from there
+        FASTF_LAUNCH(fastf_mt_jump_batch_kernel, 1, FASTF_MTJ_THREADS, 0, ctx->compute, seed, (const u64 *)ctx->mtj_polys, n_polys, first, (u64)0, state.as<u32>(), scratch.as<u32>());
+        ctx->launches++;
         FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->compute, seed, state.as<u32>(), 0u, (u64)0, pairs, (u64)0, out.as<u32>(), (u32 *)nullptr);
         ctx->launches++;
         if (cudaGetLastError() != cudaSuccess) rc = ctx_fail(ctx, "mt19937 launch failed");
     }
     if (!rc) rc = fastf_memcpy_d2h(ctx, out_words, out.p, (size_t)n * sizeof(u32));
     dev_release(ctx, state);
+    dev_release(ctx, scratch);
     dev_release(ctx, out);
     return rc;
 }

@@ -6,8 +6,8 @@
 // phi the characteristic polynomial of F (degree 19937, minimal polynomial of every output bit sequence),
 //      W_{t+J} = g(F) W_t   with   g(x) = x^J mod phi(x)  =  sum_i g_i x^i,        i.e.   W_{t+J}[j] = XOR_{i : g_i = 1} x_{t+i+j}.
 // Host side (this header): phi by Berlekamp-Massey over one output bit of the generator, and the table g_k = x^(2^k) mod phi.
-// Device side (scan_mt_sample.cuh, fastf_mt_jump_kernel): generate x_t .. x_{t+19936+623} with the normal twist and take the XOR.
-// A jump by J applies g_k for every set bit k of J (<= 40 launches of ~0.3 ms).  Published method: Haramoto, Matsumoto,
+// Device side (scan_mt_sample.cuh, fastf_mt_jump_batch_kernel): generate x_t .. x_{t+19936+623} with the normal twist and take the
+// XOR.  A jump by J applies g_k for every set bit k of J; each CTA of the kernel makes its own jump.  Published method: Haramoto, Matsumoto,
 // Nishimura, Panneton, L'Ecuyer, "Efficient jump ahead for F2-linear random number generators" (2008).
 #pragma once
 #include <stdint.h>
@@ -121,7 +121,7 @@ static inline const Tables &tables()
     for (size_t n = 0; n < N; n++) s[n] = (uint8_t)(x[n + 624] >> 31);
     Poly C;
     const size_t L = berlekamp_massey(s, C);
-    if (L != FASTF_MT_DEG) return T;   // not ok: callers fall back to sequential generation
+    if (L != FASTF_MT_DEG) return T;   // not ok (a bug: the input is a constant); callers report the error
     // C(x) = 1 + C_1 x + .. + C_L x^L is the connection polynomial; the characteristic polynomial is its reciprocal x^L C(1/x)
     T.phi.assign(FASTF_MT_POLY_WORDS + 1, 0);
     for (size_t i = 0; i <= L; i++)

@@ -76,9 +76,8 @@ __device__ __forceinline__ u32 fastf_mt_temper(u32 y)
     return y;
 }
 // Produces twist pairs [pair0, pair0 + n_pairs): stream indices [pair0*1248, (pair0+n_pairs)*1248).
-// state (624 words in global memory) carries the generator between launches so the stream can be
-// extended chunk by chunk while the inflate kernel runs on another stream; it is always stored back.  Exactly one of out_words / out_bits is non-null.
-// do_seed != 0: start from init_genrand(seed); otherwise continue from `state` (left by a previous launch or by the jump kernel).
+// The final window is always stored back to `state` (624 words in global memory).  Exactly one of out_words / out_bits is non-null.
+// do_seed != 0: start from init_genrand(seed); otherwise continue from `state` (left by the batched jump kernel).
 // pair0 only positions the output (pair p writes words [p*1248, ..) or bit words [p*39, ..)).
 __global__ void __launch_bounds__(FASTF_MT_THREADS) fastf_mt19937_kernel(u32 seed, u32 *__restrict__ state, u32 do_seed, u64 pair0, u64 n_pairs, u64 threshold,
                                                                         u32 *__restrict__ out_words, u32 *__restrict__ out_bits)
@@ -132,38 +131,11 @@ __global__ void __launch_bounds__(FASTF_MT_THREADS) fastf_mt19937_kernel(u32 see
     for (u32 i = tid; i < 624; i += FASTF_MT_THREADS) state[i] = st[a][i];
 }
 
-// Jump-ahead (mt_jump.h): state <- g(F) state for one polynomial g (FASTF_MT_POLY_WORDS 64-bit words, bit i = g_i):
+// Jump-ahead (mt_jump.h): CTA b leaves in states[b] the window at stream index origin0 + b * stride: seed, then for every set bit k
+// of the origin the window <- g(F) window with g = polys[k] (FASTF_MT_POLY_WORDS 64-bit words, bit i = g_i):
 //     new[j] = XOR over set bits i of x_{i+j},   x_0.. = the raw recurrence words generated from the current window.
-// One CTA; scratch holds FASTF_MT_DEG + 624 words.
-#define FASTF_MTJ_THREADS 1024
-__global__ void __launch_bounds__(FASTF_MTJ_THREADS) fastf_mt_jump_kernel(u32 *__restrict__ state, const u64 *__restrict__ poly, u32 *__restrict__ scratch)
-{
-    const u32 tid = threadIdx.x;
-    for (u32 i = tid; i < 624; i += FASTF_MTJ_THREADS) scratch[i] = state[i];
-    __syncthreads();
-    // x_k = x_{k-227} ^ tw(x_{k-624}, x_{k-623}): 227 independent words per step
-    for (u32 base = 624; base < 19937u + 624u; base += 227u) {
-        const u32 k = base + tid;
-        if (tid < 227u && k < 19937u + 624u) scratch[k] = scratch[k - 227] ^ fastf_mt_tw(scratch[k - 624], scratch[k - 623]);
-        __syncthreads();
-    }
-    if (tid < 624u) {
-        u32 acc = 0;
-        for (u32 w = 0; w < 312u; w++) {
-            u64 bits = poly[w];
-            const u32 b0 = w * 64u + tid;
-            while (bits) {
-                const u32 b = (u32)__ffsll((long long)bits) - 1u;
-                bits &= bits - 1ull;
-                acc ^= scratch[b0 + b];
-            }
-        }
-        state[tid] = acc;
-    }
-}
-
-// Batched jump: CTA b leaves in states[b] the window at stream index origin0 + b * stride (seed, then one polynomial per set bit).
 // scratch: gridDim.x regions of FASTF_MTJ_SCRATCH words.
+#define FASTF_MTJ_THREADS 1024
 #define FASTF_MTJ_SCRATCH (19937 + 624 + 63)
 __global__ void __launch_bounds__(FASTF_MTJ_THREADS) fastf_mt_jump_batch_kernel(u32 seed, const u64 *__restrict__ polys, u32 n_polys, u64 origin0, u64 stride, u32 *__restrict__ states,
                                                                                u32 *__restrict__ scratch_all)
@@ -183,6 +155,7 @@ __global__ void __launch_bounds__(FASTF_MTJ_THREADS) fastf_mt_jump_batch_kernel(
         const u64 *poly = polys + (size_t)kbit * 312u;
         for (u32 i = tid; i < 624; i += FASTF_MTJ_THREADS) scratch[i] = win[i];
         __syncthreads();
+        // x_k = x_{k-227} ^ tw(x_{k-624}, x_{k-623}): 227 independent words per step
         for (u32 base = 624; base < 19937u + 624u; base += 227u) {
             const u32 k = base + tid;
             if (tid < 227u && k < 19937u + 624u) scratch[k] = scratch[k - 227] ^ fastf_mt_tw(scratch[k - 624], scratch[k - 623]);
@@ -209,7 +182,8 @@ __global__ void __launch_bounds__(FASTF_MTJ_THREADS) fastf_mt_jump_batch_kernel(
 // ------------------------------------------------------------------------------------------------
 // K3b: depth sampling.  Candidate i (file order) is the (ordinal_base + i)-th CB-valid read, i.e. it
 // consumes stream index d0 + ordinal_base + i (reference src/bam2db_ds.c:385-390; SampleInt's draws
-// come first, src/utils.c:53-62).  kept && key != INVALID rows are compacted, stably, into `kept`.
+// come first, src/utils.c:53-62); the draws are generated from that index on, so draw i belongs to
+// candidate i.  kept && key != INVALID rows are compacted, stably, into `kept`.
 // Two-phase: tile counts -> row scan -> scatter.
 // ------------------------------------------------------------------------------------------------
 #define FASTF_SAMPLE_THREADS 256
@@ -218,9 +192,9 @@ __global__ void __launch_bounds__(FASTF_MTJ_THREADS) fastf_mt_jump_batch_kernel(
 
 __device__ __forceinline__ bool fastf_keep_bit(const u32 *__restrict__ bits, u64 s) { return (bits[s >> 5] >> (s & 31u)) & 1u; }
 
-// counters: [0] sampled (kept draws), [1] valid (kept && insertable)
+// counters in the depth sweep's histogram layout with one rate: [0] sampled (kept draws), [FASTF_SWEEP_MAX_RATES] valid (kept && insertable)
 __global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
-fastf_sample_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ keepbits, u64 first_draw, u32 *__restrict__ tile_valid, u64 *__restrict__ counters)
+fastf_sample_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ keepbits, u32 *__restrict__ tile_valid, u64 *__restrict__ counters)
 {
     __shared__ u32 s_kept, s_valid;
     if (threadIdx.x == 0) { s_kept = 0; s_valid = 0; }
@@ -231,7 +205,7 @@ fastf_sample_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__rest
     for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
         u64 i = base + (u64)k * FASTF_SAMPLE_THREADS + threadIdx.x;
         if (i < n) {
-            bool kp = fastf_keep_bit(keepbits, first_draw + i);
+            bool kp = fastf_keep_bit(keepbits, i);
             kept += kp;
             valid += kp && (cand[i] != FASTF_INVALID_KEY);
         }
@@ -243,12 +217,12 @@ fastf_sample_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__rest
     if (threadIdx.x == 0) {
         tile_valid[blockIdx.x] = s_valid;
         atomicAdd((unsigned long long *)&counters[0], (unsigned long long)s_kept);
-        atomicAdd((unsigned long long *)&counters[1], (unsigned long long)s_valid);
+        atomicAdd((unsigned long long *)&counters[FASTF_SWEEP_MAX_RATES], (unsigned long long)s_valid);
     }
 }
 
 __global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
-fastf_sample_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ keepbits, u64 first_draw, const u32 *__restrict__ tile_off, u64 *__restrict__ kept)
+fastf_sample_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ keepbits, const u32 *__restrict__ tile_off, u64 *__restrict__ kept)
 {
     // blocked arrangement (thread t owns ITEMS consecutive candidates) keeps file order under a single block scan
     const u64 base = (u64)blockIdx.x * FASTF_SAMPLE_TILE + (u64)threadIdx.x * FASTF_SAMPLE_ITEMS;
@@ -260,7 +234,7 @@ fastf_sample_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__re
         bool v = false;
         if (i < n) {
             keys[k] = cand[i];
-            v = fastf_keep_bit(keepbits, first_draw + i) && keys[k] != FASTF_INVALID_KEY;
+            v = fastf_keep_bit(keepbits, i) && keys[k] != FASTF_INVALID_KEY;
         }
         flags |= (u32)v << k;
         cnt += v;
@@ -295,7 +269,7 @@ __device__ __forceinline__ u32 fastf_rate_index(const u64 *t, u32 k, u32 u)
 
 // hist: u64[2][FASTF_SWEEP_MAX_RATES]: row 0 = CB-valid reads with rate index b, row 1 = those whose key is insertable
 __global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
-fastf_sweep_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, u64 first_draw, FastfSweepRates R, u32 *__restrict__ tile_valid, u64 *__restrict__ hist)
+fastf_sweep_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, FastfSweepRates R, u32 *__restrict__ tile_valid, u64 *__restrict__ hist)
 {
     __shared__ u64 s_t[FASTF_SWEEP_MAX_RATES];
     __shared__ u32 s_h[2][FASTF_SWEEP_MAX_RATES];
@@ -310,7 +284,7 @@ fastf_sweep_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restr
     for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
         u64 i = base + (u64)k * FASTF_SAMPLE_THREADS + threadIdx.x;
         if (i < n) {
-            const u32 b = fastf_rate_index(s_t, K, words[first_draw + i]);
+            const u32 b = fastf_rate_index(s_t, K, words[i]);
             if (b < K) {
                 atomicAdd(&s_h[0][b], 1u);
                 if (cand[i] != FASTF_INVALID_KEY) { atomicAdd(&s_h[1][b], 1u); valid++; }
@@ -328,7 +302,7 @@ fastf_sweep_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restr
 }
 
 __global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
-fastf_sweep_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, u64 first_draw, FastfSweepRates R, const u32 *__restrict__ tile_off, u64 *__restrict__ kept,
+fastf_sweep_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ words, FastfSweepRates R, const u32 *__restrict__ tile_off, u64 *__restrict__ kept,
                            u32 *__restrict__ kept_rate)
 {
     __shared__ u64 s_t[FASTF_SWEEP_MAX_RATES];
@@ -346,7 +320,7 @@ fastf_sweep_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__res
         bool v = false;
         rb[k] = K;
         if (i < n) {
-            rb[k] = fastf_rate_index(s_t, K, words[first_draw + i]);
+            rb[k] = fastf_rate_index(s_t, K, words[i]);
             if (rb[k] < K) { keys[k] = cand[i]; v = keys[k] != FASTF_INVALID_KEY; }
         }
         flags |= (u32)v << k;

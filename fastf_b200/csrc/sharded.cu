@@ -13,9 +13,9 @@
 //   5. local sort + run-length dedup / count per device; the COO pieces concatenate in device order (cells are range partitioned
 //      and every piece is (cell, gene)-sorted), which is the single-GPU result and the reference's `mtx` table.
 //
-// The depth sweep (fastf_bam2db_run_sharded_sweep) shares steps 1, 2 and 4: in step 3 every shard samples at all rates at once and
-// keeps each distinct key with its smallest rate index, the exchange carries that index beside the key, and in step 5 every device
-// counts each rate over the keys it received (fastf_sweep_count_device).
+// The depth sweep (fastf_bam2db_run_sharded_sweep) runs the same steps for K sorted thresholds: in step 3 every shard samples at all
+// rates at once and keeps each distinct key with its smallest rate index, the exchange carries that index beside the key, and in
+// step 5 every device counts each rate over the keys it received (fastf_sweep_count_device).  The single rate is the case K = 1.
 //
 // This translation unit uses nothing but the public C-ABI, the CUDA runtime and NCCL.  NCCL is bound at run time (dlopen of
 // libnccl.so.2: a process that already holds an NCCL -- e.g. one that imported torch -- keeps its own copy).  The emulator build
@@ -80,20 +80,19 @@ struct Shard {
     fastf_ctx *ctx = nullptr;
     fastf_bam2db_job *job = nullptr;
     size_t byte_lo = 0, byte_hi = 0;
-    uint64_t n_rec = 0, n_cbv = 0, sampled = 0, valid = 0, n_kept = 0;
+    uint64_t n_rec = 0, n_cbv = 0, n_kept = 0;
     uint64_t *kept = nullptr;              // device, owned by the job
     uint64_t *send = nullptr, *recv = nullptr;   // device
-    uint32_t *coo[3] = {nullptr, nullptr, nullptr};
     std::vector<uint64_t> part;            // keys for each destination
-    uint64_t n_send = 0, n_recv = 0, nnz = 0;
+    uint64_t n_send = 0, n_recv = 0;
     std::vector<uint64_t> rows;            // kept rows of this shard, read order (want_rows)
     fastf_bam2db_result st;                // stage clocks / byte counts of this shard
     // depth sweep: rate index (position among the sorted thresholds) of every kept / sent / received key and of every row
     uint32_t *kept_rate = nullptr;         // device, owned by the job
     uint32_t *send_rate = nullptr, *recv_rate = nullptr;   // device
     std::vector<uint32_t> row_rate;
-    std::vector<uint64_t> sampled_k, valid_k, nnz_k;       // per sorted rate
-    std::vector<uint32_t *> coo_k[3];      // per sorted rate: this device's COO piece (host, fastf_sweep_count_device)
+    std::vector<uint64_t> sampled, valid, nnz;   // per sorted rate
+    std::vector<uint32_t *> coo[3];        // per sorted rate: this device's COO piece (host, malloc'ed by the library)
     float ms_sort = 0, ms_count = 0;
     int rc = 0;
     std::string err;
@@ -136,9 +135,8 @@ struct Run {
                 if (s.recv) fastf_device_free(s.ctx, s.recv);
                 if (s.send_rate) fastf_device_free(s.ctx, s.send_rate);
                 if (s.recv_rate) fastf_device_free(s.ctx, s.recv_rate);
-                for (auto &c : s.coo) if (c) fastf_device_free(s.ctx, c);
             }
-            for (auto &v : s.coo_k) for (auto p : v) fastf_free(p);
+            for (auto &v : s.coo) for (auto p : v) fastf_free(p);
             if (s.job) fastf_bam2db_job_free(s.job);
             if (s.ctx) fastf_ctx_destroy(s.ctx);
         }
@@ -309,9 +307,12 @@ static int all_to_all(const char *who, Run &X, bool rates)
         if (r || r2) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: NCCL all-to-all: %s", who, N.GetErrorString(r ? r : r2)); return 1; }
         for (auto &s : S) { cudaSetDevice(s.device); if (fastf_synchronize(s.ctx)) { fail(s, "synchronize after the exchange"); first_error(S); return 1; } }
     } else if (S[0].n_recv) {
+        // on the compute stream, which the counting step uses next: a device-to-device cudaMemcpy may return before the copy ends,
+        // and the context's streams do not wait for the legacy default stream
         cudaSetDevice(S[0].device);
-        if (cudaMemcpy(S[0].recv, S[0].send, (size_t)S[0].n_recv * 8, cudaMemcpyDeviceToDevice) != cudaSuccess ||
-            (rates && cudaMemcpy(S[0].recv_rate, S[0].send_rate, (size_t)S[0].n_recv * 4, cudaMemcpyDeviceToDevice) != cudaSuccess)) {
+        cudaStream_t st = (cudaStream_t)fastf_compute_stream(S[0].ctx);
+        if (cudaMemcpyAsync(S[0].recv, S[0].send, (size_t)S[0].n_recv * 8, cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
+            (rates && cudaMemcpyAsync(S[0].recv_rate, S[0].send_rate, (size_t)S[0].n_recv * 4, cudaMemcpyDeviceToDevice, st) != cudaSuccess)) {
             snprintf(g_sharded_err, sizeof g_sharded_err, "%s: device copy failed", who);
             return 1;
         }
@@ -332,146 +333,64 @@ static void merge_stats(const std::vector<Shard> &S, uint32_t bits_cell, uint32_
         res->status |= s.st.status; res->n_launches += s.st.n_launches; res->n_chunks += s.st.n_chunks;
         res->ms_inflate = std::max(res->ms_inflate, s.st.ms_inflate); res->ms_parse = std::max(res->ms_parse, s.st.ms_parse); res->ms_crc = std::max(res->ms_crc, s.st.ms_crc);
         res->ms_mt = std::max(res->ms_mt, s.st.ms_mt); res->ms_sample = std::max(res->ms_sample, s.st.ms_sample); res->ms_device_total = std::max(res->ms_device_total, s.st.ms_device_total);
+        res->ms_sort = std::max(res->ms_sort, s.ms_sort); res->ms_count = std::max(res->ms_count, s.ms_count);
     }
     res->bits_cell = bits_cell; res->bits_gene = bits_gene; res->bits_umi = bits_umi; res->umi_max_bytes = (bits_umi - 4) / 8;
 }
 
-extern "C" int fastf_bam2db_run_sharded(int n_devices, const int *devices, const fastf_bam2db_params *params, const void *bgzf_bytes, size_t n_bytes, fastf_bam2db_result *res)
+// Steps 1-6 for K thresholds sorted ascending (`thr`), or with thr null (K = 1) at the keep threshold of `params`.  res->rate[p] is
+// sorted rate p; with the sweep's want_rows, row_rate holds the sorted position of every row's rate.  A key's rate index in the
+// single-job result is the minimum over all its copies in the file; the minimum is associative, so every shard reduces its own copies
+// before the exchange (fastf_unique_partition_rates_device) and the receiving device reduces again over what the senders delivered
+// (fastf_sweep_count_device).  The cell-range partition puts every (cell, gene) group on one device, whose group rates are therefore
+// computed from complete data.
+static int run_shards(const char *who, int n_devices, const int *devices, const fastf_bam2db_params *params, const void *bgzf_bytes, size_t n_bytes, uint32_t K, const uint64_t *thr,
+                      fastf_bam2db_sweep_result *res)
 {
-    const char *who = "run_sharded";
-    g_sharded_err[0] = 0;
-    memset(res, 0, sizeof *res);
-    if (n_devices < 1 || n_devices > 64) { snprintf(g_sharded_err, sizeof g_sharded_err, "run_sharded: %d devices", n_devices); return 1; }
-    const int G = n_devices;
-    const uint8_t *bytes = (const uint8_t *)bgzf_bytes;
-    Run X((size_t)G);
-    std::vector<Shard> &S = X.S;
-    if (shard_blocks(who, bytes, n_bytes, devices, S) || open_and_feed(S, params, bytes)) return 1;
-
-    // ---- 3. global draw ordinals, sampling, local unique + partition ----
-    uint32_t bits_cell = 0, bits_gene = 0, bits_umi = 0;
-    const std::vector<uint64_t> bases = ordinal_bases(S);
-    bool ok = for_all(S, [&](Shard &s, size_t g) {
-        if (fastf_bam2db_sample(s.job, bases[g])) { fail(s, "sample"); return; }
-        if (fastf_bam2db_sample_counts(s.job, &s.sampled, &s.valid) || fastf_bam2db_kept_device(s.job, &s.kept, &s.n_kept)) { fail(s, "kept"); return; }
-        uint32_t bc, bg, bu;
-        if (fastf_bam2db_key_layout(s.job, &bc, &bg, &bu)) { fail(s, "key_layout"); return; }
-        if (g == 0) { bits_cell = bc; bits_gene = bg; bits_umi = bu; }
-        if (params->want_rows && s.n_kept) {
-            s.rows.resize((size_t)s.n_kept);
-            if (fastf_memcpy_d2h(s.ctx, s.rows.data(), s.kept, (size_t)s.n_kept * 8)) { fail(s, "rows d2h"); return; }
-        }
-        void *d = nullptr;
-        if (fastf_device_alloc(s.ctx, (size_t)std::max<uint64_t>(s.n_kept, 1) * 8, &d)) { fail(s, "device_alloc"); return; }
-        s.send = (uint64_t *)d;
-        s.part.assign((size_t)G, 0);
-        if (fastf_unique_partition_device(s.ctx, s.kept, s.n_kept, bc + bg + bu, bg, bu, params->n_cells, (uint32_t)G, s.send, s.part.data())) { fail(s, "unique_partition"); return; }
-        s.n_send = 0;
-        for (auto c : s.part) s.n_send += c;
-    });
-    if (!ok) { first_error(S); return 1; }
-    const uint32_t key_bits = bits_cell + bits_gene + bits_umi;
-
-    // ---- 4. the all-to-all ----
-    if (all_to_all(who, X, false)) return 1;
-
-    // ---- 5. local sort + dedup / count; COO pieces back to the host ----
-    std::vector<std::vector<uint32_t>> piece[3];
-    for (auto &v : piece) v.resize((size_t)G);
-    ok = for_all(S, [&](Shard &s, size_t g) {
-        for (auto &c : s.coo) {
-            void *d = nullptr;
-            if (fastf_device_alloc(s.ctx, (size_t)std::max<uint64_t>(s.n_recv, 1) * 4, &d)) { fail(s, "device_alloc"); return; }
-            c = (uint32_t *)d;
-        }
-        if (s.n_recv && fastf_sort_u64_device(s.ctx, s.recv, nullptr, s.n_recv, key_bits)) { fail(s, "sort"); return; }
-        if (fastf_dedup_count_device_out(s.ctx, s.recv, s.n_recv, bits_gene, bits_umi, &s.nnz, s.coo[0], s.coo[1], s.coo[2])) { fail(s, "dedup_count"); return; }
-        for (int c = 0; c < 3; c++) {
-            piece[c][g].resize((size_t)s.nnz);
-            if (s.nnz && fastf_memcpy_d2h(s.ctx, piece[c][g].data(), s.coo[c], (size_t)s.nnz * 4)) { fail(s, "coo d2h"); return; }
-        }
-        memset(&s.st, 0, sizeof s.st);
-        if (fastf_bam2db_stats(s.job, &s.st)) { fail(s, "stats"); return; }
-    });
-    if (!ok) { first_error(S); return 1; }
-
-    // ---- 6. the result, laid out like fastf_bam2db_finish's ----
-    merge_stats(S, bits_cell, bits_gene, bits_umi, res);
-    uint64_t nnz = 0, n_rows = 0;
-    for (auto &s : S) { res->sampled += s.sampled; res->valid += s.valid; nnz += s.nnz; n_rows += s.rows.size(); }
-    res->nnz = nnz;
-    res->m_gene = (uint32_t *)malloc(std::max<uint64_t>(nnz, 1) * 4);
-    res->m_cell = (uint32_t *)malloc(std::max<uint64_t>(nnz, 1) * 4);
-    res->m_count = (uint32_t *)malloc(std::max<uint64_t>(nnz, 1) * 4);
-    res->row_keys = params->want_rows ? (uint64_t *)malloc(std::max<uint64_t>(n_rows, 1) * 8) : nullptr;
-    if (!res->m_gene || !res->m_cell || !res->m_count || (params->want_rows && !res->row_keys)) {
-        snprintf(g_sharded_err, sizeof g_sharded_err, "run_sharded: out of host memory");
-        fastf_bam2db_result_free(res);
-        return 1;
-    }
-    uint64_t o = 0, ro = 0;
-    uint32_t *dst[3] = {res->m_gene, res->m_cell, res->m_count};
-    for (int g = 0; g < G; g++) {
-        for (int c = 0; c < 3; c++) memcpy(dst[c] + o, piece[c][(size_t)g].data(), (size_t)S[(size_t)g].nnz * 4);
-        o += S[(size_t)g].nnz;
-        if (params->want_rows) { memcpy(res->row_keys + ro, S[(size_t)g].rows.data(), S[(size_t)g].rows.size() * 8); ro += S[(size_t)g].rows.size(); }
-    }
-    res->n_rows = params->want_rows ? n_rows : 0;
-    return 0;
-}
-
-// The depth sweep over the shards.  A key's rate index in the single-job result is the minimum over all its copies in the file; the
-// minimum is associative, so every shard reduces its own copies before the exchange (fastf_unique_partition_rates_device) and the
-// receiving device reduces again over what the senders delivered (fastf_sweep_count_device).  The cell-range partition puts every
-// (cell, gene) group on one device, whose group rates are therefore computed from complete data.
-extern "C" int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices, const fastf_bam2db_params *params, const void *bgzf_bytes, size_t n_bytes, uint32_t n_rates,
-                                              const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
-{
-    const char *who = "run_sharded_sweep";
     g_sharded_err[0] = 0;
     memset(res, 0, sizeof *res);
     if (n_devices < 1 || n_devices > 64) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: %d devices", who, n_devices); return 1; }
-    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES || !keep_thresholds) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: 1..%u keep thresholds", who, (unsigned)FASTF_SWEEP_MAX_RATES); return 1; }
-    for (uint32_t i = 0; i < n_rates; i++)
-        if (keep_thresholds[i] > 4294967296ull) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: keep_thresholds[%u] > 2^32", who, i); return 1; }
-    const uint32_t K = n_rates;
-    // sorted position p <-> caller index order[p]; ties keep caller order (a row's rate maps to the first of equal thresholds)
-    std::vector<uint32_t> order(K), pos(K);
-    std::vector<uint64_t> thr(K);
-    for (uint32_t i = 0; i < K; i++) order[i] = i;
-    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return keep_thresholds[a] < keep_thresholds[b]; });
-    for (uint32_t p = 0; p < K; p++) { thr[p] = keep_thresholds[order[p]]; pos[order[p]] = p; }
+    const bool sweep = thr != nullptr;
     const int G = n_devices;
     const uint8_t *bytes = (const uint8_t *)bgzf_bytes;
     Run X((size_t)G);
     std::vector<Shard> &S = X.S;
     if (shard_blocks(who, bytes, n_bytes, devices, S) || open_and_feed(S, params, bytes)) return 1;
 
-    // ---- 3. global draw ordinals, sampling at every rate, rows, local unique + partition with the smallest rate index per key ----
+    // ---- 3. global draw ordinals, sampling, rows, local unique + partition (the sweep: with the smallest rate index per key) ----
     uint32_t bits_cell = 0, bits_gene = 0, bits_umi = 0;
     const std::vector<uint64_t> bases = ordinal_bases(S);
     bool ok = for_all(S, [&](Shard &s, size_t g) {
-        s.sampled_k.assign(K, 0);
-        s.valid_k.assign(K, 0);
-        if (fastf_bam2db_sample_sweep(s.job, bases[g], K, thr.data(), s.sampled_k.data(), s.valid_k.data())) { fail(s, "sample_sweep"); return; }
-        if (fastf_bam2db_kept_sweep_device(s.job, &s.kept, &s.kept_rate, &s.n_kept)) { fail(s, "kept"); return; }
+        s.sampled.assign(K, 0);
+        s.valid.assign(K, 0);
+        if (sweep ? fastf_bam2db_sample_sweep(s.job, bases[g], K, thr, s.sampled.data(), s.valid.data()) || fastf_bam2db_kept_sweep_device(s.job, &s.kept, &s.kept_rate, &s.n_kept)
+                  : fastf_bam2db_sample(s.job, bases[g]) || fastf_bam2db_sample_counts(s.job, &s.sampled[0], &s.valid[0]) || fastf_bam2db_kept_device(s.job, &s.kept, &s.n_kept)) {
+            fail(s, "sample");
+            return;
+        }
         uint32_t bc, bg, bu;
         if (fastf_bam2db_key_layout(s.job, &bc, &bg, &bu)) { fail(s, "key_layout"); return; }
         if (g == 0) { bits_cell = bc; bits_gene = bg; bits_umi = bu; }
         if (params->want_rows && s.n_kept) {   // before the partition, which overwrites the kept keys in place
             s.rows.resize((size_t)s.n_kept);
-            s.row_rate.resize((size_t)s.n_kept);
-            if (fastf_memcpy_d2h(s.ctx, s.rows.data(), s.kept, (size_t)s.n_kept * 8) || fastf_memcpy_d2h(s.ctx, s.row_rate.data(), s.kept_rate, (size_t)s.n_kept * 4)) { fail(s, "rows d2h"); return; }
+            if (fastf_memcpy_d2h(s.ctx, s.rows.data(), s.kept, (size_t)s.n_kept * 8)) { fail(s, "rows d2h"); return; }
+            if (sweep) {
+                s.row_rate.resize((size_t)s.n_kept);
+                if (fastf_memcpy_d2h(s.ctx, s.row_rate.data(), s.kept_rate, (size_t)s.n_kept * 4)) { fail(s, "rows d2h"); return; }
+            }
         }
         void *d = nullptr;
         if (fastf_device_alloc(s.ctx, (size_t)std::max<uint64_t>(s.n_kept, 1) * 8, &d)) { fail(s, "device_alloc"); return; }
         s.send = (uint64_t *)d;
-        if (fastf_device_alloc(s.ctx, (size_t)std::max<uint64_t>(s.n_kept, 1) * 4, &d)) { fail(s, "device_alloc"); return; }
-        s.send_rate = (uint32_t *)d;
+        if (sweep) {
+            if (fastf_device_alloc(s.ctx, (size_t)std::max<uint64_t>(s.n_kept, 1) * 4, &d)) { fail(s, "device_alloc"); return; }
+            s.send_rate = (uint32_t *)d;
+        }
         s.part.assign((size_t)G, 0);
         DevClock clock(s);
-        if (fastf_unique_partition_rates_device(s.ctx, s.kept, s.kept_rate, s.n_kept, bc + bg + bu, bg, bu, params->n_cells, (uint32_t)G, s.send, s.send_rate, s.part.data())) {
-            fail(s, "unique_partition_rates");
+        if (sweep ? fastf_unique_partition_rates_device(s.ctx, s.kept, s.kept_rate, s.n_kept, bc + bg + bu, bg, bu, params->n_cells, (uint32_t)G, s.send, s.send_rate, s.part.data())
+                  : fastf_unique_partition_device(s.ctx, s.kept, s.n_kept, bc + bg + bu, bg, bu, params->n_cells, (uint32_t)G, s.send, s.part.data())) {
+            fail(s, "unique_partition");
             return;
         }
         s.ms_sort = clock.stop();
@@ -481,16 +400,18 @@ extern "C" int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices,
     if (!ok) { first_error(S); return 1; }
     const uint32_t key_bits = bits_cell + bits_gene + bits_umi;
 
-    // ---- 4. the all-to-all of (key, rate index) ----
-    if (all_to_all(who, X, true)) return 1;
+    // ---- 4. the all-to-all of the keys (the sweep: with their rate indices) ----
+    if (all_to_all(who, X, sweep)) return 1;
 
-    // ---- 5. per device: every rate's COO piece ----
+    // ---- 5. per device: every rate's COO piece, back on the host ----
     ok = for_all(S, [&](Shard &s, size_t) {
-        s.nnz_k.assign(K, 0);
-        for (auto &v : s.coo_k) v.assign(K, nullptr);
+        s.nnz.assign(K, 0);
+        for (auto &v : s.coo) v.assign(K, nullptr);
         DevClock clock(s);
-        if (fastf_sweep_count_device(s.ctx, s.recv, s.recv_rate, s.n_recv, key_bits, bits_gene, bits_umi, K, s.nnz_k.data(), s.coo_k[0].data(), s.coo_k[1].data(), s.coo_k[2].data())) {
-            fail(s, "sweep_count");
+        if (sweep ? fastf_sweep_count_device(s.ctx, s.recv, s.recv_rate, s.n_recv, key_bits, bits_gene, bits_umi, K, s.nnz.data(), s.coo[0].data(), s.coo[1].data(), s.coo[2].data())
+                  : fastf_sort_u64_device(s.ctx, s.recv, nullptr, s.n_recv, key_bits) ||
+                        fastf_dedup_count_device(s.ctx, s.recv, s.n_recv, bits_gene, bits_umi, &s.nnz[0], &s.coo[0][0], &s.coo[1][0], &s.coo[2][0])) {
+            fail(s, "count");
             return;
         }
         s.ms_count = clock.stop();
@@ -499,39 +420,38 @@ extern "C" int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices,
     });
     if (!ok) { first_error(S); return 1; }
 
-    // ---- 6. the result, laid out like fastf_bam2db_finish_sweep's ----
+    // ---- 6. the result, laid out like fastf_bam2db_finish_sweep's in sorted rate order ----
     fastf_bam2db_result st;
     memset(&st, 0, sizeof st);
     merge_stats(S, bits_cell, bits_gene, bits_umi, &st);
-    for (auto &s : S) { st.ms_sort = std::max(st.ms_sort, s.ms_sort); st.ms_count = std::max(st.ms_count, s.ms_count); }
     bool oom = false;
-    for (uint32_t i = 0; i < K; i++) {
-        const uint32_t p = pos[i];
-        fastf_bam2db_result &r = res->rate[i];
+    for (uint32_t p = 0; p < K && !oom; p++) {
+        fastf_bam2db_result &r = res->rate[p];
         r = st;
-        for (auto &s : S) { r.sampled += s.sampled_k[p]; r.valid += s.valid_k[p]; r.nnz += s.nnz_k[p]; }
+        for (auto &s : S) { r.sampled += s.sampled[p]; r.valid += s.valid[p]; r.nnz += s.nnz[p]; }
         r.m_gene = (uint32_t *)malloc(std::max<uint64_t>(r.nnz, 1) * 4);
         r.m_cell = (uint32_t *)malloc(std::max<uint64_t>(r.nnz, 1) * 4);
         r.m_count = (uint32_t *)malloc(std::max<uint64_t>(r.nnz, 1) * 4);
-        if (!r.m_gene || !r.m_cell || !r.m_count) { oom = true; break; }
+        oom = !r.m_gene || !r.m_cell || !r.m_count;
         uint32_t *dst[3] = {r.m_gene, r.m_cell, r.m_count};
         uint64_t o = 0;
         for (auto &s : S) {
-            for (int c = 0; c < 3; c++) if (s.nnz_k[p]) memcpy(dst[c] + o, s.coo_k[c][p], (size_t)s.nnz_k[p] * 4);
-            o += s.nnz_k[p];
+            if (oom) break;
+            for (int c = 0; c < 3; c++) if (s.nnz[p]) memcpy(dst[c] + o, s.coo[c][p], (size_t)s.nnz[p] * 4);
+            o += s.nnz[p];
         }
     }
     if (!oom && params->want_rows) {
         uint64_t n_rows = 0;
         for (auto &s : S) n_rows += s.rows.size();
         res->row_keys = (uint64_t *)malloc(std::max<uint64_t>(n_rows, 1) * 8);
-        res->row_rate = (uint8_t *)malloc(std::max<uint64_t>(n_rows, 1));
-        oom = !res->row_keys || !res->row_rate;
+        res->row_rate = sweep ? (uint8_t *)malloc(std::max<uint64_t>(n_rows, 1)) : nullptr;
+        oom = !res->row_keys || (sweep && !res->row_rate);
         uint64_t ro = 0;
         for (auto &s : S) {
             if (oom) break;
             memcpy(res->row_keys + ro, s.rows.data(), s.rows.size() * 8);
-            for (size_t k = 0; k < s.row_rate.size(); k++) res->row_rate[ro + k] = (uint8_t)order[s.row_rate[k]];
+            for (size_t k = 0; k < s.row_rate.size(); k++) res->row_rate[ro + k] = (uint8_t)s.row_rate[k];
             ro += s.rows.size();
         }
         res->n_rows = oom ? 0 : n_rows;
@@ -542,5 +462,40 @@ extern "C" int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices,
         return 1;
     }
     res->n_rates = K;
+    return 0;
+}
+
+extern "C" int fastf_bam2db_run_sharded(int n_devices, const int *devices, const fastf_bam2db_params *params, const void *bgzf_bytes, size_t n_bytes, fastf_bam2db_result *res)
+{
+    memset(res, 0, sizeof *res);
+    fastf_bam2db_sweep_result one;
+    if (run_shards("run_sharded", n_devices, devices, params, bgzf_bytes, n_bytes, 1, nullptr, &one)) return 1;
+    *res = one.rate[0];
+    res->row_keys = one.row_keys;
+    res->n_rows = one.n_rows;
+    return 0;
+}
+
+extern "C" int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices, const fastf_bam2db_params *params, const void *bgzf_bytes, size_t n_bytes, uint32_t n_rates,
+                                              const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+{
+    const char *who = "run_sharded_sweep";
+    g_sharded_err[0] = 0;
+    memset(res, 0, sizeof *res);
+    if (n_rates < 1 || n_rates > FASTF_SWEEP_MAX_RATES || !keep_thresholds) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: 1..%u keep thresholds", who, (unsigned)FASTF_SWEEP_MAX_RATES); return 1; }
+    for (uint32_t i = 0; i < n_rates; i++)
+        if (keep_thresholds[i] > 4294967296ull) { snprintf(g_sharded_err, sizeof g_sharded_err, "%s: keep_thresholds[%u] > 2^32", who, i); return 1; }
+    const uint32_t K = n_rates;
+    // sorted position p <-> caller index order[p]; ties keep caller order (a row's rate maps to the first of equal thresholds)
+    std::vector<uint32_t> order(K), pos(K);
+    std::vector<uint64_t> thr(K);
+    for (uint32_t i = 0; i < K; i++) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return keep_thresholds[a] < keep_thresholds[b]; });
+    for (uint32_t p = 0; p < K; p++) { thr[p] = keep_thresholds[order[p]]; pos[order[p]] = p; }
+    fastf_bam2db_sweep_result sorted;
+    if (run_shards(who, n_devices, devices, params, bgzf_bytes, n_bytes, K, thr.data(), &sorted)) return 1;
+    *res = sorted;
+    for (uint32_t i = 0; i < K; i++) res->rate[i] = sorted.rate[pos[i]];
+    for (uint64_t r = 0; r < res->n_rows; r++) res->row_rate[r] = (uint8_t)order[res->row_rate[r]];
     return 0;
 }

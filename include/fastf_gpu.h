@@ -171,15 +171,16 @@ void fastf_bam2db_result_free(fastf_bam2db_result *res);
  * locally deduplicated keys with an NCCL all-to-all (ncclSend / ncclRecv over NVLink) partitioned by cell, and count locally.
  * res is laid out exactly like fastf_bam2db_finish's and is identical to the single-GPU result (and to the reference's tables:
  * src/bam2db_ds.c:360-438,480-483).  devices == NULL means 0..n_devices-1.  p->want_rows / umi_max_bytes / inflate_lanes as in
- * fastf_bam2db_begin (FASTF_BAM_STRADDLE is single-GPU only).  Returns 0, or 1 with fastf_sharded_last_error(). */
+ * fastf_bam2db_begin (FASTF_BAM_STRADDLE is single-GPU only).  Stage clocks: the maximum over devices; ms_sort = the local unique +
+ * partition, ms_count = the receiving-side sort + count including the copy of the COO piece to the host (CUDA events on
+ * fastf_compute_stream around each call).  Returns 0, or 1 with fastf_sharded_last_error(). */
 int fastf_bam2db_run_sharded(int n_devices, const int *devices, const fastf_bam2db_params *p, const void *bgzf_bytes, size_t n_bytes, fastf_bam2db_result *res);
 /* The depth sweep over the same shards: res equals what fastf_bam2db_finish_sweep returns for one job over the whole file with these
  * keep_thresholds (caller order, validated as there): every rate[i]'s counters and COO, and n_rows / row_keys / row_rate in file order.
  * Each shard samples its reads at all rates at once (fastf_bam2db_sample_sweep), keeps every distinct key once with its smallest rate
  * index, and sends the rate index beside the key in the same all-to-all; the receiving device counts every rate
- * (fastf_sweep_count_device).  Stage clocks as in fastf_bam2db_run_sharded (maximum over devices), except ms_sort = the maximum over
- * devices of the local unique + partition, and ms_count = the maximum over devices of fastf_sweep_count_device, which includes the
- * copies of every rate's COO piece to the host (CUDA events on fastf_compute_stream around each call); the same in every rate[i]. */
+ * (fastf_sweep_count_device).  Stage clocks as in fastf_bam2db_run_sharded, ms_count over every rate's count and COO copy; the same
+ * in every rate[i]. */
 int fastf_bam2db_run_sharded_sweep(int n_devices, const int *devices, const fastf_bam2db_params *p, const void *bgzf_bytes, size_t n_bytes, uint32_t n_rates,
                                    const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res);
 const char *fastf_sharded_last_error(void);

@@ -35,7 +35,7 @@ def test_mt19937_stream_matches_reference_generator(gpu_ctx, oracle):
 
 @pytest.mark.parametrize("seed,first", [(926, 1), (926, 623), (926, 624), (926, 1000003), (5489, 123456789), (7, 3_000_000_017)])
 def test_mt19937_jump_ahead_lands_on_the_reference_stream(gpu_ctx, oracle, seed, first):
-    """GF(2) jump-ahead (mt_jump.h + fastf_mt_jump_kernel): the outputs from stream index `first` on must be the reference generator's"""
+    """GF(2) jump-ahead (mt_jump.h + fastf_mt_jump_batch_kernel): the outputs from stream index `first` on must be the reference generator's"""
     from fastf_b200 import _lib
     n = 5000
     out = np.zeros(n, dtype=np.uint32)

@@ -12,7 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 @pytest.mark.parametrize("g,n_reads,rc,rd,seed", [(2, 6000, 0.7, 0.6, 31), (3, 5000, 1.0, 0.3, 926), (5, 2500, 0.5, 0.9, 4)])
 def test_c_sharded_driver_equals_single_job_and_oracle(g, n_reads, rc, rd, seed):
     from fastf_b200 import build
-    env = dict(os.environ, FASTF_GPU_LIB=build.build_emu(), FASTF_EMU_DEVICES=str(g), FASTF_MT_JUMP_MIN="0")
+    env = dict(os.environ, FASTF_GPU_LIB=build.build_emu(), FASTF_EMU_DEVICES=str(g))
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "sharded_c_worker.py"), str(g), str(n_reads), str(rc), str(rd), str(seed)], env=env,
                        stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
     assert r.returncode == 0 and "OK sharded C driver" in r.stdout, r.stdout[-3000:]
@@ -30,7 +30,7 @@ def test_c_cli_gpus_option_on_the_emulator(name, how, tmp_path):
     case = [c for c in json.load(open(os.path.join(gold, "manifest.json")))["cases"] if c["name"] == name][0]
     d = os.path.join(gold, case["dir"])
     out = str(tmp_path)
-    env = dict(os.environ, FASTF_EMU_DEVICES="3", FASTF_MT_JUMP_MIN="0")
+    env = dict(os.environ, FASTF_EMU_DEVICES="3")
     if how == "--gpus":
         exe, extra = build.build_cli(emu=True), ["--gpus", "3"]
     else:

@@ -26,8 +26,7 @@ def test_sharded_equals_reference(name, world, tmp_path):
     emu = build.build_emu()
     case = [c for c in json.load(open(os.path.join(GOLD, "manifest.json")))["cases"] if c["name"] == name][0]
     d = os.path.join(GOLD, case["dir"])
-    # FASTF_MT_JUMP_MIN=0: later ranks reach their first draw by GF(2) jump-ahead even on these tiny inputs
-    env = dict(os.environ, FASTF_GPU_LIB=emu, OMP_NUM_THREADS="1", FASTF_MT_JUMP_MIN="0")
+    env = dict(os.environ, FASTF_GPU_LIB=emu, OMP_NUM_THREADS="1")
     port = 29600 + (os.getpid() % 300)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world), "--master-addr", "127.0.0.1", "--master-port", str(port),
            os.path.join(ROOT, "tests", "sharded_worker.py"), d, str(tmp_path), str(case["rate_cell"]), str(case["rate_depth"]), str(case["seed"])]
@@ -86,7 +85,7 @@ def test_a_failing_rank_does_not_hang_the_others(tmp_path):
     open(d / "in.bam", "wb").write(bytes(raw))
     out = tmp_path / "out"
     out.mkdir()
-    env = dict(os.environ, FASTF_GPU_LIB=emu, OMP_NUM_THREADS="1", FASTF_MT_JUMP_MIN="0")
+    env = dict(os.environ, FASTF_GPU_LIB=emu, OMP_NUM_THREADS="1")
     port = 29900 + (os.getpid() % 90)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1", "--master-port", str(port),
            os.path.join(ROOT, "tests", "sharded_worker.py"), str(d), str(out), str(case["rate_cell"]), str(case["rate_depth"]), str(case["seed"])]

@@ -16,7 +16,7 @@ KEYS = ("total", "cb_valid", "sampled", "valid", "nnz")
 
 def _emu(args, devices):
     from fastf_b200 import build
-    env = dict(os.environ, FASTF_GPU_LIB=build.build_emu(), FASTF_EMU_DEVICES=str(devices), FASTF_MT_JUMP_MIN="0")
+    env = dict(os.environ, FASTF_GPU_LIB=build.build_emu(), FASTF_EMU_DEVICES=str(devices))
     r = subprocess.run([sys.executable, WORKER] + args, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
     assert r.returncode == 0 and "ok " in r.stdout, r.stdout[-3000:]
 
