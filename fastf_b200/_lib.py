@@ -37,6 +37,13 @@ class Bam2dbSweepResult(C.Structure):
                 ("n_rows", C.c_uint64), ("row_keys", c_u64p), ("row_rate", c_u8p)]
 
 
+GRID_MAX_CELL_RATES = 32   # FASTF_GRID_MAX_CELL_RATES
+
+
+class Bam2dbCellRate(C.Structure):
+    _fields_ = [("cell_index", c_u32p), ("n_cells", C.c_uint32), ("d0", C.c_uint64)]
+
+
 class FreqResult(C.Structure):
     _fields_ = [("n_reads", C.c_uint64), ("n_keys", C.c_uint64), ("key", c_u64p), ("count", c_u32p), ("first", c_u32p),
                 ("n_exceptions", C.c_uint64), ("exc_ordinal", c_u32p), ("exc_bytes", c_u8p), ("exc_stride", C.c_uint32),
@@ -88,6 +95,8 @@ _SIGS = {
     "fastf_bam2db_sweep_result_free": (None, [C.POINTER(Bam2dbSweepResult)]),
     "fastf_bam2db_sample_sweep": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, c_u64p, c_u64p, c_u64p]),
     "fastf_bam2db_kept_sweep_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), c_u64p]),
+    "fastf_bam2db_begin_grid": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbParams), C.POINTER(C.c_void_p)]),
+    "fastf_bam2db_finish_grid": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(Bam2dbCellRate), C.c_uint32, c_u64p, C.POINTER(Bam2dbSweepResult)]),
     "fastf_bam2db_stats": (C.c_int, [C.c_void_p, C.POINTER(Bam2dbResult)]),
     "fastf_bam2db_job_free": (None, [C.c_void_p]),
     "fastf_bam2db_result_free": (None, [C.POINTER(Bam2dbResult)]),

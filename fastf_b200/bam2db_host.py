@@ -65,11 +65,28 @@ def _strtok3(line):
     return toks, line[:key_end]
 
 
+def _read_features(features_file):
+    """(features, duplicate_features): (key, id, name, type) per distinct key, in file order (src/bam2db_ds.c:296-337)"""
+    feats, fseen = [], {}
+    duplicate = False
+    for ln in gzgets_lines(_read_maybe_gz(features_file)):
+        toks, key = _strtok3(ln)
+        if toks is None:
+            raise ValueError("feature line with fewer than three tab-separated fields (the reference dereferences NULL here)")
+        toks[2] = _cut(toks[2])
+        if key not in fseen:
+            fseen[key] = len(feats) + 1
+            feats.append((key, toks[0], toks[1], toks[2]))
+        else:
+            duplicate = True
+    return feats, duplicate
+
+
 class Bam2dbInputs:
     """Barcode sample + feature table exactly as the reference builds them (src/bam2db_ds.c:229-337)."""
 
-    def __init__(self, lib, barcodes_file, features_file, rate_cell, seed):
-        lines = gzgets_lines(_read_maybe_gz(barcodes_file))
+    def __init__(self, lib, barcodes_file, features_file, rate_cell, seed, _lists=None):
+        lines, (self.features, self.duplicate_features) = _lists or (gzgets_lines(_read_maybe_gz(barcodes_file)), _read_features(features_file))
         self.n_cells = len(lines)
         samp = np.zeros(max(self.n_cells, 1), dtype=np.uint64)
         d0 = C.c_uint64(0)
@@ -94,19 +111,31 @@ class Bam2dbInputs:
             else:
                 self.duplicate_barcodes = True   # index not advanced: no later line can match (src/bam2db_ds.c:260,281-285)
         self.cells = cells
-        feats, fseen = [], {}
-        self.duplicate_features = False
-        for ln in gzgets_lines(_read_maybe_gz(features_file)):
-            toks, key = _strtok3(ln)
-            if toks is None:
-                raise ValueError("feature line with fewer than three tab-separated fields (the reference dereferences NULL here)")
-            toks[2] = _cut(toks[2])
-            if key not in fseen:
-                fseen[key] = len(feats) + 1
-                feats.append((key, toks[0], toks[1], toks[2]))
-            else:
-                self.duplicate_features = True
-        self.features = feats
+
+    @classmethod
+    def grid(cls, lib, barcodes_file, features_file, cell_rates, seed):
+        """The cell-rate grid's inputs: a Bam2dbInputs whose cell table is the UNION of the tables of `cell_rates` (every barcode of any
+        table, in order of first appearance; its d0 is unused), with `tables` = the Bam2dbInputs of each cell rate (caller order) and
+        `remaps` = per cell rate a u32 array over the union cells: the 1-based index in that rate's table, 0 = not in it.  The union is
+        not the largest rate's table: a table stops at its first duplicate barcode, so a smaller rate's table can hold a barcode that a
+        larger rate's lacks.  Raises ValueError where a single rate would."""
+        lists = (gzgets_lines(_read_maybe_gz(barcodes_file)), _read_features(features_file))
+        tables = [cls(lib, barcodes_file, features_file, r, seed, _lists=lists) for r in cell_rates]
+        u = cls.__new__(cls)
+        u.n_cells, u.features, u.duplicate_features = len(lists[0]), lists[1][0], lists[1][1]
+        index = {}
+        for t in tables:
+            for bc in t.cells:
+                index.setdefault(bc, len(index))
+        u.cells = list(index)
+        u.n_cells_sampled, u.d0, u.duplicate_barcodes = len(u.cells), 0, any(t.duplicate_barcodes for t in tables)
+        u.tables = tables
+        u.remaps = []
+        for t in tables:
+            m = np.zeros(len(u.cells), dtype=np.uint32)
+            m[[index[bc] for bc in t.cells]] = np.arange(1, len(t.cells) + 1, dtype=np.uint32)
+            u.remaps.append(m)
+        return u
 
 
 def _pack_table(keys):
@@ -225,12 +254,14 @@ def run_sharded_sweep(lib, bam_bytes, inputs, rates, seed, n_devices, want_rows=
 class Bam2dbJob:
     """One streaming bam2db job on one GPU: begin -> feed*/feed_device* -> (counts -> sample(base)) -> finish."""
 
-    def __init__(self, ctx, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, umi_max_bytes=0, headerless=False):
+    def __init__(self, ctx, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, umi_max_bytes=0, headerless=False, grid=False):
+        """grid=True: a cell-rate grid job (fastf_bam2db_begin_grid) over the union table of Bam2dbInputs.grid, finished by finish_grid"""
         self.ctx, self.lib = ctx, ctx.lib
         p, self._keep = make_params(self.lib, inputs, rate_depth, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes, headerless)
         self.want_rows = want_rows
         self.job = C.c_void_p()
-        ctx.check(self.lib.fastf_bam2db_begin(ctx.h, C.byref(p), C.byref(self.job)), "bam2db_begin")
+        begin = self.lib.fastf_bam2db_begin_grid if grid else self.lib.fastf_bam2db_begin
+        ctx.check(begin(ctx.h, C.byref(p), C.byref(self.job)), "bam2db_begin_grid" if grid else "bam2db_begin")
 
     def feed(self, host_ptr, nbytes):
         self.ctx.check(self.lib.fastf_bam2db_feed(self.job, C.c_void_p(host_ptr), nbytes), "bam2db_feed")
@@ -281,6 +312,25 @@ class Bam2dbJob:
         finally:
             self.lib.fastf_bam2db_sweep_result_free(C.byref(res))
 
+    def finish_grid(self, cell_rates, rates):
+        """The cell-rate grid instead of finish(): cell_rates = [(cell_index u32 array over the union cells, n_cells, d0)] (as
+        Bam2dbInputs.grid gives them: its remaps, and each table's len(cells) and d0).  Returns, per cell rate, what finish_sweep(rates)
+        returns for a job begun with that rate's table."""
+        thr = _thresholds(self.lib, rates)
+        idx = [np.ascontiguousarray(ci, dtype=np.uint32) for ci, _, _ in cell_rates]
+        cr = (_lib.Bam2dbCellRate * max(len(cell_rates), 1))()
+        for k, (ci, (_, n, d0)) in enumerate(zip(idx, cell_rates)):
+            cr[k].cell_index = ci.ctypes.data_as(_lib.c_u32p)
+            cr[k].n_cells = n
+            cr[k].d0 = d0
+        res = (_lib.Bam2dbSweepResult * max(len(cell_rates), 1))()
+        try:
+            self.ctx.check(self.lib.fastf_bam2db_finish_grid(self.job, len(cell_rates), cr, len(thr), thr.ctypes.data_as(_lib.c_u64p), res), "bam2db_finish_grid")
+            return [_sweep_to_python(res[k], thr, self.want_rows) for k in range(len(cell_rates))]
+        finally:
+            for k in range(len(res)):
+                self.lib.fastf_bam2db_sweep_result_free(C.byref(res[k]))
+
     def stats(self):
         res = _lib.Bam2dbResult()
         self.ctx.check(self.lib.fastf_bam2db_stats(self.job, C.byref(res)), "bam2db_stats")
@@ -319,6 +369,18 @@ def run_device_sweep(ctx, bam_bytes, inputs, rates, seed, want_rows=True, inflat
     with Bam2dbJob(ctx, inputs, 0.0, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes) as job:
         _feed_all(job, bam_bytes, feed_piece)
         return job.finish_sweep(rates)
+
+
+def grid_cell_rates(union):
+    """finish_grid's cell_rates out of Bam2dbInputs.grid"""
+    return [(m, len(t.cells), t.d0) for m, t in zip(union.remaps, union.tables)]
+
+
+def run_device_grid(ctx, bam_bytes, union, rates, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
+    """run_device_sweep for every cell rate of Bam2dbInputs.grid out of one job: [[(stats, arrays)] per depth rate] per cell rate."""
+    with Bam2dbJob(ctx, union, 0.0, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes, grid=True) as job:
+        _feed_all(job, bam_bytes, feed_piece)
+        return job.finish_grid(grid_cell_rates(union), rates)
 
 
 def matrix_header(bam_file, rate_cell, rate_depth, total, sampled, valid):
@@ -504,11 +566,11 @@ def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell,
             ctx.close()
 
 
-def sweep_layout(db_name, path_out, rates):
-    """(name, float32 value, output directory, database) per rate: rate r writes into path_out/depth_<r as given>/, its database
+def sweep_layout(db_name, path_out, rates, prefix="depth_", what="the depth sweep", check_db=True):
+    """(name, float32 value, output directory, database) per rate: rate r writes into path_out/<prefix><r as given>/, its database
     is that directory's <basename of db_name>.  Raises ValueError on what the sweep refuses."""
     if not 1 <= len(rates) <= _lib.SWEEP_MAX_RATES:
-        raise ValueError("the depth sweep takes 1..%d rates" % _lib.SWEEP_MAX_RATES)
+        raise ValueError("%s takes 1..%d rates" % (what, _lib.SWEEP_MAX_RATES))
     out, seen = [], set()
     for r in rates:
         name = r if isinstance(r, str) else str(r)
@@ -516,10 +578,10 @@ def sweep_layout(db_name, path_out, rates):
         if name in seen or val.tobytes() in seen:
             raise ValueError("the rate %s is listed twice" % name)
         seen.update((name, val.tobytes()))
-        d = os.path.join(path_out, "depth_" + name)
+        d = os.path.join(path_out, prefix + name)
         out.append((name, float(val), d, os.path.join(d, os.path.basename(db_name))))
     for _, _, _, db in out:
-        if os.path.exists(db):
+        if check_db and os.path.exists(db):
             raise ValueError("database: %s already exists, change the name of database in -d argument!" % db)
     return out
 
@@ -563,6 +625,72 @@ def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate
             print("Depth rate %s -> %s" % (name, d))
             if write_outputs(db, bam_file, d, inputs, rate_cell, val, stats, out, ctx=ctx):
                 return 1
+        return 0
+    except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
+        sys.stderr.write("bam2db: %s\n" % e)
+        return 1
+    finally:
+        for db in dbs:
+            db.close()
+        if own and ctx is not None:
+            ctx.close()
+
+
+def grid_layout(db_name, path_out, cell_rates, rates):
+    """(cell name, cell value, [(depth name, depth value, output directory, database)]) per cell rate: with a list of depth rates, set
+    (i, j) goes to path_out/cell_<Ci>/depth_<Rj>/, with one depth rate (a number or a string, as -r) to path_out/cell_<Ci>/.  Raises
+    ValueError on what the grid refuses."""
+    depths = isinstance(rates, (list, tuple))
+    out = []
+    for cname, cval, cdir, cdb in sweep_layout(db_name, path_out, cell_rates, "cell_", "the cell-rate grid", check_db=False):
+        if depths:
+            out.append((cname, cval, sweep_layout(db_name, cdir, rates)))
+        else:
+            if os.path.exists(cdb):
+                raise ValueError("database: %s already exists, change the name of database in -d argument!" % cdb)
+            out.append((cname, cval, [(str(rates), float(np.float32(float(rates))), cdir, cdb)]))
+    return out
+
+
+def bam2db_grid(bam_file, db_name, path_out, barcodes_file, features_file, cell_rates, rates, seed=926, device=0, ctx=None, gpus=1):
+    """bam2db at several cell rates x depth rates out of one pass over the BAM.  Set (i, j) is exactly what
+    bam2db(bam_file, <its database>, <its directory>, ..., cell_rates[i], rates[j], seed) writes; see grid_layout for where it goes.
+    One GPU only (gpus > 1 is refused).  Returns 0 / 1 like bam2db."""
+    own = ctx is None
+    dbs = []
+    try:
+        layout = grid_layout(db_name, path_out, cell_rates, rates)
+        if gpus != 1:
+            raise ValueError("the cell-rate grid runs on one GPU")
+        depth_vals = [v for _, v, _, _ in layout[0][2]]
+        if own:
+            ctx = _lib.Context(device)
+        union = Bam2dbInputs.grid(ctx.lib, barcodes_file, features_file, [v for _, v, _ in layout], seed)
+        print("Total number of cells: %d" % union.n_cells)
+        for (cname, _, sets), t in zip(layout, union.tables):
+            print("Cell rate %s: actual number of sampled cell barcodes: %d" % (cname, t.n_cells_sampled))
+            for _, _, d, dbf in sets:
+                os.makedirs(d, exist_ok=True)
+                db = open_database(dbf, bam_file, barcodes_file, features_file)
+                if db is None:
+                    return 1
+                dbs.append(db)
+                insert_lists(db, t)
+        if union.duplicate_barcodes:
+            print("Warning: Duplicate cell barcodes were found in %s!" % barcodes_file)
+        if union.duplicate_features:
+            print("Warning: Duplicate feature names were found in %s!" % features_file)
+        print("Start to convert bam file to sqlite3 database...")
+        sys.stdout.flush()
+        bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
+        results = _run_with_retries(lambda mb, fl: run_device_grid(ctx, bam_bytes, union, depth_vals, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+        k = 0
+        for (cname, cval, sets), t, per_depth in zip(layout, union.tables, results):
+            for (dname, dval, d, _), (stats, out) in zip(sets, per_depth):
+                print("Cell rate %s, depth rate %s -> %s" % (cname, dname, d))
+                if write_outputs(dbs[k], bam_file, d, t, cval, dval, stats, out, ctx=ctx):
+                    return 1
+                k += 1
         return 0
     except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
         sys.stderr.write("bam2db: %s\n" % e)

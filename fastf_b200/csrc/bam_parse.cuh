@@ -137,8 +137,10 @@ __global__ void fastf_bam_header_kernel(const u8 *__restrict__ infl, u64 n, u64 
 }
 
 // One alignment record [rec, rend) (after its block_size word): the reference's per-read decision up to the draw.
-// Returns 0 = not CB-valid (no candidate), 1 = candidate with *key set (FASTF_INVALID_KEY when it would not be inserted).
-template <class Acc>
+// Returns 0 = not CB-valid (no candidate), 1 = candidate with *key set.  A candidate that would not be inserted is FASTF_INVALID_KEY,
+// or with KEEP_CELL (the cell-rate grid, whose union table is remapped per cell rate later) its cell alone: cidx << (bits_gene +
+// bits_umi), gene field 0, which no insertable key has (feature indices start at 1).
+template <bool KEEP_CELL, class Acc>
 __device__ __forceinline__ u32 fastf_parse_record(const Acc &A, u64 rec, u64 rend, u32 bs, const FastfStrTableView &cells, const FastfStrTableView &genes, const FastfKeyLayout &L,
                                                   u32 c_pw1, u32 c_pw2, u32 g_pw1, u32 g_pw2, u32 lane, u32 *status, u64 *key_out)
 {
@@ -205,7 +207,7 @@ __device__ __forceinline__ u32 fastf_parse_record(const Acc &A, u64 rec, u64 ren
     if (cidx == 0) return 0;
 
     // ---- this record consumes a draw; decide whether it would be inserted if kept ----
-    u64 key = FASTF_INVALID_KEY;
+    u64 key = KEEP_CELL ? (u64)cidx << (L.bits_gene + L.bits_umi) : FASTF_INVALID_KEY;
     i64 xfv = 0;
     if (found & 2u) {
         const u64 x = xf.off;
@@ -321,6 +323,7 @@ __device__ __forceinline__ u32 fastf_table_lookup_lane(const FastfStrTableView &
 }
 
 // scalar twin of fastf_parse_record (same decisions, one thread); rec / rend are offsets into the window, bs = rend - rec
+template <bool KEEP_CELL>
 __device__ __forceinline__ u32 fastf_parse_record_lane(const FastfWin32 &A, u32 rec, u32 rend, u32 bs, const FastfStrTableView &cells, const FastfStrTableView &genes, const FastfKeyLayout &L,
                                                        u32 *status, u64 *key_out)
 {
@@ -371,7 +374,7 @@ __device__ __forceinline__ u32 fastf_parse_record_lane(const FastfWin32 &A, u32 
     if (!(found & 1u) || !(cb_type == 'Z' || cb_type == 'H')) return 0;
     const u32 cidx = fastf_table_lookup_lane(cells, A, cb_off, cb_len);
     if (cidx == 0) return 0;
-    u64 key = FASTF_INVALID_KEY;
+    u64 key = KEEP_CELL ? (u64)cidx << (L.bits_gene + L.bits_umi) : FASTF_INVALID_KEY;
     i64 xfv = 0;
     if (found & 2u) {
         const u32 x = xf_off;
@@ -423,6 +426,8 @@ __device__ __forceinline__ u32 fastf_parse_record_lane(const FastfWin32 &A, u32 
 // 32 records in flight per warp instead of 32 lanes repeating one record's scalar work), (4) the CB-valid records'
 // keys are compacted in record order with a ballot.  Records larger than the window take the warp-cooperative
 // global-memory path.  infl_total = readable bytes of the inflated buffer (>= end of the last block, multiple of 16).
+// KEEP_CELL: see fastf_parse_record (false for every job but the cell-rate grid's).
+template <bool KEEP_CELL>
 __global__ void __launch_bounds__(FASTF_PARSE_WARPS * 32)
 fastf_bam_parse_kernel(const u8 *__restrict__ infl, u64 infl_total, const u64 *__restrict__ blk_off, const u32 *__restrict__ blk_isize, u32 nblocks, const u64 *__restrict__ first_record_off_ptr,
                        FastfStrTableView cells, FastfStrTableView genes, FastfKeyLayout L,
@@ -485,7 +490,7 @@ fastf_bam_parse_kernel(const u8 *__restrict__ infl, u64 infl_total, const u64 *_
             if (p + 4 + (u64)bs > bend) { status |= FASTF_ST_REC_STRADDLE; break; }
             const FastfGlobAcc GA = {infl};
             u64 key = 0;
-            const u32 r = fastf_parse_record(GA, p + 4, p + 4 + bs, bs, cells, genes, L, cells.pw1[lane], cells.pw2[lane], genes.pw1[lane], genes.pw2[lane], lane, &status, &key);
+            const u32 r = fastf_parse_record<KEEP_CELL>(GA, p + 4, p + 4 + bs, bs, cells, genes, L, cells.pw1[lane], cells.pw2[lane], genes.pw1[lane], genes.pw2[lane], lane, &status, &key);
             if (r == 2) break;
             p += 4 + (u64)bs;
             nrec++;
@@ -499,7 +504,7 @@ fastf_bam_parse_kernel(const u8 *__restrict__ infl, u64 infl_total, const u64 *_
         // (3) one record per lane
         u64 key = 0;
         u32 r = 0, st = 0;
-        if (lane < nb) r = fastf_parse_record_lane(WA, myrec, myrec + mybs, mybs, cells, genes, L, &st, &key);
+        if (lane < nb) r = fastf_parse_record_lane<KEEP_CELL>(WA, myrec, myrec + mybs, mybs, cells, genes, L, &st, &key);
         // (4) ordered compaction; a corrupt record ends the block at that record
         const u32 badm = __ballot_sync(FASTF_FULL_MASK, r == 2);
         u32 good = nb;

@@ -1,6 +1,6 @@
 // Part of the libfastf_gpu translation unit (capi.cu includes it, in this order; it is not a header of its own):
 // the bam2db job: chunk pipeline (copy ring, inflate / CRC / parse / gather per chunk), MT19937 keep bits, sampling, sort, dedup / count, results;
-// the depth sweep (several rates out of one job).
+// the depth sweep (several rates out of one job); the cell-rate grid (several cell tables and depth rates out of one job).
 #pragma once
 
 // ---------------------------------------------------------------------------------------------------
@@ -75,6 +75,10 @@ struct fastf_bam2db_job {
     RleScratch rateS;             // depth sweep: the per-rate count over the distinct keys (held in rleS)
     PinBuf small_host;
     u64 n_sampled = 0, n_valid = 0;
+    // cell-rate grid (fastf_bam2db_begin_grid): `cand` holds the union table's candidates and stays; per cell rate, the remap table
+    // and the candidate array of that rate's own table (also the sort's ping-pong buffer once it has been sampled)
+    bool grid = false;
+    DevBuf grid_remap, grid_cand;
     SortScratch sortS;
     RleScratch rleS;
     // stats
@@ -122,6 +126,7 @@ extern "C" void fastf_bam2db_job_free(fastf_bam2db_job *job)
     dev_release(ctx, job->counters); dev_release(ctx, job->hdr_off); dev_release(ctx, job->cand); dev_release(ctx, job->keepbits); dev_release(ctx, job->mt_states); dev_release(ctx, job->mt_scratch);
     dev_release(ctx, job->tile_valid); dev_release(ctx, job->tile_tot); dev_release(ctx, job->sample_counters); dev_release(ctx, job->kept); dev_release(ctx, job->orand);
     dev_release(ctx, job->kept_rate); dev_release(ctx, job->rate_alt);
+    dev_release(ctx, job->grid_remap); dev_release(ctx, job->grid_cand);
     pin_release(ctx, job->small_host);
     sort_scratch_release(ctx, job->sortS);
     rle_scratch_release(ctx, job->rleS);
@@ -367,7 +372,8 @@ static int run_chunk(fastf_bam2db_job *job, const FastfBgzfBlock *blocks, u32 nb
     if (straddle) TRY(launch_virtual_blocks(ctx, S.virt, (const u8 *)S.infl.as<u8>(), out_total, S.idx.out_off, S.idx.isize, nb, job->hdr_off.as<u64>(), (u32 *)(job->counters.as<u64>() + 2), &p_off, &p_size,
                                             ctx->compute));
     if (nb) {
-        FASTF_LAUNCH(fastf_bam_parse_kernel, (nb + FASTF_PARSE_WARPS - 1) / FASTF_PARSE_WARPS, FASTF_PARSE_WARPS * 32, 0, ctx->compute, (const u8 *)S.infl.as<u8>(), (u64)((out_total + 15) & ~15ull),
+        const auto parse = job->grid ? fastf_bam_parse_kernel<true> : fastf_bam_parse_kernel<false>;
+        FASTF_LAUNCH(parse, (nb + FASTF_PARSE_WARPS - 1) / FASTF_PARSE_WARPS, FASTF_PARSE_WARPS * 32, 0, ctx->compute, (const u8 *)S.infl.as<u8>(), (u64)((out_total + 15) & ~15ull),
                      p_off, p_size, nb, (const u64 *)job->hdr_off.as<u64>(), job->cells.view, job->genes.view, job->L, (const u64 *)S.idx.stage_off,
                      S.stage.as<u64>(), S.idx.nrec, S.idx.ncbv, S.idx.st_parse);
         CKL("bam_parse");
@@ -590,29 +596,24 @@ extern "C" int fastf_bam2db_counts(fastf_bam2db_job *job, uint64_t *n_records, u
 
 static int report_feed_timing(fastf_bam2db_job *job);
 
-// The sampling pass of a job whose CB-valid reads meet draws d0 + ordinal_base + k: at the job's keep threshold (R null; draws as
-// keep bits), or at the depth sweep's sorted thresholds R (draws as tempered words).  hist[p] / hist[FASTF_SWEEP_MAX_RATES + p]: reads
-// / valid reads whose rate index is p (one rate: p = 0); the valid rows kept by the largest threshold land in job->kept, with the
+// The sampling pass over candidates cand[0, n) (file order) whose k-th meets draw first_draw + k: at the job's keep threshold (R null;
+// draws as keep bits), or at the depth sweep's sorted thresholds R (draws as tempered words).  hist[p] / hist[FASTF_SWEEP_MAX_RATES + p]:
+// reads / valid reads whose rate index is p (one rate: p = 0); the valid rows kept by the largest threshold land in job->kept, with the
 // sweep's rate indices in job->kept_rate (file order).
-static int sample_pass(fastf_bam2db_job *job, const char *who, u64 ordinal_base, const FastfSweepRates *R, u64 *hist)
+static int sample_cands(fastf_bam2db_job *job, const char *who, u64 first_draw, const u64 *cand, u64 n, const FastfSweepRates *R, u64 *hist)
 {
     fastf_ctx *ctx = job->ctx;
-    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already sampled", who);
-    TRY(drain_chunks(job));
-    TRY(report_feed_timing(job));
-    const u64 n = job->n_cand;
     if (n >= 0xffffffffull) return ctx_fail(ctx, "%s: %llu CB-valid reads exceed the 2^32-1 limit of one device; shard over more GPUs", who, (unsigned long long)n);
     const u32 K = R ? R->k : 1;
     const size_t hbytes = 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64);
     memset(hist, 0, hbytes);
     u64 nk = 0;
     if (n) {
-        // the number of draws is known now: generate exactly [d0 + ordinal_base, + n)
-        TRY(mt_generate_parallel(job, who, job->prm.d0 + ordinal_base, n, R != nullptr));
+        // the number of draws is known now: generate exactly [first_draw, first_draw + n)
+        TRY(mt_generate_parallel(job, who, first_draw, n, R != nullptr));
         CK(cudaEventRecord(job->ev_mt, ctx->mt));
         CK(cudaStreamWaitEvent(ctx->compute, job->ev_mt, 0));
         const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
-        const u64 *cand = job->cand.as<u64>();
         const u32 *draws = job->keepbits.as<u32>();
         TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
         TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
@@ -639,11 +640,30 @@ static int sample_pass(fastf_bam2db_job *job, const char *who, u64 ordinal_base,
         job->t_sample.stop(ctx->compute);
         CK(cudaEventRecord(job->ev_last, ctx->compute));
     }
-    job->sampled_done = true;
-    job->sweep_rates = R ? K : 0;
     job->n_sampled = 0;
     for (u32 p = 0; p < K; p++) job->n_sampled += hist[p];
     job->n_valid = nk;
+    return 0;
+}
+
+// a job begun with fastf_bam2db_begin_grid is finished by fastf_bam2db_finish_grid only: its candidates carry the union table's cells
+static int refuse_grid(fastf_bam2db_job *job, const char *who)
+{
+    if (job->grid) return ctx_fail(job->ctx, "%s: the job was begun with fastf_bam2db_begin_grid; finish it with fastf_bam2db_finish_grid", who);
+    return 0;
+}
+
+// sample_cands over the job's own candidates, once, after the last feed; its CB-valid reads meet draws d0 + ordinal_base + k
+static int sample_pass(fastf_bam2db_job *job, const char *who, u64 ordinal_base, const FastfSweepRates *R, u64 *hist)
+{
+    fastf_ctx *ctx = job->ctx;
+    TRY(refuse_grid(job, who));
+    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already sampled", who);
+    TRY(drain_chunks(job));
+    TRY(report_feed_timing(job));
+    TRY(sample_cands(job, who, job->prm.d0 + ordinal_base, job->cand.as<u64>(), job->n_cand, R, hist));
+    job->sampled_done = true;
+    job->sweep_rates = R ? R->k : 0;
     return 0;
 }
 
@@ -658,6 +678,7 @@ extern "C" int fastf_bam2db_sample(fastf_bam2db_job *job, uint64_t ordinal_base)
 extern "C" int fastf_bam2db_kept_device(fastf_bam2db_job *job, uint64_t **dev_keys, uint64_t *n)
 {
     fastf_ctx *ctx = job->ctx;
+    TRY(refuse_grid(job, "bam2db_kept_device"));
     if (!job->sampled_done) return ctx_fail(ctx, "bam2db_kept_device: call fastf_bam2db_sample first");
     if (job->sweep_rates) return ctx_fail(ctx, "bam2db_kept_device: the job was sampled by the depth sweep; use fastf_bam2db_kept_sweep_device");
     *dev_keys = job->kept.as<u64>();
@@ -787,6 +808,7 @@ extern "C" int fastf_bam2db_finish(fastf_bam2db_job *job, fastf_bam2db_result *r
     fastf_ctx *ctx = job->ctx;
     CK(cudaSetDevice(ctx->device));
     memset(res, 0, sizeof *res);
+    TRY(refuse_grid(job, "bam2db_finish"));
     if (job->sweep_rates) return ctx_fail(ctx, "bam2db_finish: the job was sampled by the depth sweep");
     if (!job->sampled_done) TRY(fastf_bam2db_sample(job, 0));
     const u64 n = job->n_valid;
@@ -883,20 +905,13 @@ static int sweep_count(fastf_ctx *ctx, SortScratch &sortS, RleScratch &rleS, Rle
     return 0;
 }
 
-extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+// The depth sweep's results out of a job that sample_cands has just sampled at the thresholds `order` came from (hist: its histograms):
+// the rows with their caller rate index, sweep_count with `alt` (a dead array of at least job->n_valid keys) as the keys' ping-pong
+// buffer, per caller rate the counters and COO, and the job's stats (cb_valid = the job's candidates).
+static int sweep_finish(fastf_bam2db_job *job, u32 K, const u32 *order, const u64 *hist, u64 *alt, fastf_bam2db_sweep_result *res)
 {
-    const char *who = "bam2db_finish_sweep";
     fastf_ctx *ctx = job->ctx;
-    CK(cudaSetDevice(ctx->device));
-    memset(res, 0, sizeof *res);
-    FastfSweepRates R;
-    u32 order[FASTF_SWEEP_MAX_RATES];
-    TRY(sweep_rates(ctx, who, n_rates, keep_thresholds, &R, order));
-    if (job->sampled_done) return ctx_fail(ctx, "bam2db_finish_sweep: the job was already sampled at one rate");
-    const u32 K = n_rates;
     const FastfKeyLayout &L = job->L;
-    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
-    TRY(sample_pass(job, who, 0, &R, hist));
     const u64 nk = job->n_valid;   // valid rows kept by the largest threshold
     // the rows in file order, each with the caller index of its rate
     if (job->prm.want_rows) {
@@ -911,11 +926,10 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         if (rc) return rc;
         res->n_rows = nk;
     }
-    // the candidate array is dead after sampling and at least as large as `kept`: the keys' ping-pong buffer
     fastf_bam2db_result *out = res->rate;
     u64 nnz[FASTF_SWEEP_MAX_RATES];
     u32 *mg[FASTF_SWEEP_MAX_RATES] = {}, *mc[FASTF_SWEEP_MAX_RATES] = {}, *mn[FASTF_SWEEP_MAX_RATES] = {};
-    const int crc = sweep_count(ctx, job->sortS, job->rleS, job->rateS, job->orand, job->small_host, job->kept.as<u64>(), job->cand.as<u64>(), job->kept_rate.as<u32>(), job->rate_alt.as<u32>(), nk,
+    const int crc = sweep_count(ctx, job->sortS, job->rleS, job->rateS, job->orand, job->small_host, job->kept.as<u64>(), alt, job->kept_rate.as<u32>(), job->rate_alt.as<u32>(), nk,
                                 L.bits_cell + L.bits_gene + L.bits_umi, L.bits_gene, L.bits_umi, K, &job->t_sort, &job->t_count, &job->ms_count, nnz, mg, mc, mn, ctx->compute);
     for (u32 p = 0; p < K; p++) { out[order[p]].m_gene = mg[p]; out[order[p]].m_cell = mc[p]; out[order[p]].m_count = mn[p]; }
     if (crc) return crc;
@@ -941,6 +955,118 @@ extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates
         r = st;
         r.sampled = keep.sampled; r.valid = keep.valid; r.nnz = keep.nnz;
         r.m_gene = keep.m_gene; r.m_cell = keep.m_cell; r.m_count = keep.m_count;
+    }
+    return 0;
+}
+
+extern "C" int fastf_bam2db_finish_sweep(fastf_bam2db_job *job, uint32_t n_rates, const uint64_t *keep_thresholds, fastf_bam2db_sweep_result *res)
+{
+    const char *who = "bam2db_finish_sweep";
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    memset(res, 0, sizeof *res);
+    FastfSweepRates R;
+    u32 order[FASTF_SWEEP_MAX_RATES];
+    TRY(sweep_rates(ctx, who, n_rates, keep_thresholds, &R, order));
+    TRY(refuse_grid(job, who));
+    if (job->sampled_done) return ctx_fail(ctx, "bam2db_finish_sweep: the job was already sampled at one rate");
+    u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+    TRY(sample_pass(job, who, 0, &R, hist));
+    // the candidate array is dead after sampling and at least as large as `kept`: the keys' ping-pong buffer
+    return sweep_finish(job, n_rates, order, hist, job->cand.as<u64>(), res);
+}
+
+// Cell-rate grid (include/fastf_gpu.h): the job parsed against the union of the cell tables, non-insertable reads keeping their cell
+// (fastf_parse_record<true>).  Per cell rate: remap + compaction into the candidate array a job begun with that rate's table would
+// have gathered (fastf_grid_count / scatter_kernel), then the depth sweep over it at the rate's d0.  job->cand is read by every rate.
+extern "C" int fastf_bam2db_begin_grid(fastf_ctx *ctx, const fastf_bam2db_params *p, fastf_bam2db_job **out)
+{
+    TRY(fastf_bam2db_begin(ctx, p, out));
+    (*out)->grid = true;
+    return 0;
+}
+
+// the caller's remap tables: 1..FASTF_GRID_MAX_CELL_RATES of them, each a one-to-one map of the union cells it holds onto 1..n_cells
+static int grid_check_cell_rates(fastf_bam2db_job *job, const char *who, uint32_t n_cell_rates, const fastf_bam2db_cell_rate *cell_rates)
+{
+    fastf_ctx *ctx = job->ctx;
+    const u32 n_union = job->prm.n_cells;
+    if (n_cell_rates < 1 || n_cell_rates > FASTF_GRID_MAX_CELL_RATES || !cell_rates) return ctx_fail(ctx, "%s: 1..%u cell rates", who, (unsigned)FASTF_GRID_MAX_CELL_RATES);
+    for (u32 i = 0; i < n_cell_rates; i++) {
+        const fastf_bam2db_cell_rate &c = cell_rates[i];
+        if (n_union && !c.cell_index) return ctx_fail(ctx, "%s: cell_rates[%u].cell_index is NULL", who, i);
+        if (c.n_cells > n_union) return ctx_fail(ctx, "%s: cell_rates[%u].n_cells = %u exceeds the union table's %u cells", who, i, c.n_cells, n_union);
+        std::vector<u8> seen((size_t)c.n_cells + 1, 0);
+        u32 held = 0;
+        for (u32 u = 0; u < n_union; u++) {
+            const u32 v = c.cell_index[u];
+            if (!v) continue;
+            if (v > c.n_cells) return ctx_fail(ctx, "%s: cell_rates[%u].cell_index[%u] = %u exceeds its n_cells = %u", who, i, u, v, c.n_cells);
+            if (seen[v]) return ctx_fail(ctx, "%s: cell_rates[%u].cell_index holds %u twice", who, i, v);
+            seen[v] = 1;
+            held++;
+        }
+        if (held != c.n_cells) return ctx_fail(ctx, "%s: cell_rates[%u] maps %u union cells onto its n_cells = %u (every cell of its table must be in the union)", who, i, held, c.n_cells);
+    }
+    return 0;
+}
+
+extern "C" int fastf_bam2db_finish_grid(fastf_bam2db_job *job, uint32_t n_cell_rates, const fastf_bam2db_cell_rate *cell_rates, uint32_t n_rates, const uint64_t *keep_thresholds,
+                                        fastf_bam2db_sweep_result *res)
+{
+    const char *who = "bam2db_finish_grid";
+    fastf_ctx *ctx = job->ctx;
+    CK(cudaSetDevice(ctx->device));
+    // zeroed before anything is checked: the caller frees every res[i], also after a refusal
+    for (u32 i = 0; res && i < std::min<u32>(n_cell_rates, FASTF_GRID_MAX_CELL_RATES); i++) memset(&res[i], 0, sizeof res[i]);
+    if (!job->grid) return ctx_fail(ctx, "%s: the job was not begun with fastf_bam2db_begin_grid", who);
+    if (!res) return ctx_fail(ctx, "%s: res is NULL", who);
+    TRY(grid_check_cell_rates(job, who, n_cell_rates, cell_rates));
+    FastfSweepRates R;
+    u32 order[FASTF_SWEEP_MAX_RATES];
+    TRY(sweep_rates(ctx, who, n_rates, keep_thresholds, &R, order));
+    if (job->sampled_done) return ctx_fail(ctx, "%s: the job was already finished", who);
+    TRY(drain_chunks(job));
+    TRY(report_feed_timing(job));
+    job->sampled_done = true;
+    const FastfKeyLayout &L = job->L;
+    const u32 n_union = job->prm.n_cells, cell_shift = L.bits_gene + L.bits_umi;
+    const u64 n = job->n_cand;
+    if (n >= 0xffffffffull) return ctx_fail(ctx, "%s: %llu CB-valid reads exceed the 2^32-1 limit of one device", who, (unsigned long long)n);
+    const u32 ntiles = (u32)((n + FASTF_SAMPLE_TILE - 1) / FASTF_SAMPLE_TILE);
+    if (n) {
+        TRY(dev_reserve(ctx, job->grid_cand, n * sizeof(u64)));
+        TRY(dev_reserve(ctx, job->grid_remap, (size_t)n_union * sizeof(u32)));
+    }
+    for (u32 i = 0; i < n_cell_rates; i++) {
+        const fastf_bam2db_cell_rate &c = cell_rates[i];
+        // this rate's own clocks (the previous rate's fill_stats collected every timer)
+        job->ms_mt = job->ms_sample = job->ms_sort = job->ms_count = 0;
+        u64 ni = 0;
+        if (n) {
+            // sample_cands of the previous rate may have left smaller tile arrays
+            TRY(dev_reserve(ctx, job->tile_valid, (size_t)ntiles * sizeof(u32)));
+            TRY(dev_reserve(ctx, job->tile_tot, sizeof(u32)));
+            CK(cudaMemcpyAsync(job->grid_remap.p, c.cell_index, (size_t)n_union * sizeof(u32), cudaMemcpyHostToDevice, ctx->compute));
+            job->t_sample.start(ctx->compute);
+            FASTF_LAUNCH(fastf_grid_count_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->grid_remap.as<u32>(), n_union, cell_shift,
+                         job->tile_valid.as<u32>());
+            CKL("grid_count");
+            TRY(launch_scan_rows(ctx, job->tile_valid.as<u32>(), ntiles, 1, job->tile_tot.as<u32>(), ctx->compute));
+            FASTF_LAUNCH(fastf_grid_scatter_kernel, ntiles, FASTF_SAMPLE_THREADS, 0, ctx->compute, (const u64 *)job->cand.as<u64>(), n, (const u32 *)job->grid_remap.as<u32>(), n_union, cell_shift,
+                         L.bits_umi, (const u32 *)job->tile_valid.as<u32>(), job->grid_cand.as<u64>());
+            CKL("grid_scatter");
+            job->t_sample.stop(ctx->compute);
+            CK(cudaMemcpyAsync(job->small_host.p, job->tile_tot.p, sizeof(u32), cudaMemcpyDeviceToHost, ctx->compute));
+            CK(cudaStreamSynchronize(ctx->compute));
+            ni = job->small_host.as<u32>()[0];
+            job->t_sample.collect(&job->ms_sample);
+        }
+        u64 hist[2 * FASTF_SWEEP_MAX_RATES];
+        TRY(sample_cands(job, who, c.d0, job->grid_cand.as<u64>(), ni, &R, hist));
+        // the compacted array is dead after sampling and holds at least `kept`: the keys' ping-pong buffer
+        TRY(sweep_finish(job, n_rates, order, hist, job->grid_cand.as<u64>(), &res[i]));
+        for (u32 j = 0; j < n_rates; j++) { res[i].rate[j].cb_valid = ni; res[i].rate[j].bits_cell = bits_for(c.n_cells); }
     }
     return 0;
 }

@@ -1,4 +1,5 @@
-// Prefix sums, the MT19937 keep-bit stream (K3), the depth-sampling compaction (K3b) and its several-rate form (the depth sweep).
+// Prefix sums, the MT19937 keep-bit stream (K3), the depth-sampling compaction (K3b), its several-rate form (the depth sweep) and the
+// per-cell-rate remap of the cell-rate grid.
 #pragma once
 #include "common.cuh"
 
@@ -332,4 +333,67 @@ fastf_sweep_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__res
 #pragma unroll
     for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++)
         if (flags & (1u << k)) { kept[o] = keys[k]; kept_rate[o] = rb[k]; o++; }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Cell-rate grid: the union job's candidates (union cell index u in the cell field; a non-insertable
+// read is its cell alone, gene field 0: fastf_parse_record<true>) -> the candidate array a job begun
+// with cell table i would have gathered: the reads whose cell table i holds, in file order, with
+// cell field cell_index[u - 1] (1-based, 0 = not in table i) and the non-insertable ones as
+// FASTF_INVALID_KEY.  Two-phase like the sampling compaction: tile counts -> row scan -> scatter.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ u32 fastf_grid_cell(const u32 *__restrict__ cell_index, u32 n_union, u64 key, u32 cell_shift)
+{
+    const u64 u = key >> cell_shift;
+    return u - 1 < (u64)n_union ? cell_index[u - 1] : 0u;   // u = 0 or beyond the table (never written by the parse): not held
+}
+
+__global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
+fastf_grid_count_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ cell_index, u32 n_union, u32 cell_shift, u32 *__restrict__ tile_cnt)
+{
+    __shared__ u32 s_cnt;
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    const u64 base = (u64)blockIdx.x * FASTF_SAMPLE_TILE;
+    u32 cnt = 0;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
+        u64 i = base + (u64)k * FASTF_SAMPLE_THREADS + threadIdx.x;
+        if (i < n) cnt += fastf_grid_cell(cell_index, n_union, cand[i], cell_shift) != 0u;
+    }
+    cnt = __reduce_add_sync(FASTF_FULL_MASK, cnt);
+    if ((threadIdx.x & 31u) == 0) atomicAdd(&s_cnt, cnt);
+    __syncthreads();
+    if (threadIdx.x == 0) tile_cnt[blockIdx.x] = s_cnt;
+}
+
+__global__ void __launch_bounds__(FASTF_SAMPLE_THREADS)
+fastf_grid_scatter_kernel(const u64 *__restrict__ cand, u64 n, const u32 *__restrict__ cell_index, u32 n_union, u32 cell_shift, u32 bits_umi, const u32 *__restrict__ tile_off,
+                          u64 *__restrict__ out)
+{
+    // blocked arrangement as in fastf_sample_scatter_kernel: file order under a single block scan
+    const u64 base = (u64)blockIdx.x * FASTF_SAMPLE_TILE + (u64)threadIdx.x * FASTF_SAMPLE_ITEMS;
+    const u64 low_mask = (1ull << cell_shift) - 1ull;
+    u64 keys[FASTF_SAMPLE_ITEMS];
+    u32 flags = 0, cnt = 0;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++) {
+        u64 i = base + k;
+        bool v = false;
+        if (i < n) {
+            const u64 key = cand[i];
+            const u32 c = fastf_grid_cell(cell_index, n_union, key, cell_shift);
+            const u64 low = key & low_mask;
+            keys[k] = (low >> bits_umi) == 0 ? FASTF_INVALID_KEY : ((u64)c << cell_shift) | low;
+            v = c != 0u;
+        }
+        flags |= (u32)v << k;
+        cnt += v;
+    }
+    u32 tot;
+    u32 ex = fastf_block_exscan<FASTF_SAMPLE_THREADS>(cnt, &tot);
+    u64 o = (u64)tile_off[blockIdx.x] + ex;
+#pragma unroll
+    for (int k = 0; k < FASTF_SAMPLE_ITEMS; k++)
+        if (flags & (1u << k)) out[o++] = keys[k];
 }

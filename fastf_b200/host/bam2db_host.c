@@ -31,11 +31,12 @@ static void sl_free(strlist *l) { free(l->buf); free(l->off); memset(l, 0, sizeo
 typedef struct { uint32_t *slot; uint32_t mask; const strlist *l; } strset;
 static uint32_t djb2(const char *s, size_t n) { uint32_t h = 5381; for (size_t i = 0; i < n; i++) h = h * 33u + (unsigned char)s[i]; return h; }
 static void ss_init(strset *s, const strlist *l, size_t expect) { uint32_t c = 64; while (c < expect * 2 + 8) c <<= 1; s->slot = (uint32_t *)calloc(c, 4); s->mask = c - 1; s->l = l; }
-static int ss_has(const strset *s, const char *k, size_t n)
+/* 1 + the string's index in the list, 0 when absent */
+static uint32_t ss_has(const strset *s, const char *k, size_t n)
 {
     for (uint32_t i = djb2(k, n) & s->mask; s->slot[i]; i = (i + 1) & s->mask) {
         uint32_t id = s->slot[i] - 1;
-        if (s->l->off[id + 1] - s->l->off[id] == n && !memcmp(s->l->buf + s->l->off[id], k, n)) return 1;
+        if (s->l->off[id + 1] - s->l->off[id] == n && !memcmp(s->l->buf + s->l->off[id], k, n)) return id + 1;
     }
     return 0;
 }
@@ -237,24 +238,89 @@ done:
     return rc;
 }
 
-/* bam2db() (n_rates == 0) and bam2db_sweep(): one device job; the sweep writes output set i into out_dir[i] / db_file[i] */
-static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
-                      const float *rates, unsigned int seed)
+/* One cell table exactly as the reference builds it (reference :229-289): the sampled lines in order, the index stalling at the first
+ * duplicate barcode.  gb is rewound first; returns 0, or 1 when fastf_sample_cells refuses the rate. */
+static int sample_cell_table(gzFile gb, size_t n_cells, float rate_cell, unsigned seed, const char *barcodes_file, strlist *cells, uint64_t *d0)
+{
+    uint64_t *samp = (uint64_t *)malloc(sizeof(uint64_t) * (n_cells ? n_cells : 1));
+    const uint64_t ns = samp ? fastf_sample_cells(n_cells, rate_cell, seed, samp, d0) : UINT64_MAX;
+    if (ns == UINT64_MAX) { free(samp); printf("Sample size must be smaller than population size when sampling without replacement."); return 1; }
+    printf("Actual number of sampled cell barcodes: %zu\n", (size_t)ns);
+    gzrewind(gb);
+    strset cset = {0};
+    ss_init(&cset, cells, ns);
+    char line[1024];
+    size_t cell_index = 1, nth = 0;
+    while (gzgets(gb, line, 1024) != NULL && cell_index <= ns) {
+        nth++;
+        if (nth - 1 != samp[cell_index - 1]) continue;
+        line[strcspn(line, "\n\r\t")] = '\0';
+        size_t n = strlen(line);
+        if (!ss_has(&cset, line, n)) {
+            sl_push(cells, line, n);
+            ss_add(&cset, line, n, cells->n - 1);
+            cell_index++;
+        } else {
+            printf("Warning: Duplicate cell barcodes were found in %s!\n", barcodes_file);
+        }
+    }
+    free(cset.slot);
+    free(samp);
+    return 0;
+}
+
+/* tables cell and feature of one output set (reference :229-337) */
+static int insert_lists(sqlite3 *db, const strlist *cells, const strlist *fid, const strlist *fname, const strlist *ftype)
+{
+    sqlite3_stmt *st = NULL;
+    int rc = 1;
+    exec_sql(db, "BEGIN TRANSACTION");
+    sqlite3_prepare_v2(db, "INSERT INTO cell VALUES (?1);", -1, &st, NULL);
+    for (uint32_t i = 0; i < cells->n; i++) {
+        sqlite3_bind_text(st, 1, cells->buf + cells->off[i], (int)(cells->off[i + 1] - cells->off[i]), SQLITE_TRANSIENT);
+        if (sqlite3_step(st) != SQLITE_DONE) { fprintf(stderr, "SQL error: %s\n", sqlite3_errmsg(db)); goto done; }
+        sqlite3_reset(st);
+    }
+    exec_sql(db, "END TRANSACTION");
+    sqlite3_finalize(st);
+    st = NULL;
+    exec_sql(db, "BEGIN TRANSACTION");
+    sqlite3_prepare_v2(db, "INSERT INTO feature VALUES (?1, ?2, ?3);", -1, &st, NULL);
+    for (uint32_t i = 0; i < fid->n; i++) {
+        sqlite3_bind_text(st, 1, fid->buf + fid->off[i], (int)(fid->off[i + 1] - fid->off[i]), SQLITE_TRANSIENT);
+        sqlite3_bind_text(st, 2, fname->buf + fname->off[i], (int)(fname->off[i + 1] - fname->off[i]), SQLITE_TRANSIENT);
+        sqlite3_bind_text(st, 3, ftype->buf + ftype->off[i], (int)(ftype->off[i + 1] - ftype->off[i]), SQLITE_TRANSIENT);
+        if (sqlite3_step(st) != SQLITE_DONE) { fprintf(stderr, "SQL error: %s\n", sqlite3_errmsg(db)); goto done; }
+        sqlite3_reset(st);
+    }
+    exec_sql(db, "END TRANSACTION");
+    rc = 0;
+done:
+    if (st) sqlite3_finalize(st);
+    return rc;
+}
+
+/* bam2db() (one output set), bam2db_sweep() (n_rates > 0: depth rates) and bam2db_grid() (n_cell_rates > 0 as well: cell rates x depth
+ * rates): one device job.  Output set (i, j) of cell rate i and depth rate j goes to out_dirs[i * K + j] / db_files[i * K + j]. */
+static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
+                      const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed)
 {
     int rc = 1;
-    const int sweep = n_rates > 0;
-    const uint32_t K = sweep ? n_rates : 1;   /* output sets */
-    sqlite3 *dbs[FASTF_SWEEP_MAX_RATES] = {NULL};
-    sqlite3_stmt *stmts[FASTF_SWEEP_MAX_RATES] = {NULL};
+    const int grid = n_cell_rates > 0, sweep = n_rates > 0;
+    const uint32_t M = grid ? n_cell_rates : 1, K = sweep ? n_rates : 1, NS = M * K;   /* cell tables, depth rates, output sets */
+    sqlite3 **dbs = (sqlite3 **)calloc(NS ? NS : 1, sizeof *dbs);
     fastf_ctx *ctx = NULL;
     fastf_bam2db_job *job = NULL;
     fastf_bam2db_result res;
     memset(&res, 0, sizeof res);
-    fastf_bam2db_sweep_result *sres = sweep ? (fastf_bam2db_sweep_result *)calloc(1, sizeof *sres) : NULL;
+    fastf_bam2db_sweep_result *sres = sweep ? (fastf_bam2db_sweep_result *)calloc(M, sizeof *sres) : NULL;
     uint64_t *rate_rows = NULL;
-    strlist cells = {0}, fkeys = {0}, fid = {0}, fname = {0}, ftype = {0};
-    strset cset = {0}, fset = {0};
-    uint64_t *samp = NULL;
+    strlist *cells = (strlist *)calloc(M, sizeof *cells);
+    strlist ucells = {0}, fkeys = {0}, fid = {0}, fname = {0}, ftype = {0};
+    strset uset = {0}, fset = {0};
+    uint64_t d0s[FASTF_GRID_MAX_CELL_RATES] = {0};
+    uint32_t *remap = NULL;
+    fastf_bam2db_cell_rate crs[FASTF_GRID_MAX_CELL_RATES];
     void *pin[2] = {NULL, NULL};
     int bam = -1;
     gzFile gb = NULL, gf = NULL;
@@ -264,11 +330,13 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         if (e && atoi(e) > 0) fastf_gpus = atoi(e);
         if ((e = getenv("FASTF_DEVICE")) != NULL) fastf_device = atoi(e);
     }
-    if (sweep && (!sres || n_rates > FASTF_SWEEP_MAX_RATES || fastf_gpus > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m the depth sweep takes 1..%d rates on one GPU\n", FASTF_SWEEP_MAX_RATES); free(sres); return 1; }
+    if (!dbs || !cells || (sweep && !sres)) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
+    if (grid && (n_cell_rates > FASTF_GRID_MAX_CELL_RATES || fastf_gpus > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m the cell-rate grid takes 1..%d cell rates on one GPU\n", FASTF_GRID_MAX_CELL_RATES); goto done; }
+    if (sweep && (n_rates > FASTF_SWEEP_MAX_RATES || fastf_gpus > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m the depth sweep takes 1..%d rates on one GPU\n", FASTF_SWEEP_MAX_RATES); goto done; }
 
     g_t_last = 0;
     phase("start");
-    for (uint32_t r = 0; r < K; r++) {
+    for (uint32_t r = 0; r < NS; r++) {
         if (sqlite3_open(db_files[r], &dbs[r])) { fprintf(stderr, "Can't open database: %s\n", sqlite3_errmsg(dbs[r])); goto done; }
         fprintf(stderr, "Opened database successfully\n");
     }
@@ -281,42 +349,18 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
     gf = gzopen(features_file, "r");
     if (!gf) { fprintf(stderr, "Can't open feature name file %s\n", features_file); goto done; }
     fprintf(stderr, "Opened feature name file %s successfully\n", features_file);
-    for (uint32_t r = 0; r < K; r++)
+    for (uint32_t r = 0; r < NS; r++)
         if (exec_sql(dbs[r], "CREATE TABLE cell (cell_barcode TEXT);") || exec_sql(dbs[r], "CREATE TABLE feature (feature_id TEXT, feature_name TEXT, feature_type);") ||
             exec_sql(dbs[r], "CREATE TABLE umi (cell_index INTEGER, feature_index INTEGER, encoded_umi TEXT);")) goto done;
 
-    /* ---- barcodes: count, sample, second pass (reference :229-289) ---- */
+    /* ---- barcodes: count, then per cell rate sample + second pass (reference :229-289) ---- */
     size_t n_cells = 0;
     while (gzgets(gb, line, 1024) != NULL) n_cells++;
     printf("Total number of cells: %zu\n", n_cells);
-    samp = (uint64_t *)malloc(sizeof(uint64_t) * (n_cells ? n_cells : 1));
-    uint64_t d0 = 0;
-    uint64_t ns = fastf_sample_cells(n_cells, rate_cell, seed, samp, &d0);
-    if (ns == UINT64_MAX) { printf("Sample size must be smaller than population size when sampling without replacement."); goto done; }
-    printf("Actual number of sampled cell barcodes: %zu\n", (size_t)ns);
-    gzrewind(gb);
-    ss_init(&cset, &cells, ns);
-    for (uint32_t r = 0; r < K; r++) { exec_sql(dbs[r], "BEGIN TRANSACTION"); sqlite3_prepare_v2(dbs[r], "INSERT INTO cell VALUES (?1);", -1, &stmts[r], NULL); }
-    size_t cell_index = 1, nth = 0;
-    while (gzgets(gb, line, 1024) != NULL && cell_index <= ns) {
-        nth++;
-        if (nth - 1 != samp[cell_index - 1]) continue;
-        line[strcspn(line, "\n\r\t")] = '\0';
-        size_t n = strlen(line);
-        if (!ss_has(&cset, line, n)) {
-            sl_push(&cells, line, n);
-            ss_add(&cset, line, n, cells.n - 1);
-            for (uint32_t r = 0; r < K; r++) {
-                sqlite3_bind_text(stmts[r], 1, line, (int)n, SQLITE_TRANSIENT);
-                if (sqlite3_step(stmts[r]) != SQLITE_DONE) { fprintf(stderr, "SQL error: %s\n", sqlite3_errmsg(dbs[r])); goto done; }
-                sqlite3_reset(stmts[r]);
-            }
-            cell_index++;
-        } else {
-            printf("Warning: Duplicate cell barcodes were found in %s!\n", barcodes_file);
-        }
+    for (uint32_t i = 0; i < M; i++) {
+        if (grid) printf("Cell rate %s:\n", cell_names[i]);
+        if (sample_cell_table(gb, n_cells, cell_rates[i], seed, barcodes_file, &cells[i], &d0s[i])) goto done;
     }
-    for (uint32_t r = 0; r < K; r++) { exec_sql(dbs[r], "END TRANSACTION"); sqlite3_finalize(stmts[r]); stmts[r] = NULL; }
 
     /* ---- features (reference :296-337): strtok on tabs, key = buffer up to its first NUL ---- */
     {
@@ -325,7 +369,6 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         gzrewind(gf);
         ss_init(&fset, &fkeys, nlines);
     }
-    for (uint32_t r = 0; r < K; r++) { exec_sql(dbs[r], "BEGIN TRANSACTION"); sqlite3_prepare_v2(dbs[r], "INSERT INTO feature VALUES (?1, ?2, ?3);", -1, &stmts[r], NULL); }
     while (gzgets(gf, line, 1024) != NULL) {
         char *id = strtok(line, "\t"), *name = strtok(NULL, "\t"), *type = strtok(NULL, "\t");
         if (!id || !name || !type) { fprintf(stderr, "\x1b[31mError:\x1b[0m feature line with fewer than three tab-separated fields in %s\n", features_file); goto done; }
@@ -335,18 +378,36 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
             sl_push(&fkeys, line, kn);
             ss_add(&fset, line, kn, fkeys.n - 1);
             sl_push(&fid, id, strlen(id)); sl_push(&fname, name, strlen(name)); sl_push(&ftype, type, strlen(type));
-            for (uint32_t r = 0; r < K; r++) {
-                sqlite3_bind_text(stmts[r], 1, id, (int)strlen(id), SQLITE_TRANSIENT);
-                sqlite3_bind_text(stmts[r], 2, name, (int)strlen(name), SQLITE_TRANSIENT);
-                sqlite3_bind_text(stmts[r], 3, type, (int)strlen(type), SQLITE_TRANSIENT);
-                if (sqlite3_step(stmts[r]) != SQLITE_DONE) { fprintf(stderr, "SQL error: %s\n", sqlite3_errmsg(dbs[r])); goto done; }
-                sqlite3_reset(stmts[r]);
-            }
         } else {
             printf("Warning: Duplicate feature names were found in %s!\n", features_file);
         }
     }
-    for (uint32_t r = 0; r < K; r++) { exec_sql(dbs[r], "END TRANSACTION"); sqlite3_finalize(stmts[r]); stmts[r] = NULL; }
+    for (uint32_t r = 0; r < NS; r++)
+        if (insert_lists(dbs[r], &cells[r / K], &fid, &fname, &ftype)) goto done;
+
+    /* the cell table the device job parses against: the one table, or the union of the grid's tables with a remap per cell rate */
+    const strlist *jcells = &cells[0];
+    if (grid) {
+        size_t tot = 0;
+        for (uint32_t i = 0; i < M; i++) tot += cells[i].n;
+        ss_init(&uset, &ucells, tot);
+        for (uint32_t i = 0; i < M; i++)
+            for (uint32_t k = 0; k < cells[i].n; k++) {
+                const char *c = cells[i].buf + cells[i].off[k];
+                const size_t n = cells[i].off[k + 1] - cells[i].off[k];
+                if (!ss_has(&uset, c, n)) { sl_push(&ucells, c, n); ss_add(&uset, c, n, ucells.n - 1); }
+            }
+        remap = (uint32_t *)calloc((size_t)M * (ucells.n ? ucells.n : 1), sizeof(uint32_t));
+        if (!remap) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
+        for (uint32_t i = 0; i < M; i++) {
+            crs[i].cell_index = remap + (size_t)i * ucells.n;
+            crs[i].n_cells = cells[i].n;
+            crs[i].d0 = d0s[i];
+            for (uint32_t k = 0; k < cells[i].n; k++)
+                remap[(size_t)i * ucells.n + ss_has(&uset, cells[i].buf + cells[i].off[k], cells[i].off[k + 1] - cells[i].off[k]) - 1] = k + 1;
+        }
+        jcells = &ucells;
+    }
 
     /* ---- the hot path: device job fed with the raw BGZF bytes ---- */
     printf("Start to convert bam file to sqlite3 database...\n");
@@ -364,9 +425,9 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
             fastf_bam2db_params p;
             memset(&p, 0, sizeof p);
             uint32_t zero_off[1] = {0};
-            p.cell_keys = cells.buf ? cells.buf : ""; p.cell_off = cells.off ? cells.off : zero_off; p.n_cells = cells.n;
+            p.cell_keys = cells[0].buf ? cells[0].buf : ""; p.cell_off = cells[0].off ? cells[0].off : zero_off; p.n_cells = cells[0].n;
             p.gene_keys = fkeys.buf ? fkeys.buf : ""; p.gene_off = fkeys.off ? fkeys.off : zero_off; p.n_genes = fkeys.n;
-            p.seed = seed; p.d0 = d0; p.keep_threshold = fastf_keep_threshold(rates[0]);
+            p.seed = seed; p.d0 = d0s[0]; p.keep_threshold = fastf_keep_threshold(rates[0]);
             p.umi_max_bytes = umi_bytes;
             p.want_rows = 1;
             failed = fastf_bam2db_run_sharded(fastf_gpus, NULL, &p, map, (size_t)sb.st_size, &res);
@@ -386,13 +447,13 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         fastf_bam2db_params p;
         memset(&p, 0, sizeof p);
         uint32_t zero_off[1] = {0};
-        p.cell_keys = cells.buf ? cells.buf : ""; p.cell_off = cells.off ? cells.off : zero_off; p.n_cells = cells.n;
+        p.cell_keys = jcells->buf ? jcells->buf : ""; p.cell_off = jcells->off ? jcells->off : zero_off; p.n_cells = jcells->n;
         p.gene_keys = fkeys.buf ? fkeys.buf : ""; p.gene_off = fkeys.off ? fkeys.off : zero_off; p.n_genes = fkeys.n;
-        p.seed = seed; p.d0 = d0; p.keep_threshold = fastf_keep_threshold(rates[0]);   /* ignored by the sweep */
+        p.seed = seed; p.d0 = d0s[0]; p.keep_threshold = fastf_keep_threshold(rates[0]);   /* ignored by the sweep (and d0 by the grid) */
         p.umi_max_bytes = umi_bytes;
         p.want_rows = 1;
         p.inflate_lanes = flags;
-        if (fastf_bam2db_begin(ctx, &p, &job)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
+        if ((grid ? fastf_bam2db_begin_grid : fastf_bam2db_begin)(ctx, &p, &job)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
         const size_t PIECE = (size_t)256 << 20;
         if (!pin[0] && (fastf_host_alloc(ctx, PIECE, &pin[0]) || fastf_host_alloc(ctx, PIECE, &pin[1]))) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
         ssize_t got;
@@ -407,8 +468,8 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         if (!failed && sweep) {
             uint64_t thr[FASTF_SWEEP_MAX_RATES];
             for (uint32_t r = 0; r < K; r++) thr[r] = fastf_keep_threshold(rates[r]);
-            failed = fastf_bam2db_finish_sweep(job, K, thr, sres);
-            if (failed) fastf_bam2db_sweep_result_free(sres);
+            failed = grid ? fastf_bam2db_finish_grid(job, M, crs, K, thr, sres) : fastf_bam2db_finish_sweep(job, K, thr, sres);
+            if (failed) for (uint32_t i = 0; i < M; i++) fastf_bam2db_sweep_result_free(&sres[i]);
         } else if (!failed) {
             failed = fastf_bam2db_finish(job, &res);
         }
@@ -428,49 +489,63 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
 
     phase("device job (ctx, read, feed, finish)");
     if (!sweep) {
-        if (write_outputs(&dbs[0], db_files[0], bam_file, out_dirs[0], rate_cell, rates[0], &res, res.row_keys, res.n_rows, &cells, &fkeys, &fid, &fname, &ftype, ctx)) goto done;
+        if (write_outputs(&dbs[0], db_files[0], bam_file, out_dirs[0], cell_rates[0], rates[0], &res, res.row_keys, res.n_rows, &cells[0], &fkeys, &fid, &fname, &ftype, ctx)) goto done;
     } else {
         uint64_t thr[FASTF_SWEEP_MAX_RATES];
         for (uint32_t r = 0; r < K; r++) thr[r] = fastf_keep_threshold(rates[r]);
-        rate_rows = (uint64_t *)malloc(sizeof(uint64_t) * (sres->n_rows ? sres->n_rows : 1));
-        if (!rate_rows) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
-        for (uint32_t r = 0; r < K; r++) {
-            /* table umi of rate r: the rows whose smallest keeping threshold is <= its own, in file order */
-            uint64_t n = 0;
-            for (uint64_t i = 0; i < sres->n_rows; i++)
-                if (thr[sres->row_rate[i]] <= thr[r]) rate_rows[n++] = sres->row_keys[i];
-            printf("Depth rate %s -> %s\n", rate_names[r], out_dirs[r]);
-            if (write_outputs(&dbs[r], db_files[r], bam_file, out_dirs[r], rate_cell, rates[r], &sres->rate[r], rate_rows, n, &cells, &fkeys, &fid, &fname, &ftype, ctx)) goto done;
+        for (uint32_t i = 0; i < M; i++) {
+            const fastf_bam2db_sweep_result *sr = &sres[i];
+            free(rate_rows);
+            rate_rows = (uint64_t *)malloc(sizeof(uint64_t) * (sr->n_rows ? sr->n_rows : 1));
+            if (!rate_rows) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
+            for (uint32_t r = 0; r < K; r++) {
+                /* table umi of rate r: the rows whose smallest keeping threshold is <= its own, in file order */
+                uint64_t n = 0;
+                for (uint64_t k = 0; k < sr->n_rows; k++)
+                    if (thr[sr->row_rate[k]] <= thr[r]) rate_rows[n++] = sr->row_keys[k];
+                if (grid) printf("Cell rate %s, depth rate %s -> %s\n", cell_names[i], rate_names[r], out_dirs[i * K + r]);
+                else printf("Depth rate %s -> %s\n", rate_names[r], out_dirs[r]);
+                if (write_outputs(&dbs[i * K + r], db_files[i * K + r], bam_file, out_dirs[i * K + r], cell_rates[i], rates[r], &sr->rate[r], rate_rows, n, &cells[i], &fkeys, &fid, &fname,
+                                  &ftype, ctx)) goto done;
+            }
         }
     }
     rc = 0;
 done:
-    for (uint32_t r = 0; r < K; r++) {
-        if (stmts[r]) sqlite3_finalize(stmts[r]);
+    for (uint32_t r = 0; dbs && r < NS; r++)
         if (dbs[r]) sqlite3_close(dbs[r]);
-    }
+    free(dbs);
     if (gb) gzclose(gb);
     if (gf) gzclose(gf);
     if (bam >= 0) close(bam);
     fastf_bam2db_result_free(&res);
-    if (sres) { fastf_bam2db_sweep_result_free(sres); free(sres); }
+    if (sres) { for (uint32_t i = 0; i < M; i++) fastf_bam2db_sweep_result_free(&sres[i]); free(sres); }
     free(rate_rows);
+    free(remap);
     if (job) fastf_bam2db_job_free(job);
     if (ctx) { fastf_host_free(ctx, pin[0]); fastf_host_free(ctx, pin[1]); fastf_ctx_destroy(ctx); }
-    free(samp);
-    free(cset.slot); free(fset.slot);
-    sl_free(&cells); sl_free(&fkeys); sl_free(&fid); sl_free(&fname); sl_free(&ftype);
+    for (uint32_t i = 0; cells && i < M; i++) sl_free(&cells[i]);
+    free(cells);
+    free(uset.slot); free(fset.slot);
+    sl_free(&ucells); sl_free(&fkeys); sl_free(&fid); sl_free(&fname); sl_free(&ftype);
     return rc;
 }
 
 int bam2db(char *bam_file, char *db_file, char *path_out, char *barcodes_file, char *features_file, float rate_cell, float rate_depth, unsigned int seed)
 {
-    return bam2db_run(bam_file, &db_file, &path_out, barcodes_file, features_file, rate_cell, 0, NULL, &rate_depth, seed);
+    return bam2db_run(bam_file, &db_file, &path_out, barcodes_file, features_file, 0, NULL, &rate_cell, 0, NULL, &rate_depth, seed);
 }
 
 int bam2db_sweep(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
                  const float *rates, unsigned int seed)
 {
     if (n_rates < 1) { fprintf(stderr, "\x1b[31mError:\x1b[0m the depth sweep needs at least one rate\n"); return 1; }
-    return bam2db_run(bam_file, db_files, out_dirs, barcodes_file, features_file, rate_cell, n_rates, rate_names, rates, seed);
+    return bam2db_run(bam_file, db_files, out_dirs, barcodes_file, features_file, 0, NULL, &rate_cell, n_rates, rate_names, rates, seed);
+}
+
+int bam2db_grid(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
+                const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed)
+{
+    if (n_cell_rates < 1 || n_rates < 1) { fprintf(stderr, "\x1b[31mError:\x1b[0m the cell-rate grid needs at least one cell rate and one depth rate\n"); return 1; }
+    return bam2db_run(bam_file, db_files, out_dirs, barcodes_file, features_file, n_cell_rates, cell_names, cell_rates, n_rates, rate_names, rates, seed);
 }

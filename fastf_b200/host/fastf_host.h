@@ -18,6 +18,11 @@ int bam2db(char *bam_file, char *db_file, char *path_out, char *barcodes_file, c
  * out_dirs[i] with database db_files[i]; 1..32 rates, one GPU.  rate_names[i] names rate i on stdout. */
 int bam2db_sweep(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
                  const float *rates, unsigned int seed);
+/* the cell-rate grid (not a reference entry point): one device job, output set (i, j) = what bam2db(..., cell_rates[i], rates[j], seed)
+ * writes, into out_dirs[i * n_rates + j] with database db_files[i * n_rates + j]; 1..32 cell rates, 1..32 depth rates, one GPU.
+ * cell_names[i] / rate_names[j] name the rates on stdout. */
+int bam2db_grid(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
+                const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed);
 /* cell_counts + print_tree in one call: histogram of the first l+u bases of every read of R1 (BGZF or plain text), written to fp
  * in the reference's BST pre-order.  Returns 0 / 1. */
 int freq_whitelist(const char *r1_path, size_t len_cellbarcode, size_t len_umi, FILE *fp);

@@ -2,17 +2,22 @@
  *   fastF bam2db  -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL -r RATE_DEPTH [-o OUT] [-s SEED] [-u]
  *   fastF bam2db  -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL --depths R1,R2,... [-o OUT] [-s SEED] [-u]
  *                 (the depth sweep, not a reference option: one pass, rate Ri written into OUT/depth_<Ri>/ with database OUT/depth_<Ri>/<basename of DB>)
+ *   fastF bam2db  -b BAM -f FEATURES -a BARCODES -d DB --cells C1,C2,... (-r RATE_DEPTH | --depths R1,R2,...) [-o OUT] [-s SEED] [-u]
+ *                 (the cell-rate grid, not a reference option: one pass, set (Ci, Rj) written into OUT/cell_<Ci>/ with -r, into
+ *                 OUT/cell_<Ci>/depth_<Rj>/ with --depths; database <that directory>/<basename of DB>)
  *   fastF freq    -R R1 -o OUT [-l LEN] [-u UMI]
  *   fastF crb     -b BAM -o OUT.gz
  *   fastF extract -b BAM -t TAG [-T 0|1]
  * Long options (--bam --feature --barcode --dbname --cell --depth --out --seed --umicopies; --R1 --out --len --umi; --tag --type) as
  * in the reference.  filter is not part of this build (out of scope: see DESIGN.md). */
 #include "fastf_host.h"
+#include "../../include/fastf_gpu.h"
 #include <errno.h>
 #include <stdlib.h>
 #include <string.h>
 #include <sys/stat.h>
 #include <unistd.h>
+#include <zlib.h>
 
 typedef struct { char s; const char *l; int has_arg; } optdef;
 /* returns the option index or -1; *val gets the argument ("-x VAL", "-xVAL", "--long VAL", "--long=VAL") */
@@ -71,35 +76,59 @@ static int cmd_freq(int argc, const char **argv)
     return rc;
 }
 
-#define MAX_DEPTHS 32   /* FASTF_SWEEP_MAX_RATES */
+#define MAX_DEPTHS 32   /* FASTF_SWEEP_MAX_RATES = FASTF_GRID_MAX_CELL_RATES */
+
+/* "R1,R2,..." of option `opt` -> names (pointers into *copy, strdup'ed) and float values as -r / -c read them; exits on what is refused */
+static uint32_t parse_rates(const char *list, const char *opt, char **copy, char **names, float *rates)
+{
+    uint32_t n = 0;
+    *copy = strdup(list);
+    for (char *save = NULL, *t = strtok_r(*copy, ",", &save); t; t = strtok_r(NULL, ",", &save)) {
+        if (n == MAX_DEPTHS) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s takes at most %d rates.\n", opt, MAX_DEPTHS); exit(1); }
+        names[n] = t;
+        rates[n] = strtof(t, NULL);
+        for (uint32_t k = 0; k < n; k++)
+            if (!strcmp(names[k], t) || !memcmp(&rates[k], &rates[n], sizeof(float))) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s lists the rate %s twice.\n", opt, t); exit(1); }
+        n++;
+    }
+    if (!n) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s needs at least one rate.\n", opt); exit(1); }
+    return n;
+}
+
+/* bam2db() lets FASTF_GPUS override --gpus: refuse either before any directory is made */
+static void one_gpu_only(const char *opt)
+{
+    const char *e = getenv("FASTF_GPUS");
+    if (fastf_gpus > 1 || (e && atoi(e) > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s runs on one GPU (--gpus 1, FASTF_GPUS unset or 1).\n", opt); exit(1); }
+}
+
+/* <dir>/<basename of db>: exits when it exists */
+static char *fresh_db(const char *dir, const char *db)
+{
+    const char *base = strrchr(db, '/') ? strrchr(db, '/') + 1 : db;
+    char *p = (char *)malloc(strlen(dir) + strlen(base) + 2);
+    sprintf(p, "%s/%s", dir, base);
+    if (access(p, F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", p); exit(1); }
+    return p;
+}
+
+static char *subdir(const char *parent, const char *prefix, const char *name)
+{
+    char *p = (char *)malloc(strlen(parent) + strlen(prefix) + strlen(name) + 2);
+    sprintf(p, "%s/%s%s", parent, prefix, name);
+    return p;
+}
 
 /* --depths R1,R2,...: one device pass, one output set per rate (bam2db_sweep) */
 static int depth_sweep(const char *bam, const char *feat, const char *bc, const char *db, const char *out, float rate_cell, const char *list, unsigned seed)
 {
-    char *names[MAX_DEPTHS + 1], *dirs[MAX_DEPTHS], *dbs[MAX_DEPTHS];
+    char *names[MAX_DEPTHS], *dirs[MAX_DEPTHS], *dbs[MAX_DEPTHS], *copy = NULL;
     float rates[MAX_DEPTHS];
-    uint32_t n = 0;
-    char *copy = strdup(list);
-    for (char *save = NULL, *t = strtok_r(copy, ",", &save); t; t = strtok_r(NULL, ",", &save)) {
-        if (n == MAX_DEPTHS) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths takes at most %d rates.\n", MAX_DEPTHS); exit(1); }
-        names[n] = t;
-        rates[n] = strtof(t, NULL);   /* as -r */
-        for (uint32_t k = 0; k < n; k++)
-            if (!strcmp(names[k], t) || !memcmp(&rates[k], &rates[n], sizeof(float))) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths lists the rate %s twice.\n", t); exit(1); }
-        n++;
-    }
-    if (!n) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths needs at least one rate.\n"); exit(1); }
-    {   /* bam2db() lets FASTF_GPUS override --gpus: refuse either here, before any directory is made */
-        const char *e = getenv("FASTF_GPUS");
-        if (fastf_gpus > 1 || (e && atoi(e) > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m --depths runs on one GPU (--gpus 1, FASTF_GPUS unset or 1).\n"); exit(1); }
-    }
-    const char *base = strrchr(db, '/') ? strrchr(db, '/') + 1 : db;
+    const uint32_t n = parse_rates(list, "--depths", &copy, names, rates);
+    one_gpu_only("--depths");
     for (uint32_t k = 0; k < n; k++) {
-        dirs[k] = (char *)malloc(strlen(out) + strlen(names[k]) + 16);
-        dbs[k] = (char *)malloc(strlen(out) + strlen(names[k]) + strlen(base) + 17);
-        sprintf(dirs[k], "%s/depth_%s", out, names[k]);
-        sprintf(dbs[k], "%s/%s", dirs[k], base);
-        if (access(dbs[k], F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", dbs[k]); exit(1); }
+        dirs[k] = subdir(out, "depth_", names[k]);
+        dbs[k] = fresh_db(dirs[k], db);
     }
     for (uint32_t k = 0; k < n; k++)
         if (mkdir(dirs[k], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", dirs[k]); exit(1); }
@@ -110,38 +139,91 @@ static int depth_sweep(const char *bam, const char *feat, const char *bc, const 
     return 0;
 }
 
+/* --cells C1,C2,... with -r R (depth_list NULL) or --depths R1,R2,...: one device pass, one output set per (cell rate, depth rate) (bam2db_grid) */
+static int cell_grid(const char *bam, const char *feat, const char *bc, const char *db, const char *out, const char *cell_list, const char *depth_list, float rate_depth,
+                     const char *rate_depth_text, unsigned seed)
+{
+    char *cnames[MAX_DEPTHS], *dnames[MAX_DEPTHS], *ccopy = NULL, *dcopy = NULL;
+    float crates[MAX_DEPTHS], drates[MAX_DEPTHS];
+    const uint32_t m = parse_rates(cell_list, "--cells", &ccopy, cnames, crates);
+    uint32_t k = 1;
+    if (depth_list) k = parse_rates(depth_list, "--depths", &dcopy, dnames, drates);
+    else { dnames[0] = (char *)rate_depth_text; drates[0] = rate_depth; }
+    one_gpu_only("--cells");
+    {   /* a cell rate the reference's SampleInt refuses is refused before anything is written */
+        gzFile g = gzopen(bc, "r");
+        char line[1024];
+        size_t n_cells = 0;
+        while (g && gzgets(g, line, 1024) != NULL) n_cells++;
+        if (g) gzclose(g);
+        uint64_t *samp = (uint64_t *)malloc(sizeof(uint64_t) * (n_cells ? n_cells : 1)), d0 = 0;
+        for (uint32_t i = 0; i < m; i++)
+            if (fastf_sample_cells(n_cells, crates[i], seed, samp, &d0) == UINT64_MAX) {
+                fprintf(stderr, "\x1b[31mError:\x1b[0m cell rate %s: Sample size must be smaller than population size when sampling without replacement.\n", cnames[i]);
+                exit(1);
+            }
+        free(samp);
+    }
+    char **cdirs = (char **)malloc(sizeof(char *) * m), **dirs = (char **)malloc(sizeof(char *) * m * k), **dbs = (char **)malloc(sizeof(char *) * m * k);
+    for (uint32_t i = 0; i < m; i++) {
+        cdirs[i] = subdir(out, "cell_", cnames[i]);
+        for (uint32_t j = 0; j < k; j++) {
+            dirs[i * k + j] = depth_list ? subdir(cdirs[i], "depth_", dnames[j]) : strdup(cdirs[i]);
+            dbs[i * k + j] = fresh_db(dirs[i * k + j], db);
+        }
+    }
+    for (uint32_t i = 0; i < m; i++) {
+        if (mkdir(cdirs[i], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", cdirs[i]); exit(1); }
+        for (uint32_t j = 0; j < k && depth_list; j++)
+            if (mkdir(dirs[i * k + j], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", dirs[i * k + j]); exit(1); }
+    }
+    const int rc = bam2db_grid((char *)bam, dbs, dirs, (char *)bc, (char *)feat, m, (const char *const *)cnames, crates, k, (const char *const *)dnames, drates, seed);
+    for (uint32_t i = 0; i < m * k; i++) { free(dirs[i]); free(dbs[i]); }
+    for (uint32_t i = 0; i < m; i++) free(cdirs[i]);
+    free(cdirs); free(dirs); free(dbs); free(ccopy); free(dcopy);
+    if (rc) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }
+    return 0;
+}
+
 static int cmd_bam2db(int argc, const char **argv)
 {
-    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".", *depths = NULL;
+    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".", *depths = NULL, *cells = NULL, *rate_depth_text = NULL;
     float rate_cell = 0.0f, rate_depth = 0.0f;   /* the reference leaves these uninitialised (src/main.c:293-294): pass -c and -r */
-    int have_r = 0;
+    int have_r = 0, have_c = 0;
     unsigned seed = 926;
-    static const optdef defs[] = {{'b', "bam", 1}, {'f', "feature", 1}, {'a', "barcode", 1}, {'d', "dbname", 1}, {'c', "cell", 1}, {'r', "depth", 1}, {'o', "out", 1}, {'s', "seed", 1}, {'u', "umicopies", 0}, {'h', "help", 0}, {'g', "gpus", 1}, {0, "depths", 1}};
+    static const optdef defs[] = {{'b', "bam", 1}, {'f', "feature", 1}, {'a', "barcode", 1}, {'d', "dbname", 1}, {'c', "cell", 1}, {'r', "depth", 1}, {'o', "out", 1}, {'s', "seed", 1}, {'u', "umicopies", 0}, {'h', "help", 0}, {'g', "gpus", 1}, {0, "depths", 1}, {0, "cells", 1}};
     for (int i = 1; i < argc; i++) {
         const char *v;
-        switch (next_opt(argc, argv, &i, defs, 12, &v)) {
+        switch (next_opt(argc, argv, &i, defs, 13, &v)) {
         case 0: bam = v; break;
         case 1: feat = v; break;
         case 2: bc = v; break;
         case 3: db = v; break;
-        case 4: rate_cell = strtof(v, NULL); break;     /* OPT_FLOAT uses strtof (src/argparse.c:101-116) */
-        case 5: rate_depth = strtof(v, NULL); have_r = 1; break;
+        case 4: rate_cell = strtof(v, NULL); have_c = 1; break;     /* OPT_FLOAT uses strtof (src/argparse.c:101-116) */
+        case 5: rate_depth = strtof(v, NULL); rate_depth_text = v; have_r = 1; break;
         case 6: out = v; break;
         case 7: seed = (unsigned)(int)strtol(v, NULL, 0); break;
         case 8: _umi_copies_flag = 1; break;
         case 10: fastf_gpus = (int)strtol(v, NULL, 0); break;   /* not a reference option: GPUs of this node to shard the BAM over */
         case 11: depths = v; break;                              /* not a reference option: the depth sweep */
+        case 12: cells = v; break;                               /* not a reference option: the cell-rate grid */
         default: printf("Usage: fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL -r RATE_DEPTH [-o OUT] [-s 926] [-u] [--gpus N]\n"
-                        "       fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL --depths R1,R2,... [-o OUT] [-s 926] [-u]\n\n"
+                        "       fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB -c RATE_CELL --depths R1,R2,... [-o OUT] [-s 926] [-u]\n"
+                        "       fastF bam2db -b BAM -f FEATURES -a BARCODES -d DB --cells C1,C2,... (-r RATE_DEPTH | --depths R1,R2,...) [-o OUT] [-s 926] [-u]\n\n"
                         "Filter bam file with desired cell proportion and read depth, then summarise it into UMI matrix.\n"
-                        "--depths writes the result of every rate Ri (up to 32, one pass over the BAM) into OUT/depth_<Ri>/, database OUT/depth_<Ri>/<basename of DB>.\n"); exit(0);
+                        "--depths writes the result of every rate Ri (up to 32, one pass over the BAM) into OUT/depth_<Ri>/, database OUT/depth_<Ri>/<basename of DB>.\n"
+                        "--cells writes the result of every cell rate Ci (up to 32, one pass over the BAM) into OUT/cell_<Ci>/ (with -r) or, for every depth\n"
+                        "rate Rj, into OUT/cell_<Ci>/depth_<Rj>/ (with --depths); database <that directory>/<basename of DB>.\n"); exit(0);
         }
     }
     if (depths && have_r) { fprintf(stderr, "\x1b[31mError:\x1b[0m -r/--depth and --depths exclude each other.\n"); exit(1); }
+    if (cells && have_c) { fprintf(stderr, "\x1b[31mError:\x1b[0m -c/--cell and --cells exclude each other.\n"); exit(1); }
+    if (cells && !depths && !have_r) { fprintf(stderr, "\x1b[31mError:\x1b[0m --cells needs -r or --depths.\n"); exit(1); }
     if (!bam || access(bam, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam file: %s does not exist.\n", bam ? bam : "(null)"); exit(1); }
     if (!feat || access(feat, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m feature file: %s does not exist.\n", feat ? feat : "(null)"); exit(1); }
     if (!bc || access(bc, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m barcode file: %s does not exist.\n", bc ? bc : "(null)"); exit(1); }
     if (!db) { fprintf(stderr, "\x1b[31mError:\x1b[0m please name the database with -d.\n"); exit(1); }
+    if (cells) return cell_grid(bam, feat, bc, db, out, cells, depths, rate_depth, rate_depth_text, seed);
     if (depths) return depth_sweep(bam, feat, bc, db, out, rate_cell, depths, seed);
     if (access(db, F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", db); exit(1); }
     if (bam2db((char *)bam, (char *)db, (char *)out, (char *)bc, (char *)feat, rate_cell, rate_depth, seed)) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }

@@ -160,6 +160,35 @@ void fastf_bam2db_sweep_result_free(fastf_bam2db_sweep_result *res);
 int fastf_bam2db_sample_sweep(fastf_bam2db_job *job, uint64_t ordinal_base, uint32_t n_rates, const uint64_t *sorted_thresholds, uint64_t *sampled, uint64_t *valid);
 /* after fastf_bam2db_sample_sweep: the valid rows kept by the largest threshold (file order) and their rate indices, owned by the job */
 int fastf_bam2db_kept_sweep_device(fastf_bam2db_job *job, uint64_t **dev_keys, uint32_t **dev_rates, uint64_t *n);
+/* ---- cell-rate grid: one job, the outputs of several cell rates x several depth rates (single GPU) ----
+ * Each cell rate -c samples its own cell table and skips its own number of draws d0 (fastf_sample_cells), so the depth sweep's subset
+ * argument does not hold across cell rates.  Inflate, CRC, record framing, the aux walk, the GX lookup and the UMI packing do not depend
+ * on the cell table, though: a grid job parses the BAM once against the UNION of the cell tables (p->cell_keys / cell_off / n_cells;
+ * p->d0 and p->keep_threshold are ignored) and keeps the cell of every CB-valid read, insertable or not.  Per cell rate it then rebuilds
+ * on the device, in file order, exactly the candidate array a job begun with that rate's table would have gathered (the reads whose
+ * cell the table holds, with the table's cell index) and runs the depth sweep over it at the rate's d0.
+ * The union is the union of the tables' barcodes, not the sampled lines of the largest rate: the host stops a table at its first
+ * duplicate barcode, so a smaller rate's table can hold a barcode that a larger rate's table lacks.
+ * After begin_grid the job is fed as any other and finished with fastf_bam2db_finish_grid only: fastf_bam2db_finish / _finish_sweep /
+ * _sample / _sample_sweep / _kept_device refuse a grid job, and finish_grid refuses any other job.  fastf_bam2db_counts on a grid job
+ * reports the union table's CB-valid reads.  FASTF_BAM_STRADDLE works as for one job.  The job sees every read of every table, so it
+ * fails with umi-too-long exactly where a single job begun with the union table would: retry with a larger umi_max_bytes as there. */
+#define FASTF_GRID_MAX_CELL_RATES 32
+typedef struct {
+    const uint32_t *cell_index;   /* p->n_cells entries: cell_index[u - 1] = 1-based index in this rate's table of union cell u, 0 = not in it */
+    uint32_t n_cells;             /* cells of this rate's table (its nonzero cell_index values are 1..n_cells, each once) */
+    uint64_t d0;                  /* MT draws consumed by this rate's cell sampling */
+} fastf_bam2db_cell_rate;
+int fastf_bam2db_begin_grid(fastf_ctx *ctx, const fastf_bam2db_params *p, fastf_bam2db_job **job);
+/* res[i] (n_cell_rates of them, caller order) is what fastf_bam2db_finish_sweep(n_rates, keep_thresholds) returns for a job begun with
+ * cell rate i's table and d0: every depth rate's counters (cb_valid = that table's CB-valid reads) and COO, bits_cell of that table, and
+ * the rows with their rate index when p->want_rows.  Stage clocks: ms_inflate / ms_crc / ms_parse / ms_gather are the shared pass's;
+ * ms_mt, ms_sample (including the remap), ms_sort and ms_count are cell rate i's own.  ms_device_total and n_launches count from the
+ * start of the job: for cell rate i they cover the shared pass and cell rates 0..i.  1..FASTF_GRID_MAX_CELL_RATES cell rates and
+ * 1..FASTF_SWEEP_MAX_RATES depth thresholds (validated as in finish_sweep).  res[0..min(n_cell_rates, FASTF_GRID_MAX_CELL_RATES)) is
+ * zeroed before anything is checked; free every res[i] with fastf_bam2db_sweep_result_free, also after a failure. */
+int fastf_bam2db_finish_grid(fastf_bam2db_job *job, uint32_t n_cell_rates, const fastf_bam2db_cell_rate *cell_rates, uint32_t n_rates, const uint64_t *keep_thresholds,
+                             fastf_bam2db_sweep_result *res);
 /* counters, sizes and per-stage device clocks so far, without finishing (multi-GPU driver); no arrays are allocated */
 int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *res);
 void fastf_bam2db_job_free(fastf_bam2db_job *job);
