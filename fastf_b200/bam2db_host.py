@@ -196,22 +196,6 @@ def _result_to_python(res, copy=True, row_keys=None):
     return stats, dict(coo, row_keys=row_keys)
 
 
-def run_sharded(lib, bam_bytes, inputs, rate_depth, seed, n_devices, want_rows=True, devices=None, **kw):
-    """bam2db over n_devices GPUs of this node in ONE process: the C driver fastf_bam2db_run_sharded (contexts, feeder threads and the
-    NCCL all-to-all live in the library).  Returns (stats, arrays) like run_device; stats gains "exchanged_keys"."""
-    p, keep = make_params(lib, inputs, rate_depth, seed, want_rows, **kw)
-    buf = np.frombuffer(bam_bytes, dtype=np.uint8)
-    res = _lib.Bam2dbResult()
-    devs = (C.c_int * n_devices)(*devices) if devices else None
-    if lib.fastf_bam2db_run_sharded(n_devices, devs, C.byref(p), C.c_void_p(buf.ctypes.data), buf.size, C.byref(res)) != 0:
-        raise _lib.FastfError("bam2db_run_sharded: " + lib.fastf_sharded_last_error().decode())
-    stats, out = _result_to_python(res)
-    lib.fastf_bam2db_result_free(C.byref(res))
-    stats["exchanged_keys"] = int(lib.fastf_sharded_exchanged())
-    del keep
-    return stats, out
-
-
 def _sweep_to_python(res, thr, want_rows):
     """[(stats, arrays)] per threshold (caller order) out of a filled Bam2dbSweepResult; rate i's rows are those whose rate's threshold is
     <= thr[i].  The caller frees res."""
@@ -229,26 +213,44 @@ def _thresholds(lib, rates):
     return np.array([lib.fastf_keep_threshold(C.c_float(r)) for r in rates], dtype=np.uint64)
 
 
-def run_sharded_sweep(lib, bam_bytes, inputs, rates, seed, n_devices, want_rows=True, devices=None, **kw):
-    """The depth sweep over n_devices GPUs of this node in ONE process (fastf_bam2db_run_sharded_sweep).  Returns what
-    Bam2dbJob.finish_sweep returns for one job over the whole file: [(stats, arrays)] in the order of `rates`; every stats gains
-    "exchanged_keys"."""
-    p, keep = make_params(lib, inputs, 0.0, seed, want_rows, **kw)
-    thr = _thresholds(lib, rates)
+def _run_sharded(lib, bam_bytes, inputs, rate_depth, rates, seed, n_devices, want_rows, devices, kw):
+    """fastf_bam2db_run_sharded at rate_depth (rates None) or fastf_bam2db_run_sharded_sweep at `rates`: [(stats, arrays)], every stats
+    with "exchanged_keys"."""
+    p, keep = make_params(lib, inputs, rate_depth, seed, want_rows, **kw)
     buf = np.frombuffer(bam_bytes, dtype=np.uint8)
-    res = _lib.Bam2dbSweepResult()
     devs = (C.c_int * n_devices)(*devices) if devices else None
+    args = (n_devices, devs, C.byref(p), C.c_void_p(buf.ctypes.data), buf.size)
+    sweep = rates is not None
+    thr = _thresholds(lib, rates) if sweep else None
+    res = _lib.Bam2dbSweepResult() if sweep else _lib.Bam2dbResult()
     try:
-        if lib.fastf_bam2db_run_sharded_sweep(n_devices, devs, C.byref(p), C.c_void_p(buf.ctypes.data), buf.size, len(thr), thr.ctypes.data_as(_lib.c_u64p), C.byref(res)) != 0:
-            raise _lib.FastfError("bam2db_run_sharded_sweep: " + lib.fastf_sharded_last_error().decode())
-        out = _sweep_to_python(res, thr, want_rows)
+        if sweep:
+            rc = lib.fastf_bam2db_run_sharded_sweep(*args, len(thr), thr.ctypes.data_as(_lib.c_u64p), C.byref(res))
+        else:
+            rc = lib.fastf_bam2db_run_sharded(*args, C.byref(res))
+        if rc != 0:
+            raise _lib.FastfError("bam2db_run_sharded%s: %s" % ("_sweep" if sweep else "", lib.fastf_sharded_last_error().decode()))
+        out = _sweep_to_python(res, thr, want_rows) if sweep else [_result_to_python(res)]
     finally:
-        lib.fastf_bam2db_sweep_result_free(C.byref(res))
+        (lib.fastf_bam2db_sweep_result_free if sweep else lib.fastf_bam2db_result_free)(C.byref(res))
     x = int(lib.fastf_sharded_exchanged())
     for stats, _ in out:
         stats["exchanged_keys"] = x
     del keep
     return out
+
+
+def run_sharded(lib, bam_bytes, inputs, rate_depth, seed, n_devices, want_rows=True, devices=None, **kw):
+    """bam2db over n_devices GPUs of this node in ONE process: the C driver fastf_bam2db_run_sharded (contexts, feeder threads and the
+    NCCL all-to-all live in the library).  Returns (stats, arrays) like run_device; stats gains "exchanged_keys"."""
+    return _run_sharded(lib, bam_bytes, inputs, rate_depth, None, seed, n_devices, want_rows, devices, kw)[0]
+
+
+def run_sharded_sweep(lib, bam_bytes, inputs, rates, seed, n_devices, want_rows=True, devices=None, **kw):
+    """The depth sweep over n_devices GPUs of this node in ONE process (fastf_bam2db_run_sharded_sweep).  Returns what
+    Bam2dbJob.finish_sweep returns for one job over the whole file: [(stats, arrays)] in the order of `rates`; every stats gains
+    "exchanged_keys"."""
+    return _run_sharded(lib, bam_bytes, inputs, 0.0, rates, seed, n_devices, want_rows, devices, kw)
 
 
 class Bam2dbJob:
@@ -357,18 +359,21 @@ def _feed_all(job, bam_bytes, feed_piece):
         job.feed(buf.ctypes.data + lo, hi - lo)
 
 
-def run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
-    """The C-ABI call sequence for one BAM image in host memory.  Returns (stats dict, dict of numpy result arrays)."""
-    with Bam2dbJob(ctx, inputs, rate_depth, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes) as job:
+def _run_job(ctx, bam_bytes, inputs, rate_depth, seed, finish, want_rows, inflate_lanes, chunk_inflated_bytes, feed_piece, umi_max_bytes, grid=False):
+    """The C-ABI call sequence for one BAM image in host memory: one job, fed the whole image, then finish(job)."""
+    with Bam2dbJob(ctx, inputs, rate_depth, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes, grid=grid) as job:
         _feed_all(job, bam_bytes, feed_piece)
-        return job.finish()
+        return finish(job)
+
+
+def run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
+    """One job at one depth rate.  Returns (stats dict, dict of numpy result arrays)."""
+    return _run_job(ctx, bam_bytes, inputs, rate_depth, seed, Bam2dbJob.finish, want_rows, inflate_lanes, chunk_inflated_bytes, feed_piece, umi_max_bytes)
 
 
 def run_device_sweep(ctx, bam_bytes, inputs, rates, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
     """run_device for several depth rates out of one job: [(stats, arrays)] in the order of `rates`."""
-    with Bam2dbJob(ctx, inputs, 0.0, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes) as job:
-        _feed_all(job, bam_bytes, feed_piece)
-        return job.finish_sweep(rates)
+    return _run_job(ctx, bam_bytes, inputs, 0.0, seed, lambda job: job.finish_sweep(rates), want_rows, inflate_lanes, chunk_inflated_bytes, feed_piece, umi_max_bytes)
 
 
 def grid_cell_rates(union):
@@ -378,9 +383,8 @@ def grid_cell_rates(union):
 
 def run_device_grid(ctx, bam_bytes, union, rates, seed, want_rows=True, inflate_lanes=0, chunk_inflated_bytes=0, feed_piece=0, umi_max_bytes=0):
     """run_device_sweep for every cell rate of Bam2dbInputs.grid out of one job: [[(stats, arrays)] per depth rate] per cell rate."""
-    with Bam2dbJob(ctx, union, 0.0, seed, want_rows, inflate_lanes, chunk_inflated_bytes, umi_max_bytes, grid=True) as job:
-        _feed_all(job, bam_bytes, feed_piece)
-        return job.finish_grid(grid_cell_rates(union), rates)
+    return _run_job(ctx, bam_bytes, union, 0.0, seed, lambda job: job.finish_grid(grid_cell_rates(union), rates), want_rows, inflate_lanes, chunk_inflated_bytes,
+                    feed_piece, umi_max_bytes, grid=True)
 
 
 def matrix_header(bam_file, rate_cell, rate_depth, total, sampled, valid):
@@ -414,23 +418,32 @@ def decode_dna10(blob_content, umi_max_bytes):
     return "".join(out)
 
 
-def open_database(db_file, bam_file, barcodes_file, features_file):
-    """the reference's opening sequence with its stderr lines (src/bam2db_ds.c:127-210); returns the sqlite connection or None"""
-    try:
-        db = sqlite3.connect(db_file, isolation_level=None)
-    except sqlite3.Error as e:
-        sys.stderr.write("Can't open database: %s\n" % e)
-        return None
-    sys.stderr.write("Opened database successfully\n")
+def open_databases(db_files, bam_file, barcodes_file, features_file, dbs):
+    """the reference's opening sequence with its stderr lines (src/bam2db_ds.c:127-210) for every database of db_files, appended to
+    dbs: the databases, the three inputs once, then the tables of every database.  Returns False after a failure."""
+    for f in db_files:
+        try:
+            dbs.append(sqlite3.connect(f, isolation_level=None))
+        except sqlite3.Error as e:
+            sys.stderr.write("Can't open database: %s\n" % e)
+            return False
+        sys.stderr.write("Opened database successfully\n")
     for path, what in ((bam_file, "BAM"), (barcodes_file, "cell barcode"), (features_file, "feature name")):
         if not os.path.exists(path):
             sys.stderr.write("Can't open %s file %s\n" % (what, path))
-            return None
+            return False
         sys.stderr.write("Opened %s file %s successfully\n" % (what, path))
-    db.execute("CREATE TABLE cell (cell_barcode TEXT);")
-    db.execute("CREATE TABLE feature (feature_id TEXT, feature_name TEXT, feature_type);")
-    db.execute("CREATE TABLE umi (cell_index INTEGER, feature_index INTEGER, encoded_umi TEXT);")
-    return db
+    for db in dbs:
+        db.execute("CREATE TABLE cell (cell_barcode TEXT);")
+        db.execute("CREATE TABLE feature (feature_id TEXT, feature_name TEXT, feature_type);")
+        db.execute("CREATE TABLE umi (cell_index INTEGER, feature_index INTEGER, encoded_umi TEXT);")
+    return True
+
+
+def open_database(db_file, bam_file, barcodes_file, features_file):
+    """open_databases for one database; returns the sqlite connection or None"""
+    dbs = []
+    return dbs[0] if open_databases([db_file], bam_file, barcodes_file, features_file, dbs) else None
 
 
 def insert_lists(db, inputs):
@@ -442,16 +455,26 @@ def insert_lists(db, inputs):
     db.execute("END TRANSACTION")
 
 
-def load_lists(db, lib, barcodes_file, features_file, rate_cell, seed):
-    inputs = Bam2dbInputs(lib, barcodes_file, features_file, rate_cell, seed)
+def cell_tables(lib, barcodes_file, features_file, cell_rates, seed, cell_names=None):
+    """The cell table of every cell rate with the reference's stdout lines (src/bam2db_ds.c:229-337).  Returns (the job's inputs, the
+    table of each cell rate): one rate's Bam2dbInputs, or with cell_names (a grid, naming each rate on stdout) Bam2dbInputs.grid."""
+    inputs = Bam2dbInputs.grid(lib, barcodes_file, features_file, cell_rates, seed) if cell_names else Bam2dbInputs(lib, barcodes_file, features_file, cell_rates[0], seed)
+    tables = inputs.tables if cell_names else [inputs]
     print("Total number of cells: %d" % inputs.n_cells)
-    print("Actual number of sampled cell barcodes: %d" % inputs.n_cells_sampled)
-    if inputs.duplicate_barcodes:
-        print("Warning: Duplicate cell barcodes were found in %s!" % barcodes_file)
+    for k, t in enumerate(tables):
+        if cell_names:
+            print("Cell rate %s:" % cell_names[k])
+        print("Actual number of sampled cell barcodes: %d" % t.n_cells_sampled)
+        if t.duplicate_barcodes:
+            print("Warning: Duplicate cell barcodes were found in %s!" % barcodes_file)
     if inputs.duplicate_features:
         print("Warning: Duplicate feature names were found in %s!" % features_file)
-    if db is not None:
-        insert_lists(db, inputs)
+    return inputs, tables
+
+
+def load_lists(db, lib, barcodes_file, features_file, rate_cell, seed):
+    inputs = cell_tables(lib, barcodes_file, features_file, [rate_cell], seed)[0]
+    insert_lists(db, inputs)
     return inputs
 
 
@@ -542,33 +565,11 @@ def _run_with_retries(run):
                 raise
 
 
-def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell, rate_depth, seed=926, device=0, ctx=None):
-    own = ctx is None
-    try:
-        if own:
-            ctx = _lib.Context(device)
-        db = open_database(db_file, bam_file, barcodes_file, features_file)
-        if db is None:
-            return 1
-        inputs = load_lists(db, ctx.lib, barcodes_file, features_file, rate_cell, seed)
-        print("Start to convert bam file to sqlite3 database...")
-        sys.stdout.flush()
-        bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
-        stats, out = _run_with_retries(lambda mb, fl: run_device(ctx, bam_bytes, inputs, rate_depth, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
-        rc = write_outputs(db, bam_file, path_out, inputs, rate_cell, rate_depth, stats, out, ctx=ctx)
-        db.close()
-        return rc
-    except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
-        sys.stderr.write("bam2db: %s\n" % e)
-        return 1
-    finally:
-        if own and ctx is not None:
-            ctx.close()
-
-
-def sweep_layout(db_name, path_out, rates, prefix="depth_", what="the depth sweep", check_db=True):
-    """(name, float32 value, output directory, database) per rate: rate r writes into path_out/<prefix><r as given>/, its database
-    is that directory's <basename of db_name>.  Raises ValueError on what the sweep refuses."""
+def _axis(rates, prefix, what):
+    """[(name, float32 value, subdirectory)] of one rate axis: a list of rates, each with its own subdirectory <prefix><rate as given>,
+    or one rate (a number or a string, as -c / -r) with none"""
+    if not isinstance(rates, (list, tuple)):
+        return [(str(rates), float(np.float32(float(rates))), "")]
     if not 1 <= len(rates) <= _lib.SWEEP_MAX_RATES:
         raise ValueError("%s takes 1..%d rates" % (what, _lib.SWEEP_MAX_RATES))
     out, seen = [], set()
@@ -578,52 +579,74 @@ def sweep_layout(db_name, path_out, rates, prefix="depth_", what="the depth swee
         if name in seen or val.tobytes() in seen:
             raise ValueError("the rate %s is listed twice" % name)
         seen.update((name, val.tobytes()))
-        d = os.path.join(path_out, prefix + name)
-        out.append((name, float(val), d, os.path.join(d, os.path.basename(db_name))))
-    for _, _, _, db in out:
-        if check_db and os.path.exists(db):
-            raise ValueError("database: %s already exists, change the name of database in -d argument!" % db)
+        out.append((name, float(val), prefix + name))
     return out
 
 
-def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, rates, seed=926, device=0, ctx=None, gpus=1):
-    """bam2db at several depth rates out of one pass over the BAM.  Rate r's output set is exactly what
-    bam2db(bam_file, <its database>, <its directory>, ..., rate_cell, r, seed) writes; see sweep_layout for where it goes.
-    gpus > 1 shards the BAM over devices 0..gpus-1 of this node (fastf_bam2db_run_sharded_sweep); `ctx` / `device` then only count
-    the copies of -u (umi.tsv, table numi).
-    Returns 0 / 1 like bam2db."""
+def rate_layout(db_name, path_out, cell_rates, rates):
+    """(cells, depths, sets) of one pass: the two axes as _axis gives them, and per output set, cell-rate major, (its directory, its
+    database).  One cell rate and one depth rate: bam2db's own path_out and db_name.  Otherwise set (i, j) goes to
+    path_out[/cell_<Ci>][/depth_<Rj>]/, a level for each axis given as a list, with database <that directory>/<basename of db_name>.
+    Raises ValueError on what the sweep and the grid refuse."""
+    cells, depths = _axis(cell_rates, "cell_", "the cell-rate grid"), _axis(rates, "depth_", "the depth sweep")
+    if not cells[0][2] and not depths[0][2]:
+        return cells, depths, [(path_out, db_name)]
+    sets = []
+    for _, _, cdir in cells:
+        for _, _, ddir in depths:
+            d = os.path.join(path_out, cdir, ddir) if ddir else os.path.join(path_out, cdir)
+            db = os.path.join(d, os.path.basename(db_name))
+            if os.path.exists(db):
+                raise ValueError("database: %s already exists, change the name of database in -d argument!" % db)
+            sets.append((d, db))
+    return cells, depths, sets
+
+
+def _bam2db_sets(bam_file, db_name, path_out, barcodes_file, features_file, cell_rates, rates, seed, device, ctx, gpus):
+    """bam2db, bam2db_sweep and bam2db_grid: the steps of the C host's bam2db_run, in its order and with its lines"""
     own = ctx is None
     dbs = []
     try:
-        layout = sweep_layout(db_name, path_out, rates)
+        cells, depths, sets = rate_layout(db_name, path_out, cell_rates, rates)
+        grid, sweep = bool(cells[0][2]), bool(depths[0][2])
+        if grid and gpus != 1:
+            raise ValueError("the cell-rate grid runs on one GPU")
         if gpus < 1:
             raise ValueError("gpus must be >= 1")
         if own and gpus == 1:
             ctx = _lib.Context(device)
         lib = ctx.lib if ctx is not None else _lib.load()   # gpus > 1: the driver opens one context per device itself
-        for _, _, d, dbf in layout:
-            os.makedirs(d, exist_ok=True)
-            db = open_database(dbf, bam_file, barcodes_file, features_file)
-            if db is None:
-                return 1
-            dbs.append(db)
-        inputs = load_lists(None, lib, barcodes_file, features_file, rate_cell, seed)
-        for db in dbs:
-            insert_lists(db, inputs)
+        if grid or sweep:
+            for d, _ in sets:
+                os.makedirs(d, exist_ok=True)
+        if not open_databases([f for _, f in sets], bam_file, barcodes_file, features_file, dbs):
+            return 1
+        inputs, tables = cell_tables(lib, barcodes_file, features_file, [v for _, v, _ in cells], seed, [n for n, _, _ in cells] if grid else None)
+        for k, db in enumerate(dbs):
+            insert_lists(db, tables[k // len(depths)])
         print("Start to convert bam file to sqlite3 database...")
         sys.stdout.flush()
         bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
-        vals = [v for _, v, _, _ in layout]
+        vals = [v for _, v, _ in depths]
+
+        def finish(job):   # one (stats, arrays) per output set, cell-rate major
+            if grid:
+                return [r for per in job.finish_grid(grid_cell_rates(inputs), vals) for r in per]
+            return job.finish_sweep(vals) if sweep else [job.finish()]
         if gpus > 1:
             # a BAM whose records straddle blocks fails here: the straddle mode (BAM_STRADDLE) needs the whole file in one job
-            results = _run_with_retries(lambda mb, fl: run_sharded_sweep(lib, bam_bytes, inputs, vals, seed, gpus, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+            results = _run_with_retries(lambda mb, fl: run_sharded_sweep(lib, bam_bytes, inputs, vals, seed, gpus, umi_max_bytes=mb, inflate_lanes=fl))
         else:
-            results = _run_with_retries(lambda mb, fl: run_device_sweep(ctx, bam_bytes, inputs, vals, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
+            results = _run_with_retries(lambda mb, fl: _run_job(ctx, bam_bytes, inputs, 0.0 if grid or sweep else vals[0], seed, finish, True, fl, 0, 0, mb, grid))
         if ctx is None and _umi_copies_flag:
             ctx = _lib.Context(device)   # numi / umi.tsv: the copies of every distinct key are counted on one device
-        for (name, val, d, _), db, (stats, out) in zip(layout, dbs, results):
-            print("Depth rate %s -> %s" % (name, d))
-            if write_outputs(db, bam_file, d, inputs, rate_cell, val, stats, out, ctx=ctx):
+        for k, ((d, _), db, (stats, out)) in enumerate(zip(sets, dbs, results)):
+            (cname, cval, _), (dname, dval, _) = cells[k // len(depths)], depths[k % len(depths)]
+            if grid:
+                print("Cell rate %s, depth rate %s -> %s" % (cname, dname, d))
+            elif sweep:
+                print("Depth rate %s -> %s" % (dname, d))
+            if write_outputs(db, bam_file, d, tables[k // len(depths)], cval, dval, stats, out, ctx=ctx):
                 return 1
         return 0
     except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
@@ -636,67 +659,22 @@ def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate
             ctx.close()
 
 
-def grid_layout(db_name, path_out, cell_rates, rates):
-    """(cell name, cell value, [(depth name, depth value, output directory, database)]) per cell rate: with a list of depth rates, set
-    (i, j) goes to path_out/cell_<Ci>/depth_<Rj>/, with one depth rate (a number or a string, as -r) to path_out/cell_<Ci>/.  Raises
-    ValueError on what the grid refuses."""
-    depths = isinstance(rates, (list, tuple))
-    out = []
-    for cname, cval, cdir, cdb in sweep_layout(db_name, path_out, cell_rates, "cell_", "the cell-rate grid", check_db=False):
-        if depths:
-            out.append((cname, cval, sweep_layout(db_name, cdir, rates)))
-        else:
-            if os.path.exists(cdb):
-                raise ValueError("database: %s already exists, change the name of database in -d argument!" % cdb)
-            out.append((cname, cval, [(str(rates), float(np.float32(float(rates))), cdir, cdb)]))
-    return out
+def bam2db(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell, rate_depth, seed=926, device=0, ctx=None):
+    return _bam2db_sets(bam_file, db_file, path_out, barcodes_file, features_file, rate_cell, rate_depth, seed, device, ctx, 1)
+
+
+def bam2db_sweep(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, rates, seed=926, device=0, ctx=None, gpus=1):
+    """bam2db at several depth rates out of one pass over the BAM.  Rate r's output set is exactly what
+    bam2db(bam_file, <its database>, <its directory>, ..., rate_cell, r, seed) writes; see rate_layout for where it goes.
+    gpus > 1 shards the BAM over devices 0..gpus-1 of this node (fastf_bam2db_run_sharded_sweep); `ctx` / `device` then only count
+    the copies of -u (umi.tsv, table numi).
+    Returns 0 / 1 like bam2db."""
+    return _bam2db_sets(bam_file, db_name, path_out, barcodes_file, features_file, rate_cell, list(rates), seed, device, ctx, gpus)
 
 
 def bam2db_grid(bam_file, db_name, path_out, barcodes_file, features_file, cell_rates, rates, seed=926, device=0, ctx=None, gpus=1):
     """bam2db at several cell rates x depth rates out of one pass over the BAM.  Set (i, j) is exactly what
-    bam2db(bam_file, <its database>, <its directory>, ..., cell_rates[i], rates[j], seed) writes; see grid_layout for where it goes.
+    bam2db(bam_file, <its database>, <its directory>, ..., cell_rates[i], rates[j], seed) writes; see rate_layout for where it goes
+    (`rates` a list: path_out/cell_<Ci>/depth_<Rj>/, one rate: path_out/cell_<Ci>/).
     One GPU only (gpus > 1 is refused).  Returns 0 / 1 like bam2db."""
-    own = ctx is None
-    dbs = []
-    try:
-        layout = grid_layout(db_name, path_out, cell_rates, rates)
-        if gpus != 1:
-            raise ValueError("the cell-rate grid runs on one GPU")
-        depth_vals = [v for _, v, _, _ in layout[0][2]]
-        if own:
-            ctx = _lib.Context(device)
-        union = Bam2dbInputs.grid(ctx.lib, barcodes_file, features_file, [v for _, v, _ in layout], seed)
-        print("Total number of cells: %d" % union.n_cells)
-        for (cname, _, sets), t in zip(layout, union.tables):
-            print("Cell rate %s: actual number of sampled cell barcodes: %d" % (cname, t.n_cells_sampled))
-            for _, _, d, dbf in sets:
-                os.makedirs(d, exist_ok=True)
-                db = open_database(dbf, bam_file, barcodes_file, features_file)
-                if db is None:
-                    return 1
-                dbs.append(db)
-                insert_lists(db, t)
-        if union.duplicate_barcodes:
-            print("Warning: Duplicate cell barcodes were found in %s!" % barcodes_file)
-        if union.duplicate_features:
-            print("Warning: Duplicate feature names were found in %s!" % features_file)
-        print("Start to convert bam file to sqlite3 database...")
-        sys.stdout.flush()
-        bam_bytes = np.fromfile(bam_file, dtype=np.uint8)
-        results = _run_with_retries(lambda mb, fl: run_device_grid(ctx, bam_bytes, union, depth_vals, seed, want_rows=True, umi_max_bytes=mb, inflate_lanes=fl))
-        k = 0
-        for (cname, cval, sets), t, per_depth in zip(layout, union.tables, results):
-            for (dname, dval, d, _), (stats, out) in zip(sets, per_depth):
-                print("Cell rate %s, depth rate %s -> %s" % (cname, dname, d))
-                if write_outputs(dbs[k], bam_file, d, t, cval, dval, stats, out, ctx=ctx):
-                    return 1
-                k += 1
-        return 0
-    except (_lib.FastfError, ValueError, OSError, sqlite3.Error) as e:
-        sys.stderr.write("bam2db: %s\n" % e)
-        return 1
-    finally:
-        for db in dbs:
-            db.close()
-        if own and ctx is not None:
-            ctx.close()
+    return _bam2db_sets(bam_file, db_name, path_out, barcodes_file, features_file, list(cell_rates), rates, seed, device, ctx, gpus)

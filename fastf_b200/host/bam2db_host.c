@@ -300,10 +300,24 @@ done:
     return rc;
 }
 
-/* bam2db() (one output set), bam2db_sweep() (n_rates > 0: depth rates) and bam2db_grid() (n_cell_rates > 0 as well: cell rates x depth
- * rates): one device job.  Output set (i, j) of cell rate i and depth rate j goes to out_dirs[i * K + j] / db_files[i * K + j]. */
-static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
-                      const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed)
+/* the job's parameters: the cell table it parses against, the feature keys, and the sampling of the first rate (ignored by the sweep,
+ * and d0 by the grid) */
+static fastf_bam2db_params job_params(const strlist *cells, const strlist *fkeys, unsigned seed, uint64_t d0, float rate, uint32_t umi_bytes, uint32_t flags)
+{
+    static const uint32_t zero_off[1] = {0};
+    fastf_bam2db_params p;
+    memset(&p, 0, sizeof p);
+    p.cell_keys = cells->buf ? cells->buf : ""; p.cell_off = cells->off ? cells->off : zero_off; p.n_cells = cells->n;
+    p.gene_keys = fkeys->buf ? fkeys->buf : ""; p.gene_off = fkeys->off ? fkeys->off : zero_off; p.n_genes = fkeys->n;
+    p.seed = seed; p.d0 = d0; p.keep_threshold = fastf_keep_threshold(rate);
+    p.umi_max_bytes = umi_bytes;
+    p.want_rows = 1;
+    p.inflate_lanes = flags;
+    return p;
+}
+
+int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
+               const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed)
 {
     int rc = 1;
     const int grid = n_cell_rates > 0, sweep = n_rates > 0;
@@ -314,14 +328,15 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
     fastf_bam2db_result res;
     memset(&res, 0, sizeof res);
     fastf_bam2db_sweep_result *sres = sweep ? (fastf_bam2db_sweep_result *)calloc(M, sizeof *sres) : NULL;
-    uint64_t *rate_rows = NULL;
+    uint64_t *rate_rows = NULL, thr[FASTF_SWEEP_MAX_RATES];
     strlist *cells = (strlist *)calloc(M, sizeof *cells);
     strlist ucells = {0}, fkeys = {0}, fid = {0}, fname = {0}, ftype = {0};
     strset uset = {0}, fset = {0};
     uint64_t d0s[FASTF_GRID_MAX_CELL_RATES] = {0};
     uint32_t *remap = NULL;
     fastf_bam2db_cell_rate crs[FASTF_GRID_MAX_CELL_RATES];
-    void *pin[2] = {NULL, NULL};
+    void *pin[2] = {NULL, NULL}, *map = MAP_FAILED;
+    size_t map_n = 0;
     int bam = -1;
     gzFile gb = NULL, gf = NULL;
     char line[1024];
@@ -331,8 +346,12 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         if ((e = getenv("FASTF_DEVICE")) != NULL) fastf_device = atoi(e);
     }
     if (!dbs || !cells || (sweep && !sres)) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
-    if (grid && (n_cell_rates > FASTF_GRID_MAX_CELL_RATES || fastf_gpus > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m the cell-rate grid takes 1..%d cell rates on one GPU\n", FASTF_GRID_MAX_CELL_RATES); goto done; }
+    if (grid && (!sweep || n_cell_rates > FASTF_GRID_MAX_CELL_RATES || fastf_gpus > 1)) {
+        fprintf(stderr, "\x1b[31mError:\x1b[0m the cell-rate grid takes 1..%d cell rates and 1..%d depth rates on one GPU\n", FASTF_GRID_MAX_CELL_RATES, FASTF_SWEEP_MAX_RATES);
+        goto done;
+    }
     if (sweep && (n_rates > FASTF_SWEEP_MAX_RATES || fastf_gpus > 1)) { fprintf(stderr, "\x1b[31mError:\x1b[0m the depth sweep takes 1..%d rates on one GPU\n", FASTF_SWEEP_MAX_RATES); goto done; }
+    for (uint32_t r = 0; r < K; r++) thr[r] = fastf_keep_threshold(rates[r]);
 
     g_t_last = 0;
     phase("start");
@@ -417,97 +436,71 @@ static int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *ba
         /* several GPUs of this node: contiguous block shards, global draw ordinals, NCCL all-to-all by cell (csrc/sharded.cu) */
         struct stat sb;
         if (fstat(bam, &sb) || sb.st_size <= 0) { fprintf(stderr, "\x1b[31mError:\x1b[0m cannot stat %s\n", bam_file); goto done; }
-        void *map = mmap(NULL, (size_t)sb.st_size, PROT_READ, MAP_PRIVATE, bam, 0);
-        if (map == MAP_FAILED) { fprintf(stderr, "\x1b[31mError:\x1b[0m cannot map %s\n", bam_file); goto done; }
-        madvise(map, (size_t)sb.st_size, MADV_SEQUENTIAL);
-        int failed = 1;
-        for (uint32_t umi_bytes = 3; umi_bytes <= 4 && failed; umi_bytes++) {
-            fastf_bam2db_params p;
-            memset(&p, 0, sizeof p);
-            uint32_t zero_off[1] = {0};
-            p.cell_keys = cells[0].buf ? cells[0].buf : ""; p.cell_off = cells[0].off ? cells[0].off : zero_off; p.n_cells = cells[0].n;
-            p.gene_keys = fkeys.buf ? fkeys.buf : ""; p.gene_off = fkeys.off ? fkeys.off : zero_off; p.n_genes = fkeys.n;
-            p.seed = seed; p.d0 = d0s[0]; p.keep_threshold = fastf_keep_threshold(rates[0]);
-            p.umi_max_bytes = umi_bytes;
-            p.want_rows = 1;
-            failed = fastf_bam2db_run_sharded(fastf_gpus, NULL, &p, map, (size_t)sb.st_size, &res);
-            if (failed && !(umi_bytes == 3 && strstr(fastf_sharded_last_error(), "umi-too-long"))) break;
-        }
-        munmap(map, (size_t)sb.st_size);
-        if (failed) {
-            fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_sharded_last_error());
-            if (strstr(fastf_sharded_last_error(), "record-straddles-bgzf-block")) fprintf(stderr, "(records cross BGZF blocks: not an htslib-written file; run it on one GPU, FASTF_GPUS=1)\n");
-            goto done;
-        }
-        if (_umi_copies_flag && fastf_ctx_create(fastf_device, &ctx)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(NULL)); goto done; }
-    } else {
-    if (fastf_ctx_create(fastf_device, &ctx)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(NULL)); goto done; }
-    uint32_t flags = 0;   /* FASTF_BAM_STRADDLE after a first attempt met records that cross BGZF blocks (htsjdk / STAR writers) */
-    for (uint32_t umi_bytes = 3; umi_bytes <= 4; umi_bytes++) {   /* 10x UMIs are 10 or 12 bases; retry once with room for 16 */
-        fastf_bam2db_params p;
-        memset(&p, 0, sizeof p);
-        uint32_t zero_off[1] = {0};
-        p.cell_keys = jcells->buf ? jcells->buf : ""; p.cell_off = jcells->off ? jcells->off : zero_off; p.n_cells = jcells->n;
-        p.gene_keys = fkeys.buf ? fkeys.buf : ""; p.gene_off = fkeys.off ? fkeys.off : zero_off; p.n_genes = fkeys.n;
-        p.seed = seed; p.d0 = d0s[0]; p.keep_threshold = fastf_keep_threshold(rates[0]);   /* ignored by the sweep (and d0 by the grid) */
-        p.umi_max_bytes = umi_bytes;
-        p.want_rows = 1;
-        p.inflate_lanes = flags;
-        if ((grid ? fastf_bam2db_begin_grid : fastf_bam2db_begin)(ctx, &p, &job)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
-        const size_t PIECE = (size_t)256 << 20;
-        if (!pin[0] && (fastf_host_alloc(ctx, PIECE, &pin[0]) || fastf_host_alloc(ctx, PIECE, &pin[1]))) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
-        ssize_t got;
-        off_t at = 0;
-        int which = 0, failed = 0;
-        while (!failed && (got = fastf_pread_parallel(bam, pin[which], PIECE, at)) > 0) {   /* several readers: one fread() cannot feed PCIe */
-            failed = fastf_bam2db_feed(job, pin[which], (size_t)got);
-            at += got;
-            which ^= 1;
-        }
-        if (!failed && got < 0) { fprintf(stderr, "\x1b[31mError:\x1b[0m reading %s failed\n", bam_file); goto done; }
-        if (!failed && sweep) {
-            uint64_t thr[FASTF_SWEEP_MAX_RATES];
-            for (uint32_t r = 0; r < K; r++) thr[r] = fastf_keep_threshold(rates[r]);
-            failed = grid ? fastf_bam2db_finish_grid(job, M, crs, K, thr, sres) : fastf_bam2db_finish_sweep(job, K, thr, sres);
-            if (failed) for (uint32_t i = 0; i < M; i++) fastf_bam2db_sweep_result_free(&sres[i]);
-        } else if (!failed) {
-            failed = fastf_bam2db_finish(job, &res);
+        map_n = (size_t)sb.st_size;
+        if ((map = mmap(NULL, map_n, PROT_READ, MAP_PRIVATE, bam, 0)) == MAP_FAILED) { fprintf(stderr, "\x1b[31mError:\x1b[0m cannot map %s\n", bam_file); goto done; }
+        madvise(map, map_n, MADV_SEQUENTIAL);
+    } else if (fastf_ctx_create(fastf_device, &ctx)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(NULL)); goto done; }
+    /* 10x UMIs are 10 or 12 bases: retried once with room for 16.  Records that cross BGZF blocks (htsjdk / STAR writers): retried once
+     * on one GPU with FASTF_BAM_STRADDLE, record starts guessed and verified per block (whole file in one chunk). */
+    for (uint32_t umi_bytes = 3, flags = 0;;) {
+        const fastf_bam2db_params p = job_params(jcells, &fkeys, seed, d0s[0], rates[0], umi_bytes, flags);
+        int failed;
+        if (fastf_gpus > 1) {
+            failed = fastf_bam2db_run_sharded(fastf_gpus, NULL, &p, map, map_n, &res);
+        } else if (!(failed = (grid ? fastf_bam2db_begin_grid : fastf_bam2db_begin)(ctx, &p, &job))) {
+            const size_t PIECE = (size_t)256 << 20;
+            if (!pin[0] && (fastf_host_alloc(ctx, PIECE, &pin[0]) || fastf_host_alloc(ctx, PIECE, &pin[1]))) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx)); goto done; }
+            ssize_t got;
+            off_t at = 0;
+            int which = 0;
+            while (!failed && (got = fastf_pread_parallel(bam, pin[which], PIECE, at)) > 0) {   /* several readers: one fread() cannot feed PCIe */
+                failed = fastf_bam2db_feed(job, pin[which], (size_t)got);
+                at += got;
+                which ^= 1;
+            }
+            if (!failed && got < 0) { fprintf(stderr, "\x1b[31mError:\x1b[0m reading %s failed\n", bam_file); goto done; }
+            if (!failed && grid) failed = fastf_bam2db_finish_grid(job, M, crs, K, thr, sres);
+            else if (!failed && sweep) failed = fastf_bam2db_finish_sweep(job, K, thr, sres);
+            else if (!failed) failed = fastf_bam2db_finish(job, &res);
         }
         if (!failed) break;
-        if (umi_bytes == 3 && strstr(fastf_last_error(ctx), "umi-too-long")) { fastf_bam2db_job_free(job); job = NULL; continue; }
-        if (!flags && strstr(fastf_last_error(ctx), "record-straddles-bgzf-block")) {
-            /* not an htslib-written file: run again with record starts guessed and verified per block (whole file in one chunk) */
-            fastf_bam2db_job_free(job); job = NULL;
-            flags = FASTF_BAM_STRADDLE;
-            umi_bytes--;
-            continue;
-        }
-        fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(ctx));
+        char err[1024];
+        snprintf(err, sizeof err, "%s", fastf_gpus > 1 ? fastf_sharded_last_error() : fastf_last_error(ctx));
+        if (job) { fastf_bam2db_job_free(job); job = NULL; }
+        fastf_bam2db_result_free(&res);
+        for (uint32_t i = 0; sweep && i < M; i++) fastf_bam2db_sweep_result_free(&sres[i]);
+        if (umi_bytes == 3 && strstr(err, "umi-too-long")) { umi_bytes = 4; continue; }
+        if (!flags && fastf_gpus == 1 && strstr(err, "record-straddles-bgzf-block")) { flags = FASTF_BAM_STRADDLE; continue; }
+        fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", err);
+        if (fastf_gpus > 1 && strstr(err, "record-straddles-bgzf-block")) fprintf(stderr, "(records cross BGZF blocks: not an htslib-written file; run it on one GPU, FASTF_GPUS=1)\n");
         goto done;
     }
-    }
+    if (!ctx && _umi_copies_flag && fastf_ctx_create(fastf_device, &ctx)) { fprintf(stderr, "\x1b[31mError:\x1b[0m %s\n", fastf_last_error(NULL)); goto done; }
 
+    /* ---- one output set per (cell rate i, depth rate r); a single-rate run is set (0, 0): the job's result and all its rows ---- */
     phase("device job (ctx, read, feed, finish)");
-    if (!sweep) {
-        if (write_outputs(&dbs[0], db_files[0], bam_file, out_dirs[0], cell_rates[0], rates[0], &res, res.row_keys, res.n_rows, &cells[0], &fkeys, &fid, &fname, &ftype, ctx)) goto done;
-    } else {
-        uint64_t thr[FASTF_SWEEP_MAX_RATES];
-        for (uint32_t r = 0; r < K; r++) thr[r] = fastf_keep_threshold(rates[r]);
-        for (uint32_t i = 0; i < M; i++) {
-            const fastf_bam2db_sweep_result *sr = &sres[i];
+    for (uint32_t i = 0; i < M; i++) {
+        const fastf_bam2db_sweep_result *sr = sweep ? &sres[i] : NULL;
+        if (sr) {
             free(rate_rows);
             rate_rows = (uint64_t *)malloc(sizeof(uint64_t) * (sr->n_rows ? sr->n_rows : 1));
             if (!rate_rows) { fprintf(stderr, "\x1b[31mError:\x1b[0m out of host memory\n"); goto done; }
-            for (uint32_t r = 0; r < K; r++) {
-                /* table umi of rate r: the rows whose smallest keeping threshold is <= its own, in file order */
-                uint64_t n = 0;
+        }
+        for (uint32_t r = 0; r < K; r++) {
+            const fastf_bam2db_result *rr = &res;
+            const uint64_t *rows = res.row_keys;
+            uint64_t n = res.n_rows;
+            if (sr) {   /* table umi of rate r: the rows whose smallest keeping threshold is <= its own, in file order */
+                rr = &sr->rate[r];
+                rows = rate_rows;
+                n = 0;
                 for (uint64_t k = 0; k < sr->n_rows; k++)
                     if (thr[sr->row_rate[k]] <= thr[r]) rate_rows[n++] = sr->row_keys[k];
-                if (grid) printf("Cell rate %s, depth rate %s -> %s\n", cell_names[i], rate_names[r], out_dirs[i * K + r]);
-                else printf("Depth rate %s -> %s\n", rate_names[r], out_dirs[r]);
-                if (write_outputs(&dbs[i * K + r], db_files[i * K + r], bam_file, out_dirs[i * K + r], cell_rates[i], rates[r], &sr->rate[r], rate_rows, n, &cells[i], &fkeys, &fid, &fname,
-                                  &ftype, ctx)) goto done;
             }
+            if (grid) printf("Cell rate %s, depth rate %s -> %s\n", cell_names[i], rate_names[r], out_dirs[i * K + r]);
+            else if (sweep) printf("Depth rate %s -> %s\n", rate_names[r], out_dirs[r]);
+            if (write_outputs(&dbs[i * K + r], db_files[i * K + r], bam_file, out_dirs[i * K + r], cell_rates[i], rates[r], rr, rows, n, &cells[i], &fkeys, &fid, &fname, &ftype,
+                              ctx)) goto done;
         }
     }
     rc = 0;
@@ -517,6 +510,7 @@ done:
     free(dbs);
     if (gb) gzclose(gb);
     if (gf) gzclose(gf);
+    if (map != MAP_FAILED) munmap(map, map_n);
     if (bam >= 0) close(bam);
     fastf_bam2db_result_free(&res);
     if (sres) { for (uint32_t i = 0; i < M; i++) fastf_bam2db_sweep_result_free(&sres[i]); free(sres); }
@@ -534,18 +528,4 @@ done:
 int bam2db(char *bam_file, char *db_file, char *path_out, char *barcodes_file, char *features_file, float rate_cell, float rate_depth, unsigned int seed)
 {
     return bam2db_run(bam_file, &db_file, &path_out, barcodes_file, features_file, 0, NULL, &rate_cell, 0, NULL, &rate_depth, seed);
-}
-
-int bam2db_sweep(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
-                 const float *rates, unsigned int seed)
-{
-    if (n_rates < 1) { fprintf(stderr, "\x1b[31mError:\x1b[0m the depth sweep needs at least one rate\n"); return 1; }
-    return bam2db_run(bam_file, db_files, out_dirs, barcodes_file, features_file, 0, NULL, &rate_cell, n_rates, rate_names, rates, seed);
-}
-
-int bam2db_grid(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
-                const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed)
-{
-    if (n_cell_rates < 1 || n_rates < 1) { fprintf(stderr, "\x1b[31mError:\x1b[0m the cell-rate grid needs at least one cell rate and one depth rate\n"); return 1; }
-    return bam2db_run(bam_file, db_files, out_dirs, barcodes_file, features_file, n_cell_rates, cell_names, cell_rates, n_rates, rate_names, rates, seed);
 }

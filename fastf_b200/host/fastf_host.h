@@ -14,15 +14,13 @@ extern int _umi_copies_flag;   /* reference src/bam2db_ds.h:23 */
 extern int fastf_device;       /* CUDA device ordinal (env FASTF_DEVICE, default 0) */
 extern int fastf_gpus;         /* bam2db over this many GPUs of the node (env FASTF_GPUS or --gpus N, default 1) */
 int bam2db(char *bam_file, char *db_file, char *path_out, char *barcodes_file, char *features_file, float rate_cell, float rate_depth, unsigned int seed);
-/* the depth sweep (not a reference entry point): one device job, output set i = what bam2db(..., rates[i], seed) writes, into
- * out_dirs[i] with database db_files[i]; 1..32 rates, one GPU.  rate_names[i] names rate i on stdout. */
-int bam2db_sweep(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, float rate_cell, uint32_t n_rates, const char *const *rate_names,
-                 const float *rates, unsigned int seed);
-/* the cell-rate grid (not a reference entry point): one device job, output set (i, j) = what bam2db(..., cell_rates[i], rates[j], seed)
- * writes, into out_dirs[i * n_rates + j] with database db_files[i * n_rates + j]; 1..32 cell rates, 1..32 depth rates, one GPU.
- * cell_names[i] / rate_names[j] name the rates on stdout. */
-int bam2db_grid(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
-                const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed);
+/* bam2db over several output sets out of one device job (not a reference entry point; bam2db() is its one-set call).  The cell axis
+ * is n_cell_rates cell rates (1..32, cell_names[i] names rate i on stdout), or with n_cell_rates = 0 the one rate cell_rates[0] and
+ * no union table.  The depth axis is n_rates depth rates (1..32, named by rate_names[j]), or with n_rates = 0 the one rate rates[0]
+ * (cell rates need n_rates >= 1).  Set (i, j) = what bam2db(..., cell_rates[i], rates[j], seed) writes, into out_dirs[i * K + j]
+ * with database db_files[i * K + j], K = max(n_rates, 1).  Several cell or depth rates run on one GPU. */
+int bam2db_run(char *bam_file, char **db_files, char **out_dirs, char *barcodes_file, char *features_file, uint32_t n_cell_rates, const char *const *cell_names,
+               const float *cell_rates, uint32_t n_rates, const char *const *rate_names, const float *rates, unsigned int seed);
 /* cell_counts + print_tree in one call: histogram of the first l+u bases of every read of R1 (BGZF or plain text), written to fp
  * in the reference's BST pre-order.  Returns 0 / 1. */
 int freq_whitelist(const char *r1_path, size_t len_cellbarcode, size_t len_umi, FILE *fp);

@@ -119,38 +119,21 @@ static char *subdir(const char *parent, const char *prefix, const char *name)
     return p;
 }
 
-/* --depths R1,R2,...: one device pass, one output set per rate (bam2db_sweep) */
-static int depth_sweep(const char *bam, const char *feat, const char *bc, const char *db, const char *out, float rate_cell, const char *list, unsigned seed)
-{
-    char *names[MAX_DEPTHS], *dirs[MAX_DEPTHS], *dbs[MAX_DEPTHS], *copy = NULL;
-    float rates[MAX_DEPTHS];
-    const uint32_t n = parse_rates(list, "--depths", &copy, names, rates);
-    one_gpu_only("--depths");
-    for (uint32_t k = 0; k < n; k++) {
-        dirs[k] = subdir(out, "depth_", names[k]);
-        dbs[k] = fresh_db(dirs[k], db);
-    }
-    for (uint32_t k = 0; k < n; k++)
-        if (mkdir(dirs[k], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", dirs[k]); exit(1); }
-    const int rc = bam2db_sweep((char *)bam, dbs, dirs, (char *)bc, (char *)feat, rate_cell, n, (const char *const *)names, rates, seed);
-    for (uint32_t k = 0; k < n; k++) { free(dirs[k]); free(dbs[k]); }
-    free(copy);
-    if (rc) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }
-    return 0;
-}
-
-/* --cells C1,C2,... with -r R (depth_list NULL) or --depths R1,R2,...: one device pass, one output set per (cell rate, depth rate) (bam2db_grid) */
-static int cell_grid(const char *bam, const char *feat, const char *bc, const char *db, const char *out, const char *cell_list, const char *depth_list, float rate_depth,
-                     const char *rate_depth_text, unsigned seed)
+/* --depths and/or --cells: one device pass, one output set per (cell rate, depth rate) (bam2db_run).  The cell axis is the --cells list
+ * (cell_list) or the one -c rate, the depth axis the --depths list (depth_list) or the one -r rate.  Set (Ci, Rj) goes to
+ * OUT[/cell_<Ci>][/depth_<Rj>]/, a level for each list.  Everything refused is refused before any directory is made. */
+static int rate_sets(const char *bam, const char *feat, const char *bc, const char *db, const char *out, const char *cell_list, float rate_cell, const char *rate_cell_text,
+                     const char *depth_list, float rate_depth, const char *rate_depth_text, unsigned seed)
 {
     char *cnames[MAX_DEPTHS], *dnames[MAX_DEPTHS], *ccopy = NULL, *dcopy = NULL;
     float crates[MAX_DEPTHS], drates[MAX_DEPTHS];
-    const uint32_t m = parse_rates(cell_list, "--cells", &ccopy, cnames, crates);
-    uint32_t k = 1;
+    uint32_t m = 1, k = 1;
+    if (cell_list) m = parse_rates(cell_list, "--cells", &ccopy, cnames, crates);
+    else { cnames[0] = (char *)rate_cell_text; crates[0] = rate_cell; }
     if (depth_list) k = parse_rates(depth_list, "--depths", &dcopy, dnames, drates);
     else { dnames[0] = (char *)rate_depth_text; drates[0] = rate_depth; }
-    one_gpu_only("--cells");
-    {   /* a cell rate the reference's SampleInt refuses is refused before anything is written */
+    one_gpu_only(cell_list ? "--cells" : "--depths");
+    {   /* a cell rate the reference's SampleInt refuses */
         gzFile g = gzopen(bc, "r");
         char line[1024];
         size_t n_cells = 0;
@@ -166,18 +149,18 @@ static int cell_grid(const char *bam, const char *feat, const char *bc, const ch
     }
     char **cdirs = (char **)malloc(sizeof(char *) * m), **dirs = (char **)malloc(sizeof(char *) * m * k), **dbs = (char **)malloc(sizeof(char *) * m * k);
     for (uint32_t i = 0; i < m; i++) {
-        cdirs[i] = subdir(out, "cell_", cnames[i]);
+        cdirs[i] = cell_list ? subdir(out, "cell_", cnames[i]) : strdup(out);
         for (uint32_t j = 0; j < k; j++) {
             dirs[i * k + j] = depth_list ? subdir(cdirs[i], "depth_", dnames[j]) : strdup(cdirs[i]);
             dbs[i * k + j] = fresh_db(dirs[i * k + j], db);
         }
     }
     for (uint32_t i = 0; i < m; i++) {
-        if (mkdir(cdirs[i], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", cdirs[i]); exit(1); }
+        if (cell_list && mkdir(cdirs[i], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", cdirs[i]); exit(1); }
         for (uint32_t j = 0; j < k && depth_list; j++)
             if (mkdir(dirs[i * k + j], 0777) && errno != EEXIST) { fprintf(stderr, "\x1b[31mError:\x1b[0m can not create directory %s\n", dirs[i * k + j]); exit(1); }
     }
-    const int rc = bam2db_grid((char *)bam, dbs, dirs, (char *)bc, (char *)feat, m, (const char *const *)cnames, crates, k, (const char *const *)dnames, drates, seed);
+    const int rc = bam2db_run((char *)bam, dbs, dirs, (char *)bc, (char *)feat, cell_list ? m : 0, (const char *const *)cnames, crates, k, (const char *const *)dnames, drates, seed);
     for (uint32_t i = 0; i < m * k; i++) { free(dirs[i]); free(dbs[i]); }
     for (uint32_t i = 0; i < m; i++) free(cdirs[i]);
     free(cdirs); free(dirs); free(dbs); free(ccopy); free(dcopy);
@@ -187,7 +170,7 @@ static int cell_grid(const char *bam, const char *feat, const char *bc, const ch
 
 static int cmd_bam2db(int argc, const char **argv)
 {
-    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".", *depths = NULL, *cells = NULL, *rate_depth_text = NULL;
+    const char *bam = NULL, *feat = NULL, *bc = NULL, *db = NULL, *out = ".", *depths = NULL, *cells = NULL, *rate_cell_text = "0", *rate_depth_text = NULL;
     float rate_cell = 0.0f, rate_depth = 0.0f;   /* the reference leaves these uninitialised (src/main.c:293-294): pass -c and -r */
     int have_r = 0, have_c = 0;
     unsigned seed = 926;
@@ -199,7 +182,7 @@ static int cmd_bam2db(int argc, const char **argv)
         case 1: feat = v; break;
         case 2: bc = v; break;
         case 3: db = v; break;
-        case 4: rate_cell = strtof(v, NULL); have_c = 1; break;     /* OPT_FLOAT uses strtof (src/argparse.c:101-116) */
+        case 4: rate_cell = strtof(v, NULL); rate_cell_text = v; have_c = 1; break;     /* OPT_FLOAT uses strtof (src/argparse.c:101-116) */
         case 5: rate_depth = strtof(v, NULL); rate_depth_text = v; have_r = 1; break;
         case 6: out = v; break;
         case 7: seed = (unsigned)(int)strtol(v, NULL, 0); break;
@@ -223,8 +206,7 @@ static int cmd_bam2db(int argc, const char **argv)
     if (!feat || access(feat, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m feature file: %s does not exist.\n", feat ? feat : "(null)"); exit(1); }
     if (!bc || access(bc, F_OK) == -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m barcode file: %s does not exist.\n", bc ? bc : "(null)"); exit(1); }
     if (!db) { fprintf(stderr, "\x1b[31mError:\x1b[0m please name the database with -d.\n"); exit(1); }
-    if (cells) return cell_grid(bam, feat, bc, db, out, cells, depths, rate_depth, rate_depth_text, seed);
-    if (depths) return depth_sweep(bam, feat, bc, db, out, rate_cell, depths, seed);
+    if (cells || depths) return rate_sets(bam, feat, bc, db, out, cells, rate_cell, rate_cell_text, depths, rate_depth, rate_depth_text, seed);
     if (access(db, F_OK) != -1) { fprintf(stderr, "\x1b[31mError:\x1b[0m database: %s already exists, change the name of database in -d argument!\n", db); exit(1); }
     if (bam2db((char *)bam, (char *)db, (char *)out, (char *)bc, (char *)feat, rate_cell, rate_depth, seed)) { fprintf(stderr, "\x1b[31mError:\x1b[0m bam2db failed.\n"); return 1; }
     return 0;

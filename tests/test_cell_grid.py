@@ -12,15 +12,9 @@ import sys
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GOLD = os.path.join(ROOT, "tests", "golden")
-FILES = ["matrix.mtx.gz", "barcodes.tsv.gz", "features.tsv.gz"]
-KEYS = ("total", "cb_valid", "sampled", "valid", "nnz")
+from bam2db_harness import FILES, GOLD, KEYS, ROOT, bam2db_cases, bam_4m, cli_refusal, dup_barcodes, emu_cli, emu_lib, same_files, single_run, spawn  # noqa: F401 (fixtures)
+
 ARRAYS = ("m_gene", "m_cell", "m_count", "row_keys")
-
-
-def _bam2db_cases():
-    return [c for c in json.load(open(os.path.join(GOLD, "manifest.json")))["cases"] if c["kind"] == "bam2db"]
 
 
 def _grid_cells(rc):
@@ -36,27 +30,12 @@ def _grid_depths(rd):
     return [r for r in (0.7, 0.25) if r != rd][:1] + [rd]
 
 
-def _same_files(a, b, files):
-    return all(gzip.open(os.path.join(a, f), "rb").read() == gzip.open(os.path.join(b, f), "rb").read() for f in files)
-
-
 # ------------------------------------------------------------------------------------------------------------------------------
 # worker (runs under the emulator build)
 # ------------------------------------------------------------------------------------------------------------------------------
 def _imports():
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-
-
-def _single(cli, rc_, rate, seed, umi, where):
-    """one `-c rc_ -r rate` run (Python host or C CLI) from the current directory into `where`"""
-    import fastf_b200
-    os.makedirs(where)
-    if cli:
-        cmd = [cli, "bam2db", "-b", "in.bam", "-f", "features.tsv.gz", "-a", "barcodes.tsv.gz", "-d", os.path.join(where, "x.db"), "-c", str(rc_), "-r", str(rate), "-o", where, "-s", str(seed)]
-        assert subprocess.run(cmd + (["-u"] if umi else []), stdout=subprocess.DEVNULL).returncode == 0
-    else:
-        assert fastf_b200.bam2db("in.bam", os.path.join(where, "x.db"), where, "barcodes.tsv.gz", "features.tsv.gz", rc_, rate, seed) == 0
 
 
 def _grid(cli, cells, depths, seed, umi, out):
@@ -88,12 +67,12 @@ def _check_against_singles(cli, d, cells, depths, seed, umi, tmp, out, golden=No
         for j, r in enumerate(depths if isinstance(depths, list) else [depths]):
             got = os.path.join(out, "cell_" + str(c)) + ("/depth_" + str(r) if isinstance(depths, list) else "")
             if golden and (c, r) == golden[:2]:
-                assert _same_files(got, golden[2], files), (d, c, r)
+                assert same_files(got, golden[2], files), (d, c, r)
                 assert db_digest(os.path.join(got, "x.db")) == json.load(open(os.path.join(golden[2], "db_digest.json"))), (d, c, r)
                 continue
             want = os.path.join(tmp, "single_%d_%d" % (i, j))
-            _single(cli, c, r, seed, umi, want)
-            assert _same_files(got, want, files), (d, c, r)
+            single_run(cli, c, r, seed, umi, want)
+            assert same_files(got, want, files), (d, c, r)
             assert db_digest(os.path.join(got, "x.db")) == db_digest(os.path.join(want, "x.db")), (d, c, r)
             o = O.bam2db(os.path.join(os.getcwd(), "in.bam"), os.path.join(os.getcwd(), "barcodes.tsv.gz"), os.path.join(os.getcwd(), "features.tsv.gz"), c, r, seed)
             st, arr = api[i][j]
@@ -106,7 +85,7 @@ def _check_against_singles(cli, d, cells, depths, seed, umi, tmp, out, golden=No
 def _worker_golden(case_name, use_cli, tmp):
     _imports()
     from fastf_b200 import bam2db_host as B
-    c = {c["name"]: c for c in _bam2db_cases()}[case_name]
+    c = {c["name"]: c for c in bam2db_cases()}[case_name]
     d = os.path.join(GOLD, c["dir"])
     rc_, rd, seed, umi = c["rate_cell"], c["rate_depth"], c["seed"], bool(c.get("umicopies"))
     cli = os.environ.get("FASTF_EMU_CLI") if use_cli else None
@@ -119,32 +98,12 @@ def _worker_golden(case_name, use_cli, tmp):
     print("ok", case_name, "cli" if cli else "python")
 
 
-def _dup_barcodes(tmp, lib):
-    """synth4k with a barcode list that repeats one barcode: the seed is chosen (deterministically, by fastf_sample_cells through
-    Bam2dbInputs) so that the 0.5 table holds a barcode the 1.0 table lacks -- the 1.0 table stops at the repeated line"""
-    from fastf_b200 import bam2db_host as B
-    g = os.path.join(GOLD, "synth4k")
-    lines = gzip.decompress(open(os.path.join(g, "barcodes.tsv.gz"), "rb").read()).splitlines(keepends=True)
-    w = os.path.join(tmp, "dup")
-    os.makedirs(w)
-    with gzip.open(os.path.join(w, "barcodes.tsv.gz"), "wb") as f:
-        f.write(b"".join(lines[:20] + [lines[3]] + lines[20:]))
-    for x in ("in.bam", "features.tsv.gz"):
-        shutil.copy(os.path.join(g, x), w)
-    for seed in range(1, 1000):
-        small = B.Bam2dbInputs(lib, os.path.join(w, "barcodes.tsv.gz"), os.path.join(w, "features.tsv.gz"), 0.5, seed)
-        full = B.Bam2dbInputs(lib, os.path.join(w, "barcodes.tsv.gz"), os.path.join(w, "features.tsv.gz"), 1.0, seed)
-        if set(small.cells) - set(full.cells):
-            return w, seed
-    raise AssertionError("no seed below 1000 gives a 0.5 table with a barcode the 1.0 table lacks")
-
-
 def _worker_duplicates(use_cli, tmp):
     _imports()
     from fastf_b200 import _lib, bam2db_host as B
     cli = os.environ.get("FASTF_EMU_CLI") if use_cli else None
     B._umi_copies_flag = 1
-    w, seed = _dup_barcodes(tmp, _lib.load())
+    w, seed = dup_barcodes(tmp, _lib.load())
     os.chdir(w)
     cells, depths = [1.0, 0.5, 0.8], [0.6, 1.0]
     out = os.path.join(tmp, "grid")
@@ -217,7 +176,7 @@ def _worker_streaming(tmp):
         for c in cells:
             for r in depths:
                 a, b = os.path.join(w, "cut", "cell_%s" % c, "depth_%s" % r), os.path.join(w, "orig", "cell_%s" % c, "depth_%s" % r)
-                assert _same_files(a, b, FILES + ["umi.tsv.gz"]), (d, c, r)
+                assert same_files(a, b, FILES + ["umi.tsv.gz"]), (d, c, r)
                 assert db_digest(os.path.join(a, "x.db")) == db_digest(os.path.join(b, "x.db")), (d, c, r)
         print("ok", d)
     ctx.close()
@@ -297,57 +256,37 @@ def _worker_library_refusals():
 # ------------------------------------------------------------------------------------------------------------------------------
 # CPU tests (emulator build)
 # ------------------------------------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def emu_lib():
-    from fastf_b200 import build
-    return build.build_emu()
-
-
-@pytest.fixture(scope="module")
-def emu_cli(emu_lib):
-    from fastf_b200 import build
-    return build.build_cli(emu=True)
-
-
-def _spawn(emu_lib, args, cli=None):
-    env = dict(os.environ, FASTF_GPU_LIB=emu_lib)
-    if cli:
-        env["FASTF_EMU_CLI"] = cli
-    r = subprocess.run([sys.executable, os.path.abspath(__file__)] + args, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
-    assert r.returncode == 0 and "ok " in r.stdout, r.stdout[-3000:]
-
-
-@pytest.mark.parametrize("case", [c["name"] for c in _bam2db_cases()])
+@pytest.mark.parametrize("case", [c["name"] for c in bam2db_cases()])
 def test_emu_grid_reproduces_golden_python(emu_lib, case, tmp_path):
     """every golden bam2db case as one set of an unsorted grid with cell rate 1.0 and a smaller one (Python host): that set equals the
     reference's recorded files and tables, every other set equals the single-rate run (files, tables) and the oracle (counters, COO)"""
-    _spawn(emu_lib, ["golden", case, "python", str(tmp_path)])
+    spawn(__file__, emu_lib, ["golden", case, "python", str(tmp_path)])
 
 
-@pytest.mark.parametrize("case", [c["name"] for c in _bam2db_cases()])
+@pytest.mark.parametrize("case", [c["name"] for c in bam2db_cases()])
 def test_emu_grid_reproduces_golden_cli(emu_lib, emu_cli, case, tmp_path):
     """the same through `fastF bam2db --cells --depths` (C host), -u where the golden case has it"""
-    _spawn(emu_lib, ["golden", case, "cli", str(tmp_path)], cli=emu_cli)
+    spawn(__file__, emu_lib, ["golden", case, "cli", str(tmp_path)], cli=emu_cli)
 
 
 @pytest.mark.parametrize("host", ["python", "cli"])
 def test_emu_grid_duplicate_barcodes(emu_lib, emu_cli, host, tmp_path):
     """a smaller cell rate's table holds a barcode the largest rate's table lacks: the union of the tables, not the largest one"""
-    _spawn(emu_lib, ["duplicates", host, str(tmp_path)], cli=emu_cli if host == "cli" else None)
+    spawn(__file__, emu_lib, ["duplicates", host, str(tmp_path)], cli=emu_cli if host == "cli" else None)
 
 
 @pytest.mark.parametrize("host", ["python", "cli"])
 def test_emu_grid_edge_cell_rates(emu_lib, emu_cli, host, tmp_path):
     """a cell rate that samples no cell, 1.0 next to 0.99, one depth rate (-r: OUT/cell_<c>/)"""
-    _spawn(emu_lib, ["edge", host, str(tmp_path)], cli=emu_cli if host == "cli" else None)
+    spawn(__file__, emu_lib, ["edge", host, str(tmp_path)], cli=emu_cli if host == "cli" else None)
 
 
 def test_emu_grid_streamed_and_straddling(emu_lib, tmp_path):
-    _spawn(emu_lib, ["streaming", str(tmp_path)])
+    spawn(__file__, emu_lib, ["streaming", str(tmp_path)])
 
 
 def test_emu_grid_library_refusals(emu_lib):
-    _spawn(emu_lib, ["refusals"])
+    spawn(__file__, emu_lib, ["refusals"])
 
 
 @pytest.mark.parametrize("extra,needle", [
@@ -364,34 +303,16 @@ def test_emu_grid_library_refusals(emu_lib):
 ])
 def test_emu_cli_grid_refusals(emu_cli, tmp_path, extra, needle):
     """refused before any work (no device job, no database written, no output directory made)"""
-    env = dict(os.environ)
-    env.pop("FASTF_GPUS", None)
-    for x in [x for x in extra if "=" in x]:
-        extra.remove(x)
-        env[x.split("=")[0]] = x.split("=")[1]
-    g = os.path.join(GOLD, "synth4k")
     if needle == "already exists":
         where = tmp_path / "out" / "cell_0.4" / ("depth_0.2" if "--depths" in extra else "")
         os.makedirs(where, exist_ok=True)
         open(where / "x.db", "wb").close()
-    cmd = [emu_cli, "bam2db", "-b", os.path.join(g, "in.bam"), "-f", os.path.join(g, "features.tsv.gz"), "-a", os.path.join(g, "barcodes.tsv.gz"), "-d", "x.db",
-           "-o", str(tmp_path / "out")] + extra
-    r = subprocess.run(cmd, cwd=tmp_path, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
-    assert r.returncode == 1 and needle in r.stderr, (r.returncode, r.stderr)
-    assert not os.path.exists(tmp_path / "out" / "cell_0.2"), "a refused grid created an output directory"
-    assert not os.path.exists(tmp_path / "x.db")
+    cli_refusal(emu_cli, tmp_path, extra, needle, tmp_path / "out" / "cell_0.2")
 
 
 # ------------------------------------------------------------------------------------------------------------------------------
 # B200
 # ------------------------------------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def bam_4m(tmp_path_factory, synth):
-    d = str(tmp_path_factory.mktemp("grid4m"))
-    paths, st = synth.write_bam_set(d, n_reads=4_000_000, n_cells=3000, n_genes=20000, seed=11, p_umi_n=0.01, n_molecules=1_500_000)
-    return paths
-
-
 @pytest.mark.gpu
 def test_gpu_grid_equals_single_rate_jobs(gpu_ctx, bam_4m, oracle):
     """about 4 M reads in several chunks, cell rates {0.25, 0.5, 0.8, 1.0} x depths {0.1, 0.3, 0.5, 0.7, 1.0} (unsorted): every set's

@@ -11,24 +11,13 @@ import sys
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GOLD = os.path.join(ROOT, "tests", "golden")
-FILES = ["matrix.mtx.gz", "barcodes.tsv.gz", "features.tsv.gz"]
-KEYS = ("total", "cb_valid", "sampled", "valid", "nnz")
-
-
-def _bam2db_cases():
-    return [c for c in json.load(open(os.path.join(GOLD, "manifest.json")))["cases"] if c["kind"] == "bam2db"]
+from bam2db_harness import FILES, GOLD, KEYS, ROOT, bam2db_cases, bam_4m, cli_refusal, emu_cli, emu_lib, same_files, single_run, spawn  # noqa: F401 (fixtures)
 
 
 def _sweep_rates(rd):
     """the golden rate among others, unsorted, golden rate second"""
     others = [r for r in (0.7, 0.0, 1.0, 0.25) if r != rd]
     return [others[0], rd] + others[1:3]
-
-
-def _same_files(a, b, files):
-    return all(gzip.open(os.path.join(a, f), "rb").read() == gzip.open(os.path.join(b, f), "rb").read() for f in files)
 
 
 # ------------------------------------------------------------------------------------------------------------------------------
@@ -41,7 +30,7 @@ def _worker_golden(case_name, use_cli, tmp):
     from fastf_b200 import _lib, bam2db_host as B
     from dbdigest import db_digest
     import oracle_binding
-    c = {c["name"]: c for c in _bam2db_cases()}[case_name]
+    c = {c["name"]: c for c in bam2db_cases()}[case_name]
     d = os.path.join(GOLD, c["dir"])
     rc_, rd, seed, umi = c["rate_cell"], c["rate_depth"], c["seed"], bool(c.get("umicopies"))
     rates = _sweep_rates(rd)
@@ -49,14 +38,6 @@ def _worker_golden(case_name, use_cli, tmp):
     cli = os.environ.get("FASTF_EMU_CLI") if use_cli else None
     B._umi_copies_flag = 1 if umi else 0
     os.chdir(d)   # the matrix header records the BAM path as passed: the golden run used "in.bam"
-
-    def single(rate, where):
-        os.makedirs(where)
-        if cli:
-            cmd = [cli, "bam2db", "-b", "in.bam", "-f", "features.tsv.gz", "-a", "barcodes.tsv.gz", "-d", os.path.join(where, "x.db"), "-c", str(rc_), "-r", str(rate), "-o", where, "-s", str(seed)]
-            assert subprocess.run(cmd + (["-u"] if umi else []), stdout=subprocess.DEVNULL).returncode == 0
-        else:
-            assert fastf_b200.bam2db("in.bam", os.path.join(where, "x.db"), where, "barcodes.tsv.gz", "features.tsv.gz", rc_, rate, seed) == 0
 
     out = os.path.join(tmp, "sweep")
     if cli:
@@ -74,12 +55,12 @@ def _worker_golden(case_name, use_cli, tmp):
         got = os.path.join(out, "depth_" + str(rate))
         if rate == rd:
             want = os.path.join(d, c["expect"])
-            assert _same_files(got, want, files), (case_name, rate)
+            assert same_files(got, want, files), (case_name, rate)
             assert db_digest(os.path.join(got, "x.db")) == json.load(open(os.path.join(want, "db_digest.json"))), (case_name, rate)
         else:
             want = os.path.join(tmp, "single_%d" % k)
-            single(rate, want)
-            assert _same_files(got, want, files), (case_name, rate)
+            single_run(cli, rc_, rate, seed, umi, want)
+            assert same_files(got, want, files), (case_name, rate)
             assert db_digest(os.path.join(got, "x.db")) == db_digest(os.path.join(want, "x.db")), (case_name, rate)
             o = O.bam2db(os.path.join(d, "in.bam"), os.path.join(d, "barcodes.tsv.gz"), os.path.join(d, "features.tsv.gz"), rc_, rate, seed)
             st, arr = api[k]
@@ -127,9 +108,9 @@ def _worker_streaming(tmp):
         assert fastf_b200.bam2db_sweep("in.bam", "x.db", os.path.join(w, "orig"), "barcodes.tsv.gz", "features.tsv.gz", rc_, rates, 926, ctx=ctx) == 0
         for r in rates:
             a, b = os.path.join(w, "cut", "depth_%s" % r), os.path.join(w, "orig", "depth_%s" % r)
-            assert _same_files(a, b, ["barcodes.tsv.gz", "features.tsv.gz", "umi.tsv.gz"]), (d, r)
+            assert same_files(a, b, ["barcodes.tsv.gz", "features.tsv.gz", "umi.tsv.gz"]), (d, r)
             # the matrix header names the BAM as passed ("in.bam" both times): identical too
-            assert _same_files(a, b, ["matrix.mtx.gz"]), (d, r)
+            assert same_files(a, b, ["matrix.mtx.gz"]), (d, r)
             assert db_digest(os.path.join(a, "x.db")) == db_digest(os.path.join(b, "x.db")), (d, r)
         print("ok", d)
     ctx.close()
@@ -167,46 +148,26 @@ def _worker_skewed():
 # ------------------------------------------------------------------------------------------------------------------------------
 # CPU tests (emulator build)
 # ------------------------------------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def emu_lib():
-    from fastf_b200 import build
-    return build.build_emu()
-
-
-@pytest.fixture(scope="module")
-def emu_cli(emu_lib):
-    from fastf_b200 import build
-    return build.build_cli(emu=True)
-
-
-def _spawn(emu_lib, args, cli=None):
-    env = dict(os.environ, FASTF_GPU_LIB=emu_lib)
-    if cli:
-        env["FASTF_EMU_CLI"] = cli
-    r = subprocess.run([sys.executable, os.path.abspath(__file__)] + args, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=1500)
-    assert r.returncode == 0 and "ok " in r.stdout, r.stdout[-3000:]
-
-
-@pytest.mark.parametrize("case", [c["name"] for c in _bam2db_cases()])
+@pytest.mark.parametrize("case", [c["name"] for c in bam2db_cases()])
 def test_emu_sweep_reproduces_golden_python(emu_lib, case, tmp_path):
     """every golden bam2db case as one rate of an unsorted sweep (Python host): that rate equals the reference's recorded files and
     tables, every other rate equals the single-rate run (files, tables) and the oracle (counters, COO)"""
-    _spawn(emu_lib, ["golden", case, "python", str(tmp_path)])
+    spawn(__file__, emu_lib, ["golden", case, "python", str(tmp_path)])
 
 
-@pytest.mark.parametrize("case", [c["name"] for c in _bam2db_cases()])
+@pytest.mark.parametrize("case", [c["name"] for c in bam2db_cases()])
 def test_emu_sweep_reproduces_golden_cli(emu_lib, emu_cli, case, tmp_path):
     """the same through `fastF bam2db --depths` (C host), -u where the golden case has it"""
-    _spawn(emu_lib, ["golden", case, "cli", str(tmp_path)], cli=emu_cli)
+    spawn(__file__, emu_lib, ["golden", case, "cli", str(tmp_path)], cli=emu_cli)
 
 
 def test_emu_sweep_streamed_and_straddling(emu_lib, tmp_path):
-    _spawn(emu_lib, ["streaming", str(tmp_path)])
+    spawn(__file__, emu_lib, ["streaming", str(tmp_path)])
 
 
 def test_emu_sweep_long_groups(emu_lib):
     """two cells x two genes: (cell, gene) groups of thousands of UMIs, read by fastf_group_rate_kernel in many warp steps"""
-    _spawn(emu_lib, ["skewed"])
+    spawn(__file__, emu_lib, ["skewed"])
 
 
 @pytest.mark.parametrize("extra,needle", [
@@ -216,24 +177,14 @@ def test_emu_sweep_long_groups(emu_lib):
     (["--depths", "0.1,0.2", "--gpus", "2"], "one GPU"),
     (["--depths", "0.1,0.2"], "already exists"),
     (["--depths", "0.1,0.2", "--gpus", "1", "FASTF_GPUS=2"], "one GPU"),
+    (["-c", "1.5", "--depths", "0.1,0.2"], "Sample size must be smaller"),
 ])
 def test_emu_cli_sweep_refusals(emu_cli, tmp_path, extra, needle):
     """refused before any work (no device job, no database written, no output directory made)"""
-    env = dict(os.environ)
-    env.pop("FASTF_GPUS", None)
-    for x in [x for x in extra if "=" in x]:
-        extra.remove(x)
-        env[x.split("=")[0]] = x.split("=")[1]
-    g = os.path.join(GOLD, "synth4k")
     os.makedirs(tmp_path / "out" / "depth_0.2")
     if needle == "already exists":
         open(tmp_path / "out" / "depth_0.2" / "x.db", "wb").close()
-    cmd = [emu_cli, "bam2db", "-b", os.path.join(g, "in.bam"), "-f", os.path.join(g, "features.tsv.gz"), "-a", os.path.join(g, "barcodes.tsv.gz"), "-d", "x.db", "-c", "1.0",
-           "-o", str(tmp_path / "out")] + extra
-    r = subprocess.run(cmd, cwd=tmp_path, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
-    assert r.returncode == 1 and needle in r.stderr, (r.returncode, r.stderr)
-    assert not os.path.exists(tmp_path / "out" / "depth_0.1"), "a refused sweep created an output directory"
-    assert not os.path.exists(tmp_path / "x.db")
+    cli_refusal(emu_cli, tmp_path, ["-c", "1.0"] + extra, needle, tmp_path / "out" / "depth_0.1")
 
 
 # ------------------------------------------------------------------------------------------------------------------------------
@@ -249,13 +200,6 @@ def _single_and_sweep(ctx, bam, inputs, rates, seed):
         for k in ("m_gene", "m_cell", "m_count", "row_keys"):
             assert np.array_equal(arr[k], arr1[k]), (r, k)
     return sweep
-
-
-@pytest.fixture(scope="module")
-def bam_4m(tmp_path_factory, synth):
-    d = str(tmp_path_factory.mktemp("sweep4m"))
-    paths, st = synth.write_bam_set(d, n_reads=4_000_000, n_cells=3000, n_genes=20000, seed=11, p_umi_n=0.01, n_molecules=1_500_000)
-    return paths
 
 
 @pytest.mark.gpu
