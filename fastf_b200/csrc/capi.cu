@@ -15,6 +15,10 @@
 // contract; capi_launch.cuh (engines, string tables, block index), capi_bam2db.cuh (the job), capi_blocks.cuh (building blocks for
 // multi-GPU hosts, single-kernel wrappers), capi_freq.cuh and capi_taghist.cuh are included at the end, in that order.  The
 // one-process multi-GPU driver is a separate unit on top of the public C-ABI (sharded.cu).
+//
+// Resources free themselves: a DevBuf / PinBuf gives its allocation back to the context's pool when it is destroyed, an Event destroys
+// its CUDA event, and the structs made of them (the job, its chunk slots, the scratch sets) need no release code.  A function that owns
+// buffers declares a DrainOnExit after them, so that none goes back to a pool while queued work can still touch it.
 #include "../../include/fastf_gpu.h"
 #include "common.cuh"
 #include "bgzf_index.h"
@@ -118,17 +122,54 @@ static size_t pool_cap_of(const std::vector<PoolEntry> &pool, size_t bytes)
         if (e.cap >= bytes && (!best || e.cap < best)) best = e.cap;
     return best;
 }
-struct DevBuf {
+// A device (DevBuf) or pinned (PinBuf) buffer that goes back to the pool of the context it was reserved on when it is destroyed or
+// released.  Move-only, so that exactly one owner gives it back.
+template <std::vector<PoolEntry> *fastf_ctx::*Pool> struct PoolBuf {
+    fastf_ctx *ctx = nullptr;   // set by the first dev_reserve / pin_reserve
     void *p = nullptr;
     size_t cap = 0;
+    PoolBuf() = default;
+    PoolBuf(const PoolBuf &) = delete;
+    PoolBuf &operator=(const PoolBuf &) = delete;
+    PoolBuf(PoolBuf &&o) noexcept : ctx(o.ctx), p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    PoolBuf &operator=(PoolBuf &&o) noexcept
+    {
+        if (this != &o) { release(); ctx = o.ctx; p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
+    ~PoolBuf() { release(); }
+    void release()
+    {
+        if (p) (ctx->*Pool)->push_back(PoolEntry{p, cap});
+        p = nullptr;
+        cap = 0;
+    }
     template <class T> T *as() const { return (T *)p; }
 };
-static void dev_release(fastf_ctx *ctx, DevBuf &b)
-{
-    if (b.p) ctx->dev_pool->push_back(PoolEntry{b.p, b.cap});
-    b.p = nullptr;
-    b.cap = 0;
-}
+using DevBuf = PoolBuf<&fastf_ctx::dev_pool>;
+using PinBuf = PoolBuf<&fastf_ctx::pin_pool>;
+
+struct DrainOnExit {   // declared after a function's buffers, so that it drains the streams before any of them goes back to the pool
+    fastf_ctx *ctx;
+    ~DrainOnExit() { cudaStreamSynchronize(ctx->compute); cudaStreamSynchronize(ctx->copy); cudaStreamSynchronize(ctx->infl); cudaStreamSynchronize(ctx->mt); }
+};
+
+struct Event {   // a CUDA event, destroyed with its holder (the driver frees a recorded event once its work has completed)
+    cudaEvent_t e = nullptr;
+    Event() = default;
+    Event(const Event &) = delete;
+    Event &operator=(const Event &) = delete;
+    Event(Event &&o) noexcept : e(o.e) { o.e = nullptr; }
+    Event &operator=(Event &&o) noexcept
+    {
+        if (this != &o) { if (e) cudaEventDestroy(e); e = o.e; o.e = nullptr; }
+        return *this;
+    }
+    ~Event() { if (e) cudaEventDestroy(e); }
+    cudaError_t create(unsigned flags = 0) { return cudaEventCreateWithFlags(&e, flags); }   // 0: cudaEventDefault, with timing
+    operator cudaEvent_t() const { return e; }
+};
+
 static int dev_reserve(fastf_ctx *ctx, DevBuf &b, size_t bytes, size_t keep_bytes = 0, cudaStream_t s = 0)
 {
     if (bytes <= b.cap) return 0;
@@ -145,22 +186,12 @@ static int dev_reserve(fastf_ctx *ctx, DevBuf &b, size_t bytes, size_t keep_byte
         CK(cudaStreamSynchronize(ctx->copy));
         CK(cudaStreamSynchronize(ctx->infl));
         CK(cudaStreamSynchronize(ctx->mt));
-        dev_release(ctx, b);
+        b.release();
     }
+    b.ctx = ctx;
     b.p = np;
     b.cap = ncap;
     return 0;
-}
-struct PinBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    template <class T> T *as() const { return (T *)p; }
-};
-static void pin_release(fastf_ctx *ctx, PinBuf &b)
-{
-    if (b.p) ctx->pin_pool->push_back(PoolEntry{b.p, b.cap});
-    b.p = nullptr;
-    b.cap = 0;
 }
 static int pin_reserve(fastf_ctx *ctx, PinBuf &b, size_t bytes)
 {
@@ -172,8 +203,9 @@ static int pin_reserve(fastf_ctx *ctx, PinBuf &b, size_t bytes)
         CK(cudaStreamSynchronize(ctx->copy));
         CK(cudaStreamSynchronize(ctx->infl));
         CK(cudaStreamSynchronize(ctx->mt));
-        pin_release(ctx, b);
+        b.release();
     }
+    b.ctx = ctx;
     size_t pc = pool_cap_of(*ctx->pin_pool, ncap);
     if (pc && pc <= 2 * ncap + (1u << 20)) { b.p = pool_take(*ctx->pin_pool, ncap); b.cap = pc; }
     if (!b.p) { CK(cudaMallocHost(&b.p, ncap)); b.cap = ncap; }
@@ -217,31 +249,28 @@ static int d2h_pageable(fastf_ctx *ctx, void *dst, const void *src_dev, size_t b
         return 0;
     }
     PinBuf bounce[2];
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    int rc = 0;
-    for (int k = 0; k < 2 && !rc; k++) { rc = pin_reserve(ctx, bounce[k], PIECE); if (!rc && cudaEventCreateWithFlags(&ev[k], cudaEventDisableTiming) != cudaSuccess) rc = ctx_fail(ctx, "d2h: event creation failed"); }
+    Event ev[2];
+    DrainOnExit drain{ctx};
+    for (int k = 0; k < 2; k++) { TRY(pin_reserve(ctx, bounce[k], PIECE)); if (ev[k].create(cudaEventDisableTiming) != cudaSuccess) return ctx_fail(ctx, "d2h: event creation failed"); }
     const size_t n_pieces = (bytes + PIECE - 1) / PIECE;
-    for (size_t k = 0; k <= n_pieces && !rc; k++) {
+    for (size_t k = 0; k <= n_pieces; k++) {
         if (k < n_pieces) {
             const size_t o = k * PIECE, m = std::min(PIECE, bytes - o);
-            if (cudaMemcpyAsync(bounce[k & 1].p, (const u8 *)src_dev + o, m, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaEventRecord(ev[k & 1], s) != cudaSuccess) rc = ctx_fail(ctx, "d2h: copy failed");
+            if (cudaMemcpyAsync(bounce[k & 1].p, (const u8 *)src_dev + o, m, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaEventRecord(ev[k & 1], s) != cudaSuccess) return ctx_fail(ctx, "d2h: copy failed");
         }
-        if (k > 0 && !rc) {
+        if (k > 0) {
             const size_t o = (k - 1) * PIECE, m = std::min(PIECE, bytes - o);
-            if (cudaEventSynchronize(ev[(k - 1) & 1]) != cudaSuccess) rc = ctx_fail(ctx, "d2h: copy failed");
-            else par_memcpy((u8 *)dst + o, bounce[(k - 1) & 1].p, m);
+            if (cudaEventSynchronize(ev[(k - 1) & 1]) != cudaSuccess) return ctx_fail(ctx, "d2h: copy failed");
+            par_memcpy((u8 *)dst + o, bounce[(k - 1) & 1].p, m);
         }
     }
-    cudaStreamSynchronize(s);
-    for (int k = 0; k < 2; k++) { if (ev[k]) cudaEventDestroy(ev[k]); pin_release(ctx, bounce[k]); }
-    return rc;
+    return 0;
 }
 
 struct Timer {   // CUDA-event stopwatch on one stream; accumulates into *acc at collect()
-    cudaEvent_t a = nullptr, b = nullptr;
+    Event a, b;
     bool armed = false;
-    int init() { return cudaEventCreate(&a) != cudaSuccess || cudaEventCreate(&b) != cudaSuccess; }
-    void destroy() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); a = b = nullptr; }
+    int init() { return a.create() != cudaSuccess || b.create() != cudaSuccess; }
     void start(cudaStream_t s) { cudaEventRecord(a, s); }
     void stop(cudaStream_t s) { cudaEventRecord(b, s); armed = true; }
     void collect(float *acc) { if (armed) { float ms = 0; cudaEventSynchronize(b); cudaEventElapsedTime(&ms, a, b); *acc += ms; armed = false; } }

@@ -15,9 +15,9 @@ struct ChunkSlot {
     DevBuf virt;          // FASTF_BAM_STRADDLE: record-start guesses and virtual blocks
     DevBuf infl;          // inflated bytes of the chunk (double buffered: chunk i+1 inflates while chunk i is parsed)
     DeScratch de;
-    cudaEvent_t ev_infl = nullptr, ev_gather = nullptr;
+    Event ev_infl, ev_gather;
     PinBuf snap;          // counters snapshot {n_records, n_candidates, status_or, chunk_candidates}
-    cudaEvent_t ev_copy = nullptr, ev_done = nullptr;
+    Event ev_copy, ev_done;
     u32 nblocks = 0;
     bool pending = false; // parse launched, gather not yet
 };
@@ -33,13 +33,13 @@ struct fastf_bam2db_job {
     u32 next_slot = 0;
     // compressed bytes of host-fed chunks: a ring of three, so that the copy of chunk i is issued before the host waits for
     // anything and overlaps the inflate of chunks i-2 and i-1
-    struct CompRing { DevBuf buf; cudaEvent_t ev_copy = nullptr, ev_free = nullptr; bool used = false; } comp_ring[3];
+    struct CompRing { DevBuf buf; Event ev_copy, ev_free; bool used = false; } comp_ring[3];
     u32 comp_seq = 0;
     u64 ring_estimate = 0;
     // FASTF_FEED_TIMING=1: where a host-fed job spends its time (stderr at finish): H2D copies by CUDA events, host waits by wall clock
     bool feed_timing = false;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ft_copy_ev, ft_infl_ev;
-    std::vector<cudaEvent_t> ft_parse_ev;
+    std::vector<std::pair<Event, Event>> ft_copy_ev, ft_infl_ev;
+    std::vector<Event> ft_parse_ev;
     std::vector<double> ft_host_submit;
     u64 ft_copy_bytes = 0;
     double ft_wait_s = 0, ft_index_s = 0, ft_feed_s = 0;
@@ -65,7 +65,7 @@ struct fastf_bam2db_job {
     std::vector<u8> carry;    // partial BGZF block left over by fastf_bam2db_feed
     // MT19937 keep bits from the job's first draw on (the depth sweep: tempered words, one u32 per draw)
     DevBuf keepbits, mt_states, mt_scratch;
-    cudaEvent_t ev_mt = nullptr;
+    Event ev_mt;
     // sampling / sort / count
     bool sampled_done = false;
     u32 sweep_rates = 0;          // sampled by the depth sweep at this many rates (0: at the job's one rate)
@@ -86,7 +86,7 @@ struct fastf_bam2db_job {
     u64 n_blocks_fed = 0, n_blocks_done = 0;   // blocks handed to run_blocks / blocks whose candidate counts have come back
     u32 launches0 = 0, n_chunks = 0;
     Timer t_infl[2], t_crc[2], t_parse[2], t_gather[2], t_mt, t_sample, t_sort, t_count;
-    cudaEvent_t ev_first = nullptr, ev_last = nullptr;
+    Event ev_first, ev_last;
     bool first_recorded = false;
     float ms_inflate = 0, ms_crc = 0, ms_parse = 0, ms_gather = 0, ms_mt = 0, ms_sample = 0, ms_sort = 0, ms_count = 0;
 };
@@ -98,39 +98,13 @@ extern "C" void fastf_bam2db_job_free(fastf_bam2db_job *job)
     if (!job) return;
     fastf_ctx *ctx = job->ctx;
     cudaSetDevice(ctx->device);
+    // the job's buffers go back to the pools when it is deleted: nothing queued may still touch them
     cudaStreamSynchronize(ctx->compute);
     cudaStreamSynchronize(ctx->copy);
     cudaStreamSynchronize(ctx->infl);
     cudaStreamSynchronize(ctx->mt);
-    for (int i = 0; i < 2; i++) {
-        ChunkSlot &S = job->slot[i];
-        index_release(ctx, S.idx); dev_release(ctx, S.stage); dev_release(ctx, S.virt); dev_release(ctx, S.infl); dev_release(ctx, S.de.counter); dev_release(ctx, S.de.sorted); pin_release(ctx, S.snap);
-        if (S.ev_copy) cudaEventDestroy(S.ev_copy);
-        if (S.ev_infl) cudaEventDestroy(S.ev_infl);
-        if (S.ev_gather) cudaEventDestroy(S.ev_gather);
-        if (S.ev_done) cudaEventDestroy(S.ev_done);
-        job->t_infl[i].destroy(); job->t_crc[i].destroy(); job->t_parse[i].destroy(); job->t_gather[i].destroy();
-    }
     ctx->hint_cand = std::max(ctx->hint_cand, job->cand.cap);
     for (auto &R : job->comp_ring) ctx->hint_ring = std::max(ctx->hint_ring, R.buf.cap);
-    for (auto &R : job->comp_ring) {
-        dev_release(ctx, R.buf);
-        if (R.ev_copy) cudaEventDestroy(R.ev_copy);
-        if (R.ev_free) cudaEventDestroy(R.ev_free);
-    }
-    job->t_mt.destroy(); job->t_sample.destroy(); job->t_sort.destroy(); job->t_count.destroy();
-    if (job->ev_mt) cudaEventDestroy(job->ev_mt);
-    if (job->ev_first) cudaEventDestroy(job->ev_first);
-    if (job->ev_last) cudaEventDestroy(job->ev_last);
-    dev_release(ctx, job->cells.slots); dev_release(ctx, job->cells.pool); dev_release(ctx, job->genes.slots); dev_release(ctx, job->genes.pool);
-    dev_release(ctx, job->counters); dev_release(ctx, job->hdr_off); dev_release(ctx, job->cand); dev_release(ctx, job->keepbits); dev_release(ctx, job->mt_states); dev_release(ctx, job->mt_scratch);
-    dev_release(ctx, job->tile_valid); dev_release(ctx, job->tile_tot); dev_release(ctx, job->sample_counters); dev_release(ctx, job->kept); dev_release(ctx, job->orand);
-    dev_release(ctx, job->kept_rate); dev_release(ctx, job->rate_alt);
-    dev_release(ctx, job->grid_remap); dev_release(ctx, job->grid_cand);
-    pin_release(ctx, job->small_host);
-    sort_scratch_release(ctx, job->sortS);
-    rle_scratch_release(ctx, job->rleS);
-    rle_scratch_release(ctx, job->rateS);
     delete job;
 }
 
@@ -180,19 +154,19 @@ extern "C" int fastf_bam2db_begin(fastf_ctx *ctx, const fastf_bam2db_params *p, 
     rc = rc || pin_reserve(ctx, job->small_host, 2 * FASTF_SWEEP_MAX_RATES * sizeof(u64));
     for (int i = 0; i < 2 && !rc; i++) {
         rc = rc || pin_reserve(ctx, job->slot[i].snap, 4 * sizeof(u64));
-        rc = rc || cudaEventCreateWithFlags(&job->slot[i].ev_copy, cudaEventDisableTiming) != cudaSuccess;
-        rc = rc || cudaEventCreateWithFlags(&job->slot[i].ev_done, cudaEventDisableTiming) != cudaSuccess;
-        rc = rc || cudaEventCreateWithFlags(&job->slot[i].ev_infl, cudaEventDisableTiming) != cudaSuccess;
-        rc = rc || cudaEventCreateWithFlags(&job->slot[i].ev_gather, cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || job->slot[i].ev_copy.create(cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || job->slot[i].ev_done.create(cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || job->slot[i].ev_infl.create(cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || job->slot[i].ev_gather.create(cudaEventDisableTiming) != cudaSuccess;
         rc = rc || job->t_infl[i].init() || job->t_crc[i].init() || job->t_parse[i].init() || job->t_gather[i].init();
     }
     for (auto &R : job->comp_ring) {
-        rc = rc || cudaEventCreateWithFlags(&R.ev_copy, cudaEventDisableTiming) != cudaSuccess;
-        rc = rc || cudaEventCreateWithFlags(&R.ev_free, cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || R.ev_copy.create(cudaEventDisableTiming) != cudaSuccess;
+        rc = rc || R.ev_free.create(cudaEventDisableTiming) != cudaSuccess;
     }
     rc = rc || job->t_mt.init() || job->t_sample.init() || job->t_sort.init() || job->t_count.init();
-    rc = rc || cudaEventCreateWithFlags(&job->ev_mt, cudaEventDisableTiming) != cudaSuccess;
-    rc = rc || cudaEventCreate(&job->ev_first) != cudaSuccess || cudaEventCreate(&job->ev_last) != cudaSuccess;
+    rc = rc || job->ev_mt.create(cudaEventDisableTiming) != cudaSuccess;
+    rc = rc || job->ev_first.create() != cudaSuccess || job->ev_last.create() != cudaSuccess;
     if (!rc) rc = cudaMemsetAsync(job->counters.p, 0, 4 * sizeof(u64), ctx->compute) != cudaSuccess;
     job->header_done = p->headerless != 0;
 
@@ -345,11 +319,11 @@ static int run_chunk(fastf_bam2db_job *job, const FastfBgzfBlock *blocks, u32 nb
     TRY(index_upload(ctx, S.idx, ctx->infl));
     job->t_infl[si].collect(&job->ms_inflate);
     job->t_infl[si].start(ctx->infl);
-    cudaEvent_t fti0 = nullptr, fti1 = nullptr;
-    if (job->feed_timing && ring) { CK(cudaEventCreate(&fti0)); CK(cudaEventCreate(&fti1)); CK(cudaEventRecord(fti0, ctx->infl)); job->ft_host_submit.push_back(wall_seconds()); }
+    std::pair<Event, Event> fti;
+    if (job->feed_timing && ring) { CK(fti.first.create()); CK(fti.second.create()); CK(cudaEventRecord(fti.first, ctx->infl)); job->ft_host_submit.push_back(wall_seconds()); }
     TRY(launch_inflate(ctx, job->lanes, comp_dev, comp_total, S.idx.in_off, S.idx.in_len, S.idx.out_off, S.idx.isize, nb, S.infl.as<u8>(), S.idx.st_infl, ctx->infl, &S.de, S.idx.h_in_off,
                        S.idx.h_in_len, S.idx.h_out_off, S.idx.h_isize));
-    if (fti0) { CK(cudaEventRecord(fti1, ctx->infl)); job->ft_infl_ev.push_back({fti0, fti1}); }
+    if (fti.first) { CK(cudaEventRecord(fti.second, ctx->infl)); job->ft_infl_ev.push_back(std::move(fti)); }
     job->t_infl[si].stop(ctx->infl);
     CK(cudaEventRecord(S.ev_infl, ctx->infl));
     CK(cudaStreamWaitEvent(ctx->compute, S.ev_infl, 0));
@@ -384,7 +358,7 @@ static int run_chunk(fastf_bam2db_job *job, const FastfBgzfBlock *blocks, u32 nb
     job->t_parse[si].stop(ctx->compute);
     CK(cudaMemcpyAsync(S.snap.p, job->counters.p, 4 * sizeof(u64), cudaMemcpyDeviceToHost, ctx->compute));
     CK(cudaEventRecord(S.ev_done, ctx->compute));
-    if (job->feed_timing && ring) { cudaEvent_t e = nullptr; CK(cudaEventCreate(&e)); CK(cudaEventRecord(e, ctx->compute)); job->ft_parse_ev.push_back(e); }
+    if (job->feed_timing && ring) { Event e; CK(e.create()); CK(cudaEventRecord(e, ctx->compute)); job->ft_parse_ev.push_back(std::move(e)); }
     S.nblocks = nb;
     S.pending = true;
     job->n_blocks += nb;
@@ -426,10 +400,10 @@ static int stage_host_bytes(fastf_bam2db_job *job, const u8 *host_base, u64 lo, 
     u64 want = P.fill + padded + 16;
     if (want > P.ring->buf.cap) want = std::max<u64>(want, std::max<u64>(ctx->hint_ring, job->ring_estimate));
     TRY(dev_reserve(ctx, P.ring->buf, want, P.fill, ctx->copy));
-    cudaEvent_t ft0 = nullptr, ft1 = nullptr;
-    if (job->feed_timing) { CK(cudaEventCreate(&ft0)); CK(cudaEventCreate(&ft1)); CK(cudaEventRecord(ft0, ctx->copy)); }
+    std::pair<Event, Event> ft;
+    if (job->feed_timing) { CK(ft.first.create()); CK(ft.second.create()); CK(cudaEventRecord(ft.first, ctx->copy)); }
     CK(cudaMemcpyAsync(P.ring->buf.as<u8>() + P.fill, host_base + lo, bytes, cudaMemcpyHostToDevice, ctx->copy));
-    if (job->feed_timing) { CK(cudaEventRecord(ft1, ctx->copy)); job->ft_copy_ev.push_back({ft0, ft1}); job->ft_copy_bytes += bytes; }
+    if (job->feed_timing) { CK(cudaEventRecord(ft.second, ctx->copy)); job->ft_copy_ev.push_back(std::move(ft)); job->ft_copy_bytes += bytes; }
     *at = P.fill;
     P.fill += padded;
     return 0;
@@ -766,7 +740,7 @@ extern "C" int fastf_bam2db_stats(fastf_bam2db_job *job, fastf_bam2db_result *re
     return fill_stats(job, res);
 }
 
-// FASTF_FEED_TIMING=1: the host-fed job's copy / inflate / parse timeline on stderr (once, when the job is sampled); releases its events
+// FASTF_FEED_TIMING=1: the host-fed job's copy / inflate / parse timeline on stderr (once, when the job is sampled)
 static int report_feed_timing(fastf_bam2db_job *job)
 {
     fastf_ctx *ctx = job->ctx;
@@ -795,10 +769,6 @@ static int report_feed_timing(fastf_bam2db_job *job)
                 fprintf(stderr, "[fastf feed timing]   copy %2zu: %.1f..%.1f\n", k, a, b);
             }
         }
-        for (auto &e : job->ft_copy_ev) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
-        for (auto &e : job->ft_infl_ev) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
-        for (auto &e : job->ft_parse_ev) cudaEventDestroy(e);
-        job->ft_copy_ev.clear(); job->ft_infl_ev.clear(); job->ft_parse_ev.clear();
     }
     return 0;
 }
@@ -1115,18 +1085,14 @@ extern "C" int fastf_sweep_count_device(fastf_ctx *ctx, uint64_t *dev_keys, uint
     RleScratch R, RR;
     DevBuf alt, ralt, orand;
     PinBuf host;
+    DrainOnExit drain{ctx};
     int rc = dev_reserve(ctx, alt, std::max<u64>(n, 1) * sizeof(u64));
     if (!rc) rc = dev_reserve(ctx, ralt, std::max<u64>(n, 1) * sizeof(u32));
     if (!rc) rc = dev_reserve(ctx, orand, 2 * sizeof(u64));
     if (!rc) rc = pin_reserve(ctx, host, 2 * sizeof(u64));
     if (!rc) rc = sweep_count(ctx, S, R, RR, orand, host, dev_keys, alt.as<u64>(), dev_rates, ralt.as<u32>(), n, key_bits, bits_gene, bits_umi, n_rates, nullptr, nullptr, nullptr, nnz, m_gene, m_cell,
                               m_count, s);
-    if (cudaStreamSynchronize(s) != cudaSuccess && !rc) rc = ctx_fail(ctx, "sweep_count_device: stream error");
-    sort_scratch_release(ctx, S);
-    rle_scratch_release(ctx, R);
-    rle_scratch_release(ctx, RR);
-    dev_release(ctx, alt); dev_release(ctx, ralt); dev_release(ctx, orand);
-    pin_release(ctx, host);
+    if (!rc && cudaStreamSynchronize(s) != cudaSuccess) rc = ctx_fail(ctx, "sweep_count_device: stream error");
     if (rc)
         for (u32 p = 0; p < n_rates; p++) { free(m_gene[p]); free(m_cell[p]); free(m_count[p]); m_gene[p] = m_cell[p] = m_count[p] = nullptr; nnz[p] = 0; }
     return rc;

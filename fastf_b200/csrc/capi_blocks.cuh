@@ -11,22 +11,20 @@ extern "C" int fastf_sort_u64_device(fastf_ctx *ctx, uint64_t *dev_keys, uint32_
     if (n == 0) return 0;
     SortScratch S;
     DevBuf alt, valt;
-    int rc = dev_reserve(ctx, alt, n * sizeof(u64));
-    if (!rc && dev_vals) rc = dev_reserve(ctx, valt, n * sizeof(u32));
+    DrainOnExit drain{ctx};
+    TRY(dev_reserve(ctx, alt, n * sizeof(u64)));
+    if (dev_vals) TRY(dev_reserve(ctx, valt, n * sizeof(u32)));
     u32 shifts[8];
     int npass = 0;
     for (u32 b = 0; b < key_bits && npass < 8; b += 8) shifts[npass++] = b;
     bool in_alt = false;
-    if (!rc) rc = sort_keys(ctx, S, dev_keys, alt.as<u64>(), dev_vals, valt.as<u32>(), n, shifts, npass, &in_alt, ctx->compute);
-    if (!rc && in_alt) {
-        rc = cudaMemcpyAsync(dev_keys, alt.p, n * sizeof(u64), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess;
-        if (!rc && dev_vals) rc = cudaMemcpyAsync(dev_vals, valt.p, n * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess;
+    TRY(sort_keys(ctx, S, dev_keys, alt.as<u64>(), dev_vals, valt.as<u32>(), n, shifts, npass, &in_alt, ctx->compute));
+    if (in_alt) {
+        CK(cudaMemcpyAsync(dev_keys, alt.p, n * sizeof(u64), cudaMemcpyDeviceToDevice, ctx->compute));
+        if (dev_vals) CK(cudaMemcpyAsync(dev_vals, valt.p, n * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute));
     }
-    if (cudaStreamSynchronize(ctx->compute) != cudaSuccess && !rc) rc = ctx_fail(ctx, "sort_u64_device: stream error");
-    sort_scratch_release(ctx, S);
-    dev_release(ctx, alt);
-    dev_release(ctx, valt);
-    return rc;
+    if (cudaStreamSynchronize(ctx->compute) != cudaSuccess) return ctx_fail(ctx, "sort_u64_device: stream error");
+    return 0;
 }
 
 // same, results left on the device in caller-provided arrays of capacity >= n (multi-GPU driver: the pieces travel over NCCL)
@@ -35,18 +33,15 @@ extern "C" int fastf_dedup_count_device_out(fastf_ctx *ctx, const uint64_t *dev_
 {
     CK(cudaSetDevice(ctx->device));
     RleScratch R;
-    u64 ng = 0;
-    int rc = rle_groups(ctx, R, dev_sorted_keys, nullptr, n, bits_umi, bits_umi - 1, bits_gene, &ng, nullptr, ctx->compute);
-    if (!rc && ng) {
-        rc = cudaMemcpyAsync(dev_gene, R.out_gene.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess ||
-             cudaMemcpyAsync(dev_cell, R.out_cell.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess ||
-             cudaMemcpyAsync(dev_count, R.count.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess;
-        if (rc) ctx_fail(ctx, "dedup_count_device_out: copy failed");
-    }
-    if (cudaStreamSynchronize(ctx->compute) != cudaSuccess && !rc) rc = ctx_fail(ctx, "dedup_count_device_out: stream error");
-    *nnz = ng;
-    rle_scratch_release(ctx, R);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(rle_groups(ctx, R, dev_sorted_keys, nullptr, n, bits_umi, bits_umi - 1, bits_gene, nnz, nullptr, ctx->compute));
+    const u64 ng = *nnz;
+    if (ng && (cudaMemcpyAsync(dev_gene, R.out_gene.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess ||
+               cudaMemcpyAsync(dev_cell, R.out_cell.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess ||
+               cudaMemcpyAsync(dev_count, R.count.p, ng * sizeof(u32), cudaMemcpyDeviceToDevice, ctx->compute) != cudaSuccess))
+        return ctx_fail(ctx, "dedup_count_device_out: copy failed");
+    if (cudaStreamSynchronize(ctx->compute) != cudaSuccess) return ctx_fail(ctx, "dedup_count_device_out: stream error");
+    return 0;
 }
 
 extern "C" int fastf_dedup_count_device(fastf_ctx *ctx, const uint64_t *dev_sorted_keys, uint64_t n, uint32_t bits_gene, uint32_t bits_umi, uint64_t *nnz, uint32_t **m_gene, uint32_t **m_cell,
@@ -54,12 +49,9 @@ extern "C" int fastf_dedup_count_device(fastf_ctx *ctx, const uint64_t *dev_sort
 {
     CK(cudaSetDevice(ctx->device));
     RleScratch R;
-    u64 ng = 0;
-    int rc = rle_groups(ctx, R, dev_sorted_keys, nullptr, n, bits_umi, bits_umi - 1, bits_gene, &ng, nullptr, ctx->compute);
-    if (!rc) rc = coo_to_host(ctx, R, ng, m_gene, m_cell, m_count, ctx->compute);
-    *nnz = ng;
-    rle_scratch_release(ctx, R);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(rle_groups(ctx, R, dev_sorted_keys, nullptr, n, bits_umi, bits_umi - 1, bits_gene, nnz, nullptr, ctx->compute));
+    return coo_to_host(ctx, R, *nnz, m_gene, m_cell, m_count, ctx->compute);
 }
 
 // Destination of a cell for the multi-GPU exchange: all keys of one (cell, gene) group must meet on one rank.  The "hash" is
@@ -106,46 +98,37 @@ static int unique_partition(fastf_ctx *ctx, const char *who, u64 *dev_keys, u32 
     RleScratch R;
     DevBuf alt, valt, orand, bounds;
     PinBuf host;
-    int rc = 0;
-    auto body = [&]() -> int {
-        TRY(dev_reserve(ctx, alt, n * sizeof(u64)));
-        if (dev_rates) TRY(dev_reserve(ctx, valt, n * sizeof(u32)));
-        TRY(dev_reserve(ctx, orand, 2 * sizeof(u64)));
-        TRY(dev_reserve(ctx, bounds, 257 * sizeof(u64)));
-        TRY(pin_reserve(ctx, host, 257 * sizeof(u64)));
-        FASTF_LAUNCH(fastf_tag_dest_kernel, (u32)((n + 255) / 256), 256, 0, s, dev_keys, n, bits_gene + bits_umi, key_bits, n_cells, nparts);
-        CKL("tag_dest");
-        u64 varying = 0;
-        TRY(varying_bits(ctx, orand, host, dev_keys, n, &varying, s));
-        u32 shifts[9];
-        int npass = 0;
-        if (dev_rates) shifts[npass++] = FASTF_SORT_VAL_DIGIT;
-        npass += plan_windows(varying, shifts + npass);
-        bool in_alt = false;
-        TRY(sort_keys(ctx, S, dev_keys, alt.as<u64>(), dev_rates, dev_rates ? valt.as<u32>() : nullptr, n, shifts, npass, &in_alt, s));
-        const u64 *sorted = in_alt ? alt.as<u64>() : dev_keys;
-        const u32 *sorted_rates = dev_rates ? (in_alt ? valt.as<u32>() : dev_rates) : nullptr;
-        // unique: every key is its own group (group_shift 0); grp_key = the distinct keys in sorted order, grp_val their first rate
-        u64 nuniq = 0;
-        TRY(rle_groups(ctx, R, sorted, sorted_rates, n, 0, 64, 0, &nuniq, nullptr, s));
-        FASTF_LAUNCH(fastf_part_bounds_kernel, 1, 256, 0, s, (const u64 *)R.grp_key.as<u64>(), nuniq, key_bits, nparts, bounds.as<u64>());
-        CKL("part_bounds");
-        CK(cudaMemcpyAsync(dev_out_keys, R.grp_key.p, nuniq * sizeof(u64), cudaMemcpyDeviceToDevice, s));
-        if (dev_rates) CK(cudaMemcpyAsync(dev_out_rates, R.grp_val.p, nuniq * sizeof(u32), cudaMemcpyDeviceToDevice, s));
-        FASTF_LAUNCH(fastf_strip_tag_kernel, (u32)((nuniq + 255) / 256), 256, 0, s, dev_out_keys, nuniq, key_bits);
-        CKL("strip_tag");
-        CK(cudaMemcpyAsync(host.p, bounds.p, (nparts + 1) * sizeof(u64), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        for (u32 p = 0; p < nparts; p++) part_counts[p] = host.as<u64>()[p + 1] - host.as<u64>()[p];
-        return 0;
-    };
-    rc = body();
-    cudaStreamSynchronize(s);
-    sort_scratch_release(ctx, S);
-    rle_scratch_release(ctx, R);
-    dev_release(ctx, alt); dev_release(ctx, valt); dev_release(ctx, orand); dev_release(ctx, bounds);
-    pin_release(ctx, host);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(dev_reserve(ctx, alt, n * sizeof(u64)));
+    if (dev_rates) TRY(dev_reserve(ctx, valt, n * sizeof(u32)));
+    TRY(dev_reserve(ctx, orand, 2 * sizeof(u64)));
+    TRY(dev_reserve(ctx, bounds, 257 * sizeof(u64)));
+    TRY(pin_reserve(ctx, host, 257 * sizeof(u64)));
+    FASTF_LAUNCH(fastf_tag_dest_kernel, (u32)((n + 255) / 256), 256, 0, s, dev_keys, n, bits_gene + bits_umi, key_bits, n_cells, nparts);
+    CKL("tag_dest");
+    u64 varying = 0;
+    TRY(varying_bits(ctx, orand, host, dev_keys, n, &varying, s));
+    u32 shifts[9];
+    int npass = 0;
+    if (dev_rates) shifts[npass++] = FASTF_SORT_VAL_DIGIT;
+    npass += plan_windows(varying, shifts + npass);
+    bool in_alt = false;
+    TRY(sort_keys(ctx, S, dev_keys, alt.as<u64>(), dev_rates, dev_rates ? valt.as<u32>() : nullptr, n, shifts, npass, &in_alt, s));
+    const u64 *sorted = in_alt ? alt.as<u64>() : dev_keys;
+    const u32 *sorted_rates = dev_rates ? (in_alt ? valt.as<u32>() : dev_rates) : nullptr;
+    // unique: every key is its own group (group_shift 0); grp_key = the distinct keys in sorted order, grp_val their first rate
+    u64 nuniq = 0;
+    TRY(rle_groups(ctx, R, sorted, sorted_rates, n, 0, 64, 0, &nuniq, nullptr, s));
+    FASTF_LAUNCH(fastf_part_bounds_kernel, 1, 256, 0, s, (const u64 *)R.grp_key.as<u64>(), nuniq, key_bits, nparts, bounds.as<u64>());
+    CKL("part_bounds");
+    CK(cudaMemcpyAsync(dev_out_keys, R.grp_key.p, nuniq * sizeof(u64), cudaMemcpyDeviceToDevice, s));
+    if (dev_rates) CK(cudaMemcpyAsync(dev_out_rates, R.grp_val.p, nuniq * sizeof(u32), cudaMemcpyDeviceToDevice, s));
+    FASTF_LAUNCH(fastf_strip_tag_kernel, (u32)((nuniq + 255) / 256), 256, 0, s, dev_out_keys, nuniq, key_bits);
+    CKL("strip_tag");
+    CK(cudaMemcpyAsync(host.p, bounds.p, (nparts + 1) * sizeof(u64), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    for (u32 p = 0; p < nparts; p++) part_counts[p] = host.as<u64>()[p + 1] - host.as<u64>()[p];
+    return 0;
 }
 
 extern "C" int fastf_unique_partition_device(fastf_ctx *ctx, uint64_t *dev_keys, uint64_t n, uint32_t key_bits, uint32_t bits_gene, uint32_t bits_umi, uint32_t n_cells, uint32_t nparts,
@@ -171,7 +154,6 @@ struct InflatedFile {
     u64 n_blocks = 0, infl_bytes = 0;
     u32 status = 0;
 };
-static void inflated_release(fastf_ctx *ctx, InflatedFile &F) { dev_release(ctx, F.comp); dev_release(ctx, F.infl); dev_release(ctx, F.de.counter); dev_release(ctx, F.de.sorted); index_release(ctx, F.idx); }
 
 // Inflate a whole BGZF image (host bytes, or device bytes + host index) into F.infl in one launch.
 // out_prefix: bytes kept free (and preserved across calls) in front of the inflated blocks -- streamed text carries the tail of the previous chunk there.
@@ -218,11 +200,10 @@ static int inflate_whole(fastf_ctx *ctx, InflatedFile &F, const void *host_bytes
     // FASTF_INFLATE_GROUP=<blocks> re-enables the grouping for experiments.)  The inflate clock is the sum of the launches.
     size_t group = std::max<size_t>(nb, 1);
     if (const char *e = getenv("FASTF_INFLATE_GROUP")) { const long v = atol(e); group = v > 0 ? (size_t)v : std::max<size_t>(nb, 1); }   // A/B knob: 0 = one launch
-    std::vector<cudaEvent_t> ev;
-    cudaEvent_t ev_copy = nullptr;
-    if (!dev_bytes) CK(cudaEventCreateWithFlags(&ev_copy, cudaEventDisableTiming));
-    int rc_l = 0;
-    for (size_t g0 = 0; g0 < nb && !rc_l; g0 += group) {
+    std::vector<Event> ev;
+    Event ev_copy;
+    if (!dev_bytes) CK(ev_copy.create(cudaEventDisableTiming));
+    for (size_t g0 = 0; g0 < nb; g0 += group) {
         const size_t g1 = std::min(nb, g0 + group);
         if (!dev_bytes) {
             // bytes of this group: from its first payload (the very first group: from lo) to the end of its last block's trailer
@@ -232,14 +213,13 @@ static int inflate_whole(fastf_ctx *ctx, InflatedFile &F, const void *host_bytes
             CK(cudaEventRecord(ev_copy, ctx->copy));
             CK(cudaStreamWaitEvent(s, ev_copy, 0));
         }
-        if (ms) { cudaEvent_t a = nullptr, b = nullptr; CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b)); ev.push_back(a); ev.push_back(b); CK(cudaEventRecord(a, s)); }
-        rc_l = launch_inflate(ctx, lanes, comp, comp_total, F.idx.in_off + g0, F.idx.in_len + g0, F.idx.out_off + g0, F.idx.isize + g0, (u32)(g1 - g0), F.infl.as<u8>(), F.idx.st_infl + g0, s, &F.de,
-                              F.idx.h_in_off + g0, F.idx.h_in_len + g0, F.idx.h_out_off + g0, F.idx.h_isize + g0);
+        if (ms) { Event a, b; CK(a.create()); CK(b.create()); CK(cudaEventRecord(a, s)); ev.push_back(std::move(a)); ev.push_back(std::move(b)); }
+        TRY(launch_inflate(ctx, lanes, comp, comp_total, F.idx.in_off + g0, F.idx.in_len + g0, F.idx.out_off + g0, F.idx.isize + g0, (u32)(g1 - g0), F.infl.as<u8>(), F.idx.st_infl + g0, s, &F.de,
+                           F.idx.h_in_off + g0, F.idx.h_in_len + g0, F.idx.h_out_off + g0, F.idx.h_isize + g0));
         if (ms) CK(cudaEventRecord(ev.back(), s));
-        if (!rc_l) rc_l = launch_crc(ctx, lanes, comp, dev_bytes ? (u64)n : comp_total, F.idx.in_off + g0, F.idx.in_len + g0, F.infl.as<u8>(), F.idx.out_off + g0, F.idx.isize + g0, (u32)(g1 - g0),
-                                     F.idx.st_infl + g0, s);
+        TRY(launch_crc(ctx, lanes, comp, dev_bytes ? (u64)n : comp_total, F.idx.in_off + g0, F.idx.in_len + g0, F.infl.as<u8>(), F.idx.out_off + g0, F.idx.isize + g0, (u32)(g1 - g0),
+                       F.idx.st_infl + g0, s));
     }
-    if (rc_l) { for (auto e : ev) cudaEventDestroy(e); if (ev_copy) cudaEventDestroy(ev_copy); return rc_l; }
     // OR of the per-block status words
     std::vector<u32> st(nb);
     if (nb) CK(cudaMemcpyAsync(st.data(), F.idx.st_infl, nb * sizeof(u32), cudaMemcpyDeviceToHost, s));
@@ -249,8 +229,6 @@ static int inflate_whole(fastf_ctx *ctx, InflatedFile &F, const void *host_bytes
         *ms = 0;
         for (size_t i = 0; i + 1 < ev.size(); i += 2) { float t = 0; cudaEventElapsedTime(&t, ev[i], ev[i + 1]); *ms += t; }
     }
-    for (auto e : ev) cudaEventDestroy(e);
-    if (ev_copy) cudaEventDestroy(ev_copy);
     F.status = 0;
     for (size_t i = 0; i < nb; i++) F.status |= st[i];
     F.n_blocks = nb;
@@ -268,15 +246,13 @@ extern "C" int fastf_inflate_host(fastf_ctx *ctx, const void *bgzf_bytes, size_t
     *out = nullptr;
     *out_n = 0;
     InflatedFile F;
-    int rc = inflate_whole(ctx, F, bgzf_bytes, n, nullptr, nullptr, (u32)lanes, ms, ctx->compute);
-    if (!rc) {
-        *out = malloc(F.infl_bytes ? F.infl_bytes : 1);
-        if (!*out) rc = ctx_fail(ctx, "inflate_host: out of host memory");
-        if (!rc && F.infl_bytes) rc = fastf_memcpy_d2h(ctx, *out, F.infl.p, F.infl_bytes);
-        *out_n = F.infl_bytes;
-    }
-    inflated_release(ctx, F);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(inflate_whole(ctx, F, bgzf_bytes, n, nullptr, nullptr, (u32)lanes, ms, ctx->compute));
+    *out = malloc(F.infl_bytes ? F.infl_bytes : 1);
+    *out_n = F.infl_bytes;
+    if (!*out) return ctx_fail(ctx, "inflate_host: out of host memory");
+    if (F.infl_bytes) TRY(fastf_memcpy_d2h(ctx, *out, F.infl.p, F.infl_bytes));
+    return 0;
 }
 
 static int mt_host_common(fastf_ctx *ctx, uint32_t seed, uint64_t n, uint64_t threshold, uint32_t *out_words, uint32_t *out_bits)
@@ -285,19 +261,15 @@ static int mt_host_common(fastf_ctx *ctx, uint32_t seed, uint64_t n, uint64_t th
     if (n == 0) return 0;
     const u64 pairs = (n + 1247) / 1248;
     DevBuf state, out;
-    int rc = dev_reserve(ctx, state, 624 * sizeof(u32));
+    DrainOnExit drain{ctx};
+    TRY(dev_reserve(ctx, state, 624 * sizeof(u32)));
     const size_t out_bytes = out_words ? (size_t)pairs * 1248 * sizeof(u32) : (size_t)pairs * 39 * sizeof(u32);
-    if (!rc) rc = dev_reserve(ctx, out, out_bytes);
-    if (!rc) {
-        FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->compute, seed, state.as<u32>(), 1u, (u64)0, pairs, threshold, out_words ? out.as<u32>() : (u32 *)nullptr,
-                     out_words ? (u32 *)nullptr : out.as<u32>());
-        ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) rc = ctx_fail(ctx, "mt19937 launch failed");
-    }
-    if (!rc) rc = out_words ? fastf_memcpy_d2h(ctx, out_words, out.p, (size_t)n * sizeof(u32)) : fastf_memcpy_d2h(ctx, out_bits, out.p, (size_t)((n + 31) / 32) * sizeof(u32));
-    dev_release(ctx, state);
-    dev_release(ctx, out);
-    return rc;
+    TRY(dev_reserve(ctx, out, out_bytes));
+    FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->compute, seed, state.as<u32>(), 1u, (u64)0, pairs, threshold, out_words ? out.as<u32>() : (u32 *)nullptr,
+                 out_words ? (u32 *)nullptr : out.as<u32>());
+    ctx->launches++;
+    if (cudaGetLastError() != cudaSuccess) return ctx_fail(ctx, "mt19937 launch failed");
+    return out_words ? fastf_memcpy_d2h(ctx, out_words, out.p, (size_t)n * sizeof(u32)) : fastf_memcpy_d2h(ctx, out_bits, out.p, (size_t)((n + 31) / 32) * sizeof(u32));
 }
 extern "C" int fastf_mt19937_host_from(fastf_ctx *ctx, uint32_t seed, uint64_t first, uint64_t n, uint32_t *out_words)
 {
@@ -307,22 +279,17 @@ extern "C" int fastf_mt19937_host_from(fastf_ctx *ctx, uint32_t seed, uint64_t f
     u32 n_polys = 0;
     TRY(mt_jump_polys(ctx, "mt19937_host_from", first, &n_polys));
     DevBuf state, scratch, out;
-    int rc = dev_reserve(ctx, state, 624 * sizeof(u32));
-    if (!rc) rc = dev_reserve(ctx, scratch, FASTF_MTJ_SCRATCH * sizeof(u32));
-    if (!rc) rc = dev_reserve(ctx, out, (size_t)pairs * 1248 * sizeof(u32));
-    if (!rc) {
-        // one CTA of the batched jump leaves the window at stream index `first`; the twist continues from there
-        FASTF_LAUNCH(fastf_mt_jump_batch_kernel, 1, FASTF_MTJ_THREADS, 0, ctx->compute, seed, (const u64 *)ctx->mtj_polys, n_polys, first, (u64)0, state.as<u32>(), scratch.as<u32>());
-        ctx->launches++;
-        FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->compute, seed, state.as<u32>(), 0u, (u64)0, pairs, (u64)0, out.as<u32>(), (u32 *)nullptr);
-        ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) rc = ctx_fail(ctx, "mt19937 launch failed");
-    }
-    if (!rc) rc = fastf_memcpy_d2h(ctx, out_words, out.p, (size_t)n * sizeof(u32));
-    dev_release(ctx, state);
-    dev_release(ctx, scratch);
-    dev_release(ctx, out);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(dev_reserve(ctx, state, 624 * sizeof(u32)));
+    TRY(dev_reserve(ctx, scratch, FASTF_MTJ_SCRATCH * sizeof(u32)));
+    TRY(dev_reserve(ctx, out, (size_t)pairs * 1248 * sizeof(u32)));
+    // one CTA of the batched jump leaves the window at stream index `first`; the twist continues from there
+    FASTF_LAUNCH(fastf_mt_jump_batch_kernel, 1, FASTF_MTJ_THREADS, 0, ctx->compute, seed, (const u64 *)ctx->mtj_polys, n_polys, first, (u64)0, state.as<u32>(), scratch.as<u32>());
+    ctx->launches++;
+    FASTF_LAUNCH(fastf_mt19937_kernel, 1, FASTF_MT_THREADS, 0, ctx->compute, seed, state.as<u32>(), 0u, (u64)0, pairs, (u64)0, out.as<u32>(), (u32 *)nullptr);
+    ctx->launches++;
+    if (cudaGetLastError() != cudaSuccess) return ctx_fail(ctx, "mt19937 launch failed");
+    return fastf_memcpy_d2h(ctx, out_words, out.p, (size_t)n * sizeof(u32));
 }
 extern "C" int fastf_mt19937_host(fastf_ctx *ctx, uint32_t seed, uint64_t n, uint32_t *out_words) { return mt_host_common(ctx, seed, n, 0, out_words, nullptr); }
 extern "C" int fastf_mt19937_keepbits_host(fastf_ctx *ctx, uint32_t seed, uint64_t n, uint64_t threshold, uint32_t *out_bits) { return mt_host_common(ctx, seed, n, threshold, nullptr, out_bits); }
@@ -332,16 +299,15 @@ extern "C" int fastf_sort_u64_host(fastf_ctx *ctx, uint64_t *keys, uint32_t *val
     CK(cudaSetDevice(ctx->device));
     if (n == 0) return 0;
     DevBuf dk, dv;
-    int rc = dev_reserve(ctx, dk, n * sizeof(u64));
-    if (!rc && vals) rc = dev_reserve(ctx, dv, n * sizeof(u32));
-    if (!rc) rc = fastf_memcpy_h2d(ctx, dk.p, keys, n * sizeof(u64));
-    if (!rc && vals) rc = fastf_memcpy_h2d(ctx, dv.p, vals, n * sizeof(u32));
-    if (!rc) rc = fastf_sort_u64_device(ctx, dk.as<u64>(), vals ? dv.as<u32>() : nullptr, n, key_bits);
-    if (!rc) rc = fastf_memcpy_d2h(ctx, keys, dk.p, n * sizeof(u64));
-    if (!rc && vals) rc = fastf_memcpy_d2h(ctx, vals, dv.p, n * sizeof(u32));
-    dev_release(ctx, dk);
-    dev_release(ctx, dv);
-    return rc;
+    DrainOnExit drain{ctx};
+    TRY(dev_reserve(ctx, dk, n * sizeof(u64)));
+    if (vals) TRY(dev_reserve(ctx, dv, n * sizeof(u32)));
+    TRY(fastf_memcpy_h2d(ctx, dk.p, keys, n * sizeof(u64)));
+    if (vals) TRY(fastf_memcpy_h2d(ctx, dv.p, vals, n * sizeof(u32)));
+    TRY(fastf_sort_u64_device(ctx, dk.as<u64>(), vals ? dv.as<u32>() : nullptr, n, key_bits));
+    TRY(fastf_memcpy_d2h(ctx, keys, dk.p, n * sizeof(u64)));
+    if (vals) TRY(fastf_memcpy_d2h(ctx, vals, dv.p, n * sizeof(u32)));
+    return 0;
 }
 
 // Distinct keys of a host array with their multiplicities: stable radix sort + run-length heads on the device (K4), the copies of
@@ -354,18 +320,17 @@ extern "C" int fastf_unique_counts_host(fastf_ctx *ctx, const uint64_t *keys, ui
     if (n == 0) return 0;
     DevBuf dk;
     RleScratch R;
+    DrainOnExit drain{ctx};
     u64 ngroups = 0;
-    int rc = dev_reserve(ctx, dk, n * sizeof(u64));
-    if (!rc) rc = fastf_memcpy_h2d(ctx, dk.p, keys, n * sizeof(u64));
-    if (!rc) rc = fastf_sort_u64_device(ctx, dk.as<u64>(), nullptr, n, key_bits);
-    if (!rc) rc = rle_groups(ctx, R, dk.as<u64>(), nullptr, n, 0, 64, 0, &ngroups, nullptr, ctx->compute);
-    u32 *first = nullptr;
-    if (!rc) {
-        *out_keys = (uint64_t *)malloc(std::max<u64>(ngroups, 1) * sizeof(uint64_t));
-        *out_counts = (uint32_t *)malloc(std::max<u64>(ngroups, 1) * sizeof(uint32_t));
-        first = (u32 *)malloc(std::max<u64>(ngroups, 1) * sizeof(u32));
-        if (!*out_keys || !*out_counts || !first) rc = ctx_fail(ctx, "unique_counts: out of host memory for %llu groups", (unsigned long long)ngroups);
-    }
+    TRY(dev_reserve(ctx, dk, n * sizeof(u64)));
+    TRY(fastf_memcpy_h2d(ctx, dk.p, keys, n * sizeof(u64)));
+    TRY(fastf_sort_u64_device(ctx, dk.as<u64>(), nullptr, n, key_bits));
+    TRY(rle_groups(ctx, R, dk.as<u64>(), nullptr, n, 0, 64, 0, &ngroups, nullptr, ctx->compute));
+    *out_keys = (uint64_t *)malloc(std::max<u64>(ngroups, 1) * sizeof(uint64_t));
+    *out_counts = (uint32_t *)malloc(std::max<u64>(ngroups, 1) * sizeof(uint32_t));
+    u32 *first = (u32 *)malloc(std::max<u64>(ngroups, 1) * sizeof(u32));
+    int rc = 0;
+    if (!*out_keys || !*out_counts || !first) rc = ctx_fail(ctx, "unique_counts: out of host memory for %llu groups", (unsigned long long)ngroups);
     if (!rc && ngroups) rc = d2h_pageable(ctx, *out_keys, R.grp_key.p, ngroups * sizeof(u64), ctx->compute);
     if (!rc && ngroups) rc = d2h_pageable(ctx, first, R.grp_first.p, ngroups * sizeof(u32), ctx->compute);
     if (!rc) {
@@ -375,8 +340,6 @@ extern "C" int fastf_unique_counts_host(fastf_ctx *ctx, const uint64_t *keys, ui
         free(*out_keys); free(*out_counts); *out_keys = nullptr; *out_counts = nullptr;
     }
     free(first);
-    dev_release(ctx, dk);
-    rle_scratch_release(ctx, R);
     return rc;
 }
 

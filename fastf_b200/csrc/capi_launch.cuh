@@ -177,7 +177,6 @@ static int sort_keys(fastf_ctx *ctx, SortScratch &S, u64 *keys, u64 *alt, u32 *v
     *sorted_in_alt = (src == alt);
     return 0;
 }
-static void sort_scratch_release(fastf_ctx *ctx, SortScratch &S) { dev_release(ctx, S.hist); dev_release(ctx, S.totals); dev_release(ctx, S.dbase); }
 
 // OR / AND of all keys -> which bit positions vary (device reduction, 16 bytes back)
 __global__ void __launch_bounds__(256) fastf_key_bits_kernel(const u64 *__restrict__ keys, u64 n, u64 *__restrict__ or_and)
@@ -193,12 +192,6 @@ struct RleScratch {
     DevBuf tile_counts, tile_totals, grp_key, grp_first, grp_dstart, grp_val, count, out_gene, out_cell;
     PinBuf totals_host;
 };
-static void rle_scratch_release(fastf_ctx *ctx, RleScratch &R)
-{
-    dev_release(ctx, R.tile_counts); dev_release(ctx, R.tile_totals); dev_release(ctx, R.grp_key); dev_release(ctx, R.grp_first); dev_release(ctx, R.grp_dstart); dev_release(ctx, R.grp_val);
-    dev_release(ctx, R.count); dev_release(ctx, R.out_gene); dev_release(ctx, R.out_cell);
-    pin_release(ctx, R.totals_host);
-}
 // After this: R.grp_key/grp_first/grp_dstart(/grp_val)/count hold ngroups entries on device; with split_bits_gene > 0
 // R.out_gene / R.out_cell hold the split group key.  pred: the depth sweep's rate predicate (radix_dedup.cuh), off by default.
 static int rle_groups(fastf_ctx *ctx, RleScratch &R, const u64 *sorted, const u32 *vals, u64 n, u32 group_shift, u32 nn_bit, u32 split_bits_gene, u64 *ngroups_out, u64 *ndistinct_out,
@@ -335,4 +328,3 @@ static int index_upload(fastf_ctx *ctx, BlockIndexDev &I, cudaStream_t s)
 #endif
     return 0;
 }
-static void index_release(fastf_ctx *ctx, BlockIndexDev &I) { dev_release(ctx, I.buf); pin_release(ctx, I.host); I.cap_blocks = 0; }
