@@ -6,10 +6,11 @@
 //
 //   decoder warps  (7 warps x 32 lanes)  lane = one BGZF block ("stream").  Pure scalar Huffman decoding out of that stream's
 //                                        own shared-memory tables; emits 4-byte TOKENS (up to three literals | match(len, dist)
-//                                        | end) into the stream's shared-memory ring.  No global stores, no warp collectives.
-//                                        One ROUND of a lane = up to two literal tokens (decoded without inner branches) plus
-//                                        the match that ends the literal run: the divergent paths of a warp execute one after
-//                                        the other and some lane always needs each of them, so every lane walks through both.
+//                                        | end) into the stream's 64-token shared-memory ring.  No global stores, no warp
+//                                        collectives.  One ROUND of a lane = up to three literal tokens (decoded without inner
+//                                        branches) plus the match that ends the literal run: the divergent paths of a warp
+//                                        execute one after the other and some lane always needs each of them, so every lane
+//                                        walks through both.
 //                                        A match whose source lies more than 512 bytes back is prefetched into L2 on the spot.
 //   service warps  (25 warps, lock step) own 9 consecutive streams each; one poll pass looks at all of them (lane k reads the
 //                                        k-th stream's control block, a ballot picks the streams with work).  (a) LZ77: take up
@@ -22,12 +23,14 @@
 //
 // Tables per stream: 8-bit literal/length table and 6-bit distance table with 16-bit entries (code length, kind, symbol) in shared
 // memory; a code longer than the table takes one lookup in the stream's second-level table in global memory (L2), with the
-// canonical walk (range limits in shared memory, symbol list in L2) as the fallback when the second level does not fit;
-// length/distance base+extra bits sit in a CTA-wide table.  224 streams x 0.9 KB + the set-up scratch fill the SM's shared memory.
-// What bounds it (profiles/r02_inflate_ab.md): a latency machine -- throughput = independent Huffman chains per SM / per-symbol
-// latency.  With 224 streams the LZ77 side co-limits: the service warps are busy 97 % of the time (5 700 cycles per batch of 22
-// tokens) and a third of the decoders' lane-rounds find their ring full; DRAM traffic is 5x the algorithmic bytes (the windows of
-// 33 152 resident streams do not fit the L2) but at 12 % of the bandwidth it is not the limit.
+// canonical walk (range limits and symbol list in L2) as the fallback when the second level does not fit (never on the synthetic
+// 10x BAM); length/distance base+extra bits sit in a CTA-wide table.  224 streams x 952 B + the set-up scratch fill the SM's shared
+// memory (229 536 of 232 448 bytes).
+// What bounds it (profiles/r02_inflate_ab.md, r05_inflate_ab.md): a latency machine -- throughput = independent Huffman chains per SM
+// / per-symbol latency.  With 224 streams the LZ77 side co-limits: with a 32-token ring a third of the decoders' lane-rounds found
+// it full (the service warps 97 % busy, 5 700 cycles per batch of 22 tokens); the 64-token ring lets every visit take a full 32
+// tokens and cuts that share to an eighth.  DRAM traffic is 5x the algorithmic bytes (the windows of 33 152 resident streams do not
+// fit the L2) but at 12 % of the bandwidth it is not the limit.
 #pragma once
 #include "bgzf_inflate.cuh"
 
@@ -37,7 +40,8 @@
 // memory limits.  8-bit literal/length and 6-bit distance tables with a 32-token ring fit 224 streams per SM (7 full decoder
 // warps + 25 service warps = 1024 threads): 179-183 GB/s algorithmic against 156 GB/s for the round-1 shape (128 streams, 9/7-bit
 // tables, 16 lanes x 8 warps + 24).  16-lane decoder warps at 224 streams leave too few service warps (138 GB/s); 256 streams need
-// a 16-token ring that starves the decoders (147 GB/s).
+// a 16-token ring that starves the decoders (147 GB/s).  Moving the canonical walk's limits to global scratch pays for a 64-token
+// ring at 224 streams: 193 -> 205 GB/s, 207 with three literal tokens per round (profiles/r05_inflate_ab.md).
 #ifndef FASTF_TPS_LBITS
 #define FASTF_TPS_LBITS 8
 #endif
@@ -69,17 +73,20 @@
 #endif
 #define FASTF_TPS_LITSUB_U16 1016u   // capacity of the literal/length sub-tables (7-bit offset field x 8)
 #define FASTF_TPS_DISTSUB_U16 512u
+// Per stream in GLOBAL scratch: symbols sorted by code length (288 lit/len + 32 dist), read only for codes longer than the tables,
+// then the two sub-table areas, then the canonical walk's range limits / index offsets (literal/length table, then distance table).
 #if FASTF_TPS_SUBTABLES
-#define FASTF_TPS_SORTED_U16 (320 + 1024 + 512)   // per stream in GLOBAL scratch: sorted symbols (288 lit/len + 32 dist), then the two sub-table areas
+#define FASTF_TPS_WALK_AT (320 + 1024 + 512)
 #else
-#define FASTF_TPS_SORTED_U16 320   // per stream in GLOBAL scratch: symbols sorted by code length (288 lit/len + 32 dist), read only for codes longer than the tables
+#define FASTF_TPS_WALK_AT 320
 #endif
+#define FASTF_TPS_SORTED_U16 (FASTF_TPS_WALK_AT + FASTF_TPS_WALK_U16(FASTF_TPS_LBITS) + FASTF_TPS_WALK_U16(FASTF_TPS_DBITS))
 #define FASTF_TPS_THREADS FASTF_TPS_THREADS_OF(FASTF_TPS_LANES, FASTF_TPS_SVC_WARPS)
 #ifndef FASTF_TPS_RING
-#define FASTF_TPS_RING 32u
+#define FASTF_TPS_RING 64u
 #endif
 #ifndef FASTF_TPS_TRIPLES
-#define FASTF_TPS_TRIPLES 2           // literal tokens (three literals each) a decoder round may produce in front of a match
+#define FASTF_TPS_TRIPLES 3           // literal tokens (three literals each) a decoder round may produce in front of a match
 #endif
 #ifndef FASTF_TPS_BATCH_MIN
 #define FASTF_TPS_BATCH_MIN (FASTF_TPS_RING >= 64u ? 32u : FASTF_TPS_RING / 2u)       // tokens that make a stream worth a visit of its service warp
@@ -119,30 +126,23 @@ enum { FASTF_TPS_NEXT = 0, FASTF_TPS_RUN = 1, FASTF_TPS_BUILD = 2, FASTF_TPS_DON
 // Codes longer than a primary table of TBITS bits have 15 - TBITS possible lengths; per length the decoder needs a range limit and
 // an index offset (fastf_tps_build).  Limits sit in [0, OFFS), offsets in [OFFS, 2 OFFS), OFFS = 8 or 12 (vector loads).
 #define FASTF_TPS_WALK_OFFS(TBITS) ((15 - (TBITS)) <= 8 ? 8 : 12)
-#define FASTF_TPS_WALK_U16(TBITS) (2 * FASTF_TPS_WALK_OFFS(TBITS) < 16 ? 16 : 2 * FASTF_TPS_WALK_OFFS(TBITS))   // >= 16: the build counts code lengths in it first
+#define FASTF_TPS_WALK_U16(TBITS) (2 * FASTF_TPS_WALK_OFFS(TBITS))   // per table in the stream's global scratch (a multiple of 4: vector loads)
+// The walk's limits live in global scratch, not in the stream structure: the hot path resolves long codes through the sub-tables,
+// so the walk is rare, and its 80 bytes per stream pay for the 64-token ring at 224 streams.
 // Lane i of a decoder warp (and lane k of a polling service warp) works on stream i: the same field of consecutive streams must
-// not fall into the same shared-memory bank.  The structure is 8-byte aligned and FASTF_TPS_PAD makes its size = 8 (mod 16) bytes,
-// i.e. a bank step of 2 between streams (an exact multiple of 128 bytes would put every lane on one bank).
-#ifndef FASTF_TPS_PAD
-#define FASTF_TPS_PAD 8
-#endif
+// not fall into the same shared-memory bank.  The structure is 8-byte aligned and its size = 8 (mod 16) bytes, i.e. a bank step
+// of 2 between streams (an exact multiple of 128 bytes would put every lane on one bank).
 struct FastfTpsStream {
     u16 lit[1 << FASTF_TPS_LBITS];
     u16 dist[1 << FASTF_TPS_DBITS];
-    alignas(8) u16 lit_cnt[FASTF_TPS_WALK_U16(FASTF_TPS_LBITS)];
-    alignas(8) u16 dist_cnt[FASTF_TPS_WALK_U16(FASTF_TPS_DBITS)];
-    u32 ring[FASTF_TPS_RING];
+    alignas(8) u32 ring[FASTF_TPS_RING];   // also the code-length counts of a table build while the stream is set up
     // control block (volatile accesses; every hand-over is fenced)
     u32 state, wr, rd, last;         // state, wr, rd: polled as ctl[0..2] by the service warps
     u32 bitpos_lo, bitpos_hi;        // absolute bit offset of the next unread bit inside `comp`
     u32 pos, isize;                  // decoder's output position / block size
-    u32 spare0, spare1;
     u32 blk, opos;                   // service side: block index, bytes written
     u32 inend_lo, inend_hi;          // absolute bit offset of the end of the payload
     u32 obase_lo, obase_hi;          // offset of the block in the inflated buffer
-#if FASTF_TPS_PAD
-    u8 pad[FASTF_TPS_PAD];
-#endif
 };
 
 // scratch of one service warp while it sets a stream up
@@ -154,6 +154,11 @@ struct FastfTpsShared {
     u8 cl_order[20];
     alignas(16) FastfTpsSvc svc[FASTF_TPS_MAX_SVC];
 };
+// largest dynamic shared memory a block may opt in to on sm_100 (227 KB): the shape must fit it at compile time, not at launch
+#define FASTF_TPS_SMEM_MAX 232448u
+#define FASTF_TPS_SMEM_BYTES (sizeof(FastfTpsStream) * FASTF_TPS_STREAMS + sizeof(FastfTpsShared))
+static_assert(sizeof(FastfTpsStream) % 16 == 8, "stream size must be 8 (mod 16) bytes: bank step of 2 between the streams of a warp");
+static_assert(FASTF_TPS_SMEM_BYTES <= FASTF_TPS_SMEM_MAX, "streams + set-up scratch exceed the shared memory of an SM");
 
 
 // Hand-over between warps of the CTA goes through shared memory only.  One thread's shared-memory stores are performed in
@@ -167,7 +172,8 @@ struct FastfTpsShared {
 // FASTF_TPS_PROF: where the lane-rounds of the decoders and the cycles of the service warps go (debug builds only; read with
 // fastf_debug_tps_prof).  [0] decoder lane-rounds decoded, [1] skipped with a full ring, [2] skipped waiting for set-up,
 // [3] service passes, [4] passes without work, [5] cycles in copies, [6] cycles in set-up, [7] cycles in passes without work,
-// [8] batches, [9] tokens, [10] total service cycles
+// [8] batches, [9] tokens, [10] total service cycles, [11] codes longer than the primary table, [12] of them resolved by the
+// canonical walk (their sub-tables did not fit)
 #ifndef FASTF_TPS_PROF
 #define FASTF_TPS_PROF 0
 #endif
@@ -212,6 +218,14 @@ __device__ __forceinline__ u32 fastf_ld_sorted(const u16 *p) { return *p; }
 __device__ __forceinline__ u32 fastf_ld_sorted(const u16 *p) { return __ldcg(p); }
 #endif
 #endif
+// the walk's limits / offsets: rewritten for every deflate block by a service warp, so always read through L2 (8-byte vectors)
+#ifdef FASTF_EMU
+__device__ __forceinline__ uint2 fastf_ld_walk2(const u16 *p) { return *reinterpret_cast<const uint2 *>(p); }
+__device__ __forceinline__ u32 fastf_ld_walk(const u16 *p) { return *p; }
+#else
+__device__ __forceinline__ uint2 fastf_ld_walk2(const u16 *p) { return __ldcg(reinterpret_cast<const uint2 *>(p)); }
+__device__ __forceinline__ u32 fastf_ld_walk(const u16 *p) { return __ldcg(p); }
+#endif
 // A decoder knows the source of a match thousands of cycles before the stream's service warp copies it: it asks the L2 for the line
 // right away (the windows of all resident streams are far larger than the L2, so a distant source is usually a DRAM access).
 #ifndef FASTF_TPS_PREFETCH_SRC
@@ -242,8 +256,10 @@ __device__ __forceinline__ u32 fastf_make16(u32 alpha, u32 sym)
 }
 
 // Cooperative (32 lanes, lock step) construction of one 16-bit decode table.  Returns non-zero for an invalid code.
+// cnt[16], first[16], start[16]: shared scratch.  lb: the stream's walk limits / offsets in global scratch
+// (null for the code-length table, whose codes all fit the table).
 // *walk = (first canonical code of length tbits+1) << 16 | (index of its first symbol in sorted[]).
-__device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n, u16 *cnt, u16 *sorted, u16 *lut, u32 tbits, u16 *first, u16 *start, u32 *walk, u32 lane,
+__device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n, u16 *cnt, u16 *lb, u16 *sorted, u16 *lut, u32 tbits, u16 *first, u16 *start, u32 *walk, u32 lane,
                                                u16 *sub = nullptr, u32 sub_cap = 0, u8 *submax = nullptr)
 {
     for (u32 i = lane; i < (1u << tbits); i += 32) lut[i] = FASTF_T16_LONG;
@@ -278,18 +294,15 @@ __device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n,
         first[0] = (u16)used;
         // For the codes longer than the table the decoder needs, per length l = tbits+1+k: the left-aligned (15-bit) end of the
         // length's code range (ranges of a canonical code follow one another in length order) and start[l] - first[l], the offset
-        // that turns a code into its index in sorted[].  They replace the counts in cnt[]: limits in [0, OFFS), offsets behind them.
-        const u32 offs_at = FASTF_TPS_WALK_OFFS(tbits);
-        u16 lim[12], off[12];
-#pragma unroll
-        for (u32 k = 0; k < 12; k++) {
-            const u32 l = tbits + 1 + k;
-            lim[k] = l <= 15 ? (u16)(((u32)first[l] + cnt[l]) << (15 - l)) : (u16)0xffff;
-            off[k] = l <= 15 ? (u16)((u32)start[l] - (u32)first[l]) : (u16)0;
+        // that turns a code into its index in sorted[].  Limits go to lb[0, OFFS), offsets behind them.
+        if (lb) {
+            const u32 offs_at = FASTF_TPS_WALK_OFFS(tbits);
+            for (u32 k = 0; k < offs_at; k++) {
+                const u32 l = tbits + 1 + k;
+                lb[k] = l <= 15 ? (u16)(((u32)first[l] + cnt[l]) << (15 - l)) : (u16)0xffff;
+                lb[offs_at + k] = l <= 15 ? (u16)((u32)start[l] - (u32)first[l]) : (u16)0;
+            }
         }
-#pragma unroll
-        for (u32 k = 0; k < 12; k++)
-            if (k < offs_at) { cnt[k] = lim[k]; cnt[offs_at + k] = off[k]; }
     }
     bad = __shfl_sync(FASTF_FULL_MASK, bad, 0);
     wk = __shfl_sync(FASTF_FULL_MASK, wk, 0);
@@ -398,6 +411,10 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
     u32 opos = S.opos, err = 0;
     u8 *lens = G.svc[sw].setup.lens;
     u16 *first = G.svc[sw].setup.scratch, *start = G.svc[sw].setup.scratch + 16;
+    // a table build counts code lengths in the stream's token ring: it is empty while the stream is set up (a batch of tokens is
+    // always copied before the set-up, and the decoder writes no token before the state says RUN)
+    u16 *cnt = reinterpret_cast<u16 *>(S.ring);
+    u16 *lit_walk = lit_sorted + FASTF_TPS_WALK_AT, *dist_walk = lit_walk + FASTF_TPS_WALK_U16(FASTF_TPS_LBITS);
     for (;;) {
         if (bitpos + 3 > in_end) { err |= FASTF_ST_IN_OVERRUN; break; }
         FastfBitReader<32> br;
@@ -445,7 +462,7 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
             }
             __syncwarp();
             u32 wk;
-            if (fastf_tps_build(FASTF_ALPHA_PLAIN, lens, 19, S.lit_cnt, dist_sorted, S.lit, 7, first, start, &wk, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+            if (fastf_tps_build(FASTF_ALPHA_PLAIN, lens, 19, cnt, nullptr, dist_sorted, S.lit, 7, first, start, &wk, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
             const u32 n = hlit + hdist;
             u32 i = 0, prev = 0;
             while (i < n) {
@@ -470,11 +487,11 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
         u32 wl, wd;
         // the distance lengths sit behind the literal/length ones in `lens`; the literal table's storage was the code-length table
 #if FASTF_TPS_SUBTABLES
-        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, S.lit_cnt, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane, lit_sorted + 320, FASTF_TPS_LITSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
-        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, S.dist_cnt, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane, lit_sorted + 320 + 1024, FASTF_TPS_DISTSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, cnt, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane, lit_sorted + 320, FASTF_TPS_LITSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, cnt, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane, lit_sorted + 320 + 1024, FASTF_TPS_DISTSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
 #else
-        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, S.lit_cnt, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
-        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, S.dist_cnt, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, cnt, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, cnt, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
 #endif
         const u64 consumed = (u64)br.widx * 32u - br.nbits - br.skip_bits;
         bitpos = origin + consumed;
@@ -682,17 +699,17 @@ struct FastfTpsReader {
     __device__ __forceinline__ u64 bitpos() const { return base_bits + (u64)widx * 32u - nbits; }
 };
 
-// Entry of a code longer than the primary table.  lb = the stream's limit / offset array written by fastf_tps_build: the code's
-// length is TBITS + 1 + the number of length ranges that end at or below the next 15 stream bits.
+// Entry of a code longer than the primary table.  lb = the stream's limit / offset array written by fastf_tps_build (global
+// scratch): the code's length is TBITS + 1 + the number of length ranges that end at or below the next 15 stream bits.
 template <int TBITS>
 __device__ __forceinline__ u32 fastf_tps_walk(u64 buf, const u16 *lb, const u16 *sorted, u32 alpha)
 {
     constexpr int NL = 15 - TBITS, OFFS = FASTF_TPS_WALK_OFFS(TBITS);
     const u32 code15 = __brev((u32)buf) >> 17;   // the next 15 stream bits, first bit most significant
-    const uint2 La = *reinterpret_cast<const uint2 *>(lb), Lb = *reinterpret_cast<const uint2 *>(lb + 4);
+    const uint2 La = fastf_ld_walk2(lb), Lb = fastf_ld_walk2(lb + 4);
     u32 w[6] = {La.x, La.y, Lb.x, Lb.y, 0xffffffffu, 0xffffffffu};
     if (NL > 8) {
-        const uint2 L2 = *reinterpret_cast<const uint2 *>(lb + 8);
+        const uint2 L2 = fastf_ld_walk2(lb + 8);
         w[4] = L2.x; w[5] = L2.y;
     }
     u32 k = 0;
@@ -700,7 +717,7 @@ __device__ __forceinline__ u32 fastf_tps_walk(u64 buf, const u16 *lb, const u16 
     for (int i = 0; i < NL; i++) k += code15 >= ((i & 1) ? (w[i >> 1] >> 16) : (w[i >> 1] & 0xffffu));
     if (k >= (u32)NL) return FASTF_T16_BAD << 4;
     const u32 len = (u32)TBITS + 1u + k;
-    const u32 idx = ((code15 >> (15u - len)) + (u32)lb[OFFS + k]) & 0xffffu;
+    const u32 idx = ((code15 >> (15u - len)) + fastf_ld_walk(lb + OFFS + k)) & 0xffffu;
     return fastf_make16(alpha, fastf_ld_sorted(sorted + idx)) | len;
 }
 
@@ -747,7 +764,7 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
         u32 wr = 0, rd_cache = 0, pos = 0, isize = 0, last = 0;
         u64 in_end = 0;
         const u8 *obase = A.out;
-        FASTF_PROF(u32 p_dec = 0; u32 p_full = 0; u32 p_wait = 0;)
+        FASTF_PROF(u32 p_dec = 0; u32 p_full = 0; u32 p_wait = 0; u32 p_long = 0; u32 p_walk = 0;)
         for (;;) {
             if (!have) {
                 const u32 st = fastf_ldv(&S.state);
@@ -767,15 +784,18 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
                 if (wr - rd_cache > FASTF_TPS_RING - (FASTF_TPS_TRIPLES + 1u)) { FASTF_PROF(p_full++;) fastf_stv(&S.wr, wr); fastf_spin_poll(); continue; }
             }
             FASTF_PROF(p_dec++;)
-            // ---- one round: up to two literal tokens (three literals each) and the match behind them ----
+            // ---- one round: up to FASTF_TPS_TRIPLES literal tokens (three literals each) and the match behind them ----
             // Both the literal and the match path of a warp run in every round anyway (some lane always needs each), so a lane
             // walks through both: literals first, then the match that ends the literal run.  Only the first symbol of a round may
             // have a code longer than the primary table (canonical walk); behind it `e` is always a PEEK of the primary table
             // ((e & 63) in 1..15 <=> literal inside the table) that the next step consumes or leaves to the next round.
-            // Bit budget: a refill leaves >= 33 bits; 15 + 9 + 9 for the first triple, 27 for the second, 9 + 5 for a length.
+            // Bit budget: a refill leaves >= 33 bits; 15 + 9 + 9 for the first triple, 27 for each further one, 9 + 5 for a length.
             br.refill();
             u32 e = S.lit[(u32)br.buf & ((1u << FASTF_TPS_LBITS) - 1u)];
-            if ((e & 15u) == 0) e = fastf_tps_long<FASTF_TPS_LBITS>(e, br.buf, S.lit_cnt, lit_sorted, lit_sorted + 320, FASTF_ALPHA_LITLEN);
+            if ((e & 15u) == 0) {
+                FASTF_PROF(p_long++; p_walk += ((e >> 6) & 7u) == 0u;)
+                e = fastf_tps_long<FASTF_TPS_LBITS>(e, br.buf, lit_sorted + FASTF_TPS_WALK_AT, lit_sorted, lit_sorted + 320, FASTF_ALPHA_LITLEN);
+            }
             u32 kind = (e >> 4) & 3u;
             u32 err = 0;
             const u32 wr0 = wr;
@@ -852,7 +872,10 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
                 const u32 len = (K >> 8) + br.take(K & 255u);
                 br.refill();
                 u32 d = S.dist[(u32)br.buf & ((1u << FASTF_TPS_DBITS) - 1u)];
-                if ((d & 15u) == 0) d = fastf_tps_long<FASTF_TPS_DBITS>(d, br.buf, S.dist_cnt, dist_sorted, lit_sorted + 320 + 1024, FASTF_ALPHA_DIST);
+                if ((d & 15u) == 0) {
+                    FASTF_PROF(p_long++; p_walk += ((d >> 6) & 7u) == 0u;)
+                    d = fastf_tps_long<FASTF_TPS_DBITS>(d, br.buf, lit_sorted + FASTF_TPS_WALK_AT + FASTF_TPS_WALK_U16(FASTF_TPS_LBITS), dist_sorted, lit_sorted + 320 + 1024, FASTF_ALPHA_DIST);
+                }
                 if (((d >> 4) & 3u) != FASTF_T16_SYM) err = FASTF_ST_BAD_SYMBOL;
                 else {
                     br.drop(d & 15u);
@@ -897,6 +920,7 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
         }
 #if FASTF_TPS_PROF
         atomicAdd(&g_fastf_tps_prof[0], (unsigned long long)p_dec); atomicAdd(&g_fastf_tps_prof[1], (unsigned long long)p_full); atomicAdd(&g_fastf_tps_prof[2], (unsigned long long)p_wait);
+        atomicAdd(&g_fastf_tps_prof[11], (unsigned long long)p_long); atomicAdd(&g_fastf_tps_prof[12], (unsigned long long)p_walk);
 #endif
     } else {
         // ---------------- service: lock-step warp, owns the streams sw, sw + SVC, sw + 2 SVC, ... ----------------

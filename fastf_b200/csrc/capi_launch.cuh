@@ -90,7 +90,7 @@ static int launch_inflate(fastf_ctx *ctx, u32 lanes, const u8 *comp, u64 comp_to
     if (lanes >= 1 && lanes <= 4) {
         // thread-per-stream kernel: persistent CTAs (one per SM), FASTF_TPS_STREAMS streams each; blocks are handed out by a global counter.
         // one shape is built: <FASTF_TPS_LANES decoding lanes per decoder warp, FASTF_TPS_SVC_WARPS service warps> (bgzf_inflate_tps.cuh); lanes 1..4 all select it
-        const size_t smem = sizeof(FastfTpsStream) * FASTF_TPS_STREAMS + sizeof(FastfTpsShared);
+        const size_t smem = FASTF_TPS_SMEM_BYTES;   // checked against the SM at compile time (bgzf_inflate_tps.cuh)
         TRY(dev_reserve(ctx, de->counter, 64));
         CK(cudaMemsetAsync(de->counter.p, 0, sizeof(u32), s));
         FastfTpsArgs A;

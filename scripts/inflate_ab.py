@@ -52,10 +52,10 @@ for r in range(a.reps):
         # -DFASTF_TPS_PROF=1 build: role counters of the last launch (the ones before are discarded by the reset)
         pr = (C.c_ulonglong * 16)()
         ctx.lib.fastf_debug_tps_prof(pr, 1)
-        d, full, wait, npass, nempty, ccopy, csetup, cempty, nb_, ntok, ctot = [int(pr[i]) for i in range(11)]
-        print("prof: decoder lane-rounds %d decoded, %d ring-full (%.1f%%), %d waiting for set-up (%.1f%%) | service passes %d, empty %.1f%%, batches %d (%.1f tokens), cycles: copy %.1f%% set-up %.1f%% empty passes %.1f%% of %.3g; per batch %.0f cycles, per set-up call avg n/a"
+        d, full, wait, npass, nempty, ccopy, csetup, cempty, nb_, ntok, ctot, nlong, nwalk = [int(pr[i]) for i in range(13)]
+        print("prof: decoder lane-rounds %d decoded, %d ring-full (%.1f%%), %d waiting for set-up (%.1f%%) | service passes %d, empty %.1f%%, batches %d (%.1f tokens), cycles: copy %.1f%% set-up %.1f%% empty passes %.1f%% of %.3g; per batch %.0f cycles | codes longer than the table %d, walks %d"
               % (d, full, 100.0 * full / max(d + full + wait, 1), wait, 100.0 * wait / max(d + full + wait, 1), npass, 100.0 * nempty / max(npass, 1), nb_, ntok / max(nb_, 1),
-                 100.0 * ccopy / max(ctot, 1), 100.0 * csetup / max(ctot, 1), 100.0 * cempty / max(ctot, 1), ctot, ccopy / max(nb_, 1)))
+                 100.0 * ccopy / max(ctot, 1), 100.0 * csetup / max(ctot, 1), 100.0 * cempty / max(ctot, 1), ctot, ccopy / max(nb_, 1), nlong, nwalk))
     elif hasattr(ctx.lib, "fastf_debug_tps_prof"):
         ctx.lib.fastf_debug_tps_prof(None, 1)
 print("lib=%s %s lanes=%d blocks=%d ms=%.2f alg_GBps=%.1f out_GBps=%.1f %s" % (os.path.basename(os.environ.get("FASTF_GPU_LIB", "default")), " ".join(f"{k}={v}" for k, v in info.items() if k != "src"),
