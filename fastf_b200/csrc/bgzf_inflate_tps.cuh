@@ -18,8 +18,9 @@
 //                                        copy the matches with all 32 lanes (the source loads of several matches, or of several
 //                                        pieces of a long one, are issued before any is stored so the L2 round trips overlap).
 //                                        (b) stream set-up: fetch the next BGZF block from a global counter, parse deflate block
-//                                        headers, copy stored blocks, build the Huffman tables cooperatively -- decoders never
-//                                        run that code.
+//                                        headers, copy stored blocks, build the Huffman tables warp-parallel -- decoders never
+//                                        run that code.  Streams whose decoder waits are served first in a pass, and the next
+//                                        deflate block of a BGZF block is set up while the previous one's tokens still drain.
 //
 // Tables per stream: 8-bit literal/length table and 6-bit distance table with 16-bit entries (code length, kind, symbol) in shared
 // memory; a code longer than the table takes one lookup in the stream's second-level table in global memory (L2), with the
@@ -135,7 +136,7 @@ enum { FASTF_TPS_NEXT = 0, FASTF_TPS_RUN = 1, FASTF_TPS_BUILD = 2, FASTF_TPS_DON
 struct FastfTpsStream {
     u16 lit[1 << FASTF_TPS_LBITS];
     u16 dist[1 << FASTF_TPS_DBITS];
-    alignas(8) u32 ring[FASTF_TPS_RING];   // also the code-length counts of a table build while the stream is set up
+    alignas(8) u32 ring[FASTF_TPS_RING];
     // control block (volatile accesses; every hand-over is fenced)
     u32 state, wr, rd, last;         // state, wr, rd: polled as ctl[0..2] by the service warps
     u32 bitpos_lo, bitpos_hi;        // absolute bit offset of the next unread bit inside `comp`
@@ -147,7 +148,7 @@ struct FastfTpsStream {
 
 // scratch of one service warp while it sets a stream up
 struct FastfTpsSvc {
-    struct { u8 lens[320]; u16 scratch[32]; u8 submax[256]; } setup;   // code lengths of the block being set up; first[16], start[16] while building; longest code per table prefix
+    struct { u8 lens[320]; u16 scratch[32]; u8 submax[256]; } setup;   // code lengths of the block being set up; first[16], start[16] of the table being built; longest code per table prefix
 };
 struct FastfTpsShared {
     u32 lenK[32], distK[32];         // base << 8 | extra bits
@@ -173,13 +174,29 @@ static_assert(FASTF_TPS_SMEM_BYTES <= FASTF_TPS_SMEM_MAX, "streams + set-up scra
 // fastf_debug_tps_prof).  [0] decoder lane-rounds decoded, [1] skipped with a full ring, [2] skipped waiting for set-up,
 // [3] service passes, [4] passes without work, [5] cycles in copies, [6] cycles in set-up, [7] cycles in passes without work,
 // [8] batches, [9] tokens, [10] total service cycles, [11] codes longer than the primary table, [12] of them resolved by the
-// canonical walk (their sub-tables did not fit)
+// canonical walk (their sub-tables did not fit).
+// Set-up in time: [13] of [2] the rounds that wait for a new BGZF block (NEXT, launch start included; the rest wait for the next
+// deflate block of the same BGZF block, BUILD), [14] / [15] decoder cycles waiting for BUILD / NEXT (summed over lanes, from the
+// hand-over or the launch start to RUN; the last wait, for DONE, is not counted), [16] decoder cycles from the launch to DONE
+// (summed over lanes), [17] BGZF blocks fetched, [18] deflate block headers parsed, [19] set-up cycles in table builds (the rest of
+// [6] is block fetch, headers, code-length decode and stored copies), [20] / [21] cycles from a BUILD hand-over to the start of its
+// set-up and their number, [22] / [23] the same for NEXT hand-overs (END token), [24] set-ups started while tokens were pending,
+// [25] of them left for later (stored block or error: set up again once the ring is empty)
 #ifndef FASTF_TPS_PROF
 #define FASTF_TPS_PROF 0
 #endif
+#define FASTF_TPS_PROF_N 32
 #if FASTF_TPS_PROF
-__device__ unsigned long long g_fastf_tps_prof[16];
+__device__ unsigned long long g_fastf_tps_prof[FASTF_TPS_PROF_N];
+// clock64 of each stream's last hand-over (0 = none yet in this launch); grids of up to 1024 CTAs
+__device__ unsigned long long g_fastf_tps_handover[1024 * FASTF_TPS_STREAMS];
 #define FASTF_PROF(x) x
+// time from a stream's hand-over to the start of its set-up: slot [at] cycles, [at + 1] count
+__device__ __forceinline__ void fastf_tps_prof_handover(u32 sidx, u32 at)
+{
+    unsigned long long &h = g_fastf_tps_handover[blockIdx.x * FASTF_TPS_STREAMS + sidx];
+    if (h) { atomicAdd(&g_fastf_tps_prof[at], (unsigned long long)(clock64() - (long long)h)); atomicAdd(&g_fastf_tps_prof[at + 1], 1ull); h = 0; }
+}
 #else
 #define FASTF_PROF(x)
 #endif
@@ -255,77 +272,69 @@ __device__ __forceinline__ u32 fastf_make16(u32 alpha, u32 sym)
     return (FASTF_T16_SYM << 4) | (sym << 8);
 }
 
-// Cooperative (32 lanes, lock step) construction of one 16-bit decode table.  Returns non-zero for an invalid code.
-// cnt[16], first[16], start[16]: shared scratch.  lb: the stream's walk limits / offsets in global scratch
-// (null for the code-length table, whose codes all fit the table).
-// *walk = (first canonical code of length tbits+1) << 16 | (index of its first symbol in sorted[]).
-__device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n, u16 *cnt, u16 *lb, u16 *sorted, u16 *lut, u32 tbits, u16 *first, u16 *start, u32 *walk, u32 lane,
+// lanes of a chunk whose code length is l, from the four ballots of the lengths' bits
+__device__ __forceinline__ u32 fastf_tps_len_peers(u32 l, u32 b0, u32 b1, u32 b2, u32 b3)
+{
+    return ((l & 1u) ? b0 : ~b0) & ((l & 2u) ? b1 : ~b1) & ((l & 4u) ? b2 : ~b2) & ((l & 8u) ? b3 : ~b3);
+}
+
+// Cooperative (32 lanes, lock step) construction of one 16-bit decode table.  Returns non-zero for an invalid code (over-subscribed,
+// or incomplete with more than one code).  No lane walks the symbols alone: symbol 32 c + k sits in lane k of chunk c, and four
+// ballots over the bits of the chunk's code lengths give every lane the lanes that share its length.  Lane l (1..15) counts the
+// codes of length l; a scan over those 15 lanes gives first[l] (first canonical code of length l) and start[l] (index of its first
+// symbol in sorted[]); a symbol's canonical code is then first[l] + the codes of length l in earlier chunks + its rank among its
+// peers, and its lane fills its table slots (and those of its sub-table) straight from registers.
+// first[16], start[16]: shared scratch, for the sub-table layout.  lb: the stream's walk limits / offsets in global scratch (null for
+// the code-length table, whose codes all fit the table).
+__device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n, u16 *lb, u16 *sorted, u16 *lut, u32 tbits, u16 *first, u16 *start, u32 lane,
                                                u16 *sub = nullptr, u32 sub_cap = 0, u8 *submax = nullptr)
 {
     for (u32 i = lane; i < (1u << tbits); i += 32) lut[i] = FASTF_T16_LONG;
-    u32 bad = 0, wk = 0;
-    if (lane == 0) {
-        for (u32 l = 0; l < 16; l++) cnt[l] = 0;
-        for (u32 s = 0; s < n; s++) cnt[lens[s]]++;
-        i32 left = 1;
-        u32 used = 0;
-        for (u32 l = 1; l < 16; l++) {
-            left = (left << 1) - (i32)cnt[l];
-            if (left < 0) bad = 1;
-            used += cnt[l];
-        }
-        if (left > 0 && used > 1) bad = 1;
-        u32 code = 0, idx = 0;
-        for (u32 l = 1; l < 16; l++) {
-            first[l] = (u16)code;
-            start[l] = (u16)idx;
-            if (l == tbits + 1) wk = (code << 16) | idx;
-            code = (code + cnt[l]) << 1;
-            idx += cnt[l];
-        }
-        if (!bad) {
-            u16 offs[16];
-            for (u32 l = 1; l < 16; l++) offs[l] = start[l];
-            for (u32 s = 0; s < n; s++) {
-                u32 l = lens[s];
-                if (l) sorted[offs[l]++] = (u16)s;
-            }
-        }
-        first[0] = (u16)used;
-        // For the codes longer than the table the decoder needs, per length l = tbits+1+k: the left-aligned (15-bit) end of the
-        // length's code range (ranges of a canonical code follow one another in length order) and start[l] - first[l], the offset
-        // that turns a code into its index in sorted[].  Limits go to lb[0, OFFS), offsets behind them.
-        if (lb) {
-            const u32 offs_at = FASTF_TPS_WALK_OFFS(tbits);
-            for (u32 k = 0; k < offs_at; k++) {
-                const u32 l = tbits + 1 + k;
-                lb[k] = l <= 15 ? (u16)(((u32)first[l] + cnt[l]) << (15 - l)) : (u16)0xffff;
-                lb[offs_at + k] = l <= 15 ? (u16)((u32)start[l] - (u32)first[l]) : (u16)0;
-            }
+    const u32 nch = (n + 31u) >> 5, ml = lane & 15u, lt = (1u << lane) - 1u;
+    u32 cnt = 0;
+    for (u32 c = 0; c < nch; c++) {
+        const u32 s = (c << 5) + lane, l = s < n ? lens[s] : 0u;
+        const u32 b0 = __ballot_sync(FASTF_FULL_MASK, l & 1u), b1 = __ballot_sync(FASTF_FULL_MASK, l & 2u);
+        const u32 b2 = __ballot_sync(FASTF_FULL_MASK, l & 4u), b3 = __ballot_sync(FASTF_FULL_MASK, l & 8u);
+        cnt += (u32)__popc(fastf_tps_len_peers(ml, b0, b1, b2, b3));
+    }
+    if (lane == 0 || lane >= 16) cnt = 0;   // length 0: symbol not used
+    // Inclusive scans over the lengths of the symbol count and of the Kraft sum: a code of length l takes 2^(15-l) of the 2^15
+    // 15-bit codes.  The code over-subscribes iff that sum exceeds 2^15 (a deficit, once negative, stays negative from one length to
+    // the next), and is incomplete iff it falls short.  first[l] = sum over k < l of cnt[k] << (l - k): the exclusive Kraft sum at
+    // l, shifted down (exactly: every term is a multiple of 2^(15-l+1)).
+    const u32 kw = cnt << (15u - ml);
+    u32 ns = cnt, ks = kw;
+#pragma unroll
+    for (int o = 1; o < 16; o <<= 1) {
+        const u32 a = __shfl_up_sync(FASTF_FULL_MASK, ns, o), k = __shfl_up_sync(FASTF_FULL_MASK, ks, o);
+        if ((int)lane >= o) { ns += a; ks += k; }
+    }
+    const u32 used = __shfl_sync(FASTF_FULL_MASK, ns, 15), kraft = __shfl_sync(FASTF_FULL_MASK, ks, 15);
+    if (kraft > 32768u || (kraft < 32768u && used > 1u)) return 1;
+    const u32 st = ns - cnt, fc = (ks - kw) >> (15u - ml);
+    if (lane < 16) { first[lane] = (u16)fc; start[lane] = (u16)st; }
+    // For the codes longer than the table the decoder needs, per length l = tbits+1+k: the left-aligned (15-bit) end of the length's
+    // code range (ranges of a canonical code follow one another in length order) and start[l] - first[l], the offset that turns a
+    // code into its index in sorted[].  Limits go to lb[0, OFFS), offsets behind them.
+    if (lb) {
+        const u32 offs_at = FASTF_TPS_WALK_OFFS(tbits), l = tbits + 1u + lane, src = l <= 15u ? l : 15u;
+        const u32 f = __shfl_sync(FASTF_FULL_MASK, fc, (int)src), c = __shfl_sync(FASTF_FULL_MASK, cnt, (int)src), s0 = __shfl_sync(FASTF_FULL_MASK, st, (int)src);
+        if (lane < offs_at) {
+            lb[lane] = l <= 15u ? (u16)((f + c) << (15u - l)) : (u16)0xffff;
+            lb[offs_at + lane] = l <= 15u ? (u16)(s0 - f) : (u16)0;
         }
     }
-    bad = __shfl_sync(FASTF_FULL_MASK, bad, 0);
-    wk = __shfl_sync(FASTF_FULL_MASK, wk, 0);
+    const u32 long_from = __shfl_sync(FASTF_FULL_MASK, st, (int)tbits + 1);
     __syncwarp();
-    if (bad) return 1;
-    const u32 used = first[0];
-    for (u32 i = lane; i < used; i += 32) {
-        const u32 sym = fastf_ld_sorted(sorted + i);
-        const u32 l = lens[sym];
-        if (l <= tbits) {
-            const u32 code = (u32)first[l] + (i - (u32)start[l]);
-            const u32 rev = __brev(code) >> (32 - l);
-            const u16 e = (u16)(fastf_make16(alpha, sym) | l);
-            for (u32 j = rev; j < (1u << tbits); j += (1u << l)) lut[j] = e;
-        }
-    }
-    const u32 long_from = start[tbits + 1];   // read before the barrier: lane 0 of the NEXT build overwrites the scratch as soon as it gets there
-    __syncwarp();
+    bool subs = false;
 #if FASTF_TPS_SUBTABLES
-    if (sub && used && long_from < used) {
+    const u32 nidx = 1u << tbits;
+    if (sub && long_from < used) {
         // (1) per table index j (the code's first tbits bits, in stream order): the longest code that starts with them.  The canonical
         // codes of length l are [first[l], first[l] + cnt[l]); the ones with the (MSB-first) prefix q are q << (l - tbits) ... .
-        const u32 nidx = 1u << tbits;
+        // The primary entry has 3 bits for the sub-table's index bits: a prefix with codes more than 7 bits longer than the table (a
+        // distance code of 14 or 15 bits) gets no sub-table, its codes take the walk.
         for (u32 j = lane; j < nidx; j += 32) {
             const u32 q = __brev(j) >> (32 - tbits);
             u32 mx = 0;
@@ -334,7 +343,7 @@ __device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n,
                 const u32 lo = q << (l - tbits), hi = (q + 1u) << (l - tbits);
                 if (c && (u32)first[l] < hi && (u32)first[l] + c > lo) mx = l;
             }
-            submax[j] = (u8)(mx ? mx - tbits : 0u);
+            submax[j] = (u8)(mx && mx - tbits <= 7u ? mx - tbits : 0u);
         }
         __syncwarp();
         // (2) sub-table offsets: sizes 2^bits padded to 8 entries, exclusive prefix sum over the indices (lane k owns a contiguous run)
@@ -345,29 +354,45 @@ __device__ __forceinline__ u32 fastf_tps_build(u32 alpha, const u8 *lens, u32 n,
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) { const u32 t = __shfl_up_sync(FASTF_FULL_MASK, inc, o); if ((int)lane >= o) inc += t; }
         const u32 total = __shfl_sync(FASTF_FULL_MASK, inc, 31);
-        if (total <= sub_cap) {
+        subs = total <= sub_cap;
+        if (subs) {
             u32 at = inc - mine;
             for (u32 j = j0; j < j0 + per && j < nidx; j++) {
                 const u32 b = submax[j];
                 if (b) { lut[j] = (u16)(FASTF_T16_LONG | (b << 6) | ((at >> 3) << 9)); at += b < 3u ? 8u : (1u << b); }
             }
-            __syncwarp();
-            // (3) every long code fills its slots of its prefix's sub-table
-            for (u32 i = long_from + lane; i < used; i += 32) {
-                const u32 sym = fastf_ld_sorted(sorted + i);
-                const u32 l = lens[sym];
-                const u32 code = (u32)first[l] + (i - (u32)start[l]);
-                const u32 rev = __brev(code) >> (32 - l);
-                const u32 pe = lut[rev & (nidx - 1u)];
-                const u32 b = (pe >> 6) & 7u, at = (pe >> 9) << 3;
-                const u16 e = (u16)(fastf_make16(alpha, sym) | l);
-                for (u32 k = rev >> tbits; k < (1u << b); k += 1u << (l - tbits)) sub[at + k] = e;
-            }
         }
         __syncwarp();
     }
 #endif
-    *walk = wk;
+    // (3) every symbol: its place in sorted[], its primary-table slots, or (a long code) its slots of its prefix's sub-table.
+    // Lane l carries the code and the sorted[] index of the next symbol of length l.
+    u32 nf = fc, nsrt = st;
+    for (u32 c = 0; c < nch; c++) {
+        const u32 s = (c << 5) + lane, l = s < n ? lens[s] : 0u;
+        const u32 b0 = __ballot_sync(FASTF_FULL_MASK, l & 1u), b1 = __ballot_sync(FASTF_FULL_MASK, l & 2u);
+        const u32 b2 = __ballot_sync(FASTF_FULL_MASK, l & 4u), b3 = __ballot_sync(FASTF_FULL_MASK, l & 8u);
+        const u32 rank = (u32)__popc(fastf_tps_len_peers(l, b0, b1, b2, b3) & lt);
+        const u32 code = __shfl_sync(FASTF_FULL_MASK, nf, (int)l) + rank, idx = __shfl_sync(FASTF_FULL_MASK, nsrt, (int)l) + rank;
+        const u32 here = (u32)__popc(fastf_tps_len_peers(ml, b0, b1, b2, b3));
+        nf += here; nsrt += here;
+        if (l) {
+            sorted[idx] = (u16)s;
+            const u32 rev = __brev(code) >> (32 - l);
+            const u16 e = (u16)(fastf_make16(alpha, s) | l);
+            if (l <= tbits) {
+                for (u32 j = rev; j < (1u << tbits); j += (1u << l)) lut[j] = e;
+            }
+#if FASTF_TPS_SUBTABLES
+            else if (subs) {
+                const u32 pe = lut[rev & (nidx - 1u)];
+                const u32 b = (pe >> 6) & 7u, at = (pe >> 9) << 3;
+                if (b) for (u32 k = rev >> tbits; k < (1u << b); k += 1u << (l - tbits)) sub[at + k] = e;
+            }
+#endif
+        }
+    }
+    __syncwarp();
     return 0;
 }
 
@@ -401,19 +426,20 @@ struct FastfTpsArgs {
 
 // Parse deflate block headers of stream S from its current bit position until a Huffman block is ready for the decoder
 // (state RUN) or the BGZF block is finished / broken (status written, state NEXT).  Stored blocks are copied here.
-__device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsStream &S, u16 *lit_sorted, FastfTpsShared &G, u32 sw, u32 lane)
+// pending: the previous deflate block's tokens are still in the ring (a BUILD hand-over set up before the ring drains, so that the
+// decoder does not wait for the copies).  Then only the tables and the bit position change: the copy side keeps reading the ring
+// in FIFO order at S.opos, the decoder goes on at S.pos.  A stored block or an error then leaves everything as it was and
+// returns non-zero: the stream stays in BUILD and is set up again from the same bit position once the ring is empty.
+__device__ __forceinline__ u32 fastf_tps_setup(const FastfTpsArgs &A, FastfTpsStream &S, u16 *lit_sorted, FastfTpsShared &G, u32 sw, u32 lane, bool pending)
 {
     u16 *dist_sorted = lit_sorted + 288;
     const u32 b = S.blk;
     u8 *out = A.out + (((u64)S.obase_hi << 32) | S.obase_lo);
     const u64 in_end = ((u64)S.inend_hi << 32) | S.inend_lo;
     u64 bitpos = ((u64)S.bitpos_hi << 32) | S.bitpos_lo;
-    u32 opos = S.opos, err = 0;
+    u32 opos = S.pos, err = 0;
     u8 *lens = G.svc[sw].setup.lens;
     u16 *first = G.svc[sw].setup.scratch, *start = G.svc[sw].setup.scratch + 16;
-    // a table build counts code lengths in the stream's token ring: it is empty while the stream is set up (a batch of tokens is
-    // always copied before the set-up, and the decoder writes no token before the state says RUN)
-    u16 *cnt = reinterpret_cast<u16 *>(S.ring);
     u16 *lit_walk = lit_sorted + FASTF_TPS_WALK_AT, *dist_walk = lit_walk + FASTF_TPS_WALK_U16(FASTF_TPS_LBITS);
     for (;;) {
         if (bitpos + 3 > in_end) { err |= FASTF_ST_IN_OVERRUN; break; }
@@ -424,8 +450,10 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
         br.refill();
         const u32 last = br.take(1);
         const u32 btype = br.take(2);
+        FASTF_PROF(if (lane == 0) atomicAdd(&g_fastf_tps_prof[18], 1ull);)
         if (btype == 3) { err |= FASTF_ST_BAD_BTYPE; break; }
         if (btype == 0) {
+            if (pending) return 1;
             br.drop(br.nbits & 7u);
             br.refill();
             const u32 len = br.take(16);
@@ -461,8 +489,10 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
                 if (lane == 0) lens[G.cl_order[i]] = (u8)v;
             }
             __syncwarp();
-            u32 wk;
-            if (fastf_tps_build(FASTF_ALPHA_PLAIN, lens, 19, cnt, nullptr, dist_sorted, S.lit, 7, first, start, &wk, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+            FASTF_PROF(const long long p_tb = clock64();)
+            const u32 clbad = fastf_tps_build(FASTF_ALPHA_PLAIN, lens, 19, nullptr, dist_sorted, S.lit, 7, first, start, lane);
+            FASTF_PROF(if (lane == 0) atomicAdd(&g_fastf_tps_prof[19], (u64)(clock64() - p_tb));)
+            if (clbad) { err |= FASTF_ST_BAD_CODELENS; break; }
             const u32 n = hlit + hdist;
             u32 i = 0, prev = 0;
             while (i < n) {
@@ -484,26 +514,29 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
             __syncwarp();
             if (lens[256] == 0) { err |= FASTF_ST_BAD_CODELENS; break; }
         }
-        u32 wl, wd;
+        FASTF_PROF(const long long p_tb = clock64();)
         // the distance lengths sit behind the literal/length ones in `lens`; the literal table's storage was the code-length table
 #if FASTF_TPS_SUBTABLES
-        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, cnt, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane, lit_sorted + 320, FASTF_TPS_LITSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
-        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, cnt, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane, lit_sorted + 320 + 1024, FASTF_TPS_DISTSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, lane, lit_sorted + 320, FASTF_TPS_LITSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, lane, lit_sorted + 320 + 1024, FASTF_TPS_DISTSUB_U16, G.svc[sw].setup.submax)) { err |= FASTF_ST_BAD_CODELENS; break; }
 #else
-        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, cnt, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, &wl, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
-        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, cnt, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, &wd, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_LITLEN, lens, hlit, lit_walk, lit_sorted, S.lit, FASTF_TPS_LBITS, first, start, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
+        if (fastf_tps_build(FASTF_ALPHA_DIST, lens + hlit, hdist, dist_walk, dist_sorted, S.dist, FASTF_TPS_DBITS, first, start, lane)) { err |= FASTF_ST_BAD_CODELENS; break; }
 #endif
+        FASTF_PROF(if (lane == 0) atomicAdd(&g_fastf_tps_prof[19], (u64)(clock64() - p_tb));)
         const u64 consumed = (u64)br.widx * 32u - br.nbits - br.skip_bits;
         bitpos = origin + consumed;
         if (lane == 0) {
             S.bitpos_lo = (u32)bitpos; S.bitpos_hi = (u32)(bitpos >> 32);
-            S.last = last; S.pos = opos; S.opos = opos;
+            S.last = last; S.pos = opos;
+            if (!pending) S.opos = opos;
             __threadfence_block();
             fastf_stv(&S.state, FASTF_TPS_RUN);
         }
         __syncwarp();
-        return;
+        return 0;
     }
+    if (pending) return 1;
     // the BGZF block ended inside this routine (stored-only block, or an error)
     if (!err && opos != S.isize) err |= FASTF_ST_SIZE_MISMATCH;
     if (lane == 0) {
@@ -513,6 +546,7 @@ __device__ __forceinline__ void fastf_tps_setup(const FastfTpsArgs &A, FastfTpsS
         fastf_stv(&S.state, FASTF_TPS_NEXT);
     }
     __syncwarp();
+    return 0;
 }
 
 // LZ77 resolution of up to 32 tokens of one stream by a whole warp.  Returns the number of tokens consumed.
@@ -748,6 +782,7 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
     if (threadIdx.x < FASTF_TPS_STREAMS) {
         FastfTpsStream &S = streams[threadIdx.x];
         S.state = FASTF_TPS_NEXT; S.wr = 0; S.rd = 0; S.last = 0; S.pos = 0; S.isize = 0; S.opos = 0; S.blk = 0;
+        FASTF_PROF(g_fastf_tps_handover[blockIdx.x * FASTF_TPS_STREAMS + threadIdx.x] = 0;)
     }
     __syncthreads();
 
@@ -764,12 +799,14 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
         u32 wr = 0, rd_cache = 0, pos = 0, isize = 0, last = 0;
         u64 in_end = 0;
         const u8 *obase = A.out;
-        FASTF_PROF(u32 p_dec = 0; u32 p_full = 0; u32 p_wait = 0; u32 p_long = 0; u32 p_walk = 0;)
+        FASTF_PROF(u32 p_dec = 0; u32 p_full = 0; u32 p_wait = 0; u32 p_long = 0; u32 p_walk = 0; u32 p_waitn = 0; bool p_next = true;
+                   u64 p_cbuild = 0; u64 p_cnext = 0; const long long p_t00 = clock64(); long long p_tw = p_t00;)
         for (;;) {
             if (!have) {
                 const u32 st = fastf_ldv(&S.state);
                 if (st == FASTF_TPS_DONE) break;
-                if (st != FASTF_TPS_RUN) { FASTF_PROF(p_wait++;) fastf_spin_poll(); continue; }
+                if (st != FASTF_TPS_RUN) { FASTF_PROF(p_wait++; p_waitn += p_next;) fastf_spin_poll(); continue; }
+                FASTF_PROF(if (p_next) p_cnext += (u64)(clock64() - p_tw); else p_cbuild += (u64)(clock64() - p_tw);)
                 __threadfence_block();
                 br.init(A.comp, A.comp_total, ((u64)S.bitpos_hi << 32) | S.bitpos_lo);
                 pos = S.pos; isize = S.isize; last = S.last;
@@ -912,6 +949,7 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
             }
             S.bitpos_lo = (u32)bp; S.bitpos_hi = (u32)(bp >> 32);
             S.pos = pos;
+            FASTF_PROF(p_next = end_stream; p_tw = clock64(); g_fastf_tps_handover[blockIdx.x * FASTF_TPS_STREAMS + sidx] = (u64)p_tw;)
             __threadfence_block();
             fastf_stv(&S.wr, wr);
             __threadfence_block();
@@ -921,6 +959,8 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
 #if FASTF_TPS_PROF
         atomicAdd(&g_fastf_tps_prof[0], (unsigned long long)p_dec); atomicAdd(&g_fastf_tps_prof[1], (unsigned long long)p_full); atomicAdd(&g_fastf_tps_prof[2], (unsigned long long)p_wait);
         atomicAdd(&g_fastf_tps_prof[11], (unsigned long long)p_long); atomicAdd(&g_fastf_tps_prof[12], (unsigned long long)p_walk);
+        atomicAdd(&g_fastf_tps_prof[13], (unsigned long long)p_waitn); atomicAdd(&g_fastf_tps_prof[14], p_cbuild); atomicAdd(&g_fastf_tps_prof[15], p_cnext);
+        atomicAdd(&g_fastf_tps_prof[16], (u64)(clock64() - p_t00));
 #endif
     } else {
         // ---------------- service: lock-step warp, owns the streams sw, sw + SVC, sw + 2 SVC, ... ----------------
@@ -956,8 +996,14 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
                 FASTF_PROF(p_empty++; p_cempty += (u64)(clock64() - p_t0);)
                 continue;
             }
-            const u32 work = avail ? 1u : (st == FASTF_TPS_NEXT ? 2u : 3u);
-            while (m) {
+            // Streams whose decoder waits (set-up, or the drain of an ended BGZF block) go first: a stream with a partly full ring
+            // still decodes.  A BUILD hand-over is set up at once, its tokens stay in the ring; a NEXT hand-over drains first, because
+            // the copy side still reads the old block's blk / isize / obase.
+            u32 rest = m & ~__ballot_sync(FASTF_FULL_MASK, mine && (st & 1u) == 0);
+            m &= ~rest;
+            const u32 work = st == FASTF_TPS_BUILD ? 3u : (avail ? 1u : 2u);
+            while (m | rest) {
+                if (!m) { m = rest; rest = 0; }
                 const u32 k = (u32)__ffs((int)m) - 1u;
                 m &= m - 1u;
                 const u32 w = __shfl_sync(FASTF_FULL_MASK, work, (int)k);
@@ -972,6 +1018,7 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
                     fastf_tps_copy(A, S, krd, kav < 32u ? kav : 32u, lane);
                 } else if (w == 2) {
                     // fetch the next BGZF block for this stream
+                    FASTF_PROF(if (lane == 0) fastf_tps_prof_handover(sidx, 22);)
                     u32 b = 0;
                     if (lane == 0) b = atomicAdd(A.next_block, 1u);
                     b = __shfl_sync(FASTF_FULL_MASK, b, 0);
@@ -986,11 +1033,15 @@ __global__ void __launch_bounds__(FASTF_TPS_THREADS_OF(L, SVC), 1) fastf_bgzf_in
                             S.inend_lo = (u32)be; S.inend_hi = (u32)(be >> 32);
                             S.obase_lo = (u32)ob; S.obase_hi = (u32)(ob >> 32);
                         }
+                        FASTF_PROF(if (lane == 0) atomicAdd(&g_fastf_tps_prof[17], 1ull);)
                         __syncwarp();
-                        fastf_tps_setup(A, S, ssorted, G, sw, lane);
+                        fastf_tps_setup(A, S, ssorted, G, sw, lane, false);
                     }
                 } else {
-                    fastf_tps_setup(A, S, ssorted, G, sw, lane);
+                    FASTF_PROF(if (lane == 0) fastf_tps_prof_handover(sidx, 20);)
+                    const u32 later = fastf_tps_setup(A, S, ssorted, G, sw, lane, kav != 0);
+                    FASTF_PROF(if (lane == 0 && kav) { atomicAdd(&g_fastf_tps_prof[24], 1ull); atomicAdd(&g_fastf_tps_prof[25], (unsigned long long)later); })
+                    if (later) fastf_tps_copy(A, S, krd, kav < 32u ? kav : 32u, lane);   // drain, then set up again
                 }
                 FASTF_PROF(if (w == 1) p_ccopy += (u64)(clock64() - p_t1); else p_csetup += (u64)(clock64() - p_t1);)
             }

@@ -287,10 +287,10 @@ extern "C" int fastf_abi_version(void) { return FASTF_ABI_VERSION; }
 #define FASTF_STR(x) FASTF_STR2(x)
 #if FASTF_TPS_PROF
 // debug builds only (-DFASTF_TPS_PROF=1, scripts/inflate_ab.py): the kernel's role counters, see bgzf_inflate_tps.cuh
-extern "C" int fastf_debug_tps_prof(unsigned long long *out16, int reset)
+extern "C" int fastf_debug_tps_prof(unsigned long long *out32, int reset)
 {
-    if (out16 && cudaMemcpyFromSymbol(out16, g_fastf_tps_prof, 16 * sizeof(unsigned long long)) != cudaSuccess) return 1;
-    if (reset) { unsigned long long z[16] = {0}; if (cudaMemcpyToSymbol(g_fastf_tps_prof, z, sizeof z) != cudaSuccess) return 1; }
+    if (out32 && cudaMemcpyFromSymbol(out32, g_fastf_tps_prof, FASTF_TPS_PROF_N * sizeof(unsigned long long)) != cudaSuccess) return 1;
+    if (reset) { unsigned long long z[FASTF_TPS_PROF_N] = {0}; if (cudaMemcpyToSymbol(g_fastf_tps_prof, z, sizeof z) != cudaSuccess) return 1; }
     return 0;
 }
 #endif

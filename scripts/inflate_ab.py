@@ -50,12 +50,17 @@ for r in range(a.reps):
     best = ms.value if best is None else min(best, ms.value)
     if hasattr(ctx.lib, "fastf_debug_tps_prof") and r == a.reps - 1:
         # -DFASTF_TPS_PROF=1 build: role counters of the last launch (the ones before are discarded by the reset)
-        pr = (C.c_ulonglong * 16)()
+        pr = (C.c_ulonglong * 32)()   # FASTF_TPS_PROF_N
         ctx.lib.fastf_debug_tps_prof(pr, 1)
-        d, full, wait, npass, nempty, ccopy, csetup, cempty, nb_, ntok, ctot, nlong, nwalk = [int(pr[i]) for i in range(13)]
-        print("prof: decoder lane-rounds %d decoded, %d ring-full (%.1f%%), %d waiting for set-up (%.1f%%) | service passes %d, empty %.1f%%, batches %d (%.1f tokens), cycles: copy %.1f%% set-up %.1f%% empty passes %.1f%% of %.3g; per batch %.0f cycles | codes longer than the table %d, walks %d"
-              % (d, full, 100.0 * full / max(d + full + wait, 1), wait, 100.0 * wait / max(d + full + wait, 1), npass, 100.0 * nempty / max(npass, 1), nb_, ntok / max(nb_, 1),
+        (d, full, wait, npass, nempty, ccopy, csetup, cempty, nb_, ntok, ctot, nlong, nwalk, waitn, cwb, cwn, cdec, nbgzf, nhdr, cbuild,
+         hob, nhob, hon, nhon, nearly, nlater) = [int(pr[i]) for i in range(26)]
+        rounds = max(d + full + wait, 1)
+        print("prof: decoder lane-rounds %d decoded, %d ring-full (%.1f%%), %d waiting for set-up (%.1f%%: BUILD %.1f%%, NEXT %.1f%%) | service passes %d, empty %.1f%%, batches %d (%.1f tokens), cycles: copy %.1f%% set-up %.1f%% empty passes %.1f%% of %.3g; per batch %.0f cycles | codes longer than the table %d, walks %d"
+              % (d, full, 100.0 * full / rounds, wait, 100.0 * wait / rounds, 100.0 * (wait - waitn) / rounds, 100.0 * waitn / rounds, npass, 100.0 * nempty / max(npass, 1), nb_, ntok / max(nb_, 1),
                  100.0 * ccopy / max(ctot, 1), 100.0 * csetup / max(ctot, 1), 100.0 * cempty / max(ctot, 1), ctot, ccopy / max(nb_, 1), nlong, nwalk))
+        print("prof-time: decoder cycles waiting for set-up %.1f%% (BUILD %.1f%%, NEXT %.1f%%) of %.3g | %d BGZF blocks, %.2f deflate blocks each | set-up cycles: headers + code lengths %.1f%%, table builds %.1f%% of %.3g (%.0f per deflate block) | hand-over to set-up start: BUILD %.0f cycles (%d), NEXT %.0f cycles (%d) | set-ups with tokens pending %d, %d of them left for later"
+              % (100.0 * (cwb + cwn) / max(cdec, 1), 100.0 * cwb / max(cdec, 1), 100.0 * cwn / max(cdec, 1), cdec, nbgzf, nhdr / max(nbgzf, 1),
+                 100.0 * (csetup - cbuild) / max(csetup, 1), 100.0 * cbuild / max(csetup, 1), csetup, csetup / max(nhdr, 1), hob / max(nhob, 1), nhob, hon / max(nhon, 1), nhon, nearly, nlater))
     elif hasattr(ctx.lib, "fastf_debug_tps_prof"):
         ctx.lib.fastf_debug_tps_prof(None, 1)
 print("lib=%s %s lanes=%d blocks=%d ms=%.2f alg_GBps=%.1f out_GBps=%.1f %s" % (os.path.basename(os.environ.get("FASTF_GPU_LIB", "default")), " ".join(f"{k}={v}" for k, v in info.items() if k != "src"),
